@@ -4,6 +4,7 @@
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload conus3|conus12|weak2048|deep120|tiny]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference ...      # the reference's own CPU C code on the host cores
+    python bench.py ... --dump-outputs DIR    # also write the last timed step's output fields to DIR/<name>.npy
 
 A "step" is one pass of the hot path over the workload: for the default workload (conus3, the
 CONUS-3km-class 1800x1060x50 grid BASELINE.json's target is quoted on) that is the device-resident
@@ -51,6 +52,10 @@ METRIC = "advance_mu_t grid-points/s"
 UNIT = "grid-points/s"
 C_UV = 0.25                     # coefficient of the advance_uv stand-in
 KERNEL_NAMES = {0: "auto", 1: "amt_column_kernel", 2: "amt_tile_kernel", 3: "amt_pipe_kernel"}
+OUTPUTS = ("ww", "t", "t_ave", "mu", "muave", "muts", "mudf")     # what advance_mu_t hands back to its caller
+DUMP_BYTES = 64_000_000          # all files of one --dump-outputs run, .npy headers included
+NPY_HEADER_BYTES = 4096         # room kept per file; numpy writes 128 bytes for these arrays
+DUMP_SEED = 20240617
 
 
 def peaks():
@@ -121,6 +126,22 @@ class ClockSampler:
                 "samples": len(sm), "reasons": sorted(reasons)}
 
 
+def dump_outputs(out_dir, fields, prefix="", share=1):
+    """Write the output fields to out_dir/<prefix><name>.npy as float32, so that two builds run with the same
+    arguments can be compared value for value.  All files of a run (`share` writers) stay within DUMP_BYTES: a
+    field larger than its part is replaced by a stratified sample of its flattened [j,k,i] values, one value from
+    each of `cap` equal runs at offsets drawn with a fixed seed, so the same positions are sampled in every run."""
+    os.makedirs(out_dir, exist_ok=True)
+    cap = (DUMP_BYTES // (len(OUTPUTS) * share) - NPY_HEADER_BYTES) // 4
+    for name in OUTPUTS:
+        a = np.ascontiguousarray(fields[name], dtype=np.float32)
+        if a.size > cap:
+            run = a.size // cap
+            idx = np.arange(cap, dtype=np.int64) * run + np.random.default_rng(DUMP_SEED).integers(0, run, cap)
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(out_dir, prefix + name + ".npy"), a)
+
+
 def global_grid(workload, n_gpus):
     """(Grid, scalars, small steps per bench step, dx).  Grid is index arithmetic only (no library call)."""
     from wrf_model_cuda_sample_b200.advance_mu_t import Grid
@@ -180,10 +201,12 @@ def run_reference_arm(args):
         return
     from oracle import synth_np
     g, scalars, nsmall, dx = global_grid(args.workload, 1)
-    steps = max(1, min(args.steps, 60))        # each step is one small step over the full grid: bounded sample
+    steps = args.steps                         # each step is one small step over the full grid
     warmup = max(1, args.warmup)
     fields = synth_np.synth_fields(g)
     r = cpu_reference_run(g, scalars, fields, steps, warmup)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, fields)
     line = {
         "impl": "reference", "metric": METRIC, "value": r["value"], "unit": UNIT, "n_gpus": args.gpus,
         "steps": steps, "warmup": warmup, "ms_per_step": r["ms_per_small_step"],
@@ -579,6 +602,11 @@ def run_ours(args):
     l2_note = ("inputs larger than L2 (%.2f GB touched per small step vs 126 MB L2)" % (bytes_local / 1e9)
                if flush is None else "L2 flushed (256 MB write) before every timed step")
     halo_timeouts = patch.comm_status()[0] if world > 1 else 0
+    if args.dump_outputs:                                      # the state the last timed step left on the device
+        out = {n: np.empty(pg.shape_of(n), dtype=np.float32) for n in OUTPUTS}
+        patch.download(out, names=OUTPUTS)
+        dump_outputs(args.dump_outputs, out, prefix=f"rank{rank}_" if world > 1 else "", share=world)
+        del out
 
     elapsed_ms = max_over_ranks(elapsed_ms, dev, world)
     ms_per_step = elapsed_ms / args.steps
@@ -752,7 +780,12 @@ def main():
     ap.add_argument("--no-ref-cuda", action="store_true")
     ap.add_argument("--no-extras", action="store_true",
                     help="skip the stand-in loop, the other BASELINE configs and the pageable e2e variants")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write the output fields of the last one to DIR/<name>.npy "
+                         "(float32, at most 64 MB in all: larger fields are sampled at fixed seeded positions)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if os.environ.get("BENCH_HANG_DUMP"):                       # debugging aid: dump all stacks after N seconds
         import faulthandler
         faulthandler.dump_traceback_later(int(os.environ["BENCH_HANG_DUMP"]), exit=True)

@@ -33,7 +33,7 @@ _cache = {}
 def _load(path):
     if path not in _cache:
         if not os.path.exists(path):
-            raise FileNotFoundError(f"{path} missing: run `make -C oracle` (needs /root/reference for _ref/)")
+            raise FileNotFoundError(f"{path} missing: run `make -C oracle` (_ref/ needs REF=<reference checkout>)")
         _cache[path] = C.CDLL(path)
     return _cache[path]
 

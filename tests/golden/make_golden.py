@@ -1,12 +1,11 @@
 """Generate (or --check) the golden vectors in tests/golden/.
 
 The reference ships no golden data (its .bin dumps live in an un-shipped /data2 directory,
-advance_mu_t_driver.f90:36), so the vectors are OUTPUTS OF THE REFERENCE ITSELF run in the build
-container: /root/reference/advance_mu_t.c, unmodified, compiled in place by oracle/Makefile into
-oracle/_ref/libref_advance_mu_t.so, executed on seeded numpy inputs.  /root/reference cannot travel to the
-GPU box; these files can.
+advance_mu_t_driver.f90:36), so the vectors are OUTPUTS OF THE REFERENCE ITSELF: its advance_mu_t.c,
+unmodified, compiled in place by oracle/Makefile into oracle/_ref/libref_advance_mu_t.so, executed on seeded
+numpy inputs.  The reference sources are not part of this repository; these files are.
 
-    python tests/golden/make_golden.py          # regenerate (needs oracle/_ref, i.e. /root/reference)
+    python tests/golden/make_golden.py          # regenerate (needs oracle/_ref: make -C oracle REF=<reference checkout>)
     python tests/golden/make_golden.py --check  # verify the committed files against a fresh run
 """
 import os

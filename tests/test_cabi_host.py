@@ -3,6 +3,7 @@ its host-side utilities work, and compute entry points fail LOUDLY (no CPU fallb
 import ctypes as C
 import os
 import re
+import threading
 
 import numpy as np
 import pytest
@@ -210,5 +211,9 @@ def test_comm_and_residency_entry_points_fail_cleanly_without_state():
     assert lib.wrfb200_comm_step(None) == _lib.ERR_INVALID_ARG
     assert lib.wrfb200_comm_connect(None, None, 0) == _lib.ERR_INVALID_ARG
     assert lib.wrfb200_acoustic_loop_begin() == 0 and lib.wrfb200_acoustic_loop_end() == 0
-    k = C.c_int(-1)
-    assert lib.wrfb200_default_last_kernel(C.byref(k)) == 0 and k.value == 0
+    # the last kernel is per thread: ask from one that has made no call, whatever ran earlier in this process
+    k, rc = C.c_int(-1), []
+    t = threading.Thread(target=lambda: rc.append(lib.wrfb200_default_last_kernel(C.byref(k))))
+    t.start()
+    t.join()
+    assert rc == [0] and k.value == 0

@@ -1,6 +1,6 @@
 """The oracle is pinned before it is trusted (not gpu):
   1. against the committed golden vectors = outputs of the reference's own advance_mu_t.c (tests/golden/),
-  2. against that reference C executed live when oracle/_ref is present (build container),
+  2. against that reference C executed live when oracle/_ref is built (`make -C oracle REF=<reference checkout>`),
   3. C restatement == numpy restatement, single call == j-tiled calls,
   4. in/out contract: inputs untouched, cells outside the index sets untouched, empty tiles legal.
 """
@@ -11,7 +11,7 @@ from oracle import loader
 from tests import cases
 from tests.golden import make_golden
 
-needs_ref = pytest.mark.skipif(not loader.have_ref(), reason="oracle/_ref not built (no /root/reference here)")
+needs_ref = pytest.mark.skipif(not loader.have_ref(), reason="oracle/_ref not built (needs REF=<reference checkout>)")
 
 
 @pytest.mark.parametrize("name", sorted(make_golden.CASES))
