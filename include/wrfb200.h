@@ -34,6 +34,11 @@
  *   - Every function returns a wrfb200_status (0 = ok).  After a non-zero status,
  *     wrfb200_last_error() gives a human-readable message (thread-local).
  *   - No CPU fallback exists: without a CUDA device every compute entry point fails with WRFB200_ERR_CUDA.
+ *   - Precision: the unsuffixed entry points take binary32 (`float`, WRF's default REAL = 4 bytes).  WRF built
+ *     with -r8 (REAL = 8 bytes) calls the `_r8` entry points, which take `double` and compute every operation
+ *     in binary64, in the same order.  A handle holds one precision, fixed by wrfb200_create / _create_r8;
+ *     a verb typed for the other precision fails with WRFB200_ERR_STATE.  The multi-GPU, halo, stand-in and
+ *     resident-bundle verbs are binary32 only (WRFB200_ERR_UNSUPPORTED on an r8 handle).
  */
 #ifndef WRFB200_H
 #define WRFB200_H
@@ -84,9 +89,11 @@ typedef struct wrfb200_domain {
 typedef enum wrfb200_kernel {
     WRFB200_KERNEL_AUTO = 0,
     WRFB200_KERNEL_COLUMN = 1,   /* one thread per (i,j) column, any layout */
-    WRFB200_KERNEL_TILE = 2,     /* k-parallel float4 tile kernel (register staged), needs 16-byte aligned rows */
+    WRFB200_KERNEL_TILE = 2,     /* k-parallel float4 tile kernel (register staged), needs 16-byte aligned rows;
+                                    on an r8 handle the double2 tile kernel (the AUTO choice there), which needs
+                                    16-byte aligned fields, pitches of an even number of doubles and nk <= 220 */
     WRFB200_KERNEL_PIPE = 3      /* tile kernel with per-warp TMA bulk-copy pipelines (the AUTO choice when the
-                                    layout allows it) */
+                                    layout allows it); binary32 only */
 } wrfb200_kernel;
 
 /* Halo sides of a patch. */
@@ -125,6 +132,33 @@ int wrfb200_advance_mu_t_loop(
     float rdx, float rdy, float dts, float epssm,
     const float *dnw, const float *fnm, const float *fnp, const float *rdnw,
     const float *msfuy, const float *msfvx_inv, const float *msftx, const float *msfty,
+    int periodic_x, int specified, int nested,
+    int ids, int ide, int jds, int jde, int kde,
+    int ims, int ime, int jms, int jme, int kms, int kme,
+    int its, int ite, int jts, int jte, int kts, int kte,
+    int nsteps);
+
+/* The same two entry points in double precision, for WRF built with -r8.  Same semantics (host pointers in
+ * compat mode with cached per-thread mirrors, residency and pinning as below; device pointers launched in place),
+ * every operation rounded once in binary64. */
+int wrfb200_advance_mu_t_r8(
+    double *ww, const double *ww_1, const double *u, const double *u_1, const double *v, const double *v_1,
+    double *mu, const double *mut, double *muave, double *muts, const double *muu, const double *muv,
+    double *mudf, double *t, const double *t_1, double *t_ave, const double *ft, const double *mu_tend,
+    double rdx, double rdy, double dts, double epssm,
+    const double *dnw, const double *fnm, const double *fnp, const double *rdnw,
+    const double *msfuy, const double *msfvx_inv, const double *msftx, const double *msfty,
+    int periodic_x, int specified, int nested,
+    int ids, int ide, int jds, int jde, int kde,
+    int ims, int ime, int jms, int jme, int kms, int kme,
+    int its, int ite, int jts, int jte, int kts, int kte);
+int wrfb200_advance_mu_t_loop_r8(
+    double *ww, const double *ww_1, const double *u, const double *u_1, const double *v, const double *v_1,
+    double *mu, const double *mut, double *muave, double *muts, const double *muu, const double *muv,
+    double *mudf, double *t, const double *t_1, double *t_ave, const double *ft, const double *mu_tend,
+    double rdx, double rdy, double dts, double epssm,
+    const double *dnw, const double *fnm, const double *fnp, const double *rdnw,
+    const double *msfuy, const double *msfvx_inv, const double *msftx, const double *msfty,
     int periodic_x, int specified, int nested,
     int ids, int ide, int jds, int jde, int kde,
     int ims, int ime, int jms, int jme, int kms, int kme,
@@ -208,6 +242,18 @@ int wrfb200_step(wrfb200_handle *h, int its, int ite, int jts, int jte, int kts,
 /* `nsteps` back-to-back steps replayed from a CUDA graph captured on first use for this tile. */
 int wrfb200_step_graph(wrfb200_handle *h, int its, int ite, int jts, int jte, int kts, int kte, int nsteps);
 int wrfb200_sync(wrfb200_handle *h);
+
+/* real*8 handles: the verbs above that carry a precision, with double arrays / scalars.  create_r8 pads rows to
+ * a multiple of 16 doubles (128 bytes); pitches are in doubles.  step, step_graph, sync, set_stream,
+ * set_kernel, destroy, launch_count and last_kernel work on handles of either precision. */
+int wrfb200_create_r8(wrfb200_handle **out, const wrfb200_domain *dom, int device, int allocate);
+int wrfb200_set_scalars_r8(wrfb200_handle *h, double rdx, double rdy, double dts, double epssm);
+int wrfb200_bind_device_r8(wrfb200_handle *h, int field, double *device_ptr, long pitch);
+int wrfb200_device_ptr_r8(wrfb200_handle *h, int field, double **device_ptr, long *pitch);
+int wrfb200_upload_r8(wrfb200_handle *h, int field, const double *host);
+int wrfb200_download_r8(wrfb200_handle *h, int field, double *host);
+int wrfb200_upload_range_r8(wrfb200_handle *h, int field, const double *host, int i0, int i1, int k0, int k1, int j0, int j1);
+int wrfb200_download_range_r8(wrfb200_handle *h, int field, double *host, int i0, int i1, int k0, int k1, int j0, int j1);
 
 /* Number of kernels this library has launched on behalf of `h` since creation (bench accounting). */
 int wrfb200_launch_count(wrfb200_handle *h, long *count);

@@ -51,11 +51,14 @@ class WrfB200Error(RuntimeError):
 
 _P = C.c_void_p
 _ADV_ARGS = ([_P] * 18 + [C.c_float] * 4 + [_P] * 8 + [C.c_int] * 3 + [C.c_int] * 5 + [C.c_int] * 6 + [C.c_int] * 6)
+_ADV_ARGS_R8 = ([_P] * 18 + [C.c_double] * 4 + [_P] * 8 + [C.c_int] * 3 + [C.c_int] * 5 + [C.c_int] * 6 + [C.c_int] * 6)
 
 # every symbol include/wrfb200.h declares, with its ctypes prototype
 PROTOTYPES = {
     "wrfb200_advance_mu_t": (C.c_int, _ADV_ARGS),
     "wrfb200_advance_mu_t_loop": (C.c_int, _ADV_ARGS + [C.c_int]),
+    "wrfb200_advance_mu_t_r8": (C.c_int, _ADV_ARGS_R8),
+    "wrfb200_advance_mu_t_loop_r8": (C.c_int, _ADV_ARGS_R8 + [C.c_int]),
     "wrfb200_set_default_stream": (C.c_int, [_P]),
     "wrfb200_set_default_kernel": (C.c_int, [C.c_int]),
     "wrfb200_release_cache": (C.c_int, []),
@@ -81,6 +84,14 @@ PROTOTYPES = {
     "wrfb200_download": (C.c_int, [_P, C.c_int, _P]),
     "wrfb200_upload_range": (C.c_int, [_P, C.c_int, _P] + [C.c_int] * 6),
     "wrfb200_download_range": (C.c_int, [_P, C.c_int, _P] + [C.c_int] * 6),
+    "wrfb200_create_r8": (C.c_int, [C.POINTER(_P), C.POINTER(Domain), C.c_int, C.c_int]),
+    "wrfb200_set_scalars_r8": (C.c_int, [_P, C.c_double, C.c_double, C.c_double, C.c_double]),
+    "wrfb200_bind_device_r8": (C.c_int, [_P, C.c_int, _P, C.c_long]),
+    "wrfb200_device_ptr_r8": (C.c_int, [_P, C.c_int, C.POINTER(_P), C.POINTER(C.c_long)]),
+    "wrfb200_upload_r8": (C.c_int, [_P, C.c_int, _P]),
+    "wrfb200_download_r8": (C.c_int, [_P, C.c_int, _P]),
+    "wrfb200_upload_range_r8": (C.c_int, [_P, C.c_int, _P] + [C.c_int] * 6),
+    "wrfb200_download_range_r8": (C.c_int, [_P, C.c_int, _P] + [C.c_int] * 6),
     "wrfb200_step": (C.c_int, [_P] + [C.c_int] * 6),
     "wrfb200_step_graph": (C.c_int, [_P] + [C.c_int] * 7),
     "wrfb200_sync": (C.c_int, [_P]),

@@ -8,6 +8,8 @@ object with ``periodic_x / specified / nested`` members, the only ones the routi
 
 Arrays are numpy float32 in C order ``[j, k, i]`` / ``[j, i]`` / ``[k]`` -- byte-identical to the Fortran
 ``(i,k,j)`` / ``(i,j)`` / ``(k)`` layout -- or torch CUDA tensors of the same shape (launched in place).
+float64 arrays (WRF built with -r8) take the ``_r8`` entry points and are computed in binary64; one call's
+arrays must all have the same precision.
 All compute happens in the CUDA library; nothing here falls back to the CPU.
 """
 from __future__ import annotations
@@ -113,18 +115,38 @@ class Grid:
         return replace(self, its=its, ite=ite, jts=jts, jte=jte)
 
 
-def _ptr(a) -> int:
-    """Raw address of a numpy array (host) or torch tensor (host or device)."""
+def _dtype(a):
+    """np.float32 / np.float64 for a numpy array or torch tensor of that precision, else None."""
     if isinstance(a, np.ndarray):
-        if a.dtype != np.float32 or not a.flags["C_CONTIGUOUS"]:
-            raise TypeError("fields must be C-contiguous float32 arrays")
-        return a.ctypes.data
+        return a.dtype.type if a.dtype in (np.float32, np.float64) else None
     if hasattr(a, "data_ptr"):
         import torch
-        if a.dtype != torch.float32 or not a.is_contiguous():
-            raise TypeError("fields must be contiguous float32 tensors")
+        return {torch.float32: np.float32, torch.float64: np.float64}.get(a.dtype)
+    return None
+
+
+def _ptr(a, dtype=np.float32) -> int:
+    """Raw address of a numpy array (host) or torch tensor (host or device) of precision ``dtype``."""
+    name = np.dtype(dtype).name
+    if isinstance(a, np.ndarray):
+        if a.dtype != dtype or not a.flags["C_CONTIGUOUS"]:
+            raise TypeError(f"fields must be C-contiguous {name} arrays")
+        return a.ctypes.data
+    if hasattr(a, "data_ptr"):
+        if _dtype(a) is not dtype or not a.is_contiguous():
+            raise TypeError(f"fields must be contiguous {name} tensors")
         return a.data_ptr()
     raise TypeError(f"unsupported array type {type(a)!r}")
+
+
+def _precision(arrays) -> type:
+    """The one precision (np.float32 or np.float64) shared by every array of a call."""
+    kinds = {_dtype(a) for a in arrays}
+    if len(kinds) != 1 or None in kinds:
+        names = sorted({str(getattr(a, "dtype", type(a).__name__)) for a in arrays})
+        raise TypeError("advance_mu_t needs all arrays float32 (default REAL) or all float64 (-r8), "
+                        f"got {', '.join(names)}")
+    return kinds.pop()
 
 
 def advance_mu_t(ww, ww_1, u, u_1, v, v_1, mu, mut, muave, muts, muu, muv, mudf, t, t_1, t_ave, ft, mu_tend,
@@ -134,18 +156,21 @@ def advance_mu_t(ww, ww_1, u, u_1, v, v_1, mu, mut, muave, muts, muu, muv, mudf,
     """The reference operator (module_small_step_em.f90:7-18), executed on the GPU.
 
     Updates ww, mu, muave, muts, mudf, t, t_ave in place.  ``nsteps`` > 1 repeats the step on
-    device-resident state with a single upload/download (host arrays only).
+    device-resident state with a single upload/download (host arrays only).  All-float32 arrays run the
+    binary32 operator, all-float64 arrays the real*8 one (``wrfb200_advance_mu_t_r8``); a mix raises TypeError.
     """
     arrays_a = (ww, ww_1, u, u_1, v, v_1, mu, mut, muave, muts, muu, muv, mudf, t, t_1, t_ave, ft, mu_tend)
     arrays_b = (dnw, fnm, fnp, rdnw, msfuy, msfvx_inv, msftx, msfty)
-    args = ([_ptr(a) for a in arrays_a] + [float(rdx), float(rdy), float(dts), float(epssm)]
-            + [_ptr(a) for a in arrays_b]
+    dt = _precision(arrays_a + arrays_b)
+    args = ([_ptr(a, dt) for a in arrays_a] + [float(rdx), float(rdy), float(dts), float(epssm)]
+            + [_ptr(a, dt) for a in arrays_b]
             + [int(bool(config_flags.periodic_x)), int(bool(config_flags.specified)), int(bool(config_flags.nested))]
             + [int(x) for x in (ids, ide, jds, jde, kde, ims, ime, jms, jme, kms, kme, its, ite, jts, jte, kts, kte)])
+    sfx = "_r8" if dt is np.float64 else ""
     if nsteps == 1:
-        check(lib().wrfb200_advance_mu_t(*args))
+        check(getattr(lib(), "wrfb200_advance_mu_t" + sfx)(*args))
     else:
-        check(lib().wrfb200_advance_mu_t_loop(*args, int(nsteps)))
+        check(getattr(lib(), "wrfb200_advance_mu_t_loop" + sfx)(*args, int(nsteps)))
 
 
 def call_with_fields(fields: Dict[str, object], grid: Grid, rdx, rdy, dts, epssm, nsteps: int = 1) -> None:
@@ -156,13 +181,19 @@ def call_with_fields(fields: Dict[str, object], grid: Grid, rdx, rdy, dts, epssm
 
 
 class Patch:
-    """Device-resident state of one patch (one rank): wrfb200_create / upload / step / download."""
+    """Device-resident state of one patch (one rank): wrfb200_create / upload / step / download.
 
-    def __init__(self, grid: Grid, device: int = -1, allocate: bool = True, stream: Optional[int] = None):
+    ``dtype`` np.float64 (or torch.float64) makes a real*8 patch (wrfb200_create_r8): fields are float64 and the
+    step runs in binary64.  The multi-GPU, halo, stand-in and resident-bundle verbs are binary32 only."""
+
+    def __init__(self, grid: Grid, device: int = -1, allocate: bool = True, stream: Optional[int] = None,
+                 dtype=np.float32):
         self.grid = grid
+        self.dtype = _patch_dtype(dtype)
+        self._sfx = "_r8" if self.dtype is np.float64 else ""
         self._h = C.c_void_p()
         dom = grid.domain()
-        check(lib().wrfb200_create(C.byref(self._h), C.byref(dom), device, int(allocate)))
+        check(getattr(lib(), "wrfb200_create" + self._sfx)(C.byref(self._h), C.byref(dom), device, int(allocate)))
         if stream is not None:
             self.set_stream(stream)
 
@@ -188,8 +219,12 @@ class Patch:
     def set_stream(self, cuda_stream: int):
         check(lib().wrfb200_set_stream(self._h, C.c_void_p(cuda_stream)))
 
+    def _fn(self, name):
+        """The C verb of this patch's precision."""
+        return getattr(lib(), name + self._sfx)
+
     def set_scalars(self, rdx, rdy, dts, epssm):
-        check(lib().wrfb200_set_scalars(self._h, float(rdx), float(rdy), float(dts), float(epssm)))
+        check(self._fn("wrfb200_set_scalars")(self._h, float(rdx), float(rdy), float(dts), float(epssm)))
 
     def set_kernel(self, kernel: int):
         check(lib().wrfb200_set_kernel(self._h, int(kernel)))
@@ -198,11 +233,12 @@ class Patch:
         """Adopt a caller-owned device buffer (e.g. a torch CUDA tensor) for ``field``."""
         if pitch is None:
             pitch = tensor.shape[-1]
-        check(lib().wrfb200_bind_device(self._h, FIELD_ID[field], C.c_void_p(_ptr(tensor)), int(pitch)))
+        check(self._fn("wrfb200_bind_device")(self._h, FIELD_ID[field], C.c_void_p(_ptr(tensor, self.dtype)),
+                                              int(pitch)))
 
     def device_ptr(self, field: str):
         p, pitch = C.c_void_p(), C.c_long()
-        check(lib().wrfb200_device_ptr(self._h, FIELD_ID[field], C.byref(p), C.byref(pitch)))
+        check(self._fn("wrfb200_device_ptr")(self._h, FIELD_ID[field], C.byref(p), C.byref(pitch)))
         return p.value, pitch.value
 
     # ---- copies (async on the patch stream) ----
@@ -211,19 +247,21 @@ class Patch:
             a = fields[n]
             if tuple(a.shape) != self.grid.shape_of(n):
                 raise ValueError(f"{n}: shape {tuple(a.shape)} != {self.grid.shape_of(n)}")
-            check(lib().wrfb200_upload(self._h, FIELD_ID[n], C.c_void_p(_ptr(a))))
+            check(self._fn("wrfb200_upload")(self._h, FIELD_ID[n], C.c_void_p(_ptr(a, self.dtype))))
 
     def download(self, fields: Dict[str, np.ndarray], names: Iterable[str] = OUTPUT_FIELDS, sync: bool = True):
         for n in names:
-            check(lib().wrfb200_download(self._h, FIELD_ID[n], C.c_void_p(_ptr(fields[n]))))
+            check(self._fn("wrfb200_download")(self._h, FIELD_ID[n], C.c_void_p(_ptr(fields[n], self.dtype))))
         if sync:
             self.sync()
 
     def download_range(self, field: str, host, i0, i1, k0, k1, j0, j1):
-        check(lib().wrfb200_download_range(self._h, FIELD_ID[field], C.c_void_p(_ptr(host)), i0, i1, k0, k1, j0, j1))
+        check(self._fn("wrfb200_download_range")(self._h, FIELD_ID[field], C.c_void_p(_ptr(host, self.dtype)),
+                                                 i0, i1, k0, k1, j0, j1))
 
     def upload_range(self, field: str, host, i0, i1, k0, k1, j0, j1):
-        check(lib().wrfb200_upload_range(self._h, FIELD_ID[field], C.c_void_p(_ptr(host)), i0, i1, k0, k1, j0, j1))
+        check(self._fn("wrfb200_upload_range")(self._h, FIELD_ID[field], C.c_void_p(_ptr(host, self.dtype)),
+                                               i0, i1, k0, k1, j0, j1))
 
     # ---- resident-state verbs (the three cadences of the acoustic loop) ----
     CONSTANTS = ("ww_1", "u_1", "v_1", "t_1", "ft", "mut", "muu", "muv", "mu_tend",
@@ -324,6 +362,19 @@ class Patch:
         t, n = C.c_int(), C.c_long()
         check(lib().wrfb200_comm_status(self._h, C.byref(t), C.byref(n)))
         return t.value, n.value
+
+
+def _patch_dtype(dtype):
+    """np.float32 / np.float64 from a numpy or torch dtype."""
+    if dtype in (np.float32, np.float64):
+        return np.dtype(dtype).type
+    if hasattr(dtype, "is_floating_point"):         # torch.dtype
+        import torch
+        if dtype in (torch.float32, torch.float64):
+            return np.float32 if dtype == torch.float32 else np.float64
+    if isinstance(dtype, np.dtype) and dtype.type in (np.float32, np.float64):
+        return dtype.type
+    raise TypeError(f"Patch dtype must be float32 or float64, got {dtype!r}")
 
 
 class acoustic_loop:

@@ -48,34 +48,40 @@ struct AmtHalo {
     unsigned long long timeout_ns;     // a flag wait gives up after this long (never hang the GPU)
 };
 
-struct AmtParams {
+// Argument block of one launch, for element type T (float: the real*4 kernels; double: the real*8 kernels of a
+// handle created with wrfb200_create_r8).  AmtParams / AmtParamsR8 below are the two instances; the float one keeps
+// its own struct name so the float kernels' symbols do not change.
+template <class T>
+struct AmtFields {
     // 3-D fields, (i fastest, k, j): element (i,k,j) at  j*jstride + k*pitch + i
-    float *ww;
-    const float *ww_1, *u, *u_1, *v, *v_1;
-    float *t;
-    const float *t_1;
-    float *t_ave;
-    const float *ft;
+    T *ww;
+    const T *ww_1, *u, *u_1, *v, *v_1;
+    T *t;
+    const T *t_1;
+    T *t_ave;
+    const T *ft;
     // 2-D fields: element (i,j) at  j*pitch2 + i
-    float *mu;
-    const float *mut;
-    float *muave, *muts;
-    const float *muu, *muv;
-    float *mudf;
-    const float *mu_tend, *msfuy, *msfvx_inv, *msftx, *msfty;
+    T *mu;
+    const T *mut;
+    T *muave, *muts;
+    const T *muu, *muv;
+    T *mudf;
+    const T *mu_tend, *msfuy, *msfvx_inv, *msftx, *msfty;
     // 1-D fields, index 0 = level kms
-    const float *dnw, *fnm, *fnp, *rdnw;
-    float rdx, rdy, dts, epssm;
-    long long pitch;    // 3-D row stride in floats
-    long long jstride;  // 3-D plane stride in floats (= pitch * kdim)
-    long long pitch2;   // 2-D row stride in floats
+    const T *dnw, *fnm, *fnp, *rdnw;
+    T rdx, rdy, dts, epssm;
+    long long pitch;    // 3-D row stride in elements
+    long long jstride;  // 3-D plane stride in elements (= pitch * kdim)
+    long long pitch2;   // 2-D row stride in elements
     int i0, i1;         // computed i range (i_start..i_end), inclusive, memory index
     int j0, j1;         // computed j range
     int k0;             // memory index of level kts
     int nk;             // number of computed levels: k_start..k_end = kts..kte-1
     int kdim, jdim;     // memory extents in k and j (jstride == pitch * kdim)
-    AmtHalo halo;       // fused multi-GPU halo exchange (enabled == 0 on a single GPU)
+    AmtHalo halo;       // fused multi-GPU halo exchange (enabled == 0 on a single GPU; always 0 for double)
 };
+struct AmtParams : AmtFields<float> {};
+struct AmtParamsR8 : AmtFields<double> {};
 
 // Tensor maps of the TMA-staged kernel (amt_pipe.cu): boxes are [columns x 1 level x rows].
 struct AmtTmaMaps {
@@ -97,6 +103,13 @@ __device__ __forceinline__ float f_add(float a, float b) { return __fadd_rn(a, b
 __device__ __forceinline__ float f_sub(float a, float b) { return __fsub_rn(a, b); }
 __device__ __forceinline__ float f_mul(float a, float b) { return __fmul_rn(a, b); }
 __device__ __forceinline__ float f_div(float a, float b) { return __fdiv_rn(a, b); }
+// The same four in binary64 for the real*8 kernels.  Division stays the IEEE __ddiv_rn: its correctly rounded
+// sequence is built from DFMA internally (as __fdiv_rn's is from FFMA), but no operation of the formula itself is
+// ever contracted.
+__device__ __forceinline__ double f_add(double a, double b) { return __dadd_rn(a, b); }
+__device__ __forceinline__ double f_sub(double a, double b) { return __dsub_rn(a, b); }
+__device__ __forceinline__ double f_mul(double a, double b) { return __dmul_rn(a, b); }
+__device__ __forceinline__ double f_div(double a, double b) { return __ddiv_rn(a, b); }
 
 // ---- cross-GPU flag helpers (system scope: the peer is another GPU on NVLink) ----
 __device__ __forceinline__ unsigned ld_acquire_sys(const unsigned *p)
@@ -170,3 +183,7 @@ bool amt_tile_supported(const AmtParams &p);
 bool amt_pipe_supported(const AmtParams &p);
 bool amt_build_tma_maps(const AmtParams &p, AmtTmaMaps *maps);                    // cached: rebuilds only on change
 cudaError_t amt_launch_pipe(const AmtParams &p, const AmtTmaMaps &maps, cudaStream_t stream, int cfg);   // cfg 0 = automatic
+// real*8 kernels (amt_column.cu, amt_tile_r8.cu)
+cudaError_t amt_launch_column(const AmtParamsR8 &p, cudaStream_t stream);
+cudaError_t amt_launch_tile(const AmtParamsR8 &p, cudaStream_t stream);
+bool amt_tile_supported(const AmtParamsR8 &p);

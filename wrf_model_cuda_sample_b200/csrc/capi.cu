@@ -18,6 +18,7 @@
 #include <new>
 #include <string>
 #include <tuple>
+#include <type_traits>
 
 #include "amt_params.h"
 #include "capi_internal.h"
@@ -60,11 +61,15 @@ int check_domain(const wrfb200_domain &d)
 
 }  // namespace
 
+namespace {
+
 // Build the kernel argument block for the tile its:ite x jts:jte.  Returns >0 status on error,
-// sets *empty when the index sets are empty (legal: nothing to do).
-int wrfb200_make_params(const wrfb200_handle *h, int its, int ite, int jts, int jte, int kts, int kte,
-                AmtParams *out, bool *empty)
+// sets *empty when the index sets are empty (legal: nothing to do).  P = AmtParams or AmtParamsR8, matching
+// the handle's element size (the callers check it).
+template <class P>
+int make_params(const wrfb200_handle *h, int its, int ite, int jts, int jte, int kts, int kte, P *out, bool *empty)
 {
+    using T = std::remove_pointer_t<decltype(P::ww)>;
     const wrfb200_domain &d = h->dom;
     if (kts != 1) return fail(WRFB200_ERR_UNSUPPORTED, "kts=%d: the routine addresses levels 1 and 2 literally (module_small_step_em.f90:159,168,209)", kts);
     if (kte != d.kde) return fail(WRFB200_ERR_UNSUPPORTED, "kte=%d != kde=%d: wdtn(kde) is the top boundary flux (module_small_step_em.f90:221)", kte, d.kde);
@@ -80,23 +85,25 @@ int wrfb200_make_params(const wrfb200_handle *h, int its, int ite, int jts, int 
                     is, ie, js, je, d.ims, d.ime, d.jms, d.jme);
     for (int f = 0; f < WRFB200_NUM_FIELDS; ++f)
         if (!h->d[f]) return fail(WRFB200_ERR_STATE, "field %d has no device buffer (allocate or bind it)", f);
-    if (!h->scalars_set) return fail(WRFB200_ERR_STATE, "rdx/rdy/dts/epssm not set (wrfb200_set_scalars)");
+    if (!h->scalars_set)
+        return fail(WRFB200_ERR_STATE, "rdx/rdy/dts/epssm not set (wrfb200_set_scalars%s)", sizeof(T) == 8 ? "_r8" : "");
 
-    AmtParams p{};
-    p.ww = h->d[WRFB200_WW];       p.ww_1 = h->d[WRFB200_WW_1];
-    p.u = h->d[WRFB200_U];         p.u_1 = h->d[WRFB200_U_1];
-    p.v = h->d[WRFB200_V];         p.v_1 = h->d[WRFB200_V_1];
-    p.t = h->d[WRFB200_T];         p.t_1 = h->d[WRFB200_T_1];
-    p.t_ave = h->d[WRFB200_T_AVE]; p.ft = h->d[WRFB200_FT];
-    p.mu = h->d[WRFB200_MU];       p.mut = h->d[WRFB200_MUT];
-    p.muave = h->d[WRFB200_MUAVE]; p.muts = h->d[WRFB200_MUTS];
-    p.muu = h->d[WRFB200_MUU];     p.muv = h->d[WRFB200_MUV];
-    p.mudf = h->d[WRFB200_MUDF];   p.mu_tend = h->d[WRFB200_MU_TEND];
-    p.msfuy = h->d[WRFB200_MSFUY]; p.msfvx_inv = h->d[WRFB200_MSFVX_INV];
-    p.msftx = h->d[WRFB200_MSFTX]; p.msfty = h->d[WRFB200_MSFTY];
-    p.dnw = h->d[WRFB200_DNW];     p.fnm = h->d[WRFB200_FNM];
-    p.fnp = h->d[WRFB200_FNP];     p.rdnw = h->d[WRFB200_RDNW];
-    p.rdx = h->rdx; p.rdy = h->rdy; p.dts = h->dts; p.epssm = h->epssm;
+    auto F = [h](int f) { return reinterpret_cast<T *>(h->d[f]); };
+    P p{};
+    p.ww = F(WRFB200_WW);       p.ww_1 = F(WRFB200_WW_1);
+    p.u = F(WRFB200_U);         p.u_1 = F(WRFB200_U_1);
+    p.v = F(WRFB200_V);         p.v_1 = F(WRFB200_V_1);
+    p.t = F(WRFB200_T);         p.t_1 = F(WRFB200_T_1);
+    p.t_ave = F(WRFB200_T_AVE); p.ft = F(WRFB200_FT);
+    p.mu = F(WRFB200_MU);       p.mut = F(WRFB200_MUT);
+    p.muave = F(WRFB200_MUAVE); p.muts = F(WRFB200_MUTS);
+    p.muu = F(WRFB200_MUU);     p.muv = F(WRFB200_MUV);
+    p.mudf = F(WRFB200_MUDF);   p.mu_tend = F(WRFB200_MU_TEND);
+    p.msfuy = F(WRFB200_MSFUY); p.msfvx_inv = F(WRFB200_MSFVX_INV);
+    p.msftx = F(WRFB200_MSFTX); p.msfty = F(WRFB200_MSFTY);
+    p.dnw = F(WRFB200_DNW);     p.fnm = F(WRFB200_FNM);
+    p.fnp = F(WRFB200_FNP);     p.rdnw = F(WRFB200_RDNW);
+    p.rdx = (T)h->rdx; p.rdy = (T)h->rdy; p.dts = (T)h->dts; p.epssm = (T)h->epssm;   // exact: stored from a T
     p.pitch = h->pitch3;
     p.jstride = h->pitch3 * (long long)h->kdim;
     p.pitch2 = h->pitch2;
@@ -110,13 +117,15 @@ int wrfb200_make_params(const wrfb200_handle *h, int its, int ite, int jts, int 
     return WRFB200_OK;
 }
 
-namespace {
+}  // namespace
 
-inline int make_params(const wrfb200_handle *h, int its, int ite, int jts, int jte, int kts, int kte,
-                       AmtParams *out, bool *empty)
+int wrfb200_make_params(const wrfb200_handle *h, int its, int ite, int jts, int jte, int kts, int kte,
+                AmtParams *out, bool *empty)
 {
-    return wrfb200_make_params(h, its, ite, jts, jte, kts, kte, out, empty);
+    return make_params(h, its, ite, jts, jte, kts, kte, out, empty);
 }
+
+namespace {
 
 // Tuning override for the pipelined kernel: WRFB200_PIPE_CFG = TJ*10 + STAGES (0 / unset = automatic).
 int pipe_cfg()
@@ -159,7 +168,67 @@ int launch(wrfb200_handle *h, const AmtParams &p, cudaStream_t s, int kernel)
     return WRFB200_OK;
 }
 
+// real*8: the double2 tile kernel where the layout allows it, else the any-layout column kernel.  The TMA pipe
+// kernel is binary32 only.
+int launch(wrfb200_handle *h, const AmtParamsR8 &p, cudaStream_t s, int kernel)
+{
+    cudaError_t e;
+    int ran = kernel;
+    if (kernel == WRFB200_KERNEL_PIPE) {
+        return fail(WRFB200_ERR_UNSUPPORTED, "the pipe kernel is binary32 only; a real*8 handle runs the tile or column kernel");
+    } else if (kernel == WRFB200_KERNEL_COLUMN) {
+        e = amt_launch_column(p, s);
+    } else if (kernel == WRFB200_KERNEL_TILE) {
+        if (!amt_tile_supported(p))
+            return fail(WRFB200_ERR_UNSUPPORTED, "real*8 tile kernel needs 16-byte aligned fields, pitches of an even "
+                                                 "number of doubles and at most 220 levels (nk=%d)", p.nk);
+        e = amt_launch_tile(p, s);
+    } else {
+        // AUTO: tiles narrower than a warp of columns take the column kernel, as for binary32
+        const bool wide = (p.i1 - p.i0 + 1) >= 32;
+        if (wide && amt_tile_supported(p)) {
+            e = amt_launch_tile(p, s);
+            ran = WRFB200_KERNEL_TILE;
+        } else {
+            e = amt_launch_column(p, s);
+            ran = WRFB200_KERNEL_COLUMN;
+        }
+    }
+    if (e != cudaSuccess) return fail(WRFB200_ERR_CUDA, "kernel launch failed: %s", cudaGetErrorString(e));
+    h->launches += 1;
+    h->last_kernel = ran;
+    return WRFB200_OK;
+}
+
+// validate the tile and launch one step on `s` in the handle's precision
+int step_on(wrfb200_handle *h, int its, int ite, int jts, int jte, int kts, int kte, cudaStream_t s, int kernel)
+{
+    bool empty = false;
+    if (h->esize == 8) {
+        AmtParamsR8 p;
+        if (int rc = make_params(h, its, ite, jts, jte, kts, kte, &p, &empty)) return rc;
+        return empty ? WRFB200_OK : launch(h, p, s, kernel);
+    }
+    AmtParams p;
+    if (int rc = make_params(h, its, ite, jts, jte, kts, kte, &p, &empty)) return rc;
+    return empty ? WRFB200_OK : launch(h, p, s, kernel);
+}
+
+// A verb typed for one precision applied to a handle of the other.
+int wrong_precision(const wrfb200_handle *h, const char *verb)
+{
+    return fail(WRFB200_ERR_STATE, "%s: this is a %s handle (created by %s); use the %s verbs", verb,
+                h->esize == 8 ? "real*8" : "real*4", h->esize == 8 ? "wrfb200_create_r8" : "wrfb200_create",
+                h->esize == 8 ? "_r8" : "binary32 (no _r8 suffix)");
+}
+
 }  // namespace
+
+int wrfb200_require_r4(const wrfb200_handle *h, const char *what)
+{
+    if (h->esize == 4) return WRFB200_OK;
+    return fail(WRFB200_ERR_UNSUPPORTED, "%s is binary32 only and not available on a real*8 handle", what);
+}
 
 int wrfb200_launch_params(wrfb200_handle *h, const AmtParams &p, cudaStream_t s, int kernel)
 {
@@ -184,8 +253,9 @@ struct DeviceGuard {
     DeviceGuard guard_((h)->device);                                                                 \
     if (!guard_.ok) return fail(WRFB200_ERR_CUDA, "cannot select CUDA device %d", (h)->device)
 
-// Copy a Fortran-numbered sub-box between a dense host array and the (pitched) device mirror.
-int copy_range(wrfb200_handle *h, int field, const float *host_src, float *host_dst,
+// Copy a Fortran-numbered sub-box between a dense host array and the (pitched) device mirror, in elements of
+// the handle's size (4 or 8 bytes).
+int copy_range(wrfb200_handle *h, int field, const void *host_src, void *host_dst,
                int i0, int i1, int k0, int k1, int j0, int j1)
 {
     const wrfb200_domain &d = h->dom;
@@ -193,53 +263,58 @@ int copy_range(wrfb200_handle *h, int field, const float *host_src, float *host_
     if (!h->d[field]) return fail(WRFB200_ERR_STATE, "field %d has no device buffer", field);
     const bool to_dev = host_src != nullptr;
     const cudaMemcpyKind kind = to_dev ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToHost;
+    const size_t es = (size_t)h->esize;
+    char *dev = reinterpret_cast<char *>(h->d[field]);
+    char *host = to_dev ? const_cast<char *>(static_cast<const char *>(host_src)) : static_cast<char *>(host_dst);
     if (is1d(field)) {
         if (k0 < d.kms || k1 > d.kme || k0 > k1) return fail(WRFB200_ERR_INVALID_ARG, "bad k range %d..%d", k0, k1);
-        const size_t off = (size_t)(k0 - d.kms), n = (size_t)(k1 - k0 + 1) * sizeof(float);
-        if (to_dev) CU(cudaMemcpyAsync(h->d[field] + off, host_src + off, n, kind, h->stream));
-        else        CU(cudaMemcpyAsync(host_dst + off, h->d[field] + off, n, kind, h->stream));
+        const size_t off = (size_t)(k0 - d.kms) * es, n = (size_t)(k1 - k0 + 1) * es;
+        if (to_dev) CU(cudaMemcpyAsync(dev + off, host + off, n, kind, h->stream));
+        else        CU(cudaMemcpyAsync(host + off, dev + off, n, kind, h->stream));
         return WRFB200_OK;
     }
     if (i0 < d.ims || i1 > d.ime || i0 > i1 || j0 < d.jms || j1 > d.jme || j0 > j1)
         return fail(WRFB200_ERR_INVALID_ARG, "bad i/j range %d..%d, %d..%d", i0, i1, j0, j1);
-    const size_t w = (size_t)(i1 - i0 + 1) * sizeof(float);
+    const size_t w = (size_t)(i1 - i0 + 1) * es;
     if (is2d(field)) {
-        const size_t hoff = (size_t)(j0 - d.jms) * h->idim + (size_t)(i0 - d.ims);
-        const size_t doff = (size_t)(j0 - d.jms) * h->pitch2 + (size_t)(i0 - d.ims);
+        const size_t hoff = ((size_t)(j0 - d.jms) * h->idim + (size_t)(i0 - d.ims)) * es;
+        const size_t doff = ((size_t)(j0 - d.jms) * h->pitch2 + (size_t)(i0 - d.ims)) * es;
         const size_t rows = (size_t)(j1 - j0 + 1);
         if (to_dev)
-            CU(cudaMemcpy2DAsync(h->d[field] + doff, h->pitch2 * sizeof(float), host_src + hoff,
-                                 h->idim * sizeof(float), w, rows, kind, h->stream));
+            CU(cudaMemcpy2DAsync(dev + doff, h->pitch2 * es, host + hoff, h->idim * es, w, rows, kind, h->stream));
         else
-            CU(cudaMemcpy2DAsync(host_dst + hoff, h->idim * sizeof(float), h->d[field] + doff,
-                                 h->pitch2 * sizeof(float), w, rows, kind, h->stream));
+            CU(cudaMemcpy2DAsync(host + hoff, h->idim * es, dev + doff, h->pitch2 * es, w, rows, kind, h->stream));
         return WRFB200_OK;
     }
     if (k0 < d.kms || k1 > d.kme || k0 > k1) return fail(WRFB200_ERR_INVALID_ARG, "bad k range %d..%d", k0, k1);
     const size_t nkc = (size_t)(k1 - k0 + 1), njc = (size_t)(j1 - j0 + 1);
-    const size_t hoff = ((size_t)(j0 - d.jms) * h->kdim + (size_t)(k0 - d.kms)) * h->idim + (size_t)(i0 - d.ims);
-    const size_t doff = ((size_t)(j0 - d.jms) * h->kdim + (size_t)(k0 - d.kms)) * h->pitch3 + (size_t)(i0 - d.ims);
+    const size_t hoff = (((size_t)(j0 - d.jms) * h->kdim + (size_t)(k0 - d.kms)) * h->idim + (size_t)(i0 - d.ims)) * es;
+    const size_t doff = (((size_t)(j0 - d.jms) * h->kdim + (size_t)(k0 - d.kms)) * h->pitch3 + (size_t)(i0 - d.ims)) * es;
     if (nkc == (size_t)h->kdim) {
         // whole columns: rows of one field are equally spaced across k AND j -> a single 2-D copy
         const size_t rows = nkc * njc;
         if (to_dev)
-            CU(cudaMemcpy2DAsync(h->d[field] + doff, h->pitch3 * sizeof(float), host_src + hoff,
-                                 h->idim * sizeof(float), w, rows, kind, h->stream));
+            CU(cudaMemcpy2DAsync(dev + doff, h->pitch3 * es, host + hoff, h->idim * es, w, rows, kind, h->stream));
         else
-            CU(cudaMemcpy2DAsync(host_dst + hoff, h->idim * sizeof(float), h->d[field] + doff,
-                                 h->pitch3 * sizeof(float), w, rows, kind, h->stream));
+            CU(cudaMemcpy2DAsync(host + hoff, h->idim * es, dev + doff, h->pitch3 * es, w, rows, kind, h->stream));
         return WRFB200_OK;
     }
     cudaMemcpy3DParms cp{};
-    float *hp = to_dev ? const_cast<float *>(host_src) : host_dst;
-    cudaPitchedPtr hostp = make_cudaPitchedPtr(hp + hoff, h->idim * sizeof(float), h->idim * sizeof(float), h->kdim);
-    cudaPitchedPtr devp = make_cudaPitchedPtr(h->d[field] + doff, h->pitch3 * sizeof(float), h->pitch3 * sizeof(float), h->kdim);
+    cudaPitchedPtr hostp = make_cudaPitchedPtr(host + hoff, h->idim * es, h->idim * es, h->kdim);
+    cudaPitchedPtr devp = make_cudaPitchedPtr(dev + doff, h->pitch3 * es, h->pitch3 * es, h->kdim);
     cp.srcPtr = to_dev ? hostp : devp;
     cp.dstPtr = to_dev ? devp : hostp;
     cp.extent = make_cudaExtent(w, nkc, njc);
     cp.kind = kind;
     CU(cudaMemcpy3DAsync(&cp, h->stream));
     return WRFB200_OK;
+}
+
+// whole-field copy
+int copy_field(wrfb200_handle *h, int field, const void *host_src, void *host_dst)
+{
+    const wrfb200_domain &d = h->dom;
+    return copy_range(h, field, host_src, host_dst, d.ims, d.ime, d.kms, d.kme, d.jms, d.jme);
 }
 
 }  // namespace
@@ -288,7 +363,9 @@ extern "C" int wrfb200_bounds(int periodic_x, int specified, int nested,
 // -------------------------------------------------------------------------------------------------
 // exported: handle life cycle
 // -------------------------------------------------------------------------------------------------
-extern "C" int wrfb200_create(wrfb200_handle **out, const wrfb200_domain *dom, int device, int allocate)
+namespace {
+
+int create(wrfb200_handle **out, const wrfb200_domain *dom, int device, int allocate, int esize)
 {
     if (!out || !dom) return fail(WRFB200_ERR_INVALID_ARG, "null argument");
     *out = nullptr;
@@ -302,24 +379,25 @@ extern "C" int wrfb200_create(wrfb200_handle **out, const wrfb200_domain *dom, i
     if (!h) return fail(WRFB200_ERR_NOMEM, "out of host memory");
     h->dom = *dom;
     h->device = device;
+    h->esize = esize;
     h->idim = dom->ime - dom->ims + 1;
     h->jdim = dom->jme - dom->jms + 1;
     h->kdim = dom->kme - dom->kms + 1;
     if (allocate) {
         DeviceGuard g(device);
         if (!g.ok) { delete h; return fail(WRFB200_ERR_CUDA, "cannot select CUDA device %d", device); }
-        h->pitch3 = h->pitch2 = round_up(h->idim, 32);          // 128-byte rows
+        h->pitch3 = h->pitch2 = round_up(h->idim, 128 / esize);  // 128-byte rows
         for (int f = 0; f < WRFB200_NUM_FIELDS; ++f) {
             size_t n = is3d(f) ? (size_t)h->pitch3 * h->kdim * h->jdim
                      : is2d(f) ? (size_t)h->pitch2 * h->jdim
                                : (size_t)h->kdim;
-            cudaError_t e = cudaMalloc(&h->d[f], n * sizeof(float));
-            if (e == cudaSuccess) e = cudaMemsetAsync(h->d[f], 0, n * sizeof(float), nullptr);
+            cudaError_t e = cudaMalloc(&h->d[f], n * esize);
+            if (e == cudaSuccess) e = cudaMemsetAsync(h->d[f], 0, n * esize, nullptr);
             if (e != cudaSuccess) {
                 for (int q = 0; q < f; ++q) cudaFree(h->d[q]);
                 delete h;
                 return fail(e == cudaErrorMemoryAllocation ? WRFB200_ERR_NOMEM : WRFB200_ERR_CUDA,
-                            "cudaMalloc of field %d (%zu bytes) failed: %s", f, n * sizeof(float), cudaGetErrorString(e));
+                            "cudaMalloc of field %d (%zu bytes) failed: %s", f, n * esize, cudaGetErrorString(e));
             }
             h->owned[f] = true;
         }
@@ -327,6 +405,18 @@ extern "C" int wrfb200_create(wrfb200_handle **out, const wrfb200_domain *dom, i
     }
     *out = h;
     return WRFB200_OK;
+}
+
+}  // namespace
+
+extern "C" int wrfb200_create(wrfb200_handle **out, const wrfb200_domain *dom, int device, int allocate)
+{
+    return create(out, dom, device, allocate, 4);
+}
+
+extern "C" int wrfb200_create_r8(wrfb200_handle **out, const wrfb200_domain *dom, int device, int allocate)
+{
+    return create(out, dom, device, allocate, 8);
 }
 
 extern "C" int wrfb200_destroy(wrfb200_handle *h)
@@ -349,9 +439,10 @@ extern "C" int wrfb200_set_stream(wrfb200_handle *h, void *cuda_stream)
     return WRFB200_OK;
 }
 
-extern "C" int wrfb200_set_scalars(wrfb200_handle *h, float rdx, float rdy, float dts, float epssm)
+namespace {
+
+int set_scalars(wrfb200_handle *h, double rdx, double rdy, double dts, double epssm)
 {
-    if (!h) return fail(WRFB200_ERR_INVALID_ARG, "null handle");
     if (h->scalars_set && (rdx != h->rdx || rdy != h->rdy || dts != h->dts || epssm != h->epssm)) {
         for (auto &kv : h->graphs) cudaGraphExecDestroy(kv.second);     // captured kernels hold the old values
         h->graphs.clear();
@@ -359,6 +450,22 @@ extern "C" int wrfb200_set_scalars(wrfb200_handle *h, float rdx, float rdy, floa
     h->rdx = rdx; h->rdy = rdy; h->dts = dts; h->epssm = epssm;
     h->scalars_set = true;
     return WRFB200_OK;
+}
+
+}  // namespace
+
+extern "C" int wrfb200_set_scalars(wrfb200_handle *h, float rdx, float rdy, float dts, float epssm)
+{
+    if (!h) return fail(WRFB200_ERR_INVALID_ARG, "null handle");
+    if (h->esize != 4) return wrong_precision(h, "wrfb200_set_scalars");
+    return set_scalars(h, rdx, rdy, dts, epssm);
+}
+
+extern "C" int wrfb200_set_scalars_r8(wrfb200_handle *h, double rdx, double rdy, double dts, double epssm)
+{
+    if (!h) return fail(WRFB200_ERR_INVALID_ARG, "null handle");
+    if (h->esize != 8) return wrong_precision(h, "wrfb200_set_scalars_r8");
+    return set_scalars(h, rdx, rdy, dts, epssm);
 }
 
 extern "C" int wrfb200_set_kernel(wrfb200_handle *h, int kernel)
@@ -370,9 +477,10 @@ extern "C" int wrfb200_set_kernel(wrfb200_handle *h, int kernel)
     return WRFB200_OK;
 }
 
-extern "C" int wrfb200_bind_device(wrfb200_handle *h, int field, float *device_ptr, long pitch)
+namespace {
+
+int bind_device(wrfb200_handle *h, int field, void *device_ptr, long pitch)
 {
-    if (!h) return fail(WRFB200_ERR_INVALID_ARG, "null handle");
     if (field < 0 || field >= WRFB200_NUM_FIELDS) return fail(WRFB200_ERR_INVALID_ARG, "bad field id %d", field);
     if (!device_ptr) return fail(WRFB200_ERR_INVALID_ARG, "null device pointer");
     if (!is1d(field)) {
@@ -391,52 +499,122 @@ extern "C" int wrfb200_bind_device(wrfb200_handle *h, int field, float *device_p
         cudaFree(h->d[field]);
     }
     h->owned[field] = false;
-    h->d[field] = device_ptr;
+    h->d[field] = static_cast<float *>(device_ptr);
     for (auto &kv : h->graphs) cudaGraphExecDestroy(kv.second);
     h->graphs.clear();
     return WRFB200_OK;
 }
 
-extern "C" int wrfb200_device_ptr(wrfb200_handle *h, int field, float **device_ptr, long *pitch)
+int device_ptr(wrfb200_handle *h, int field, void **ptr, long *pitch)
 {
-    if (!h) return fail(WRFB200_ERR_INVALID_ARG, "null handle");
     if (field < 0 || field >= WRFB200_NUM_FIELDS) return fail(WRFB200_ERR_INVALID_ARG, "bad field id %d", field);
-    if (device_ptr) *device_ptr = h->d[field];
+    if (ptr) *ptr = h->d[field];
     if (pitch) *pitch = is3d(field) ? h->pitch3 : is2d(field) ? h->pitch2 : h->kdim;
     return WRFB200_OK;
+}
+
+}  // namespace
+
+extern "C" int wrfb200_bind_device(wrfb200_handle *h, int field, float *device_ptr, long pitch)
+{
+    if (!h) return fail(WRFB200_ERR_INVALID_ARG, "null handle");
+    if (h->esize != 4) return wrong_precision(h, "wrfb200_bind_device");
+    return bind_device(h, field, device_ptr, pitch);
+}
+
+extern "C" int wrfb200_bind_device_r8(wrfb200_handle *h, int field, double *device_ptr, long pitch)
+{
+    if (!h) return fail(WRFB200_ERR_INVALID_ARG, "null handle");
+    if (h->esize != 8) return wrong_precision(h, "wrfb200_bind_device_r8");
+    return bind_device(h, field, device_ptr, pitch);
+}
+
+extern "C" int wrfb200_device_ptr(wrfb200_handle *h, int field, float **ptr, long *pitch)
+{
+    if (!h) return fail(WRFB200_ERR_INVALID_ARG, "null handle");
+    if (h->esize != 4) return wrong_precision(h, "wrfb200_device_ptr");
+    void *p = nullptr;
+    const int rc = device_ptr(h, field, &p, pitch);
+    if (ptr) *ptr = static_cast<float *>(p);
+    return rc;
+}
+
+extern "C" int wrfb200_device_ptr_r8(wrfb200_handle *h, int field, double **ptr, long *pitch)
+{
+    if (!h) return fail(WRFB200_ERR_INVALID_ARG, "null handle");
+    if (h->esize != 8) return wrong_precision(h, "wrfb200_device_ptr_r8");
+    void *p = nullptr;
+    const int rc = device_ptr(h, field, &p, pitch);
+    if (ptr) *ptr = static_cast<double *>(p);
+    return rc;
 }
 
 // -------------------------------------------------------------------------------------------------
 // exported: copies
 // -------------------------------------------------------------------------------------------------
+// Every copy verb checks the handle's precision against its own and then runs the one copy_range.
+namespace {
+
+int copy_verb(wrfb200_handle *h, int esize, const char *verb, int field, const void *src, void *dst,
+              int i0, int i1, int k0, int k1, int j0, int j1)
+{
+    GUARD(h);
+    if (h->esize != esize) return wrong_precision(h, verb);
+    if (!src && !dst) return fail(WRFB200_ERR_INVALID_ARG, "null host pointer");
+    return copy_range(h, field, src, dst, i0, i1, k0, k1, j0, j1);
+}
+
+int copy_verb_all(wrfb200_handle *h, int esize, const char *verb, int field, const void *src, void *dst)
+{
+    if (!h) return fail(WRFB200_ERR_INVALID_ARG, "null handle");
+    const wrfb200_domain &d = h->dom;
+    return copy_verb(h, esize, verb, field, src, dst, d.ims, d.ime, d.kms, d.kme, d.jms, d.jme);
+}
+
+}  // namespace
+
 extern "C" int wrfb200_upload_range(wrfb200_handle *h, int field, const float *host,
                                     int i0, int i1, int k0, int k1, int j0, int j1)
 {
-    GUARD(h);
-    if (!host) return fail(WRFB200_ERR_INVALID_ARG, "null host pointer");
-    return copy_range(h, field, host, nullptr, i0, i1, k0, k1, j0, j1);
+    return copy_verb(h, 4, "wrfb200_upload_range", field, host, nullptr, i0, i1, k0, k1, j0, j1);
 }
 
 extern "C" int wrfb200_download_range(wrfb200_handle *h, int field, float *host,
                                       int i0, int i1, int k0, int k1, int j0, int j1)
 {
-    GUARD(h);
-    if (!host) return fail(WRFB200_ERR_INVALID_ARG, "null host pointer");
-    return copy_range(h, field, nullptr, host, i0, i1, k0, k1, j0, j1);
+    return copy_verb(h, 4, "wrfb200_download_range", field, nullptr, host, i0, i1, k0, k1, j0, j1);
 }
 
 extern "C" int wrfb200_upload(wrfb200_handle *h, int field, const float *host)
 {
-    if (!h) return fail(WRFB200_ERR_INVALID_ARG, "null handle");
-    const wrfb200_domain &d = h->dom;
-    return wrfb200_upload_range(h, field, host, d.ims, d.ime, d.kms, d.kme, d.jms, d.jme);
+    return copy_verb_all(h, 4, "wrfb200_upload", field, host, nullptr);
 }
 
 extern "C" int wrfb200_download(wrfb200_handle *h, int field, float *host)
 {
-    if (!h) return fail(WRFB200_ERR_INVALID_ARG, "null handle");
-    const wrfb200_domain &d = h->dom;
-    return wrfb200_download_range(h, field, host, d.ims, d.ime, d.kms, d.kme, d.jms, d.jme);
+    return copy_verb_all(h, 4, "wrfb200_download", field, nullptr, host);
+}
+
+extern "C" int wrfb200_upload_range_r8(wrfb200_handle *h, int field, const double *host,
+                                       int i0, int i1, int k0, int k1, int j0, int j1)
+{
+    return copy_verb(h, 8, "wrfb200_upload_range_r8", field, host, nullptr, i0, i1, k0, k1, j0, j1);
+}
+
+extern "C" int wrfb200_download_range_r8(wrfb200_handle *h, int field, double *host,
+                                         int i0, int i1, int k0, int k1, int j0, int j1)
+{
+    return copy_verb(h, 8, "wrfb200_download_range_r8", field, nullptr, host, i0, i1, k0, k1, j0, j1);
+}
+
+extern "C" int wrfb200_upload_r8(wrfb200_handle *h, int field, const double *host)
+{
+    return copy_verb_all(h, 8, "wrfb200_upload_r8", field, host, nullptr);
+}
+
+extern "C" int wrfb200_download_r8(wrfb200_handle *h, int field, double *host)
+{
+    return copy_verb_all(h, 8, "wrfb200_download_r8", field, nullptr, host);
 }
 
 // Resident-state verbs (SURVEY.md section 8b): the groups of arrays a host-resident caller moves at the three
@@ -448,6 +626,8 @@ extern "C" int wrfb200_upload_constants(
     const float *msfuy, const float *msfvx_inv, const float *msftx, const float *msfty,
     const float *dnw, const float *fnm, const float *fnp, const float *rdnw)
 {
+    if (!h) return fail(WRFB200_ERR_INVALID_ARG, "null handle");
+    if (int rc = wrfb200_require_r4(h, "wrfb200_upload_constants")) return rc;
     const int ids[] = {WRFB200_WW_1, WRFB200_U_1, WRFB200_V_1, WRFB200_T_1, WRFB200_FT, WRFB200_MUT, WRFB200_MUU,
                        WRFB200_MUV, WRFB200_MU_TEND, WRFB200_MSFUY, WRFB200_MSFVX_INV, WRFB200_MSFTX, WRFB200_MSFTY,
                        WRFB200_DNW, WRFB200_FNM, WRFB200_FNP, WRFB200_RDNW};
@@ -459,6 +639,8 @@ extern "C" int wrfb200_upload_constants(
 
 extern "C" int wrfb200_upload_state(wrfb200_handle *h, const float *ww, const float *t, const float *mu)
 {
+    if (!h) return fail(WRFB200_ERR_INVALID_ARG, "null handle");
+    if (int rc = wrfb200_require_r4(h, "wrfb200_upload_state")) return rc;
     if (ww) if (int rc = wrfb200_upload(h, WRFB200_WW, ww)) return rc;
     if (t) if (int rc = wrfb200_upload(h, WRFB200_T, t)) return rc;
     if (mu) if (int rc = wrfb200_upload(h, WRFB200_MU, mu)) return rc;
@@ -467,6 +649,8 @@ extern "C" int wrfb200_upload_state(wrfb200_handle *h, const float *ww, const fl
 
 extern "C" int wrfb200_set_uv(wrfb200_handle *h, const float *u, const float *v)
 {
+    if (!h) return fail(WRFB200_ERR_INVALID_ARG, "null handle");
+    if (int rc = wrfb200_require_r4(h, "wrfb200_set_uv")) return rc;
     if (u) if (int rc = wrfb200_upload(h, WRFB200_U, u)) return rc;
     if (v) if (int rc = wrfb200_upload(h, WRFB200_V, v)) return rc;
     return WRFB200_OK;
@@ -478,6 +662,7 @@ extern "C" int wrfb200_download_outputs(wrfb200_handle *h, int its, int ite, int
                                         float *ww, float *t, float *t_ave, float *mu, float *muave, float *muts, float *mudf)
 {
     if (!h) return fail(WRFB200_ERR_INVALID_ARG, "null handle");
+    if (int rc = wrfb200_require_r4(h, "wrfb200_download_outputs")) return rc;
     const wrfb200_domain &d = h->dom;
     int is, ie, js, je, ks, ke;
     wrfb200_bounds(d.periodic_x, d.specified, d.nested, d.ids, d.ide, d.jds, d.jde,
@@ -496,11 +681,7 @@ extern "C" int wrfb200_download_outputs(wrfb200_handle *h, int its, int ite, int
 extern "C" int wrfb200_step(wrfb200_handle *h, int its, int ite, int jts, int jte, int kts, int kte)
 {
     GUARD(h);
-    AmtParams p;
-    bool empty = false;
-    if (int rc = make_params(h, its, ite, jts, jte, kts, kte, &p, &empty)) return rc;
-    if (empty) return WRFB200_OK;
-    return launch(h, p, h->stream, h->kernel);
+    return step_on(h, its, ite, jts, jte, kts, kte, h->stream, h->kernel);
 }
 
 extern "C" int wrfb200_step_graph(wrfb200_handle *h, int its, int ite, int jts, int jte, int kts, int kte, int nsteps)
@@ -508,8 +689,11 @@ extern "C" int wrfb200_step_graph(wrfb200_handle *h, int its, int ite, int jts, 
     GUARD(h);
     if (nsteps <= 0) return WRFB200_OK;
     AmtParams p;
+    AmtParamsR8 p8;
     bool empty = false;
-    if (int rc = make_params(h, its, ite, jts, jte, kts, kte, &p, &empty)) return rc;
+    const int rc0 = h->esize == 8 ? make_params(h, its, ite, jts, jte, kts, kte, &p8, &empty)
+                                  : make_params(h, its, ite, jts, jte, kts, kte, &p, &empty);
+    if (rc0) return rc0;
     if (empty) return WRFB200_OK;
     const auto key = std::make_tuple(its, ite, jts, jte, kte, nsteps, h->kernel);
     auto it = h->graphs.find(key);
@@ -521,7 +705,8 @@ extern "C" int wrfb200_step_graph(wrfb200_handle *h, int its, int ite, int jts, 
         cudaError_t e = cudaStreamBeginCapture(cs, cudaStreamCaptureModeThreadLocal);
         int rc = WRFB200_OK;
         if (e == cudaSuccess) {
-            for (int s = 0; s < nsteps && rc == WRFB200_OK; ++s) rc = launch(h, p, cs, h->kernel);
+            for (int s = 0; s < nsteps && rc == WRFB200_OK; ++s)
+                rc = h->esize == 8 ? launch(h, p8, cs, h->kernel) : launch(h, p, cs, h->kernel);
             h->launches -= nsteps;                      // counted again on every replay below
             e = cudaStreamEndCapture(cs, &graph);
         }
@@ -564,8 +749,8 @@ thread_local int g_default_kernel = WRFB200_KERNEL_AUTO;
 constexpr int kMaxSlabs = 16;
 
 struct Args {
-    float *f[WRFB200_NUM_FIELDS];
-    float rdx, rdy, dts, epssm;
+    void *f[WRFB200_NUM_FIELDS];       // float or double arrays (the entry point's precision)
+    double rdx, rdy, dts, epssm;
     wrfb200_domain dom;
     int its, ite, jts, jte, kts, kte;
 };
@@ -576,8 +761,8 @@ struct CompatCache {
     wrfb200_handle *h = nullptr;
     cudaStream_t up = nullptr, comp = nullptr, down = nullptr;      // upload / compute / download lanes
     cudaEvent_t ev_up[kMaxSlabs] = {}, ev_comp[kMaxSlabs] = {};
-    float *stage[2] = {nullptr, nullptr};                           // dense landing buffers for H2D slabs
-    size_t stage_floats = 0;
+    void *stage[2] = {nullptr, nullptr};                            // dense landing buffers for H2D slabs
+    size_t stage_bytes = 0;
     // acoustic-loop residency (wrfb200_acoustic_loop_begin/end): after the first call of a loop the device
     // mirrors hold everything; later calls with the SAME arrays and index sets move only u, v up
     bool loop_active = false, primed = false;
@@ -590,8 +775,8 @@ struct CompatCache {
             h->stream = nullptr;               // never synchronise on one of the lanes destroyed below
             wrfb200_destroy(h);                // device-wide sync, frees the mirrors
             h = nullptr;
-            for (float *&b : stage) if (b) { cudaFree(b); b = nullptr; }
-            stage_floats = 0;
+            for (void *&b : stage) if (b) { cudaFree(b); b = nullptr; }
+            stage_bytes = 0;
             for (cudaEvent_t &e : ev_up) if (e) { cudaEventDestroy(e); e = nullptr; }
             for (cudaEvent_t &e : ev_comp) if (e) { cudaEventDestroy(e); e = nullptr; }
             for (cudaStream_t *st : {&up, &comp, &down}) if (*st) { cudaStreamDestroy(*st); *st = nullptr; }
@@ -600,18 +785,19 @@ struct CompatCache {
     }
     ~CompatCache() { release(); }
 };
-thread_local CompatCache g_cache;
+thread_local CompatCache g_cache[2];        // [0]: binary32 calls, [1]: real*8 calls
 
 // Device-pointer callers: the handle that wraps the caller's arrays (and its six TMA tensor maps) is kept
 // between calls and re-used while the pointers and extents stay the same -- a 25-830 us step must not pay
 // six cuTensorMapEncodeTiled and 26 cudaPointerGetAttributes every time.
 struct DeviceCallCache {
     wrfb200_handle h;
-    float *ptrs[WRFB200_NUM_FIELDS] = {};
+    void *ptrs[WRFB200_NUM_FIELDS] = {};
     wrfb200_domain dom{};
     bool valid = false;
 };
-thread_local DeviceCallCache g_devcall;
+thread_local DeviceCallCache g_devcall[2];   // indexed like g_cache
+thread_local int g_last_prec = 0;              // which of the two the most recent call used
 
 bool same_shape(const wrfb200_domain &a, const wrfb200_domain &b)
 {
@@ -671,14 +857,14 @@ void unpin_all()
 size_t field_bytes(const wrfb200_handle *h, int f)
 {
     const size_t n = is3d(f) ? (size_t)h->idim * h->kdim * h->jdim : is2d(f) ? (size_t)h->idim * h->jdim : (size_t)h->kdim;
-    return n * sizeof(float);
+    return n * h->esize;
 }
 
-int run_device_in_place(const Args &a)
+int run_device_in_place(const Args &a, int prec)
 {
     // Caller-owned device arrays in the dense Fortran layout, wrapped in a (cached) handle.
     if (int rc = check_domain(a.dom)) return rc;
-    DeviceCallCache &c = g_devcall;
+    DeviceCallCache &c = g_devcall[prec];
     int dev = 0;
     CU(cudaGetDevice(&dev));
     const bool hit = c.valid && c.h.device == dev && same_domain(c.dom, a.dom) &&
@@ -691,18 +877,15 @@ int run_device_in_place(const Args &a)
         c.h.jdim = a.dom.jme - a.dom.jms + 1;
         c.h.kdim = a.dom.kme - a.dom.kms + 1;
         c.h.pitch3 = c.h.pitch2 = c.h.idim;
-        for (int f = 0; f < WRFB200_NUM_FIELDS; ++f) c.h.d[f] = a.f[f];
+        c.h.esize = prec ? 8 : 4;
+        for (int f = 0; f < WRFB200_NUM_FIELDS; ++f) c.h.d[f] = static_cast<float *>(a.f[f]);
         c.h.maps.valid = 0;
         std::memcpy(c.ptrs, a.f, sizeof(c.ptrs));
         c.dom = a.dom;
         c.valid = true;
     }
     c.h.rdx = a.rdx; c.h.rdy = a.rdy; c.h.dts = a.dts; c.h.epssm = a.epssm; c.h.scalars_set = true;
-    AmtParams p;
-    bool empty = false;
-    if (int rc = make_params(&c.h, a.its, a.ite, a.jts, a.jte, a.kts, a.kte, &p, &empty)) return rc;
-    if (empty) return WRFB200_OK;
-    return launch(&c.h, p, g_default_stream, g_default_kernel);
+    return step_on(&c.h, a.its, a.ite, a.jts, a.jte, a.kts, a.kte, g_default_stream, g_default_kernel);
 }
 
 // Host-pointer form of the operator.  The reference does alloc -> 26 blocking H2D copies -> launch ->
@@ -717,7 +900,7 @@ int run_device_in_place(const Args &a)
 // arrays upload only u and v (what advance_uv changed; everything else on the device is this routine's own
 // previous output or a loop constant) -- the per-small-step drop-in pattern of a host-resident model:
 // 0.76 GB up and 1.15 GB down per step on 1800x1060x50 instead of 3.2 GB up.
-int run_host_compat_body(const Args &a, int nsteps, wrfb200_handle *h)
+int run_host_compat_body(const Args &a, int nsteps, wrfb200_handle *h, CompatCache &cc)
 {
     const wrfb200_domain &d = a.dom;
     int is, ie, js, je, ks, ke;
@@ -740,7 +923,6 @@ int run_host_compat_body(const Args &a, int nsteps, wrfb200_handle *h)
     static const int out2[] = {WRFB200_MU, WRFB200_MUAVE, WRFB200_MUTS, WRFB200_MUDF};
 
     // resident step: same arrays, same index sets, same scalars as the call that primed the mirrors
-    CompatCache &cc = g_cache;
     const bool resident = cc.loop_active && cc.primed && std::memcmp(cc.primed_args.f, a.f, sizeof(a.f)) == 0 &&
                           same_domain(cc.primed_args.dom, a.dom) && cc.primed_args.its == a.its &&
                           cc.primed_args.ite == a.ite && cc.primed_args.jts == a.jts && cc.primed_args.jte == a.jte &&
@@ -758,13 +940,14 @@ int run_host_compat_body(const Args &a, int nsteps, wrfb200_handle *h)
     // reads, module_small_step_em.f90:159-161)
     h->stream = cc.up;
     if (!resident) {
-        for (int f : in2) if (int rc = wrfb200_upload(h, f, a.f[f])) return rc;
-        for (int f : in1) if (int rc = wrfb200_upload(h, f, a.f[f])) return rc;
-        if (int rc = wrfb200_upload_range(h, WRFB200_WW, a.f[WRFB200_WW], d.ims, d.ime, a.kts, a.kts, d.jms, d.jme)) return rc;
+        for (int f : in2) if (int rc = copy_field(h, f, a.f[f], nullptr)) return rc;
+        for (int f : in1) if (int rc = copy_field(h, f, a.f[f], nullptr)) return rc;
+        if (int rc = copy_range(h, WRFB200_WW, a.f[WRFB200_WW], nullptr, d.ims, d.ime, a.kts, a.kts, d.jms, d.jme)) return rc;
     }
 
     const int nj = je - js + 1;
-    const size_t bytes3 = (size_t)h->idim * h->kdim * h->jdim * sizeof(float);
+    const size_t es = (size_t)h->esize;
+    const size_t bytes3 = (size_t)h->idim * h->kdim * h->jdim * es;
     int nslab = 1;
     if (bytes3 >= ((size_t)16 << 20) && nj >= 32) nslab = nj / 16 < kMaxSlabs ? nj / 16 : kMaxSlabs;
     if (nslab > kMaxSlabs) nslab = kMaxSlabs;             // one event pair per slab
@@ -773,13 +956,14 @@ int run_host_compat_body(const Args &a, int nsteps, wrfb200_handle *h)
     // measured, tools/pcie_probe.py).  When the mirror is padded, land each slab densely in a staging buffer
     // with ONE contiguous copy and re-pitch it on the device (HBM speed, negligible).
     const bool staged = (h->pitch3 != h->idim) && nslab > 1;
-    const size_t slab_floats = (size_t)(nj / nslab + 3) * h->kdim * h->idim;
-    if (staged && cc.stage_floats < slab_floats) {
-        for (float *&b : cc.stage) { if (b) cudaFree(b); b = nullptr; }
-        cc.stage_floats = 0;
-        for (float *&b : cc.stage) CU(cudaMalloc(&b, slab_floats * sizeof(float)));
-        cc.stage_floats = slab_floats;
+    const size_t slab_bytes = (size_t)(nj / nslab + 3) * h->kdim * h->idim * es;
+    if (staged && cc.stage_bytes < slab_bytes) {
+        for (void *&b : cc.stage) { if (b) cudaFree(b); b = nullptr; }
+        cc.stage_bytes = 0;
+        for (void *&b : cc.stage) CU(cudaMalloc(&b, slab_bytes));
+        cc.stage_bytes = slab_bytes;
     }
+    const int fpe = h->esize / (int)sizeof(float);         // the re-pitch kernel moves 4-byte words
     int flip = 0;
     for (int s = 0; s < nslab; ++s) {
         const int ja = js + (int)((long long)nj * s / nslab);
@@ -794,14 +978,14 @@ int run_host_compat_body(const Args &a, int nsteps, wrfb200_handle *h)
             for (int x = 0; x < n_in3; ++x) {
                 const int f = in3[x];
                 if (!staged) {
-                    if (int rc = wrfb200_upload_range(h, f, a.f[f], d.ims, d.ime, d.kms, d.kme, next_row, hi)) return rc;
+                    if (int rc = copy_range(h, f, a.f[f], nullptr, d.ims, d.ime, d.kms, d.kme, next_row, hi)) return rc;
                     continue;
                 }
-                float *st = cc.stage[flip];
+                float *st = static_cast<float *>(cc.stage[flip]);
                 flip ^= 1;
-                CU(cudaMemcpyAsync(st, a.f[f] + hoff, (size_t)nrows * h->idim * sizeof(float),
+                CU(cudaMemcpyAsync(st, static_cast<const char *>(a.f[f]) + hoff * es, (size_t)nrows * h->idim * es,
                                    cudaMemcpyHostToDevice, cc.up));
-                CU(wrfb200_repitch_rows(h->d[f] + doff, st, h->pitch3, h->idim, nrows, cc.up));
+                CU(wrfb200_repitch_rows(h->d[f] + doff * fpe, st, h->pitch3 * fpe, h->idim * fpe, nrows, cc.up));
                 h->launches += 1;
             }
             next_row = hi + 1;
@@ -816,8 +1000,8 @@ int run_host_compat_body(const Args &a, int nsteps, wrfb200_handle *h)
         // outputs: exactly the cells the Fortran writes
         CU(cudaStreamWaitEvent(cc.down, cc.ev_comp[s], 0));
         h->stream = cc.down;
-        for (int f : out3) if (int rc = wrfb200_download_range(h, f, a.f[f], is, ie, ks, ke, ja, jb)) return rc;
-        for (int f : out2) if (int rc = wrfb200_download_range(h, f, a.f[f], is, ie, 0, 0, ja, jb)) return rc;
+        for (int f : out3) if (int rc = copy_range(h, f, nullptr, a.f[f], is, ie, ks, ke, ja, jb)) return rc;
+        for (int f : out2) if (int rc = copy_range(h, f, nullptr, a.f[f], is, ie, 0, 0, ja, jb)) return rc;
     }
     CU(cudaStreamSynchronize(cc.up));
     CU(cudaStreamSynchronize(cc.comp));
@@ -826,44 +1010,48 @@ int run_host_compat_body(const Args &a, int nsteps, wrfb200_handle *h)
     return WRFB200_OK;
 }
 
-int run_host_compat(const Args &a, int nsteps)
+int run_host_compat(const Args &a, int nsteps, int prec)
 {
     if (int rc = check_domain(a.dom)) return rc;
-    if (g_cache.h && !same_shape(g_cache.h->dom, a.dom)) g_cache.release();
-    if (!g_cache.h) {
-        if (int rc = wrfb200_create(&g_cache.h, &a.dom, -1, 1)) return rc;
-        DeviceGuard g(g_cache.h->device);
-        for (cudaStream_t *st : {&g_cache.up, &g_cache.comp, &g_cache.down})
+    CompatCache &cc = g_cache[prec];
+    if (cc.h && !same_shape(cc.h->dom, a.dom)) cc.release();
+    if (!cc.h) {
+        if (int rc = create(&cc.h, &a.dom, -1, 1, prec ? 8 : 4)) return rc;
+        DeviceGuard g(cc.h->device);
+        for (cudaStream_t *st : {&cc.up, &cc.comp, &cc.down})
             CU(cudaStreamCreateWithFlags(st, cudaStreamNonBlocking));
         for (int i = 0; i < kMaxSlabs; ++i) {
-            CU(cudaEventCreateWithFlags(&g_cache.ev_up[i], cudaEventDisableTiming));
-            CU(cudaEventCreateWithFlags(&g_cache.ev_comp[i], cudaEventDisableTiming));
+            CU(cudaEventCreateWithFlags(&cc.ev_up[i], cudaEventDisableTiming));
+            CU(cudaEventCreateWithFlags(&cc.ev_comp[i], cudaEventDisableTiming));
         }
     }
-    wrfb200_handle *h = g_cache.h;
+    wrfb200_handle *h = cc.h;
     GUARD(h);
     h->dom = a.dom;                       // same extents; domain dims / flags may differ between calls
     h->kernel = g_default_kernel;
-    wrfb200_set_scalars(h, a.rdx, a.rdy, a.dts, a.epssm);
-    const int rc = run_host_compat_body(a, nsteps, h);
+    set_scalars(h, a.rdx, a.rdy, a.dts, a.epssm);
+    const int rc = run_host_compat_body(a, nsteps, h, cc);
     if (rc != WRFB200_OK) {
         // an early return must not leave copies on the caller's arrays in flight, nor the cached handle
         // pointing at one of the internal lanes
         const std::string msg = wrfb200_last_error();
-        for (cudaStream_t st : {g_cache.up, g_cache.comp, g_cache.down}) if (st) cudaStreamSynchronize(st);
+        for (cudaStream_t st : {cc.up, cc.comp, cc.down}) if (st) cudaStreamSynchronize(st);
         (void)cudaGetLastError();
-        g_cache.primed = false;
+        cc.primed = false;
         wrfb200_fail(rc, "%s", msg.c_str());
     }
     h->stream = g_default_stream;
     return rc;
 }
 
-int dispatch(Args &a, int nsteps, bool allow_device)
+// prec: 0 = binary32 entry points, 1 = real*8 entry points
+int dispatch(Args &a, int nsteps, bool allow_device, int prec)
 {
+    g_last_prec = prec;
+    DeviceCallCache &dc = g_devcall[prec];
     // device-pointer fast path: the very same arrays as the previous call need no re-classification
-    if (allow_device && nsteps == 1 && g_devcall.valid && std::memcmp(g_devcall.ptrs, a.f, sizeof(a.f)) == 0)
-        return run_device_in_place(a);
+    if (allow_device && nsteps == 1 && dc.valid && std::memcmp(dc.ptrs, a.f, sizeof(a.f)) == 0)
+        return run_device_in_place(a, prec);
     PtrKind kind = classify(a.f[0]);
     for (int f = 0; f < WRFB200_NUM_FIELDS; ++f) {
         PtrKind k = classify(a.f[f]);
@@ -878,31 +1066,31 @@ int dispatch(Args &a, int nsteps, bool allow_device)
     if (kind == PTR_DEVICE) {
         if (!allow_device || nsteps != 1)
             return fail(WRFB200_ERR_INVALID_ARG, "this entry point takes host pointers; device-resident callers use wrfb200_step");
-        return run_device_in_place(a);
+        return run_device_in_place(a, prec);
     }
-    g_devcall.valid = false;
-    return run_host_compat(a, nsteps);
+    dc.valid = false;
+    return run_host_compat(a, nsteps, prec);
 }
 
 }  // namespace
 
 #define WRFB200_PACK_ARGS(a)                                                                              \
     Args a{};                                                                                             \
-    a.f[WRFB200_WW] = ww;            a.f[WRFB200_WW_1] = const_cast<float *>(ww_1);                       \
-    a.f[WRFB200_U] = const_cast<float *>(u);       a.f[WRFB200_U_1] = const_cast<float *>(u_1);           \
-    a.f[WRFB200_V] = const_cast<float *>(v);       a.f[WRFB200_V_1] = const_cast<float *>(v_1);           \
-    a.f[WRFB200_T] = t;              a.f[WRFB200_T_1] = const_cast<float *>(t_1);                         \
-    a.f[WRFB200_T_AVE] = t_ave;      a.f[WRFB200_FT] = const_cast<float *>(ft);                           \
-    a.f[WRFB200_MU] = mu;            a.f[WRFB200_MUT] = const_cast<float *>(mut);                         \
-    a.f[WRFB200_MUAVE] = muave;      a.f[WRFB200_MUTS] = muts;                                            \
-    a.f[WRFB200_MUU] = const_cast<float *>(muu);   a.f[WRFB200_MUV] = const_cast<float *>(muv);           \
-    a.f[WRFB200_MUDF] = mudf;        a.f[WRFB200_MU_TEND] = const_cast<float *>(mu_tend);                 \
-    a.f[WRFB200_MSFUY] = const_cast<float *>(msfuy);                                                      \
-    a.f[WRFB200_MSFVX_INV] = const_cast<float *>(msfvx_inv);                                              \
-    a.f[WRFB200_MSFTX] = const_cast<float *>(msftx);                                                      \
-    a.f[WRFB200_MSFTY] = const_cast<float *>(msfty);                                                      \
-    a.f[WRFB200_DNW] = const_cast<float *>(dnw);   a.f[WRFB200_FNM] = const_cast<float *>(fnm);           \
-    a.f[WRFB200_FNP] = const_cast<float *>(fnp);   a.f[WRFB200_RDNW] = const_cast<float *>(rdnw);         \
+    a.f[WRFB200_WW] = (void *)ww;            a.f[WRFB200_WW_1] = (void *)ww_1;                            \
+    a.f[WRFB200_U] = (void *)u;       a.f[WRFB200_U_1] = (void *)u_1;                                     \
+    a.f[WRFB200_V] = (void *)v;       a.f[WRFB200_V_1] = (void *)v_1;                                     \
+    a.f[WRFB200_T] = (void *)t;              a.f[WRFB200_T_1] = (void *)t_1;                              \
+    a.f[WRFB200_T_AVE] = (void *)t_ave;      a.f[WRFB200_FT] = (void *)ft;                                \
+    a.f[WRFB200_MU] = (void *)mu;            a.f[WRFB200_MUT] = (void *)mut;                              \
+    a.f[WRFB200_MUAVE] = (void *)muave;      a.f[WRFB200_MUTS] = (void *)muts;                            \
+    a.f[WRFB200_MUU] = (void *)muu;   a.f[WRFB200_MUV] = (void *)muv;                                     \
+    a.f[WRFB200_MUDF] = (void *)mudf;        a.f[WRFB200_MU_TEND] = (void *)mu_tend;                      \
+    a.f[WRFB200_MSFUY] = (void *)msfuy;                                                                   \
+    a.f[WRFB200_MSFVX_INV] = (void *)msfvx_inv;                                                           \
+    a.f[WRFB200_MSFTX] = (void *)msftx;                                                                   \
+    a.f[WRFB200_MSFTY] = (void *)msfty;                                                                   \
+    a.f[WRFB200_DNW] = (void *)dnw;   a.f[WRFB200_FNM] = (void *)fnm;                                     \
+    a.f[WRFB200_FNP] = (void *)fnp;   a.f[WRFB200_RDNW] = (void *)rdnw;                                   \
     a.rdx = rdx; a.rdy = rdy; a.dts = dts; a.epssm = epssm;                                               \
     a.dom.ids = ids; a.dom.ide = ide; a.dom.jds = jds; a.dom.jde = jde; a.dom.kde = kde;                  \
     a.dom.ims = ims; a.dom.ime = ime; a.dom.jms = jms; a.dom.jme = jme; a.dom.kms = kms; a.dom.kme = kme; \
@@ -922,7 +1110,7 @@ extern "C" int wrfb200_advance_mu_t(
     int its, int ite, int jts, int jte, int kts, int kte)
 {
     WRFB200_PACK_ARGS(a);
-    return dispatch(a, 1, true);
+    return dispatch(a, 1, true, 0);
 }
 
 extern "C" int wrfb200_advance_mu_t_loop(
@@ -940,7 +1128,43 @@ extern "C" int wrfb200_advance_mu_t_loop(
 {
     if (nsteps < 1) return fail(WRFB200_ERR_INVALID_ARG, "nsteps=%d", nsteps);
     WRFB200_PACK_ARGS(a);
-    return dispatch(a, nsteps, false);
+    return dispatch(a, nsteps, false, 0);
+}
+
+// The same two entry points for WRF built with -r8 (default REAL = 8 bytes): double arrays and scalars,
+// evaluated in binary64 by the real*8 kernels.
+extern "C" int wrfb200_advance_mu_t_r8(
+    double *ww, const double *ww_1, const double *u, const double *u_1, const double *v, const double *v_1,
+    double *mu, const double *mut, double *muave, double *muts, const double *muu, const double *muv,
+    double *mudf, double *t, const double *t_1, double *t_ave, const double *ft, const double *mu_tend,
+    double rdx, double rdy, double dts, double epssm,
+    const double *dnw, const double *fnm, const double *fnp, const double *rdnw,
+    const double *msfuy, const double *msfvx_inv, const double *msftx, const double *msfty,
+    int periodic_x, int specified, int nested,
+    int ids, int ide, int jds, int jde, int kde,
+    int ims, int ime, int jms, int jme, int kms, int kme,
+    int its, int ite, int jts, int jte, int kts, int kte)
+{
+    WRFB200_PACK_ARGS(a);
+    return dispatch(a, 1, true, 1);
+}
+
+extern "C" int wrfb200_advance_mu_t_loop_r8(
+    double *ww, const double *ww_1, const double *u, const double *u_1, const double *v, const double *v_1,
+    double *mu, const double *mut, double *muave, double *muts, const double *muu, const double *muv,
+    double *mudf, double *t, const double *t_1, double *t_ave, const double *ft, const double *mu_tend,
+    double rdx, double rdy, double dts, double epssm,
+    const double *dnw, const double *fnm, const double *fnp, const double *rdnw,
+    const double *msfuy, const double *msfvx_inv, const double *msftx, const double *msfty,
+    int periodic_x, int specified, int nested,
+    int ids, int ide, int jds, int jde, int kde,
+    int ims, int ime, int jms, int jme, int kms, int kme,
+    int its, int ite, int jts, int jte, int kts, int kte,
+    int nsteps)
+{
+    if (nsteps < 1) return fail(WRFB200_ERR_INVALID_ARG, "nsteps=%d", nsteps);
+    WRFB200_PACK_ARGS(a);
+    return dispatch(a, nsteps, false, 1);
 }
 
 extern "C" int wrfb200_set_default_stream(void *cuda_stream)
@@ -959,23 +1183,21 @@ extern "C" int wrfb200_set_default_kernel(int kernel)
 
 extern "C" int wrfb200_release_cache(void)
 {
-    g_cache.release();
-    g_devcall.valid = false;
+    for (CompatCache &c : g_cache) c.release();
+    for (DeviceCallCache &c : g_devcall) c.valid = false;
     unpin_all();
     return WRFB200_OK;
 }
 
 extern "C" int wrfb200_acoustic_loop_begin(void)
 {
-    g_cache.loop_active = true;
-    g_cache.primed = false;
+    for (CompatCache &c : g_cache) { c.loop_active = true; c.primed = false; }
     return WRFB200_OK;
 }
 
 extern "C" int wrfb200_acoustic_loop_end(void)
 {
-    g_cache.loop_active = false;
-    g_cache.primed = false;
+    for (CompatCache &c : g_cache) { c.loop_active = false; c.primed = false; }
     return WRFB200_OK;
 }
 
@@ -1041,6 +1263,8 @@ extern "C" int wrfb200_last_kernel(wrfb200_handle *h, int *kernel)
 extern "C" int wrfb200_default_last_kernel(int *kernel)
 {
     if (!kernel) return fail(WRFB200_ERR_INVALID_ARG, "null argument");
-    *kernel = g_devcall.valid ? g_devcall.h.last_kernel : (g_cache.h ? g_cache.h->last_kernel : 0);
+    const DeviceCallCache &dc = g_devcall[g_last_prec];
+    const CompatCache &cc = g_cache[g_last_prec];
+    *kernel = dc.valid ? dc.h.last_kernel : (cc.h ? cc.h->last_kernel : 0);
     return WRFB200_OK;
 }

@@ -14,11 +14,12 @@ struct wrfb200_handle {
     wrfb200_domain dom{};
     int device = 0;
     cudaStream_t stream = nullptr;
-    float *d[WRFB200_NUM_FIELDS] = {};
+    int esize = 4;                     // bytes per element: 4 (wrfb200_create) or 8 (wrfb200_create_r8)
+    float *d[WRFB200_NUM_FIELDS] = {};   // device fields; they hold doubles when esize == 8
     bool owned[WRFB200_NUM_FIELDS] = {};
-    long pitch3 = 0, pitch2 = 0;       // row strides in floats (0 = not yet known)
+    long pitch3 = 0, pitch2 = 0;       // row strides in elements (0 = not yet known)
     int idim = 0, jdim = 0, kdim = 0;
-    float rdx = 0, rdy = 0, dts = 0, epssm = 0;
+    double rdx = 0, rdy = 0, dts = 0, epssm = 0;   // exact for either precision
     bool scalars_set = false;
     int kernel = WRFB200_KERNEL_AUTO;
     long launches = 0;
@@ -44,3 +45,5 @@ cudaError_t wrfb200_halo_preload();
 
 // thread-local error message; returns `code`
 int wrfb200_fail(int code, const char *fmt, ...);
+// WRFB200_OK for a binary32 handle; WRFB200_ERR_UNSUPPORTED naming `what` for a real*8 one
+int wrfb200_require_r4(const wrfb200_handle *h, const char *what);

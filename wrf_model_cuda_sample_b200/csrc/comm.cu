@@ -267,6 +267,7 @@ __global__ void barrier_kernel(const __grid_constant__ BarrierArgs a)
 int need_comm(wrfb200_handle *h, bool connected)
 {
     if (!h) return wrfb200_fail(WRFB200_ERR_INVALID_ARG, "null handle");
+    if (int rc = wrfb200_require_r4(h, "multi-GPU halo exchange (wrfb200_comm_*)")) return rc;
     if (!h->comm) return wrfb200_fail(WRFB200_ERR_STATE, "wrfb200_comm_init has not been called on this handle");
     if (connected && !h->comm->connected) return wrfb200_fail(WRFB200_ERR_STATE, "wrfb200_comm_connect has not been called");
     return WRFB200_OK;
@@ -503,6 +504,7 @@ extern "C" int wrfb200_comm_init(wrfb200_handle *h, int px, int py, int rank,
                                  int ips, int ipe, int jps, int jpe, void *info_out)
 {
     if (!h || !info_out) return wrfb200_fail(WRFB200_ERR_INVALID_ARG, "null argument");
+    if (int rc = wrfb200_require_r4(h, "multi-GPU halo exchange (wrfb200_comm_*)")) return rc;
     if (px < 1 || py < 1 || rank < 0 || rank >= px * py)
         return wrfb200_fail(WRFB200_ERR_INVALID_ARG, "bad process grid %dx%d / rank %d", px, py, rank);
     const wrfb200_domain &d = h->dom;

@@ -77,6 +77,7 @@ int halo_copy(wrfb200_handle *h, int field, int side, int width, int ips, int ip
               float *buf, bool pack)
 {
     if (!h || !buf) return wrfb200_fail(WRFB200_ERR_INVALID_ARG, "null argument");
+    if (int rc = wrfb200_require_r4(h, pack ? "wrfb200_pack_halo" : "wrfb200_unpack_halo")) return rc;
     const bool f3 = field >= WRFB200_WW && field <= WRFB200_FT;
     const bool f2 = field >= WRFB200_MU && field <= WRFB200_MSFTY;
     if (!f3 && !f2) return wrfb200_fail(WRFB200_ERR_INVALID_ARG, "field %d has no horizontal halo", field);
@@ -147,6 +148,7 @@ extern "C" int wrfb200_unpack_halo(wrfb200_handle *h, int field, int side, int w
 extern "C" int wrfb200_standin_advance_uv(wrfb200_handle *h, int field, float c, int i0, int i1, int j0, int j1)
 {
     if (!h) return wrfb200_fail(WRFB200_ERR_INVALID_ARG, "null handle");
+    if (int rc = wrfb200_require_r4(h, "wrfb200_standin_advance_uv")) return rc;
     if (field != WRFB200_U && field != WRFB200_V)
         return wrfb200_fail(WRFB200_ERR_INVALID_ARG, "stand-in update applies to u or v only");
     if (i0 > i1 || j0 > j1) return WRFB200_OK;

@@ -7,13 +7,15 @@
 !     CALL advance_mu_t( grid_ww, ww1, grid_u_2, ... , its, ite, jts, jte, kts, kte )
 ! (advance_mu_t_driver.f90:193-205), or WRF's solve_em -- compiles and links unchanged.  The body does no
 ! arithmetic: it pulls the three logicals the routine reads out of config_flags
-! (module_small_step_em.f90:97-106; module_configure.f90:434,436,447) and calls the C ABI entry
-! wrfb200_advance_mu_t of libwrfb200.so (include/wrfb200.h), which runs the CUDA path.
+! (module_small_step_em.f90:97-106; module_configure.f90:434,436,447) and calls the C ABI of
+! libwrfb200.so (include/wrfb200.h), which runs the CUDA path.
 !
-! The dummies are explicit-shape arrays, so they are contiguous and can be passed by reference as
-! real(c_float); default REAL must be 4 bytes (the reference is real*4; do not build with -r8 /
-! -fdefault-real-8).  grid_config_rec_type is not BIND(C)-interoperable (1 796 components, 110 of them
-! character*256): it never crosses the boundary.
+! The dummies are explicit-shape arrays, so they are contiguous and are passed by reference.  The C entry
+! is reached through the generic interface wrfb200_amt, whose two specific bodies take REAL(c_float)
+! (wrfb200_advance_mu_t) and REAL(c_double) (wrfb200_advance_mu_t_r8): the compiler picks the one that
+! matches default REAL, so the same source builds for WRF's default real*4 and for `configure -r8`
+! (-fdefault-real-8 / -r8), which then runs in binary64.  grid_config_rec_type is not BIND(C)-interoperable
+! (1 796 components, 110 of them character*256): it never crosses the boundary.
 !
 ! Build (any Fortran 2003 compiler; none is available in the build container, see INTEGRATION.md):
 !     gfortran -c module_configure.f90 module_small_step_em.F90
@@ -23,13 +25,14 @@
 MODULE module_small_step_em
 
 USE module_configure, ONLY : grid_config_rec_type
-USE, INTRINSIC :: iso_c_binding, ONLY : c_float, c_int, c_char, c_ptr, c_null_char, c_f_pointer, c_size_t
+USE, INTRINSIC :: iso_c_binding, ONLY : c_float, c_double, c_int, c_char, c_ptr, c_null_char, c_f_pointer, &
+                                        c_size_t
 
 IMPLICIT NONE
 PRIVATE
 PUBLIC :: advance_mu_t
 
-INTERFACE
+INTERFACE wrfb200_amt
    ! int wrfb200_advance_mu_t(float *ww, const float *ww_1, ..., int kts, int kte);   include/wrfb200.h
    FUNCTION wrfb200_advance_mu_t( ww, ww_1, u, u_1, v, v_1, mu, mut, muave, muts, muu, muv,        &
                                   mudf, t, t_1, t_ave, ft, mu_tend,                               &
@@ -50,6 +53,28 @@ INTERFACE
       INTEGER(c_int) :: status
    END FUNCTION wrfb200_advance_mu_t
 
+   ! int wrfb200_advance_mu_t_r8(double *ww, const double *ww_1, ..., int kts, int kte);   include/wrfb200.h
+   FUNCTION wrfb200_advance_mu_t_r8( ww, ww_1, u, u_1, v, v_1, mu, mut, muave, muts, muu, muv,     &
+                                     mudf, t, t_1, t_ave, ft, mu_tend,                            &
+                                     rdx, rdy, dts, epssm, dnw, fnm, fnp, rdnw,                   &
+                                     msfuy, msfvx_inv, msftx, msfty,                              &
+                                     periodic_x, specified, nested,                               &
+                                     ids, ide, jds, jde, kde, ims, ime, jms, jme, kms, kme,       &
+                                     its, ite, jts, jte, kts, kte )                               &
+            BIND(C, NAME="wrfb200_advance_mu_t_r8") RESULT(status)
+      IMPORT :: c_double, c_int
+      REAL(c_double), DIMENSION(*), INTENT(INOUT) :: ww, mu, muave, muts, mudf, t, t_ave
+      REAL(c_double), DIMENSION(*), INTENT(IN)    :: ww_1, u, u_1, v, v_1, mut, muu, muv, t_1, ft, mu_tend
+      REAL(c_double), DIMENSION(*), INTENT(IN)    :: dnw, fnm, fnp, rdnw, msfuy, msfvx_inv, msftx, msfty
+      REAL(c_double), VALUE :: rdx, rdy, dts, epssm
+      INTEGER(c_int), VALUE :: periodic_x, specified, nested
+      INTEGER(c_int), VALUE :: ids, ide, jds, jde, kde, ims, ime, jms, jme, kms, kme
+      INTEGER(c_int), VALUE :: its, ite, jts, jte, kts, kte
+      INTEGER(c_int) :: status
+   END FUNCTION wrfb200_advance_mu_t_r8
+END INTERFACE wrfb200_amt
+
+INTERFACE
    ! const char *wrfb200_last_error(void);
    FUNCTION wrfb200_last_error() BIND(C, NAME="wrfb200_last_error") RESULT(msg)
       IMPORT :: c_ptr
@@ -95,16 +120,17 @@ SUBROUTINE advance_mu_t( ww, ww_1, u, u_1, v, v_1,            &
   sp = MERGE(1_c_int, 0_c_int, config_flags%specified)
   ne = MERGE(1_c_int, 0_c_int, config_flags%nested)
 
-  status = wrfb200_advance_mu_t( ww, ww_1, u, u_1, v, v_1, mu, mut, muave, muts, muu, muv,            &
-                                 mudf, t, t_1, t_ave, ft, mu_tend,                                    &
-                                 REAL(rdx, c_float), REAL(rdy, c_float), REAL(dts, c_float),          &
-                                 REAL(epssm, c_float), dnw, fnm, fnp, rdnw,                           &
-                                 msfuy, msfvx_inv, msftx, msfty, px, sp, ne,                          &
-                                 INT(ids, c_int), INT(ide, c_int), INT(jds, c_int), INT(jde, c_int),  &
-                                 INT(kde, c_int), INT(ims, c_int), INT(ime, c_int), INT(jms, c_int),  &
-                                 INT(jme, c_int), INT(kms, c_int), INT(kme, c_int), INT(its, c_int),  &
-                                 INT(ite, c_int), INT(jts, c_int), INT(jte, c_int), INT(kts, c_int),  &
-                                 INT(kte, c_int) )
+  ! resolved at compile time by the kind of default REAL: c_float -> wrfb200_advance_mu_t,
+  ! c_double (-r8) -> wrfb200_advance_mu_t_r8
+  status = wrfb200_amt( ww, ww_1, u, u_1, v, v_1, mu, mut, muave, muts, muu, muv,                     &
+                        mudf, t, t_1, t_ave, ft, mu_tend,                                             &
+                        rdx, rdy, dts, epssm, dnw, fnm, fnp, rdnw,                                    &
+                        msfuy, msfvx_inv, msftx, msfty, px, sp, ne,                                   &
+                        INT(ids, c_int), INT(ide, c_int), INT(jds, c_int), INT(jde, c_int),           &
+                        INT(kde, c_int), INT(ims, c_int), INT(ime, c_int), INT(jms, c_int),           &
+                        INT(jme, c_int), INT(kms, c_int), INT(kme, c_int), INT(its, c_int),           &
+                        INT(ite, c_int), INT(jts, c_int), INT(jte, c_int), INT(kts, c_int),           &
+                        INT(kte, c_int) )
 
   IF ( status /= 0 ) CALL advance_mu_t_fail( status )
 

@@ -40,7 +40,7 @@
 !-----------------------------------------------------------------------------------------------------------
 MODULE module_small_step_em_resident
 
-USE, INTRINSIC :: iso_c_binding, ONLY : c_float, c_int, c_long, c_ptr, c_size_t
+USE, INTRINSIC :: iso_c_binding, ONLY : c_float, c_double, c_int, c_long, c_ptr, c_size_t
 
 IMPLICIT NONE
 PUBLIC
@@ -145,6 +145,70 @@ INTERFACE
    FUNCTION wrfb200_sync(handle) BIND(C, NAME="wrfb200_sync") RESULT(status)
       IMPORT :: c_int, c_ptr
       TYPE(c_ptr), VALUE :: handle
+      INTEGER(c_int) :: status
+   END FUNCTION
+
+   ! ---- (B') the same patch in double precision (WRF built with -r8); step / step_graph / sync / destroy
+   !      above work on it too.  Field ids: enum wrfb200_field of include/wrfb200.h.
+   FUNCTION wrfb200_create_r8(handle, dom, device, allocate) BIND(C, NAME="wrfb200_create_r8") RESULT(status)
+      IMPORT :: c_int, c_ptr, wrfb200_domain
+      TYPE(c_ptr), INTENT(OUT) :: handle
+      TYPE(wrfb200_domain), INTENT(IN) :: dom
+      INTEGER(c_int), VALUE :: device, allocate
+      INTEGER(c_int) :: status
+   END FUNCTION
+   FUNCTION wrfb200_set_scalars_r8(handle, rdx, rdy, dts, epssm) BIND(C, NAME="wrfb200_set_scalars_r8")      &
+            RESULT(status)
+      IMPORT :: c_int, c_ptr, c_double
+      TYPE(c_ptr), VALUE :: handle
+      REAL(c_double), VALUE :: rdx, rdy, dts, epssm
+      INTEGER(c_int) :: status
+   END FUNCTION
+   FUNCTION wrfb200_upload_r8(handle, field, host) BIND(C, NAME="wrfb200_upload_r8") RESULT(status)
+      IMPORT :: c_int, c_ptr, c_double
+      TYPE(c_ptr), VALUE :: handle
+      INTEGER(c_int), VALUE :: field
+      REAL(c_double), DIMENSION(*), INTENT(IN) :: host
+      INTEGER(c_int) :: status
+   END FUNCTION
+   FUNCTION wrfb200_download_r8(handle, field, host) BIND(C, NAME="wrfb200_download_r8") RESULT(status)
+      IMPORT :: c_int, c_ptr, c_double
+      TYPE(c_ptr), VALUE :: handle
+      INTEGER(c_int), VALUE :: field
+      REAL(c_double), DIMENSION(*), INTENT(INOUT) :: host
+      INTEGER(c_int) :: status
+   END FUNCTION
+   FUNCTION wrfb200_upload_range_r8(handle, field, host, i0, i1, k0, k1, j0, j1)                       &
+            BIND(C, NAME="wrfb200_upload_range_r8") RESULT(status)
+      IMPORT :: c_int, c_ptr, c_double
+      TYPE(c_ptr), VALUE :: handle
+      INTEGER(c_int), VALUE :: field, i0, i1, k0, k1, j0, j1
+      REAL(c_double), DIMENSION(*), INTENT(IN) :: host
+      INTEGER(c_int) :: status
+   END FUNCTION
+   FUNCTION wrfb200_download_range_r8(handle, field, host, i0, i1, k0, k1, j0, j1)                     &
+            BIND(C, NAME="wrfb200_download_range_r8") RESULT(status)
+      IMPORT :: c_int, c_ptr, c_double
+      TYPE(c_ptr), VALUE :: handle
+      INTEGER(c_int), VALUE :: field, i0, i1, k0, k1, j0, j1
+      REAL(c_double), DIMENSION(*), INTENT(INOUT) :: host
+      INTEGER(c_int) :: status
+   END FUNCTION
+   FUNCTION wrfb200_bind_device_r8(handle, field, device_ptr, pitch) BIND(C, NAME="wrfb200_bind_device_r8") &
+            RESULT(status)
+      IMPORT :: c_int, c_long, c_ptr
+      TYPE(c_ptr), VALUE :: handle, device_ptr
+      INTEGER(c_int), VALUE :: field
+      INTEGER(c_long), VALUE :: pitch
+      INTEGER(c_int) :: status
+   END FUNCTION
+   FUNCTION wrfb200_device_ptr_r8(handle, field, device_ptr, pitch) BIND(C, NAME="wrfb200_device_ptr_r8")    &
+            RESULT(status)
+      IMPORT :: c_int, c_long, c_ptr
+      TYPE(c_ptr), VALUE :: handle
+      INTEGER(c_int), VALUE :: field
+      TYPE(c_ptr), INTENT(OUT) :: device_ptr
+      INTEGER(c_long), INTENT(OUT) :: pitch
       INTEGER(c_int) :: status
    END FUNCTION
 
