@@ -192,8 +192,30 @@ int wrfb200_set_host_pinning(int enable);
 int wrfb200_host_register(const float *host, size_t bytes);
 int wrfb200_host_unregister_all(void);
 
-/* Kernel the most recent wrfb200_advance_mu_t call of this thread ran (a wrfb200_kernel id; AUTO resolved). */
+/* Kernel the most recent wrfb200_advance_mu_t call of this thread ran (a wrfb200_kernel id; AUTO resolved; for a
+ * call split over several devices, the first part's). */
 int wrfb200_default_last_kernel(int *kernel);
+
+/* Devices the HOST-pointer form of wrfb200_advance_mu_t / _loop (and the _r8 pair) spreads its j-rows over.
+ * Thread-local, like wrfb200_set_default_stream / _kernel.  n = 0 (devices may be NULL): back to the current
+ * device only (the default).  Ids may repeat (several parts on one device).  Device-pointer calls ignore it and
+ * run in place on the current device; the multi-GPU comm path (3b) is unaffected.
+ * Each part is the single-device call applied to its rows: its own cached mirrors on its device, its rows plus
+ * the one-row ring copied straight from the caller's arrays (no GPU-to-GPU traffic), issued from a host thread
+ * of its own; every thread is joined before the call returns.  Results are bit-identical to the single-device
+ * call.  Acoustic-loop residency, pinning (registered portable, so every device copies at the pinned rate) and
+ * wrfb200_release_cache cover every part.  A failing part makes the call return its status, with the device and
+ * rows in the message, after every part has finished.
+ * n < 0, n > 64, devices == NULL with n > 0, or an id outside [0, device count): WRFB200_ERR_INVALID_ARG; no
+ * device at all: WRFB200_ERR_CUDA.  Changing the list releases this thread's cached mirrors. */
+int wrfb200_set_default_devices(const int *devices, int n);
+
+/* Host-only: how a host-pointer call of this tile is split over n parts (1 <= n <= 64).  rows4[4p..4p+3] =
+ * {first computed row, last computed row, first memory row, last memory row} of part p (Fortran j; a part
+ * without rows has first > last).  The computed rows j_start..j_end are cut with j_start + nj*p/n; a part's
+ * memory is its rows plus one ring row on each side (in i it keeps ims..ime).  Needs no GPU. */
+int wrfb200_host_split_plan(const wrfb200_domain *dom, int its, int ite, int jts, int jte, int kts, int kte,
+                            int n, int *rows4);
 
 /* ------------------------------------------------------------------------------------------------
  * 2. Device-resident state (replaces the per-call malloc/H2D/D2H/free of advance_mu_t_no_async.cu).

@@ -14,10 +14,12 @@ All compute happens in the CUDA library; nothing here falls back to the CPU.
 """
 from __future__ import annotations
 
+import contextlib
 import ctypes as C
+import threading
 from dataclasses import dataclass, replace
 from types import SimpleNamespace
-from typing import Dict, Iterable, Optional
+from typing import Dict, Iterable, Optional, Sequence
 
 import numpy as np
 
@@ -388,6 +390,40 @@ class acoustic_loop:
 
     def __exit__(self, *exc):
         check(lib().wrfb200_acoustic_loop_end())
+
+
+_devices_state = threading.local()
+
+
+def set_default_devices(devices: Optional[Sequence[int]]) -> None:
+    """Spread this thread's host-array ``advance_mu_t`` calls over the CUDA devices ``devices`` (j-rows split
+    into ``len(devices)`` parts; ids may repeat).  ``None`` or ``[]``: the current device only (the default).
+    Device-array calls ignore it (wrfb200_set_default_devices)."""
+    ids = [int(d) for d in (devices or ())]
+    arr = (C.c_int * max(1, len(ids)))(*ids)
+    check(lib().wrfb200_set_default_devices(arr if ids else None, len(ids)))
+    _devices_state.devices = ids
+
+
+@contextlib.contextmanager
+def default_devices(devices: Optional[Sequence[int]]):
+    """``with default_devices([0, 1]):`` -- ``set_default_devices`` for the block, then the previous list."""
+    prev = list(getattr(_devices_state, "devices", []))
+    set_default_devices(devices)
+    try:
+        yield
+    finally:
+        set_default_devices(prev)
+
+
+def host_split_plan(grid: Grid, n: int):
+    """The split of a host-array call of ``grid``'s tile over ``n`` parts: one (first row, last row, first memory
+    row, last memory row) per part, Fortran j; a part without rows has first > last.  Needs no GPU."""
+    rows4 = (C.c_int * (4 * max(1, int(n))))()
+    dom = grid.domain()
+    check(lib().wrfb200_host_split_plan(C.byref(dom), grid.its, grid.ite, grid.jts, grid.jte, grid.kts, grid.kte,
+                                        int(n), rows4))
+    return [tuple(rows4[4 * p:4 * p + 4]) for p in range(int(n))]
 
 
 def default_last_kernel() -> int:

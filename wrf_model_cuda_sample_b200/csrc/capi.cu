@@ -14,11 +14,14 @@
 #include <cstdlib>
 #include <cstring>
 #include <map>
+#include <memory>
 #include <mutex>
 #include <new>
 #include <string>
+#include <thread>
 #include <tuple>
 #include <type_traits>
+#include <vector>
 
 #include "amt_params.h"
 #include "capi_internal.h"
@@ -840,7 +843,8 @@ int pin_host(const void *p, size_t bytes)
     bool already = false;
     if (classify(p, &already) != PTR_HOST || already) return WRFB200_OK;       // already page-locked by the caller
     if (it != g_pinned.end()) { cudaHostUnregister(const_cast<void *>(p)); g_pinned.erase(it); }
-    cudaError_t e = cudaHostRegister(const_cast<void *>(p), bytes, cudaHostRegisterDefault);
+    // portable: every device treats the range as page-locked (a host call may be split over several GPUs)
+    cudaError_t e = cudaHostRegister(const_cast<void *>(p), bytes, cudaHostRegisterPortable);
     if (e != cudaSuccess) { (void)cudaGetLastError(); return WRFB200_OK; }     // stays pageable: slower, still correct
     g_pinned[p] = bytes;
     return WRFB200_OK;
@@ -854,10 +858,11 @@ void unpin_all()
     (void)cudaGetLastError();
 }
 
-size_t field_bytes(const wrfb200_handle *h, int f)
+// bytes of the dense host array of `field` with the memory extents of `d`
+size_t field_bytes(const wrfb200_domain &d, int f, size_t esize)
 {
-    const size_t n = is3d(f) ? (size_t)h->idim * h->kdim * h->jdim : is2d(f) ? (size_t)h->idim * h->jdim : (size_t)h->kdim;
-    return n * h->esize;
+    const size_t idim = d.ime - d.ims + 1, jdim = d.jme - d.jms + 1, kdim = d.kme - d.kms + 1;
+    return (is3d(f) ? idim * kdim * jdim : is2d(f) ? idim * jdim : kdim) * esize;
 }
 
 int run_device_in_place(const Args &a, int prec)
@@ -900,7 +905,10 @@ int run_device_in_place(const Args &a, int prec)
 // arrays upload only u and v (what advance_uv changed; everything else on the device is this routine's own
 // previous output or a loop constant) -- the per-small-step drop-in pattern of a host-resident model:
 // 0.76 GB up and 1.15 GB down per step on 1800x1060x50 instead of 3.2 GB up.
-int run_host_compat_body(const Args &a, int nsteps, wrfb200_handle *h, CompatCache &cc)
+//
+// `part`: this is one device's share of a split call (run_host_split), whose calling thread has already
+// synchronised the caller's stream and page-locked the caller's whole arrays.
+int run_host_compat_body(const Args &a, int nsteps, wrfb200_handle *h, CompatCache &cc, bool part)
 {
     const wrfb200_domain &d = a.dom;
     int is, ie, js, je, ks, ke;
@@ -911,7 +919,7 @@ int run_host_compat_body(const Args &a, int nsteps, wrfb200_handle *h, CompatCac
         return fail(WRFB200_ERR_INVALID_ARG,
                     "computed range i=%d..%d j=%d..%d needs a one-cell ring inside memory i=%d..%d j=%d..%d",
                     is, ie, js, je, d.ims, d.ime, d.jms, d.jme);
-    CU(cudaStreamSynchronize(g_default_stream));          // the caller's earlier work on its stream is done
+    if (!part) CU(cudaStreamSynchronize(g_default_stream));   // the caller's earlier work on its stream is done
 
     static const int in3_all[] = {WRFB200_WW_1, WRFB200_U, WRFB200_U_1, WRFB200_V, WRFB200_V_1,
                                   WRFB200_T, WRFB200_T_1, WRFB200_FT};
@@ -933,8 +941,8 @@ int run_host_compat_body(const Args &a, int nsteps, wrfb200_handle *h, CompatCac
     const int *in3 = resident ? in3_uv : in3_all;
     const int n_in3 = resident ? 2 : 8;
 
-    if (pin_enabled())
-        for (int f = 0; f < WRFB200_NUM_FIELDS; ++f) pin_host(a.f[f], field_bytes(h, f));
+    if (pin_enabled() && !part)
+        for (int f = 0; f < WRFB200_NUM_FIELDS; ++f) pin_host(a.f[f], field_bytes(d, f, h->esize));
 
     // small operands first: 2-D and 1-D inputs, and ww at level 1 (the only level of ww the routine
     // reads, module_small_step_em.f90:159-161)
@@ -1010,13 +1018,16 @@ int run_host_compat_body(const Args &a, int nsteps, wrfb200_handle *h, CompatCac
     return WRFB200_OK;
 }
 
-int run_host_compat(const Args &a, int nsteps, int prec)
+// One host-pointer call, or one device's share of a split call, on the cached mirrors `cc`.  device < 0: the
+// current device, and a cache of the same memory shape is re-used wherever it lives (the single-device call);
+// device >= 0: the cache is re-created when it lives on another device.  `kernel` is the calling thread's
+// choice, passed in because a part may run in a worker thread.
+int run_host_part(const Args &a, int nsteps, int prec, CompatCache &cc, int device, int kernel, bool part)
 {
     if (int rc = check_domain(a.dom)) return rc;
-    CompatCache &cc = g_cache[prec];
-    if (cc.h && !same_shape(cc.h->dom, a.dom)) cc.release();
+    if (cc.h && (!same_shape(cc.h->dom, a.dom) || (device >= 0 && cc.h->device != device))) cc.release();
     if (!cc.h) {
-        if (int rc = create(&cc.h, &a.dom, -1, 1, prec ? 8 : 4)) return rc;
+        if (int rc = create(&cc.h, &a.dom, device, 1, prec ? 8 : 4)) return rc;
         DeviceGuard g(cc.h->device);
         for (cudaStream_t *st : {&cc.up, &cc.comp, &cc.down})
             CU(cudaStreamCreateWithFlags(st, cudaStreamNonBlocking));
@@ -1028,9 +1039,9 @@ int run_host_compat(const Args &a, int nsteps, int prec)
     wrfb200_handle *h = cc.h;
     GUARD(h);
     h->dom = a.dom;                       // same extents; domain dims / flags may differ between calls
-    h->kernel = g_default_kernel;
+    h->kernel = kernel;
     set_scalars(h, a.rdx, a.rdy, a.dts, a.epssm);
-    const int rc = run_host_compat_body(a, nsteps, h, cc);
+    const int rc = run_host_compat_body(a, nsteps, h, cc, part);
     if (rc != WRFB200_OK) {
         // an early return must not leave copies on the caller's arrays in flight, nor the cached handle
         // pointing at one of the internal lanes
@@ -1040,8 +1051,131 @@ int run_host_compat(const Args &a, int nsteps, int prec)
         cc.primed = false;
         wrfb200_fail(rc, "%s", msg.c_str());
     }
-    h->stream = g_default_stream;
+    h->stream = part ? nullptr : g_default_stream;
     return rc;
+}
+
+// ---- one host-pointer call split over several devices (wrfb200_set_default_devices) --------------------
+constexpr int kMaxParts = 64;
+
+thread_local std::vector<int> g_default_devices;                         // empty: the current device only
+// parts 1.. of a split call (part 0 is g_cache), indexed like g_cache
+thread_local std::vector<std::unique_ptr<CompatCache>> g_parts[2];
+
+// The split rule, shared by wrfb200_host_split_plan and the call: the computed rows j_start..j_end are cut into n
+// contiguous parts with the slab loop's formula; a part's memory is its rows plus the one-row ring on each side.
+int host_split(const wrfb200_domain &d, int its, int ite, int jts, int jte, int kts, int kte, int n, int *rows4)
+{
+    int is, ie, js, je, ks, ke;
+    wrfb200_bounds(d.periodic_x, d.specified, d.nested, d.ids, d.ide, d.jds, d.jde,
+                   its, ite, jts, jte, kts, kte, &is, &ie, &js, &je, &ks, &ke);
+    const bool empty = is > ie || js > je || ks > ke;
+    if (!empty && (is - 1 < d.ims || ie + 1 > d.ime || js - 1 < d.jms || je + 1 > d.jme))
+        return fail(WRFB200_ERR_INVALID_ARG,
+                    "computed range i=%d..%d j=%d..%d needs a one-cell ring inside memory i=%d..%d j=%d..%d",
+                    is, ie, js, je, d.ims, d.ime, d.jms, d.jme);
+    const int nj = empty ? 0 : je - js + 1;
+    for (int p = 0; p < n; ++p) {
+        const int ja = js + (int)((long long)nj * p / n);
+        const int jb = js + (int)((long long)nj * (p + 1) / n) - 1;
+        int *r = rows4 + 4 * p;
+        r[0] = ja; r[1] = jb;
+        r[2] = ja <= jb ? ja - 1 : ja; r[3] = ja <= jb ? jb + 1 : jb;
+    }
+    return WRFB200_OK;
+}
+
+// The host-pointer call as one sub-call per used part.  A part is the single-device call on a sub-domain: field
+// pointers offset to the part's first memory row (j is the slowest index, so that slice of a dense array is
+// dense), jms..jme narrowed to the part's memory and jts..jte to its rows; ids..jde, the flags, its..ite and
+// kts..kte unchanged.  Part 0 runs in the calling thread, every other part in a thread of its own, so that each
+// device's copies and launches are issued concurrently (a pageable cudaMemcpyAsync blocks its thread); all are
+// joined before the call returns.
+int run_host_split(const Args &a, int nsteps, int prec)
+{
+    if (int rc = check_domain(a.dom)) return rc;
+    const int n = (int)g_default_devices.size();
+    int rows4[4 * kMaxParts];
+    if (int rc = host_split(a.dom, a.its, a.ite, a.jts, a.jte, a.kts, a.kte, n, rows4)) return rc;
+    CU(cudaStreamSynchronize(g_default_stream));          // the caller's earlier work on its stream is done
+    const size_t es = prec ? 8 : 4;
+    // the caller's WHOLE arrays, once: part slices overlap by the ring rows, and a second registration of an
+    // overlapping range would fail
+    if (pin_enabled())
+        for (int f = 0; f < WRFB200_NUM_FIELDS; ++f) pin_host(a.f[f], field_bytes(a.dom, f, es));
+
+    struct Part {
+        Args a;
+        int device, rc = WRFB200_OK;
+        std::string err;
+    };
+    std::vector<Part> parts;
+    for (int p = 0; p < n; ++p) {
+        const int *r = rows4 + 4 * p;
+        if (r[0] > r[1]) continue;                        // no rows: not used
+        Part q;
+        q.a = a;
+        q.device = g_default_devices[p];
+        const size_t row3 = field_bytes(a.dom, WRFB200_U, es) / (a.dom.jme - a.dom.jms + 1);
+        const size_t row2 = field_bytes(a.dom, WRFB200_MU, es) / (a.dom.jme - a.dom.jms + 1);
+        for (int f = 0; f < WRFB200_NUM_FIELDS; ++f)
+            if (!is1d(f)) q.a.f[f] = static_cast<char *>(a.f[f]) + (size_t)(r[2] - a.dom.jms) * (is3d(f) ? row3 : row2);
+        q.a.dom.jms = r[2]; q.a.dom.jme = r[3];
+        q.a.jts = r[0]; q.a.jte = r[1];
+        parts.push_back(q);
+    }
+    if (parts.empty()) return WRFB200_OK;
+
+    std::vector<std::unique_ptr<CompatCache>> &pool = g_parts[prec];
+    while (pool.size() + 1 < parts.size()) {
+        pool.emplace_back(new (std::nothrow) CompatCache());
+        if (!pool.back()) { pool.pop_back(); return fail(WRFB200_ERR_NOMEM, "out of host memory"); }
+        pool.back()->loop_active = g_cache[prec].loop_active;
+    }
+    auto cache = [&](size_t q) -> CompatCache & { return q == 0 ? g_cache[prec] : *pool[q - 1]; };
+    const int kernel = g_default_kernel;
+    auto run = [&](size_t q) {
+        Part &p = parts[q];
+        p.rc = run_host_part(p.a, nsteps, prec, cache(q), p.device, kernel, true);
+        if (p.rc != WRFB200_OK) p.err = wrfb200_last_error();
+    };
+    std::vector<std::thread> workers;
+    workers.reserve(parts.size());
+    for (size_t q = 1; q < parts.size(); ++q) {
+        try {
+            workers.emplace_back(run, q);
+        } catch (const std::exception &) {
+            parts[q].rc = WRFB200_ERR_NOMEM;
+            parts[q].err = "cannot start a host thread";
+        }
+    }
+    run(0);
+    for (std::thread &t : workers) t.join();
+
+    for (size_t q = 0; q < parts.size(); ++q) {
+        if (parts[q].rc == WRFB200_OK) continue;
+        for (size_t r = 0; r < parts.size(); ++r) cache(r).primed = false;
+        const Part &p = parts[q];
+        return fail(p.rc, "device %d, rows j=%d..%d: %s", p.device, p.a.jts, p.a.jte, p.err.c_str());
+    }
+    return WRFB200_OK;
+}
+
+int run_host_compat(const Args &a, int nsteps, int prec)
+{
+    if (!g_default_devices.empty()) {
+        int cur = 0;
+        CU(cudaGetDevice(&cur));
+        if (g_default_devices.size() > 1 || g_default_devices[0] != cur) return run_host_split(a, nsteps, prec);
+    }
+    return run_host_part(a, nsteps, prec, g_cache[prec], -1, g_default_kernel, false);
+}
+
+void release_parts()
+{
+    for (CompatCache &c : g_cache) c.release();
+    for (auto &pool : g_parts)
+        for (auto &c : pool) c->release();
 }
 
 // prec: 0 = binary32 entry points, 1 = real*8 entry points
@@ -1181,9 +1315,40 @@ extern "C" int wrfb200_set_default_kernel(int kernel)
     return WRFB200_OK;
 }
 
+extern "C" int wrfb200_set_default_devices(const int *devices, int n)
+{
+    if (n < 0 || n > kMaxParts) return fail(WRFB200_ERR_INVALID_ARG, "n=%d: 0..%d devices", n, kMaxParts);
+    if (n > 0 && !devices) return fail(WRFB200_ERR_INVALID_ARG, "null device list with n=%d", n);
+    if (n > 0) {
+        int ndev = 0;
+        if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
+            cudaGetLastError();
+            return fail(WRFB200_ERR_CUDA, "no CUDA device available (this library has no CPU fallback)");
+        }
+        for (int p = 0; p < n; ++p)
+            if (devices[p] < 0 || devices[p] >= ndev)
+                return fail(WRFB200_ERR_INVALID_ARG, "device %d out of range (%d devices)", devices[p], ndev);
+    }
+    std::vector<int> list(devices, devices + n);
+    if (list != g_default_devices) {
+        release_parts();
+        g_default_devices.swap(list);
+    }
+    return WRFB200_OK;
+}
+
+extern "C" int wrfb200_host_split_plan(const wrfb200_domain *dom, int its, int ite, int jts, int jte, int kts, int kte,
+                                       int n, int *rows4)
+{
+    if (!dom || !rows4) return fail(WRFB200_ERR_INVALID_ARG, "null argument");
+    if (n < 1 || n > kMaxParts) return fail(WRFB200_ERR_INVALID_ARG, "n=%d: 1..%d parts", n, kMaxParts);
+    if (int rc = check_domain(*dom)) return rc;
+    return host_split(*dom, its, ite, jts, jte, kts, kte, n, rows4);
+}
+
 extern "C" int wrfb200_release_cache(void)
 {
-    for (CompatCache &c : g_cache) c.release();
+    release_parts();
     for (DeviceCallCache &c : g_devcall) c.valid = false;
     unpin_all();
     return WRFB200_OK;
@@ -1192,12 +1357,16 @@ extern "C" int wrfb200_release_cache(void)
 extern "C" int wrfb200_acoustic_loop_begin(void)
 {
     for (CompatCache &c : g_cache) { c.loop_active = true; c.primed = false; }
+    for (auto &pool : g_parts)
+        for (auto &c : pool) { c->loop_active = true; c->primed = false; }
     return WRFB200_OK;
 }
 
 extern "C" int wrfb200_acoustic_loop_end(void)
 {
     for (CompatCache &c : g_cache) { c.loop_active = false; c.primed = false; }
+    for (auto &pool : g_parts)
+        for (auto &c : pool) { c->loop_active = false; c->primed = false; }
     return WRFB200_OK;
 }
 

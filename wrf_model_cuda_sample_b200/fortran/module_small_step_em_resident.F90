@@ -79,6 +79,22 @@ INTERFACE
       IMPORT :: c_int
       INTEGER(c_int) :: status
    END FUNCTION
+   ! the host-array call split over several GPUs of the box: call once at start-up (e.g. ids 0..7 on an
+   ! 8-GPU box), the advance_mu_t call itself is unchanged
+   FUNCTION wrfb200_set_default_devices(devices, n) BIND(C, NAME="wrfb200_set_default_devices") RESULT(status)
+      IMPORT :: c_int
+      INTEGER(c_int), DIMENSION(*), INTENT(IN) :: devices
+      INTEGER(c_int), VALUE :: n
+      INTEGER(c_int) :: status
+   END FUNCTION
+   FUNCTION wrfb200_host_split_plan(dom, its, ite, jts, jte, kts, kte, n, rows4)                      &
+            BIND(C, NAME="wrfb200_host_split_plan") RESULT(status)
+      IMPORT :: c_int, wrfb200_domain
+      TYPE(wrfb200_domain), INTENT(IN) :: dom
+      INTEGER(c_int), VALUE :: its, ite, jts, jte, kts, kte, n
+      INTEGER(c_int), DIMENSION(*), INTENT(OUT) :: rows4
+      INTEGER(c_int) :: status
+   END FUNCTION
 
    ! ---- (B) explicit device-resident patch ----
    FUNCTION wrfb200_create(handle, dom, device, allocate) BIND(C, NAME="wrfb200_create") RESULT(status)
