@@ -382,11 +382,6 @@ int wrfb200_compare(const float *a, const float *b, long n, wrfb200_compare_resu
 int wrfb200_pipe_plan(const wrfb200_domain *dom, int its, int ite, int jts, int jte, int kts, int kte,
                       int resident_blocks, long long *plan10);
 
-/* Device self-test of the kernel's division by a loop-invariant divisor (reciprocal hoisted out of the level
- * loop, csrc/amt_pipe.cu) against IEEE division: all 2^23 divisor mantissas at three exponents, each with
- * `dividends_per_divisor` dividends.  *mismatches must come back 0. */
-int wrfb200_selftest_division(long long *mismatches, long long *checked, int dividends_per_divisor);
-
 const char *wrfb200_last_error(void);
 int wrfb200_version(void);
 

@@ -1,9 +1,12 @@
-"""Compare the binary32 kernels' SASS of two builds of libwrfb200.so, function by function.
+"""Compare the kernels' SASS of two builds of libwrfb200.so, function by function.
 
-    python tools/sass_diff.py OLD.so NEW.so      # exit 0 when every float kernel is identical
+    python tools/sass_diff.py OLD.so NEW.so      # exit 0 when both builds hold the same kernels with identical SASS
 
-Instruction text and encodings are compared; code addresses and cuobjdump's column padding (which depends on the
-longest instruction in the module) are stripped.  Used to show that a change leaves the float kernels untouched."""
+Kernels are matched by their demangled name without the parameter list or an anonymous namespace: the hash nvcc
+puts into the name of an anonymous namespace (`_GLOBAL__N__<hex>_`) depends on the path of the source file, and a
+kernel whose parameters or linkage change is still the same kernel.  Instruction text and both 64-bit halves of
+every encoding are compared; code addresses and cuobjdump's column padding (which depends on the longest
+instruction in the module) are stripped.  Kernels found in only one build are listed separately."""
 import re
 import subprocess
 import sys
@@ -17,13 +20,24 @@ def funcs(so):
         if m:
             name = m.group(1)
             res[name] = []
-        elif name and re.match(r"\s+/\*[0-9a-f]{4}\*/", ln):
+        elif name and re.match(r"\s+/\*[0-9a-f]{4,}\*/", ln):
             res[name].append(" ".join(re.sub(r"/\*[0-9a-f]{4,}\*/", "", ln).split()))
-    return res
+        elif name and res[name] and re.fullmatch(r"\s+/\* 0x[0-9a-f]{16} \*/", ln):
+            res[name][-1] += " " + ln.strip()       # second half of the encoding: the scheduling control bits
+    names = subprocess.run(["cu++filt"], input="\n".join(res), capture_output=True, text=True,
+                           check=True).stdout.splitlines()
+    return {re.sub(r"^void |<unnamed>::|\([^()]*\)$", "", d): res[m] for m, d in zip(res, names)}
 
 
 a, b = funcs(sys.argv[1]), funcs(sys.argv[2])
-sel = [n for n in a if re.search(r"amt_pipe_|amt_tile_kernel|amt_column_kernel", n) and "_r8" not in n]
-bad = [n for n in sel if a[n] != b.get(n)]
-print(f"{len(sel)} float kernels compared, {sum(len(a[n]) for n in sel)} instructions; differing: {bad}")
-sys.exit(1 if bad else 0)
+both = [n for n in a if n in b]
+same = [n for n in both if a[n] == b[n]]
+only_a = [n for n in a if n not in b]
+only_b = [n for n in b if n not in a]
+print(f"{len(both)} kernels in both builds, {len(same)} identical "
+      f"({sum(len(a[n]) for n in same)} instructions)")
+for title, names in (("differing", [n for n in both if a[n] != b[n]]), (f"only in {sys.argv[1]}", only_a),
+                     (f"only in {sys.argv[2]}", only_b)):
+    for n in names:
+        print(f"  {title}: {n}" + (f" ({len(a[n])} -> {len(b[n])} instructions)" if n in a and n in b else ""))
+sys.exit(0 if len(same) == len(a) == len(b) else 1)

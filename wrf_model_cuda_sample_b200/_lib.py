@@ -116,7 +116,6 @@ PROTOTYPES = {
     "wrfb200_synth_field": (C.c_int, [C.c_int, C.c_uint64, C.POINTER(Domain), C.c_float, _P]),
     "wrfb200_compare": (C.c_int, [_P, _P, C.c_long, C.POINTER(CompareResult)]),
     "wrfb200_pipe_plan": (C.c_int, [C.POINTER(Domain)] + [C.c_int] * 7 + [C.POINTER(C.c_longlong)]),
-    "wrfb200_selftest_division": (C.c_int, [C.POINTER(C.c_longlong), C.POINTER(C.c_longlong), C.c_int]),
     "wrfb200_last_error": (C.c_char_p, []),
     "wrfb200_version": (C.c_int, []),
 }

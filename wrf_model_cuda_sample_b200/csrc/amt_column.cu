@@ -30,6 +30,10 @@ amt_column_kernel(const AmtParams p, const int nbx)
     amt_column_thread(p, i, j, s_dvdxi + tid, kColThreads);
 }
 
+}  // namespace
+
+// Outside the anonymous namespace, like amt_tile_kernel_r8: the symbol then carries no hash of the source path, so
+// the library's kernel and this file compiled elsewhere (tests/test_r8.py compares their SASS) have the same name.
 __global__ void __launch_bounds__(kColThreads)
 amt_column_kernel_r8(const AmtParamsR8 p, const int nbx)
 {
@@ -43,6 +47,8 @@ amt_column_kernel_r8(const AmtParamsR8 p, const int nbx)
 
     amt_column_thread(p, i, j, s_dvdxi_r8 + tid, kColThreads);
 }
+
+namespace {
 
 // One launcher for both element types (the two kernels differ in their argument block only).
 template <class P, class T, class K>

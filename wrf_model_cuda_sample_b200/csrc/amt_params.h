@@ -159,9 +159,8 @@ inline cudaError_t amt_raise_smem_limit(K kernel, bool (&done)[64])
 }
 
 // Launchers (defined in the kernel translation units).
-cudaError_t amt_division_selftest(unsigned long long *mismatches, unsigned long long *checked, int dividends_per_divisor);
-bool amt_pipe_plan(const AmtParams &p, int cfg, int slots, long long out[10]);   // host-only launch description
-cudaError_t amt_pipe_preload();
+bool amt_pipe_plan(const AmtParams &p, int slots, long long out[10]);   // host-only launch description
+cudaError_t amt_pipe_preload();                                         // load all kernels of amt_pipe.cu (see there)
 // blocks of a fused launch that own the patch's east column / north row signal the neighbours when they finish
 __device__ __forceinline__ void amt_halo_block_done(const AmtHalo &hx, bool owns_east, bool owns_north, unsigned step)
 {
@@ -176,13 +175,13 @@ __device__ __forceinline__ void amt_halo_block_done(const AmtHalo &hx, bool owns
         __threadfence_system();
         st_release_sys(hx.out_flag_to_east, step);
     }
-}   // load all kernels of amt_pipe.cu (see there)
+}
 cudaError_t amt_launch_column(const AmtParams &p, cudaStream_t stream);
 cudaError_t amt_launch_tile(const AmtParams &p, cudaStream_t stream);
 bool amt_tile_supported(const AmtParams &p);
 bool amt_pipe_supported(const AmtParams &p);
 bool amt_build_tma_maps(const AmtParams &p, AmtTmaMaps *maps);                    // cached: rebuilds only on change
-cudaError_t amt_launch_pipe(const AmtParams &p, const AmtTmaMaps &maps, cudaStream_t stream, int cfg);   // cfg 0 = automatic
+cudaError_t amt_launch_pipe(const AmtParams &p, const AmtTmaMaps &maps, cudaStream_t stream);
 // real*8 kernels (amt_column.cu, amt_tile_r8.cu)
 cudaError_t amt_launch_column(const AmtParamsR8 &p, cudaStream_t stream);
 cudaError_t amt_launch_tile(const AmtParamsR8 &p, cudaStream_t stream);

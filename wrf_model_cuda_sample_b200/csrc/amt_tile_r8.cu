@@ -17,8 +17,8 @@
 // rows per tile and two resident blocks per SM while nk <= 55, one row otherwise.
 //
 // Arithmetic: every operation is one __d*_rn intrinsic in the Fortran's order (amt_params.h), so the result is
-// the Fortran's evaluated in real*8 bit for bit.  Division is the IEEE __ddiv_rn; the float pipe
-// kernel's hoisted reciprocal is proven for the 2^23 binary32 mantissas only and is not used here.
+// the Fortran's evaluated in real*8 bit for bit.  Division is the IEEE __ddiv_rn, as the float kernels use
+// __fdiv_rn.
 //
 // Layout requirement: 16-byte aligned base pointers and row pitches that are even numbers of doubles.
 // WRF's default halo-5 patch (ims = ids-5 .. ime = ide+5, e.g. 1810 points on a 1800-point domain) is such

@@ -130,13 +130,6 @@ int wrfb200_make_params(const wrfb200_handle *h, int its, int ite, int jts, int 
 
 namespace {
 
-// Tuning override for the pipelined kernel: WRFB200_PIPE_CFG = TJ*10 + STAGES (0 / unset = automatic).
-int pipe_cfg()
-{
-    static const int cfg = [] { const char *e = getenv("WRFB200_PIPE_CFG"); return e ? atoi(e) : 0; }();
-    return cfg;
-}
-
 int launch(wrfb200_handle *h, const AmtParams &p, cudaStream_t s, int kernel)
 {
     cudaError_t e;
@@ -151,14 +144,14 @@ int launch(wrfb200_handle *h, const AmtParams &p, cudaStream_t s, int kernel)
         if (!amt_pipe_supported(p))
             return fail(WRFB200_ERR_UNSUPPORTED, "pipe kernel needs 16-byte aligned fields and pitches that are multiples of 4");
         if (!amt_build_tma_maps(p, &h->maps)) return fail(WRFB200_ERR_CUDA, "cuTensorMapEncodeTiled failed");
-        e = amt_launch_pipe(p, h->maps, s, pipe_cfg());
+        e = amt_launch_pipe(p, h->maps, s);
     } else {
         // AUTO: the TMA-pipelined tile kernel wherever the layout allows it; tiles narrower than a warp
         // of columns (e.g. the one-column strips behind an east halo) would stage 128-wide rows for
         // nothing, and unaligned caller layouts cannot be bulk-copied: those take the column kernel.
         const bool wide = (p.i1 - p.i0 + 1) >= 32;
         if (wide && amt_pipe_supported(p) && amt_build_tma_maps(p, &h->maps)) {
-            e = amt_launch_pipe(p, h->maps, s, pipe_cfg());
+            e = amt_launch_pipe(p, h->maps, s);
             ran = WRFB200_KERNEL_PIPE;
         } else {
             e = amt_launch_column(p, s);
@@ -1402,23 +1395,8 @@ extern "C" int wrfb200_pipe_plan(const wrfb200_domain *dom, int its, int ite, in
     p.i0 = is - dom->ims; p.i1 = ie - dom->ims;
     p.j0 = js - dom->jms; p.j1 = je - dom->jms;
     p.k0 = ks - dom->kms; p.nk = ke - ks + 1;
-    if (!amt_pipe_plan(p, 0, resident_blocks > 0 ? resident_blocks : 2 * 148, plan10))
-        return fail(WRFB200_ERR_INVALID_ARG, "empty index sets or no launch shape");
-    return WRFB200_OK;
-}
-
-extern "C" int wrfb200_selftest_division(long long *mismatches, long long *checked, int dividends_per_divisor)
-{
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-        cudaGetLastError();
-        return fail(WRFB200_ERR_CUDA, "no CUDA device available (this library has no CPU fallback)");
-    }
-    if (dividends_per_divisor < 1) dividends_per_divisor = 1;
-    unsigned long long bad = 0, n = 0;
-    CU(amt_division_selftest(&bad, &n, dividends_per_divisor));
-    if (mismatches) *mismatches = (long long)bad;
-    if (checked) *checked = (long long)n;
+    if (!amt_pipe_plan(p, resident_blocks > 0 ? resident_blocks : 2 * 148, plan10))
+        return fail(WRFB200_ERR_INVALID_ARG, "empty index sets");
     return WRFB200_OK;
 }
 
