@@ -37,8 +37,9 @@
  *   - Precision: the unsuffixed entry points take binary32 (`float`, WRF's default REAL = 4 bytes).  WRF built
  *     with -r8 (REAL = 8 bytes) calls the `_r8` entry points, which take `double` and compute every operation
  *     in binary64, in the same order.  A handle holds one precision, fixed by wrfb200_create / _create_r8;
- *     a verb typed for the other precision fails with WRFB200_ERR_STATE.  The multi-GPU, halo, stand-in and
- *     resident-bundle verbs are binary32 only (WRFB200_ERR_UNSUPPORTED on an r8 handle).
+ *     a verb typed for the other precision fails with WRFB200_ERR_STATE.  The multi-GPU, stand-in and
+ *     resident-bundle verbs have `_r8` twins (wrfb200_comm_init_r8, ..., section 3b); their binary32 forms
+ *     return WRFB200_ERR_UNSUPPORTED on an r8 handle.  The halo pack / unpack verbs (section 3) are binary32 only.
  */
 #ifndef WRFB200_H
 #define WRFB200_H
@@ -258,6 +259,17 @@ int wrfb200_upload_state(wrfb200_handle *h, const float *ww, const float *t, con
 int wrfb200_set_uv(wrfb200_handle *h, const float *u, const float *v);
 int wrfb200_download_outputs(wrfb200_handle *h, int its, int ite, int jts, int jte, int kts, int kte,
                              float *ww, float *t, float *t_ave, float *mu, float *muave, float *muts, float *mudf);
+/* The same four verbs for a real*8 handle (double arrays). */
+int wrfb200_upload_constants_r8(
+    wrfb200_handle *h, const double *ww_1, const double *u_1, const double *v_1, const double *t_1, const double *ft,
+    const double *mut, const double *muu, const double *muv, const double *mu_tend,
+    const double *msfuy, const double *msfvx_inv, const double *msftx, const double *msfty,
+    const double *dnw, const double *fnm, const double *fnp, const double *rdnw);
+int wrfb200_upload_state_r8(wrfb200_handle *h, const double *ww, const double *t, const double *mu);
+int wrfb200_set_uv_r8(wrfb200_handle *h, const double *u, const double *v);
+int wrfb200_download_outputs_r8(wrfb200_handle *h, int its, int ite, int jts, int jte, int kts, int kte,
+                                double *ww, double *t, double *t_ave, double *mu, double *muave, double *muts,
+                                double *mudf);
 
 /* One advance_mu_t over the tile its:ite x jts:jte (kts:kte as the Fortran), asynchronous on the stream. */
 int wrfb200_step(wrfb200_handle *h, int its, int ite, int jts, int jte, int kts, int kte);
@@ -300,6 +312,8 @@ int wrfb200_unpack_halo(wrfb200_handle *h, int field, int side, int width,
  * field = WRFB200_V: v(i,k,j) += c*(mudf(i,j)-mudf(i,j-1)); over i0..i1 x all memory levels x j0..j1.
  * It makes the multi-step loop and the halo exchange load-bearing in tests (SURVEY.md section 8d). */
 int wrfb200_standin_advance_uv(wrfb200_handle *h, int field, float c, int i0, int i1, int j0, int j1);
+/* The same on a real*8 handle, every operation rounded once in binary64. */
+int wrfb200_standin_advance_uv_r8(wrfb200_handle *h, int field, double c, int i0, int i1, int j0, int j1);
 
 /* ------------------------------------------------------------------------------------------------
  * 3b. Multi-GPU behind the boundary: one rank per GPU of one NVLink box, 2-D (i,j) patches, the one-cell
@@ -325,6 +339,13 @@ int wrfb200_standin_advance_uv(wrfb200_handle *h, int field, float c, int i0, in
  *     asynchronous on the handle's stream; there is no host synchronisation and no NCCL call inside the loop.
  *     All ranks must issue the same sequence of steps (the flags are step counters).  A halo wait gives up
  *     after 5 s (WRFB200_FLAG_TIMEOUT_MS) and is reported by wrfb200_comm_status.
+ *
+ *     Real*8 ranks (wrfb200_create_r8, allocate=1): wrfb200_comm_init_r8 instead of wrfb200_comm_init, and the
+ *     _r8 forms of the loop and the stand-in (double c).  connect, barrier, push_constants, push_uv,
+ *     wait_outputs, step and status take no floating-point argument and serve both precisions.  Each step runs
+ *     the double2 tile kernel with the exchange fused in, so wrfb200_comm_init_r8 fails with
+ *     WRFB200_ERR_UNSUPPORTED when the patch has more than 220 computed levels.  All ranks must hold the same
+ *     precision: connect rejects a neighbour's blob of the other one with WRFB200_ERR_INVALID_ARG.
  * ---------------------------------------------------------------------------------------------- */
 #define WRFB200_COMM_INFO_BYTES 2048
 int wrfb200_comm_info_bytes(void);
@@ -346,6 +367,11 @@ int wrfb200_comm_loop(wrfb200_handle *h, int nsteps, int standin, float c, int u
 /* Synchronises the stream; flag_timeouts != 0 means some halo wait gave up (results are then invalid);
  * steps_done = advance_mu_t launches completed since wrfb200_comm_init. */
 int wrfb200_comm_status(wrfb200_handle *h, int *flag_timeouts, long *steps_done);
+/* real*8 ranks */
+int wrfb200_comm_init_r8(wrfb200_handle *h, int px, int py, int rank,
+                         int ips, int ipe, int jps, int jpe, void *info_out /* WRFB200_COMM_INFO_BYTES */);
+int wrfb200_comm_standin_advance_uv_r8(wrfb200_handle *h, double c);
+int wrfb200_comm_loop_r8(wrfb200_handle *h, int nsteps, int standin, double c, int use_graph);
 
 /* ------------------------------------------------------------------------------------------------
  * 4. Harness utilities (host side; usable without a GPU).

@@ -2,24 +2,47 @@
 
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         tools/multi_gpu_check.py [--pgrid PXxPY] [--shape NXxNYxNZ] [--steps S] [--mode fused|nccl]
+        [--dtype float32|float64]
 
 Every rank runs the CUDA path on its patch (tile = patch, domain = global) and applies the advance_uv stand-in
 between steps.  --mode fused (default): the one-cell ring moves by peer-mapped stores fused into the kernels
 (csrc/comm.cu; torch.distributed only all-gathers the bootstrap blobs).  --mode nccl: pack / NCCL send-recv /
 unpack through HaloExchanger, overlapped with the interior tile (the round-1 path).  Each rank then checks its
-patch BIT FOR BIT against the single-domain oracle loop.  Exit code 0 = every rank identical.
+patch BIT FOR BIT against the single-domain oracle loop.  --dtype float64 (fused mode only): real*8 patches
+(wrfb200_comm_init_r8 / wrfb200_comm_loop_r8) on float64 inputs with full 53-bit mantissas, checked against the
+binary64 checker loop (tests/r8_checkers.py).  Exit code 0 = every rank identical.
 """
 import argparse
 import os
 import sys
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 import torch.distributed as dist  # noqa: E402
 
 import wrf_model_cuda_sample_b200 as wrf  # noqa: E402
 from wrf_model_cuda_sample_b200 import parallel  # noqa: E402
 from tests import cases  # noqa: E402
+
+SCALARS_3KM_R8 = (1.0 / 3000.0, 1.0 / 3000.0, 3.0, 0.1)
+
+
+def widen64(f):
+    """float32 fields -> float64 with low mantissa bits a float cannot hold (x * (1 + 2^-40), one rounding)."""
+    return {n: a.astype(np.float64) * (1.0 + 2.0 ** -40) for n, a in f.items() if isinstance(a, np.ndarray)}
+
+
+def checker_loop64(G, whole, scalars, nsteps, c):
+    """The binary64 checker over the whole domain, with the stand-in advance_uv between steps."""
+    from tests import r8_checkers
+    f = cases.copy_fields(whole)
+    ubox, vbox = cases.standin_boxes(G, G.ids, G.ide, G.jds, G.jde)
+    for s in range(nsteps):
+        r8_checkers.oracle_c_r8(f, G, scalars, tiles=64)
+        if s + 1 < nsteps:
+            cases.standin_advance_uv_numpy(f, G, c, ubox, vbox)
+    return f
 
 
 def run_fused(patch, decomp, rank, dev, steps, c_uv, graph):
@@ -64,7 +87,11 @@ def main():
     ap.add_argument("--variant", default="specified")
     ap.add_argument("--mode", choices=("fused", "nccl"), default="fused")
     ap.add_argument("--no-graph", action="store_true")
+    ap.add_argument("--dtype", choices=("float32", "float64"), default="float32")
     args = ap.parse_args()
+    r8 = args.dtype == "float64"
+    if r8 and args.mode != "fused":
+        ap.error("--dtype float64 runs the fused mode only (the pack / unpack path is binary32)")
     rank, world = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"])
     local = int(os.environ.get("LOCAL_RANK", rank))
     torch.cuda.set_device(local)
@@ -79,15 +106,18 @@ def main():
     c_uv = 0.25
 
     whole = wrf.synth_fields(G, seed=99)
+    if r8:
+        whole = widen64(whole)
+    scalars = SCALARS_3KM_R8 if r8 else cases.SCALARS_3KM
     f = cases.carve_patch(whole, G, pg)
     # poison every halo that a neighbour must fill, so a missing exchange cannot go unnoticed
     cases.poison_neighbour_halos(f, decomp, rank, pg,
                                  (parallel.CONSTANT_HALOS, parallel.STEP_HALOS, parallel.OUTPUT_HALOS))
 
     main_stream = torch.cuda.current_stream()
-    with wrf.Patch(pg, device=local) as patch:
+    with wrf.Patch(pg, device=local, dtype=np.float64 if r8 else np.float32) as patch:
         patch.set_stream(main_stream.cuda_stream)
-        patch.set_scalars(*cases.SCALARS_3KM)
+        patch.set_scalars(*scalars)
         patch.upload(f)
         if args.mode == "fused":
             timeouts = run_fused(patch, decomp, rank, dev, args.steps, c_uv, not args.no_graph)
@@ -96,7 +126,10 @@ def main():
         patch.download(f, names=cases.OUTPUTS + ("u", "v"))
         dist.barrier()                               # nobody unmaps a neighbour that is still storing into it
 
-    want = cases.oracle_loop(G, whole, cases.SCALARS_3KM, args.steps, c=c_uv)
+    if r8:
+        want = checker_loop64(G, whole, scalars, args.steps, c_uv)
+    else:
+        want = cases.oracle_loop(G, whole, cases.SCALARS_3KM, args.steps, c=c_uv)
     mism = cases.patch_mismatches(f, want, G, pg, ext)
     for n, nb in mism.items():
         print(f"rank {rank}: field {n}: {nb} values differ", flush=True)
@@ -106,8 +139,10 @@ def main():
     t = torch.tensor([bad], device=dev, dtype=torch.int64)
     dist.all_reduce(t)
     if rank == 0:
-        print(f"multi_gpu_check [{args.mode}] {px}x{py} on {nx}x{ny}x{nz}, {args.steps} steps: "
-              f"{'BIT-IDENTICAL to the single-domain oracle' if t.item() == 0 else str(t.item()) + ' MISMATCHES'}", flush=True)
+        ref = "binary64 checker" if r8 else "oracle"
+        mode = f"{args.mode}, float64" if r8 else args.mode
+        print(f"multi_gpu_check [{mode}] {px}x{py} on {nx}x{ny}x{nz}, {args.steps} steps: "
+              f"{f'BIT-IDENTICAL to the single-domain {ref}' if t.item() == 0 else str(t.item()) + ' MISMATCHES'}", flush=True)
     dist.destroy_process_group()
     sys.exit(0 if t.item() == 0 else 1)
 

@@ -74,6 +74,10 @@ PROTOTYPES = {
     "wrfb200_upload_state": (C.c_int, [_P, _P, _P, _P]),
     "wrfb200_set_uv": (C.c_int, [_P, _P, _P]),
     "wrfb200_download_outputs": (C.c_int, [_P] + [C.c_int] * 6 + [_P] * 7),
+    "wrfb200_upload_constants_r8": (C.c_int, [_P] + [_P] * 17),
+    "wrfb200_upload_state_r8": (C.c_int, [_P, _P, _P, _P]),
+    "wrfb200_set_uv_r8": (C.c_int, [_P, _P, _P]),
+    "wrfb200_download_outputs_r8": (C.c_int, [_P] + [C.c_int] * 6 + [_P] * 7),
     "wrfb200_last_kernel": (C.c_int, [_P, C.POINTER(C.c_int)]),
     "wrfb200_create": (C.c_int, [C.POINTER(_P), C.POINTER(Domain), C.c_int, C.c_int]),
     "wrfb200_destroy": (C.c_int, [_P]),
@@ -101,6 +105,7 @@ PROTOTYPES = {
     "wrfb200_pack_halo": (C.c_int, [_P, C.c_int, C.c_int, C.c_int] + [C.c_int] * 4 + [_P]),
     "wrfb200_unpack_halo": (C.c_int, [_P, C.c_int, C.c_int, C.c_int] + [C.c_int] * 4 + [_P]),
     "wrfb200_standin_advance_uv": (C.c_int, [_P, C.c_int, C.c_float] + [C.c_int] * 4),
+    "wrfb200_standin_advance_uv_r8": (C.c_int, [_P, C.c_int, C.c_double] + [C.c_int] * 4),
     "wrfb200_comm_info_bytes": (C.c_int, []),
     "wrfb200_comm_init": (C.c_int, [_P, C.c_int, C.c_int, C.c_int] + [C.c_int] * 4 + [_P]),
     "wrfb200_comm_connect": (C.c_int, [_P, _P, C.c_int]),
@@ -112,6 +117,9 @@ PROTOTYPES = {
     "wrfb200_comm_standin_advance_uv": (C.c_int, [_P, C.c_float]),
     "wrfb200_comm_loop": (C.c_int, [_P, C.c_int, C.c_int, C.c_float, C.c_int]),
     "wrfb200_comm_status": (C.c_int, [_P, C.POINTER(C.c_int), C.POINTER(C.c_long)]),
+    "wrfb200_comm_init_r8": (C.c_int, [_P, C.c_int, C.c_int, C.c_int] + [C.c_int] * 4 + [_P]),
+    "wrfb200_comm_standin_advance_uv_r8": (C.c_int, [_P, C.c_double]),
+    "wrfb200_comm_loop_r8": (C.c_int, [_P, C.c_int, C.c_int, C.c_double, C.c_int]),
     "wrfb200_bounds": (C.c_int, [C.c_int] * 13 + [C.POINTER(C.c_int)] * 6),
     "wrfb200_synth_field": (C.c_int, [C.c_int, C.c_uint64, C.POINTER(Domain), C.c_float, _P]),
     "wrfb200_compare": (C.c_int, [_P, _P, C.c_long, C.POINTER(CompareResult)]),

@@ -186,7 +186,8 @@ class Patch:
     """Device-resident state of one patch (one rank): wrfb200_create / upload / step / download.
 
     ``dtype`` np.float64 (or torch.float64) makes a real*8 patch (wrfb200_create_r8): fields are float64 and the
-    step runs in binary64.  The multi-GPU, halo, stand-in and resident-bundle verbs are binary32 only."""
+    step runs in binary64.  Every verb with a precision calls the C verb of the patch's precision (the ``_r8``
+    entry points for float64), the fused multi-GPU verbs included; halo pack / unpack are binary32 only."""
 
     def __init__(self, grid: Grid, device: int = -1, allocate: bool = True, stream: Optional[int] = None,
                  dtype=np.float32):
@@ -271,22 +272,23 @@ class Patch:
 
     def upload_constants(self, fields: Dict[str, np.ndarray]):
         """Once per RK sub-step: everything advance_mu_t reads and nobody changes inside the acoustic loop."""
-        ptrs = [C.c_void_p(_ptr(fields[n])) if n in fields else None for n in self.CONSTANTS]
-        check(lib().wrfb200_upload_constants(self._h, *ptrs))
+        ptrs = [C.c_void_p(_ptr(fields[n], self.dtype)) if n in fields else None for n in self.CONSTANTS]
+        check(self._fn("wrfb200_upload_constants")(self._h, *ptrs))
 
     def upload_state(self, fields: Dict[str, np.ndarray]):
         """Once per RK sub-step: the state the loop starts from (ww, t, mu)."""
-        check(lib().wrfb200_upload_state(self._h, *[C.c_void_p(_ptr(fields[n])) for n in ("ww", "t", "mu")]))
+        check(self._fn("wrfb200_upload_state")(self._h, *[C.c_void_p(_ptr(fields[n], self.dtype))
+                                                          for n in ("ww", "t", "mu")]))
 
     def set_uv(self, u, v):
         """Every small step: what advance_uv changed."""
-        check(lib().wrfb200_set_uv(self._h, C.c_void_p(_ptr(u)), C.c_void_p(_ptr(v))))
+        check(self._fn("wrfb200_set_uv")(self._h, C.c_void_p(_ptr(u, self.dtype)), C.c_void_p(_ptr(v, self.dtype))))
 
     def download_outputs(self, fields: Dict[str, np.ndarray], tile: Optional[Grid] = None, sync: bool = True):
         """Every small step: exactly the cells the routine writes, into the caller's arrays."""
         g = tile or self.grid
-        ptrs = [C.c_void_p(_ptr(fields[n])) if n in fields else None for n in OUTPUT_FIELDS]
-        check(lib().wrfb200_download_outputs(self._h, g.its, g.ite, g.jts, g.jte, g.kts, g.kte, *ptrs))
+        ptrs = [C.c_void_p(_ptr(fields[n], self.dtype)) if n in fields else None for n in OUTPUT_FIELDS]
+        check(self._fn("wrfb200_download_outputs")(self._h, g.its, g.ite, g.jts, g.jte, g.kts, g.kte, *ptrs))
         if sync:
             self.sync()
 
@@ -322,14 +324,14 @@ class Patch:
                                         C.c_void_p(_ptr(device_buf))))
 
     def standin_advance_uv(self, field: str, c: float, i0, i1, j0, j1):
-        check(lib().wrfb200_standin_advance_uv(self._h, FIELD_ID[field], float(c), i0, i1, j0, j1))
+        check(self._fn("wrfb200_standin_advance_uv")(self._h, FIELD_ID[field], float(c), i0, i1, j0, j1))
 
     # ---- multi-GPU: halo exchange fused into the kernels over peer-mapped memory (csrc/comm.cu) ----
     def comm_init(self, px: int, py: int, rank: int, ips, ipe, jps, jpe) -> bytes:
         """-> this rank's opaque info blob; all-gather the blobs in rank order and pass them to comm_connect."""
         n = lib().wrfb200_comm_info_bytes()
         buf = C.create_string_buffer(n)
-        check(lib().wrfb200_comm_init(self._h, px, py, rank, ips, ipe, jps, jpe, buf))
+        check(self._fn("wrfb200_comm_init")(self._h, px, py, rank, ips, ipe, jps, jpe, buf))
         return buf.raw
 
     def comm_connect(self, infos) -> None:
@@ -354,10 +356,10 @@ class Patch:
         check(lib().wrfb200_comm_step(self._h))
 
     def comm_standin_advance_uv(self, c: float):
-        check(lib().wrfb200_comm_standin_advance_uv(self._h, float(c)))
+        check(self._fn("wrfb200_comm_standin_advance_uv")(self._h, float(c)))
 
     def comm_loop(self, nsteps: int, standin: bool = False, c: float = 0.0, graph: bool = True):
-        check(lib().wrfb200_comm_loop(self._h, int(nsteps), int(bool(standin)), float(c), int(bool(graph))))
+        check(self._fn("wrfb200_comm_loop")(self._h, int(nsteps), int(bool(standin)), float(c), int(bool(graph))))
 
     def comm_status(self):
         """(flag_timeouts, steps_done) after synchronising the stream."""

@@ -78,7 +78,8 @@ struct AmtFields {
     int k0;             // memory index of level kts
     int nk;             // number of computed levels: k_start..k_end = kts..kte-1
     int kdim, jdim;     // memory extents in k and j (jstride == pitch * kdim)
-    AmtHalo halo;       // fused multi-GPU halo exchange (enabled == 0 on a single GPU; always 0 for double)
+    AmtHalo halo;       // fused multi-GPU halo exchange (enabled == 0 on a single GPU); for double its peer
+                        // pointers address doubles (pitches stay in elements)
 };
 struct AmtParams : AmtFields<float> {};
 struct AmtParamsR8 : AmtFields<double> {};
@@ -158,6 +159,19 @@ inline cudaError_t amt_raise_smem_limit(K kernel, bool (&done)[64])
     return e;
 }
 
+// Dispatch order of the block rows in a fused multi-GPU launch: south row first (its blocks push v to the south
+// neighbour before anything else), NORTH ROW SECOND, then the rest.  The north-row blocks are the ones that wait
+// for the north neighbour's v (pushed by ITS first blocks, i.e. at about the same time) and the ones whose
+// completion tells that neighbour "step done": run early, neither their wait nor their system-scope fence and
+// flag store sit at the end of the launch, and the neighbour's write-after-read guard is released a whole
+// launch ahead of its use.  Used by the binary32 pipe kernels and the fused real*8 tile kernel alike.
+template <class T>
+__device__ __forceinline__ int north_row_second(const AmtFields<T> &p, const int by, const int nby)
+{
+    if (!p.halo.enabled || !p.halo.north_second || !p.halo.out_flag_to_north || nby < 3) return by;
+    return by == 0 ? 0 : (by == 1 ? nby - 1 : by - 1);
+}
+
 // Launchers (defined in the kernel translation units).
 bool amt_pipe_plan(const AmtParams &p, int slots, long long out[10]);   // host-only launch description
 cudaError_t amt_pipe_preload();                                         // load all kernels of amt_pipe.cu (see there)
@@ -186,3 +200,5 @@ cudaError_t amt_launch_pipe(const AmtParams &p, const AmtTmaMaps &maps, cudaStre
 cudaError_t amt_launch_column(const AmtParamsR8 &p, cudaStream_t stream);
 cudaError_t amt_launch_tile(const AmtParamsR8 &p, cudaStream_t stream);
 bool amt_tile_supported(const AmtParamsR8 &p);
+cudaError_t amt_launch_tile_fused(const AmtParamsR8 &p, cudaStream_t stream);    // p.halo.enabled: multi-GPU
+cudaError_t amt_tile_r8_preload();                                               // see amt_pipe_preload

@@ -128,6 +128,12 @@ int wrfb200_make_params(const wrfb200_handle *h, int its, int ite, int jts, int 
     return make_params(h, its, ite, jts, jte, kts, kte, out, empty);
 }
 
+int wrfb200_make_params(const wrfb200_handle *h, int its, int ite, int jts, int jte, int kts, int kte,
+                AmtParamsR8 *out, bool *empty)
+{
+    return make_params(h, its, ite, jts, jte, kts, kte, out, empty);
+}
+
 namespace {
 
 int launch(wrfb200_handle *h, const AmtParams &p, cudaStream_t s, int kernel)
@@ -170,7 +176,14 @@ int launch(wrfb200_handle *h, const AmtParamsR8 &p, cudaStream_t s, int kernel)
 {
     cudaError_t e;
     int ran = kernel;
-    if (kernel == WRFB200_KERNEL_PIPE) {
+    if (p.halo.enabled) {
+        // a multi-GPU rank (comm.cu): the tile kernel with the halo exchange fused in; wrfb200_comm_init_r8 has
+        // checked that the patch's layout and level count suit it
+        if (!amt_tile_supported(p))
+            return fail(WRFB200_ERR_UNSUPPORTED, "the fused real*8 exchange needs the tile kernel's layout and nk <= 220 (nk=%d)", p.nk);
+        e = amt_launch_tile_fused(p, s);
+        ran = WRFB200_KERNEL_TILE;
+    } else if (kernel == WRFB200_KERNEL_PIPE) {
         return fail(WRFB200_ERR_UNSUPPORTED, "the pipe kernel is binary32 only; a real*8 handle runs the tile or column kernel");
     } else if (kernel == WRFB200_KERNEL_COLUMN) {
         e = amt_launch_column(p, s);
@@ -227,6 +240,11 @@ int wrfb200_require_r4(const wrfb200_handle *h, const char *what)
 }
 
 int wrfb200_launch_params(wrfb200_handle *h, const AmtParams &p, cudaStream_t s, int kernel)
+{
+    return launch(h, p, s, kernel);
+}
+
+int wrfb200_launch_params(wrfb200_handle *h, const AmtParamsR8 &p, cudaStream_t s, int kernel)
 {
     return launch(h, p, s, kernel);
 }
@@ -668,6 +686,61 @@ extern "C" int wrfb200_download_outputs(wrfb200_handle *h, int its, int ite, int
     float *ptr[] = {ww, t, t_ave, mu, muave, muts, mudf};
     for (int x = 0; x < 7; ++x)
         if (ptr[x]) if (int rc = wrfb200_download_range(h, ids[x], ptr[x], is, ie, ks, ke, js, je)) return rc;
+    return WRFB200_OK;
+}
+
+// The same four verbs for real*8 handles (WRF built with -r8): double arrays, the _r8 copies.
+extern "C" int wrfb200_upload_constants_r8(
+    wrfb200_handle *h, const double *ww_1, const double *u_1, const double *v_1, const double *t_1, const double *ft,
+    const double *mut, const double *muu, const double *muv, const double *mu_tend,
+    const double *msfuy, const double *msfvx_inv, const double *msftx, const double *msfty,
+    const double *dnw, const double *fnm, const double *fnp, const double *rdnw)
+{
+    if (!h) return fail(WRFB200_ERR_INVALID_ARG, "null handle");
+    if (h->esize != 8) return wrong_precision(h, "wrfb200_upload_constants_r8");
+    const int ids[] = {WRFB200_WW_1, WRFB200_U_1, WRFB200_V_1, WRFB200_T_1, WRFB200_FT, WRFB200_MUT, WRFB200_MUU,
+                       WRFB200_MUV, WRFB200_MU_TEND, WRFB200_MSFUY, WRFB200_MSFVX_INV, WRFB200_MSFTX, WRFB200_MSFTY,
+                       WRFB200_DNW, WRFB200_FNM, WRFB200_FNP, WRFB200_RDNW};
+    const double *ptr[] = {ww_1, u_1, v_1, t_1, ft, mut, muu, muv, mu_tend, msfuy, msfvx_inv, msftx, msfty, dnw, fnm, fnp, rdnw};
+    for (int x = 0; x < 17; ++x)
+        if (ptr[x]) if (int rc = wrfb200_upload_r8(h, ids[x], ptr[x])) return rc;
+    return WRFB200_OK;
+}
+
+extern "C" int wrfb200_upload_state_r8(wrfb200_handle *h, const double *ww, const double *t, const double *mu)
+{
+    if (!h) return fail(WRFB200_ERR_INVALID_ARG, "null handle");
+    if (h->esize != 8) return wrong_precision(h, "wrfb200_upload_state_r8");
+    if (ww) if (int rc = wrfb200_upload_r8(h, WRFB200_WW, ww)) return rc;
+    if (t) if (int rc = wrfb200_upload_r8(h, WRFB200_T, t)) return rc;
+    if (mu) if (int rc = wrfb200_upload_r8(h, WRFB200_MU, mu)) return rc;
+    return WRFB200_OK;
+}
+
+extern "C" int wrfb200_set_uv_r8(wrfb200_handle *h, const double *u, const double *v)
+{
+    if (!h) return fail(WRFB200_ERR_INVALID_ARG, "null handle");
+    if (h->esize != 8) return wrong_precision(h, "wrfb200_set_uv_r8");
+    if (u) if (int rc = wrfb200_upload_r8(h, WRFB200_U, u)) return rc;
+    if (v) if (int rc = wrfb200_upload_r8(h, WRFB200_V, v)) return rc;
+    return WRFB200_OK;
+}
+
+extern "C" int wrfb200_download_outputs_r8(wrfb200_handle *h, int its, int ite, int jts, int jte, int kts, int kte,
+                                           double *ww, double *t, double *t_ave, double *mu, double *muave,
+                                           double *muts, double *mudf)
+{
+    if (!h) return fail(WRFB200_ERR_INVALID_ARG, "null handle");
+    if (h->esize != 8) return wrong_precision(h, "wrfb200_download_outputs_r8");
+    const wrfb200_domain &d = h->dom;
+    int is, ie, js, je, ks, ke;
+    wrfb200_bounds(d.periodic_x, d.specified, d.nested, d.ids, d.ide, d.jds, d.jde,
+                   its, ite, jts, jte, kts, kte, &is, &ie, &js, &je, &ks, &ke);
+    if (is > ie || js > je || ks > ke) return WRFB200_OK;
+    const int ids[] = {WRFB200_WW, WRFB200_T, WRFB200_T_AVE, WRFB200_MU, WRFB200_MUAVE, WRFB200_MUTS, WRFB200_MUDF};
+    double *ptr[] = {ww, t, t_ave, mu, muave, muts, mudf};
+    for (int x = 0; x < 7; ++x)
+        if (ptr[x]) if (int rc = wrfb200_download_range_r8(h, ids[x], ptr[x], is, ie, ks, ke, js, je)) return rc;
     return WRFB200_OK;
 }
 

@@ -34,6 +34,10 @@ struct wrfb200_handle {
 int wrfb200_make_params(const wrfb200_handle *h, int its, int ite, int jts, int jte, int kts, int kte,
                         AmtParams *out, bool *empty);
 int wrfb200_launch_params(wrfb200_handle *h, const AmtParams &p, cudaStream_t s, int kernel);
+// ... and their real*8 twins (a block with p.halo.enabled runs the fused tile kernel whatever `kernel` says)
+int wrfb200_make_params(const wrfb200_handle *h, int its, int ite, int jts, int jte, int kts, int kte,
+                        AmtParamsR8 *out, bool *empty);
+int wrfb200_launch_params(wrfb200_handle *h, const AmtParamsR8 &p, cudaStream_t s, int kernel);
 // comm.cu: called by wrfb200_destroy
 void wrfb200_comm_release(wrfb200_handle *h);
 

@@ -14,7 +14,8 @@
 //         advance_mu_t kernel itself before they start; the u west column (read at i+1, :145-146; only for
 //         px > 1) by the small kernel `push_kernel`,
 //       - mu, muts, mudf east column / north row (what the neighbour's next advance_uv reads) by the
-//         advance_mu_t kernel itself, from the scan thread that has just computed them (amt_pipe.cu),
+//         advance_mu_t kernel itself, from the scan thread that has just computed them (amt_pipe.cu; real*8:
+//         amt_tile_r8.cu),
 //       - the loop constants u_1, muu, msfuy, v_1, muv, msfvx_inv, t_1 once per RK sub-step;
 //   * orders everything with monotonically increasing epoch flags in device memory (st.release.sys /
 //     ld.acquire.sys): only the blocks of advance_mu_t that own the patch's east column / north row wait
@@ -35,6 +36,11 @@
 //   out_from_west / out_from_south = n : the west / south neighbour's blocks that own its east column / north
 //                                       row have all finished step n: its mu, muts, mudf edges are in my halo AND
 //                                       it no longer reads the u / v halo I filled for step n
+//
+// Real*8 ranks (wrfb200_create_r8 + wrfb200_comm_init_r8) run the same protocol with the same flags: the step is
+// the fused double2 tile kernel (amt_tile_kernel_r8_fused, amt_tile_r8.cu), the peer addresses are computed with
+// the element size, and push_kernel moves double edges as pairs of 4-byte words.  Both ranks of a pair must hold
+// the same precision (checked at connect).
 #include <unistd.h>
 
 #include <cstdint>
@@ -67,6 +73,7 @@ struct CommInfo {
     uint32_t magic;
     int rank, px, py;
     int pid, device;
+    int esize;                       // bytes per element: 4 (binary32) or 8 (real*8); neighbours must agree
     uint64_t host_id;
     int ims, ime, jms, jme, kms, kme;
     int ips, ipe, jps, jpe;
@@ -152,7 +159,7 @@ struct wrfb200_comm {
     AmtHalo halo{};
     std::vector<std::string> opened;           // keys into ipc_cache()
     struct LoopGraph { cudaGraphExec_t exec; long launches; };
-    std::map<std::tuple<int, int, unsigned>, LoopGraph> graphs;         // (nsteps, standin, bits of c)
+    std::map<std::tuple<int, int, unsigned long long>, LoopGraph> graphs;   // (nsteps, standin, bits of c)
 };
 
 namespace {
@@ -264,10 +271,19 @@ __global__ void barrier_kernel(const __grid_constant__ BarrierArgs a)
 // ---------------------------------------------------------------------------------------------------
 // host helpers
 // ---------------------------------------------------------------------------------------------------
-int need_comm(wrfb200_handle *h, bool connected)
+// `verb` is the calling entry point.  typed: 4 for the verbs with a float argument, 8 for the _r8 verbs, 0 for the
+// verbs without a floating-point argument, which serve a real*8 handle once wrfb200_comm_init_r8 made its comm state.
+int need_comm(wrfb200_handle *h, bool connected, const char *verb, int typed = 0)
 {
     if (!h) return wrfb200_fail(WRFB200_ERR_INVALID_ARG, "null handle");
-    if (int rc = wrfb200_require_r4(h, "multi-GPU halo exchange (wrfb200_comm_*)")) return rc;
+    if (typed == 8 && h->esize != 8)
+        return wrfb200_fail(WRFB200_ERR_STATE, "%s: this is a real*4 handle (created by wrfb200_create); use the "
+                            "binary32 verb without the _r8 suffix", verb);
+    if (typed == 4)
+        if (int rc = wrfb200_require_r4(h, verb)) return rc;
+    if (!h->comm && h->esize == 8)
+        return wrfb200_fail(WRFB200_ERR_UNSUPPORTED, "%s: the state of wrfb200_comm_init is binary32 only; a real*8 "
+                            "handle needs wrfb200_comm_init_r8 first", verb);
     if (!h->comm) return wrfb200_fail(WRFB200_ERR_STATE, "wrfb200_comm_init has not been called on this handle");
     if (connected && !h->comm->connected) return wrfb200_fail(WRFB200_ERR_STATE, "wrfb200_comm_connect has not been called");
     return WRFB200_OK;
@@ -289,9 +305,11 @@ cudaError_t launch_push(const PushArgs &a, cudaStream_t s)
 }
 
 // The box of `field` that goes to the neighbour on `side`: this rank's edge column / row of the patch,
-// addressed in both memories by its Fortran indices.
+// addressed in both memories by its Fortran indices.  Boxes count 4-byte words: push_kernel moves a real*8 edge as
+// pairs of words, bit for bit, with the extents and strides doubled.
 Box edge_box(const wrfb200_handle *h, const Peer &pr, int field, int side)
 {
+    const int w = h->esize / 4;
     const wrfb200_comm *c = h->comm;
     const wrfb200_domain &d = h->dom;
     const CommInfo &q = pr.info;
@@ -307,10 +325,10 @@ Box edge_box(const wrfb200_handle *h, const Peer &pr, int field, int side)
     default:            j0 = j1 = c->jpe; i0 = c->ips; i1 = c->ipe; break;
     }
     Box b{};
-    b.src = h->d[field] + (long long)(j0 - d.jms) * sj + (i0 - d.ims);
-    b.dst = pr.f[field] + (long long)(j0 - q.jms) * dj + (i0 - q.ims);
-    b.sp = sp; b.sj = sj; b.dp = dp; b.dj = dj;
-    b.ni = i1 - i0 + 1; b.nk = nk; b.nj = j1 - j0 + 1;
+    b.src = h->d[field] + ((long long)(j0 - d.jms) * sj + (i0 - d.ims)) * w;
+    b.dst = pr.f[field] + ((long long)(j0 - q.jms) * dj + (i0 - q.ims)) * w;
+    b.sp = sp * w; b.sj = sj * w; b.dp = dp * w; b.dj = dj * w;
+    b.ni = (i1 - i0 + 1) * w; b.nk = nk; b.nj = j1 - j0 + 1;
     return b;
 }
 
@@ -402,7 +420,8 @@ int enqueue_push_uv(wrfb200_handle *h, cudaStream_t s, unsigned index)
         a.sig0 = w.flags + F_UV_E;
     }
     // (the v south row goes to the south neighbour from inside advance_mu_t itself: its south-row blocks push it
-    // before they start, amt_pipe.cu -- no separate launch for j-slab decompositions)
+    // before they start, amt_pipe.cu for binary32 and amt_tile_r8.cu for real*8 -- no separate launch for j-slab
+    // decompositions)
     if (a.nbox == 0) return WRFB200_OK;
     a.epoch = c->flags + F_EPOCH;
     a.index = index;
@@ -429,16 +448,23 @@ int enqueue_wait_outputs(wrfb200_handle *h, cudaStream_t s, unsigned done_index)
     return WRFB200_OK;
 }
 
-int enqueue_step(wrfb200_handle *h, cudaStream_t s, unsigned index)
+// binary32: the TMA pipe kernel; real*8: the fused tile kernel (amt_tile_r8.cu)
+template <class P>
+int enqueue_step_as(wrfb200_handle *h, cudaStream_t s, unsigned index)
 {
     wrfb200_comm *c = h->comm;
-    AmtParams p;
+    P p;
     bool empty = false;
     if (int rc = wrfb200_make_params(h, c->ips, c->ipe, c->jps, c->jpe, 1, h->dom.kde, &p, &empty)) return rc;
     if (empty) return wrfb200_fail(WRFB200_ERR_UNSUPPORTED, "rank %d: patch has no computed columns", c->rank);
     p.halo = c->halo;
     p.halo.step_index = index;
     return wrfb200_launch_params(h, p, s, WRFB200_KERNEL_PIPE);
+}
+
+int enqueue_step(wrfb200_handle *h, cudaStream_t s, unsigned index)
+{
+    return h->esize == 8 ? enqueue_step_as<AmtParamsR8>(h, s, index) : enqueue_step_as<AmtParams>(h, s, index);
 }
 
 int enqueue_epoch(wrfb200_handle *h, cudaStream_t s, unsigned nsteps)
@@ -452,20 +478,25 @@ int enqueue_epoch(wrfb200_handle *h, cudaStream_t s, unsigned nsteps)
     return WRFB200_OK;
 }
 
-int enqueue_standin(wrfb200_handle *h, cudaStream_t s, float cc, unsigned done_index)
+// cc: the caller's float (binary32 handle) or double (real*8 handle), exact in a double either way
+int enqueue_standin(wrfb200_handle *h, cudaStream_t s, double cc, unsigned done_index)
 {
     int ub[4], vb[4];
     standin_boxes(h, ub, vb);
     if (int rc = enqueue_wait_outputs(h, s, done_index)) return rc;          // the mudf halo the stand-in reads has arrived
     cudaStream_t keep = h->stream;
     h->stream = s;
-    int rc = wrfb200_standin_advance_uv(h, WRFB200_U, cc, ub[0], ub[1], ub[2], ub[3]);
-    if (rc == WRFB200_OK) rc = wrfb200_standin_advance_uv(h, WRFB200_V, cc, vb[0], vb[1], vb[2], vb[3]);
+    auto advance = [&](int field, const int *b) {
+        return h->esize == 8 ? wrfb200_standin_advance_uv_r8(h, field, cc, b[0], b[1], b[2], b[3])
+                             : wrfb200_standin_advance_uv(h, field, (float)cc, b[0], b[1], b[2], b[3]);
+    };
+    int rc = advance(WRFB200_U, ub);
+    if (rc == WRFB200_OK) rc = advance(WRFB200_V, vb);
     h->stream = keep;
     return rc;
 }
 
-int enqueue_loop(wrfb200_handle *h, cudaStream_t s, int nsteps, int standin, float cc)
+int enqueue_loop(wrfb200_handle *h, cudaStream_t s, int nsteps, int standin, double cc)
 {
     for (int n = 0; n < nsteps; ++n) {
         if (int rc = enqueue_push_uv(h, s, (unsigned)n)) return rc;
@@ -500,11 +531,11 @@ void wrfb200_comm_release(wrfb200_handle *h)
 
 extern "C" int wrfb200_comm_info_bytes(void) { return WRFB200_COMM_INFO_BYTES; }
 
-extern "C" int wrfb200_comm_init(wrfb200_handle *h, int px, int py, int rank,
-                                 int ips, int ipe, int jps, int jpe, void *info_out)
+namespace {
+
+// wrfb200_comm_init / _init_r8 after the precision checks
+int comm_init(wrfb200_handle *h, int px, int py, int rank, int ips, int ipe, int jps, int jpe, void *info_out)
 {
-    if (!h || !info_out) return wrfb200_fail(WRFB200_ERR_INVALID_ARG, "null argument");
-    if (int rc = wrfb200_require_r4(h, "multi-GPU halo exchange (wrfb200_comm_*)")) return rc;
     if (px < 1 || py < 1 || rank < 0 || rank >= px * py)
         return wrfb200_fail(WRFB200_ERR_INVALID_ARG, "bad process grid %dx%d / rank %d", px, py, rank);
     const wrfb200_domain &d = h->dom;
@@ -546,7 +577,7 @@ extern "C" int wrfb200_comm_init(wrfb200_handle *h, int px, int py, int rank,
     CommInfo q{};
     q.magic = kMagic;
     q.rank = rank; q.px = px; q.py = py;
-    q.pid = (int)getpid(); q.device = h->device; q.host_id = host_id();
+    q.pid = (int)getpid(); q.device = h->device; q.esize = h->esize; q.host_id = host_id();
     q.ims = d.ims; q.ime = d.ime; q.jms = d.jms; q.jme = d.jme; q.kms = d.kms; q.kme = d.kme;
     q.ips = ips; q.ipe = ipe; q.jps = jps; q.jpe = jpe;
     q.pitch3 = h->pitch3; q.pitch2 = h->pitch2;
@@ -568,9 +599,45 @@ extern "C" int wrfb200_comm_init(wrfb200_handle *h, int px, int py, int rank,
     return WRFB200_OK;
 }
 
+}  // namespace
+
+extern "C" int wrfb200_comm_init(wrfb200_handle *h, int px, int py, int rank,
+                                 int ips, int ipe, int jps, int jpe, void *info_out)
+{
+    if (!h || !info_out) return wrfb200_fail(WRFB200_ERR_INVALID_ARG, "null argument");
+    if (int rc = wrfb200_require_r4(h, "multi-GPU halo exchange (wrfb200_comm_*)")) return rc;
+    return comm_init(h, px, py, rank, ips, ipe, jps, jpe, info_out);
+}
+
+extern "C" int wrfb200_comm_init_r8(wrfb200_handle *h, int px, int py, int rank,
+                                    int ips, int ipe, int jps, int jpe, void *info_out)
+{
+    if (!h || !info_out) return wrfb200_fail(WRFB200_ERR_INVALID_ARG, "null argument");
+    if (h->esize != 8)
+        return wrfb200_fail(WRFB200_ERR_STATE, "wrfb200_comm_init_r8: this is a real*4 handle (created by "
+                            "wrfb200_create); use wrfb200_comm_init");
+    // every step runs the fused tile kernel: refuse a patch it cannot take now rather than at the first step.
+    // Handle-owned mirrors are 128-byte aligned with even pitches, so the level count is what can fail.
+    AmtParamsR8 p{};
+    auto F = [h](int f) { return reinterpret_cast<double *>(h->d[f]); };
+    p.ww = F(WRFB200_WW); p.ww_1 = F(WRFB200_WW_1); p.u = F(WRFB200_U); p.u_1 = F(WRFB200_U_1);
+    p.v = F(WRFB200_V); p.v_1 = F(WRFB200_V_1); p.t = F(WRFB200_T); p.t_1 = F(WRFB200_T_1);
+    p.t_ave = F(WRFB200_T_AVE); p.ft = F(WRFB200_FT); p.mu = F(WRFB200_MU); p.mut = F(WRFB200_MUT);
+    p.muave = F(WRFB200_MUAVE); p.muts = F(WRFB200_MUTS); p.muu = F(WRFB200_MUU); p.muv = F(WRFB200_MUV);
+    p.mudf = F(WRFB200_MUDF); p.mu_tend = F(WRFB200_MU_TEND); p.msfuy = F(WRFB200_MSFUY);
+    p.msfvx_inv = F(WRFB200_MSFVX_INV); p.msftx = F(WRFB200_MSFTX); p.msfty = F(WRFB200_MSFTY);
+    p.pitch = h->pitch3; p.jstride = h->pitch3 * (long long)h->kdim; p.pitch2 = h->pitch2;
+    p.nk = h->dom.kde - 1;                                      // levels 1 .. kde-1
+    if (!amt_tile_supported(p))
+        return wrfb200_fail(WRFB200_ERR_UNSUPPORTED, "the real*8 multi-GPU path runs the double2 tile kernel, which "
+                            "needs 16-byte aligned fields, pitches of an even number of doubles and at most 220 levels "
+                            "(this patch computes %d)", p.nk);
+    return comm_init(h, px, py, rank, ips, ipe, jps, jpe, info_out);
+}
+
 extern "C" int wrfb200_comm_connect(wrfb200_handle *h, const void *all_infos, int nranks)
 {
-    if (int rc = need_comm(h, false)) return rc;
+    if (int rc = need_comm(h, false, "wrfb200_comm_connect")) return rc;
     wrfb200_comm *c = h->comm;
     if (!all_infos || nranks != c->nranks)
         return wrfb200_fail(WRFB200_ERR_INVALID_ARG, "expected the info blobs of all %d ranks, in rank order", c->nranks);
@@ -583,8 +650,9 @@ extern "C" int wrfb200_comm_connect(wrfb200_handle *h, const void *all_infos, in
         CUC(cudaFuncGetAttributes(&fa, (const void *)wait_outputs_kernel));
         CUC(cudaFuncGetAttributes(&fa, (const void *)barrier_kernel));
         CUC(cudaFuncGetAttributes(&fa, (const void *)epoch_kernel));
-        CUC(amt_pipe_preload());
         CUC(wrfb200_halo_preload());
+        if (h->esize == 8) CUC(amt_tile_r8_preload());
+        else CUC(amt_pipe_preload());
     }
     const wrfb200_domain &d = h->dom;
     const int kdim = h->kdim;
@@ -596,6 +664,10 @@ extern "C" int wrfb200_comm_connect(wrfb200_handle *h, const void *all_infos, in
         const CommInfo &q = pr.info;
         if (q.magic != kMagic || q.rank != c->nbr[side] || q.px != c->px || q.py != c->py)
             return wrfb200_fail(WRFB200_ERR_INVALID_ARG, "info blob %d is not rank %d of a %dx%d grid", c->nbr[side], c->nbr[side], c->px, c->py);
+        if (q.esize != h->esize)
+            return wrfb200_fail(WRFB200_ERR_INVALID_ARG, "rank %d holds %s data and this rank %s: ranks of mixed "
+                                "precision are not supported", q.rank, q.esize == 8 ? "real*8" : "binary32",
+                                h->esize == 8 ? "real*8" : "binary32");
         if (q.kms != d.kms || q.kme - q.kms + 1 != kdim)
             return wrfb200_fail(WRFB200_ERR_INVALID_ARG, "rank %d has different vertical memory extents", q.rank);
         bool adjacent = false;
@@ -612,6 +684,9 @@ extern "C" int wrfb200_comm_connect(wrfb200_handle *h, const void *all_infos, in
         pr.present = true;
     }
 
+    // peer addresses: element offsets into the neighbour's arrays, scaled to 4-byte words (the kernels read the
+    // float pointers of AmtHalo as double pointers on a real*8 rank; pitches stay in elements)
+    const int w = h->esize / 4;
     AmtHalo hx{};
     hx.enabled = 1;
     hx.ipe_mem = c->ipe - d.ims;
@@ -622,7 +697,7 @@ extern "C" int wrfb200_comm_connect(wrfb200_handle *h, const void *all_infos, in
     if (so.present) {
         const CommInfo &q = so.info;
         // south neighbour's v at (my memory column 0, level 0, Fortran row jps = its north halo row)
-        hx.s_v = so.f[WRFB200_V] + (long long)(c->jps - q.jms) * (q.kme - q.kms + 1) * q.pitch3 + (d.ims - q.ims);
+        hx.s_v = so.f[WRFB200_V] + ((long long)(c->jps - q.jms) * (q.kme - q.kms + 1) * q.pitch3 + (d.ims - q.ims)) * w;
         hx.s_pitch3 = q.pitch3;
         hx.war_flag_south = c->flags + F_OUT_S;
         hx.uv_flag_to_south = so.flags + F_UV_N;
@@ -632,14 +707,14 @@ extern "C" int wrfb200_comm_connect(wrfb200_handle *h, const void *all_infos, in
     if (e.present) {
         const CommInfo &q = e.info;
         hx.uv_flag_east = c->flags + F_UV_E;
-        const long long o = (long long)(d.jms - q.jms) * q.pitch2 + (c->ipe - q.ims);    // my memory row 0, column ipe
+        const long long o = ((long long)(d.jms - q.jms) * q.pitch2 + (c->ipe - q.ims)) * w;  // my memory row 0, column ipe
         hx.e_mu = e.f[WRFB200_MU] + o; hx.e_muts = e.f[WRFB200_MUTS] + o; hx.e_mudf = e.f[WRFB200_MUDF] + o;
         hx.e_pitch2 = q.pitch2;
     }
     if (n.present) {
         const CommInfo &q = n.info;
         hx.uv_flag_north = c->flags + F_UV_N;
-        const long long o = (long long)(c->jpe - q.jms) * q.pitch2 + (d.ims - q.ims);    // row jpe, my memory column 0
+        const long long o = ((long long)(c->jpe - q.jms) * q.pitch2 + (d.ims - q.ims)) * w;  // row jpe, my memory column 0
         hx.n_mu = n.f[WRFB200_MU] + o; hx.n_muts = n.f[WRFB200_MUTS] + o; hx.n_mudf = n.f[WRFB200_MUDF] + o;
     }
     if (e.present) { hx.out_flag_to_east = e.flags + F_OUT_W; hx.east_counter = c->flags + F_EAST_DONE; }
@@ -660,7 +735,7 @@ extern "C" int wrfb200_comm_connect(wrfb200_handle *h, const void *all_infos, in
 
 extern "C" int wrfb200_comm_barrier(wrfb200_handle *h)
 {
-    if (int rc = need_comm(h, true)) return rc;
+    if (int rc = need_comm(h, true, "wrfb200_comm_barrier")) return rc;
     wrfb200_comm *c = h->comm;
     DevGuard g(h->device);
     BarrierArgs a{};
@@ -684,7 +759,7 @@ extern "C" int wrfb200_comm_barrier(wrfb200_handle *h)
 
 extern "C" int wrfb200_comm_push_constants(wrfb200_handle *h)
 {
-    if (int rc = need_comm(h, true)) return rc;
+    if (int rc = need_comm(h, true, "wrfb200_comm_push_constants")) return rc;
     wrfb200_comm *c = h->comm;
     DevGuard g(h->device);
     // (field, side the edge goes to): what advance_mu_t reads across a patch edge and nobody changes inside
@@ -716,21 +791,21 @@ extern "C" int wrfb200_comm_push_constants(wrfb200_handle *h)
 
 extern "C" int wrfb200_comm_push_uv(wrfb200_handle *h)
 {
-    if (int rc = need_comm(h, true)) return rc;
+    if (int rc = need_comm(h, true, "wrfb200_comm_push_uv")) return rc;
     DevGuard g(h->device);
     return enqueue_push_uv(h, h->stream, 0u);
 }
 
 extern "C" int wrfb200_comm_wait_outputs(wrfb200_handle *h)
 {
-    if (int rc = need_comm(h, true)) return rc;
+    if (int rc = need_comm(h, true, "wrfb200_comm_wait_outputs")) return rc;
     DevGuard g(h->device);
     return enqueue_wait_outputs(h, h->stream, 0u);     // the epoch already counts every completed step here
 }
 
 extern "C" int wrfb200_comm_step(wrfb200_handle *h)
 {
-    if (int rc = need_comm(h, true)) return rc;
+    if (int rc = need_comm(h, true, "wrfb200_comm_step")) return rc;
     DevGuard g(h->device);
     if (int rc = enqueue_step(h, h->stream, 0u)) return rc;
     return enqueue_epoch(h, h->stream, 1u);
@@ -738,21 +813,30 @@ extern "C" int wrfb200_comm_step(wrfb200_handle *h)
 
 extern "C" int wrfb200_comm_standin_advance_uv(wrfb200_handle *h, float c)
 {
-    if (int rc = need_comm(h, true)) return rc;
+    if (int rc = need_comm(h, true, "wrfb200_comm_standin_advance_uv", 4)) return rc;
     DevGuard g(h->device);
     return enqueue_standin(h, h->stream, c, 0u);
 }
 
-extern "C" int wrfb200_comm_loop(wrfb200_handle *h, int nsteps, int standin, float cc, int use_graph)
+extern "C" int wrfb200_comm_standin_advance_uv_r8(wrfb200_handle *h, double c)
 {
-    if (int rc = need_comm(h, true)) return rc;
+    if (int rc = need_comm(h, true, "wrfb200_comm_standin_advance_uv_r8", 8)) return rc;
+    DevGuard g(h->device);
+    return enqueue_standin(h, h->stream, c, 0u);
+}
+
+namespace {
+
+// wrfb200_comm_loop / _loop_r8 after the checks; cc is the caller's float or double, held exactly
+int comm_loop(wrfb200_handle *h, int nsteps, int standin, double cc, int use_graph)
+{
     if (nsteps <= 0) return WRFB200_OK;
     wrfb200_comm *c = h->comm;
     DevGuard g(h->device);
     if (!use_graph) return enqueue_loop(h, h->stream, nsteps, standin, cc);
-    unsigned cbits;
-    std::memcpy(&cbits, &cc, 4);
-    const auto key = std::make_tuple(nsteps, standin ? 1 : 0, standin ? cbits : 0u);
+    unsigned long long cbits;
+    std::memcpy(&cbits, &cc, 8);
+    const auto key = std::make_tuple(nsteps, standin ? 1 : 0, standin ? cbits : 0ull);
     auto it = c->graphs.find(key);
     if (it == c->graphs.end()) {
         cudaStream_t cs;
@@ -781,9 +865,23 @@ extern "C" int wrfb200_comm_loop(wrfb200_handle *h, int nsteps, int standin, flo
     return WRFB200_OK;
 }
 
+}  // namespace
+
+extern "C" int wrfb200_comm_loop(wrfb200_handle *h, int nsteps, int standin, float cc, int use_graph)
+{
+    if (int rc = need_comm(h, true, "wrfb200_comm_loop", 4)) return rc;
+    return comm_loop(h, nsteps, standin, cc, use_graph);
+}
+
+extern "C" int wrfb200_comm_loop_r8(wrfb200_handle *h, int nsteps, int standin, double cc, int use_graph)
+{
+    if (int rc = need_comm(h, true, "wrfb200_comm_loop_r8", 8)) return rc;
+    return comm_loop(h, nsteps, standin, cc, use_graph);
+}
+
 extern "C" int wrfb200_comm_status(wrfb200_handle *h, int *flag_timeouts, long *steps_done)
 {
-    if (int rc = need_comm(h, false)) return rc;
+    if (int rc = need_comm(h, false, "wrfb200_comm_status")) return rc;
     wrfb200_comm *c = h->comm;
     DevGuard g(h->device);
     unsigned host[F_WORDS];

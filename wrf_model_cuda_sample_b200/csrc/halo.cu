@@ -44,6 +44,21 @@ __global__ void standin_uv_kernel(float *f, const float *mudf, long long pitch, 
     }
 }
 
+// the same in binary64 (real*8 handles): one rounding per operation, as the float kernel
+__global__ void standin_uv_kernel_r8(double *f, const double *mudf, long long pitch, long long jstride,
+                                     long long pitch2, long long dshift, double c,
+                                     int i0, int j0, int ni, int nk, int nj)
+{
+    for (long long r = blockIdx.x; r < (long long)nk * nj; r += gridDim.x) {
+        const int k = (int)(r % nk);
+        const int j = (int)(r / nk);
+        double *row = f + (long long)(j0 + j) * jstride + (long long)k * pitch + i0;
+        const double *m = mudf + (long long)(j0 + j) * pitch2 + i0;
+        for (int i = threadIdx.x; i < ni; i += blockDim.x)
+            row[i] = __dadd_rn(row[i], __dmul_rn(c, __dsub_rn(m[i], m[i - dshift])));
+    }
+}
+
 // rows of `ni` floats, dense in `src`, to rows `pitch` floats apart in `dst`
 __global__ void repitch_rows_kernel(float *dst, const float *src, long long pitch, int ni, long long nrows)
 {
@@ -128,6 +143,7 @@ cudaError_t wrfb200_halo_preload()
 {
     cudaFuncAttributes a;
     cudaError_t e = cudaFuncGetAttributes(&a, (const void *)standin_uv_kernel);
+    if (e == cudaSuccess) e = cudaFuncGetAttributes(&a, (const void *)standin_uv_kernel_r8);
     if (e == cudaSuccess) e = cudaFuncGetAttributes(&a, (const void *)box_copy_kernel<true>);
     if (e == cudaSuccess) e = cudaFuncGetAttributes(&a, (const void *)box_copy_kernel<false>);
     return e;
@@ -145,10 +161,11 @@ extern "C" int wrfb200_unpack_halo(wrfb200_handle *h, int field, int side, int w
     return halo_copy(h, field, side, width, ips, ipe, jps, jpe, const_cast<float *>(device_buf), false);
 }
 
-extern "C" int wrfb200_standin_advance_uv(wrfb200_handle *h, int field, float c, int i0, int i1, int j0, int j1)
+namespace {
+
+// u or v += c * (one-sided mudf difference) over i0..i1 x j0..j1, in the handle's precision (checked by the callers)
+int standin(wrfb200_handle *h, int field, double c, int i0, int i1, int j0, int j1)
 {
-    if (!h) return wrfb200_fail(WRFB200_ERR_INVALID_ARG, "null handle");
-    if (int rc = wrfb200_require_r4(h, "wrfb200_standin_advance_uv")) return rc;
     if (field != WRFB200_U && field != WRFB200_V)
         return wrfb200_fail(WRFB200_ERR_INVALID_ARG, "stand-in update applies to u or v only");
     if (i0 > i1 || j0 > j1) return WRFB200_OK;
@@ -158,21 +175,42 @@ extern "C" int wrfb200_standin_advance_uv(wrfb200_handle *h, int field, float c,
         return wrfb200_fail(WRFB200_ERR_INVALID_ARG, "stand-in box outside memory");
     if (!h->d[field] || !h->d[WRFB200_MUDF]) return wrfb200_fail(WRFB200_ERR_STATE, "fields not allocated");
     const int ni = i1 - i0 + 1, nj = j1 - j0 + 1, nk = h->kdim;
-    const long long n = (long long)ni * nk * nj;
     int prev = -1;
     cudaGetDevice(&prev);
     if (prev != h->device) cudaSetDevice(h->device);
     const int threads = ni >= 256 ? 256 : (ni >= 64 ? 64 : 32);
     const long long rows = (long long)nk * nj;
     const unsigned blocks = (unsigned)(rows < 148 * 64 ? rows : 148 * 64);
-    (void)n;
+    const long long jstride = h->pitch3 * (long long)h->kdim, dshift = field == WRFB200_U ? 1 : h->pitch2;
     (void)cudaGetLastError();   // a launch status must not inherit a stale error of some earlier, unrelated call
-    standin_uv_kernel<<<blocks, threads, 0, h->stream>>>(
-        h->d[field], h->d[WRFB200_MUDF], h->pitch3, h->pitch3 * (long long)h->kdim, h->pitch2,
-        field == WRFB200_U ? 1 : h->pitch2, c, i0 - d.ims, j0 - d.jms, ni, nk, nj);
+    if (h->esize == 8)
+        standin_uv_kernel_r8<<<blocks, threads, 0, h->stream>>>(
+            reinterpret_cast<double *>(h->d[field]), reinterpret_cast<const double *>(h->d[WRFB200_MUDF]), h->pitch3,
+            jstride, h->pitch2, dshift, c, i0 - d.ims, j0 - d.jms, ni, nk, nj);
+    else
+        standin_uv_kernel<<<blocks, threads, 0, h->stream>>>(
+            h->d[field], h->d[WRFB200_MUDF], h->pitch3, jstride, h->pitch2, dshift, (float)c, i0 - d.ims, j0 - d.jms,
+            ni, nk, nj);
     cudaError_t e = cudaGetLastError();
     if (prev != h->device && prev >= 0) cudaSetDevice(prev);
     if (e != cudaSuccess) return wrfb200_fail(WRFB200_ERR_CUDA, "stand-in kernel launch failed: %s", cudaGetErrorString(e));
     h->launches += 1;
     return WRFB200_OK;
+}
+
+}  // namespace
+
+extern "C" int wrfb200_standin_advance_uv(wrfb200_handle *h, int field, float c, int i0, int i1, int j0, int j1)
+{
+    if (!h) return wrfb200_fail(WRFB200_ERR_INVALID_ARG, "null handle");
+    if (int rc = wrfb200_require_r4(h, "wrfb200_standin_advance_uv")) return rc;
+    return standin(h, field, c, i0, i1, j0, j1);
+}
+
+extern "C" int wrfb200_standin_advance_uv_r8(wrfb200_handle *h, int field, double c, int i0, int i1, int j0, int j1)
+{
+    if (!h) return wrfb200_fail(WRFB200_ERR_INVALID_ARG, "null handle");
+    if (h->esize != 8) return wrfb200_fail(WRFB200_ERR_STATE, "wrfb200_standin_advance_uv_r8: this is a real*4 handle "
+                                           "(created by wrfb200_create); use wrfb200_standin_advance_uv");
+    return standin(h, field, c, i0, i1, j0, j1);
 }

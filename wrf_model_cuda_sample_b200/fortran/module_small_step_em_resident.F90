@@ -34,8 +34,24 @@
 !           st = wrfb200_comm_push_constants( h )
 !           st = wrfb200_comm_loop( h, number_of_small_timesteps, 0_c_int, 0.0_c_float, 1_c_int )
 !
-! Source only: no Fortran compiler exists in the build image (INTEGRATION.md); tests/c_abi_harness.c and
-! tests/c_comm_harness.c drive exactly these entry points from C, and tests/test_cabi_host.py checks that every
+!       In a build configured with -r8 the same sequence uses the real*8 patch (section (B') below): create_r8,
+!       the _r8 uploads, comm_init_r8 and comm_loop_r8; connect, push_constants, push_uv, step and status are
+!       shared by both precisions.  All ranks must be built alike (connect rejects a rank of the other precision):
+!
+!           st = wrfb200_create_r8( h, dom, MOD(myrank, gpus_per_node), 1_c_int )
+!           st = wrfb200_set_scalars_r8( h, rdx, rdy, dts, epssm )
+!           st = wrfb200_upload_constants_r8( h, ww1, u_1, v_1, t_1, ft, mut, muu, muv, mu_tend, &
+!                                             msfuy, msfvx_inv, msftx, msfty, dnw, fnm, fnp, rdnw )
+!           st = wrfb200_upload_state_r8( h, ww, t_2, mu_2 )
+!           st = wrfb200_set_uv_r8( h, u_2, v_2 )
+!           st = wrfb200_comm_init_r8( h, px, py, myrank, ips, ipe, jps, jpe, C_LOC(mine) )
+!           CALL MPI_Allgather( mine, WRFB200_COMM_INFO_BYTES, MPI_BYTE, everyone, WRFB200_COMM_INFO_BYTES, MPI_BYTE, comm, ierr )
+!           st = wrfb200_comm_connect( h, C_LOC(everyone), nproc )
+!           st = wrfb200_comm_push_constants( h )
+!           st = wrfb200_comm_loop_r8( h, number_of_small_timesteps, 0_c_int, 0.0_c_double, 1_c_int )
+!
+! Source only: no Fortran compiler exists in the build image (INTEGRATION.md); tests/c_abi_harness.c,
+! tests/c_comm_harness.c and tests/c_comm_harness_r8.c drive exactly these entry points from C, and tests/test_cabi_host.py checks that every
 ! NAME= below is an exported symbol of the built library.
 !-----------------------------------------------------------------------------------------------------------
 MODULE module_small_step_em_resident
@@ -228,6 +244,46 @@ INTERFACE
       INTEGER(c_int) :: status
    END FUNCTION
 
+   FUNCTION wrfb200_upload_constants_r8(handle, ww_1, u_1, v_1, t_1, ft, mut, muu, muv, mu_tend,     &
+                                        msfuy, msfvx_inv, msftx, msfty, dnw, fnm, fnp, rdnw)        &
+            BIND(C, NAME="wrfb200_upload_constants_r8") RESULT(status)
+      IMPORT :: c_int, c_ptr, c_double
+      TYPE(c_ptr), VALUE :: handle
+      REAL(c_double), DIMENSION(*), INTENT(IN) :: ww_1, u_1, v_1, t_1, ft, mut, muu, muv, mu_tend
+      REAL(c_double), DIMENSION(*), INTENT(IN) :: msfuy, msfvx_inv, msftx, msfty, dnw, fnm, fnp, rdnw
+      INTEGER(c_int) :: status
+   END FUNCTION
+   FUNCTION wrfb200_upload_state_r8(handle, ww, t, mu) BIND(C, NAME="wrfb200_upload_state_r8") RESULT(status)
+      IMPORT :: c_int, c_ptr, c_double
+      TYPE(c_ptr), VALUE :: handle
+      REAL(c_double), DIMENSION(*), INTENT(IN) :: ww, t, mu
+      INTEGER(c_int) :: status
+   END FUNCTION
+   FUNCTION wrfb200_set_uv_r8(handle, u, v) BIND(C, NAME="wrfb200_set_uv_r8") RESULT(status)
+      IMPORT :: c_int, c_ptr, c_double
+      TYPE(c_ptr), VALUE :: handle
+      REAL(c_double), DIMENSION(*), INTENT(IN) :: u, v
+      INTEGER(c_int) :: status
+   END FUNCTION
+   FUNCTION wrfb200_download_outputs_r8(handle, its, ite, jts, jte, kts, kte,                         &
+                                        ww, t, t_ave, mu, muave, muts, mudf)                         &
+            BIND(C, NAME="wrfb200_download_outputs_r8") RESULT(status)
+      IMPORT :: c_int, c_ptr, c_double
+      TYPE(c_ptr), VALUE :: handle
+      INTEGER(c_int), VALUE :: its, ite, jts, jte, kts, kte
+      REAL(c_double), DIMENSION(*), INTENT(INOUT) :: ww, t, t_ave, mu, muave, muts, mudf
+      INTEGER(c_int) :: status
+   END FUNCTION
+   FUNCTION wrfb200_standin_advance_uv_r8(handle, field, c, i0, i1, j0, j1)                           &
+            BIND(C, NAME="wrfb200_standin_advance_uv_r8") RESULT(status)
+      IMPORT :: c_int, c_ptr, c_double
+      TYPE(c_ptr), VALUE :: handle
+      INTEGER(c_int), VALUE :: field
+      REAL(c_double), VALUE :: c
+      INTEGER(c_int), VALUE :: i0, i1, j0, j1
+      INTEGER(c_int) :: status
+   END FUNCTION
+
    ! ---- (C) one rank per GPU: halo exchange fused into the kernels over peer-mapped memory ----
    FUNCTION wrfb200_comm_init(handle, px, py, rank, ips, ipe, jps, jpe, info_out)                     &
             BIND(C, NAME="wrfb200_comm_init") RESULT(status)
@@ -282,6 +338,33 @@ INTERFACE
       TYPE(c_ptr), VALUE :: handle
       INTEGER(c_int), INTENT(OUT) :: flag_timeouts
       INTEGER(c_long), INTENT(OUT) :: steps_done
+      INTEGER(c_int) :: status
+   END FUNCTION
+
+   ! ---- (C') the same on real*8 ranks (-r8 builds); connect / barrier / push_* / wait_outputs / step / status
+   !      above serve them too
+   FUNCTION wrfb200_comm_init_r8(handle, px, py, rank, ips, ipe, jps, jpe, info_out)                  &
+            BIND(C, NAME="wrfb200_comm_init_r8") RESULT(status)
+      IMPORT :: c_int, c_ptr
+      TYPE(c_ptr), VALUE :: handle
+      INTEGER(c_int), VALUE :: px, py, rank, ips, ipe, jps, jpe
+      TYPE(c_ptr), VALUE :: info_out                      ! WRFB200_COMM_INFO_BYTES bytes
+      INTEGER(c_int) :: status
+   END FUNCTION
+   FUNCTION wrfb200_comm_standin_advance_uv_r8(handle, c) BIND(C, NAME="wrfb200_comm_standin_advance_uv_r8")  &
+            RESULT(status)
+      IMPORT :: c_int, c_ptr, c_double
+      TYPE(c_ptr), VALUE :: handle
+      REAL(c_double), VALUE :: c
+      INTEGER(c_int) :: status
+   END FUNCTION
+   FUNCTION wrfb200_comm_loop_r8(handle, nsteps, standin, c, use_graph) BIND(C, NAME="wrfb200_comm_loop_r8")   &
+            RESULT(status)
+      IMPORT :: c_int, c_ptr, c_double
+      TYPE(c_ptr), VALUE :: handle
+      INTEGER(c_int), VALUE :: nsteps, standin
+      REAL(c_double), VALUE :: c
+      INTEGER(c_int), VALUE :: use_graph
       INTEGER(c_int) :: status
    END FUNCTION
 END INTERFACE
