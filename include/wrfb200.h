@@ -37,9 +37,10 @@
  *   - Precision: the unsuffixed entry points take binary32 (`float`, WRF's default REAL = 4 bytes).  WRF built
  *     with -r8 (REAL = 8 bytes) calls the `_r8` entry points, which take `double` and compute every operation
  *     in binary64, in the same order.  A handle holds one precision, fixed by wrfb200_create / _create_r8;
- *     a verb typed for the other precision fails with WRFB200_ERR_STATE.  The multi-GPU, stand-in and
- *     resident-bundle verbs have `_r8` twins (wrfb200_comm_init_r8, ..., section 3b); their binary32 forms
- *     return WRFB200_ERR_UNSUPPORTED on an r8 handle.  The halo pack / unpack verbs (section 3) are binary32 only.
+ *     a verb typed for the other precision fails with WRFB200_ERR_STATE.  The multi-GPU, halo pack / unpack,
+ *     stand-in and resident-bundle verbs have `_r8` twins (wrfb200_pack_halo_r8, ..., section 3;
+ *     wrfb200_comm_init_r8, ..., section 3b); their binary32 forms return WRFB200_ERR_UNSUPPORTED on an r8 handle.
+ *     wrfb200_compare_r8 is the error report over doubles.
  */
 #ifndef WRFB200_H
 #define WRFB200_H
@@ -301,11 +302,19 @@ int wrfb200_last_kernel(wrfb200_handle *h, int *kernel);
  *    Buffer layout is [j][k][i] over the packed sub-box (i fastest); ips..ipe/jps..jpe is the patch.
  *    Buffer sizes: WEST/EAST width*nk*(jpe-jps+1) floats, SOUTH/NORTH (ipe-ips+1)*nk*width floats
  *    (nk = kme-kms+1 for 3-D fields, 1 for 2-D).
+ *    The caller moves the buffers between ranks with its own transport (MPI or NCCL send/recv, a device copy),
+ *    so ranks may sit on different hosts.  Asynchronous on the handle's stream.
  * ---------------------------------------------------------------------------------------------- */
 int wrfb200_pack_halo(wrfb200_handle *h, int field, int side, int width,
                       int ips, int ipe, int jps, int jpe, float *device_buf);
 int wrfb200_unpack_halo(wrfb200_handle *h, int field, int side, int width,
                         int ips, int ipe, int jps, int jpe, const float *device_buf);
+/* The same on a real*8 handle: same box, layout and sizes, counted in doubles.  On a real*4 handle they return
+ * WRFB200_ERR_STATE; the two verbs above return WRFB200_ERR_UNSUPPORTED on a real*8 one. */
+int wrfb200_pack_halo_r8(wrfb200_handle *h, int field, int side, int width,
+                         int ips, int ipe, int jps, int jpe, double *device_buf);
+int wrfb200_unpack_halo_r8(wrfb200_handle *h, int field, int side, int width,
+                           int ips, int ipe, int jps, int jpe, const double *device_buf);
 
 /* Deterministic stand-in for advance_uv (which in WRF updates u,v between two advance_mu_t calls but is
  * not part of the reference): field = WRFB200_U: u(i,k,j) += c*(mudf(i,j)-mudf(i-1,j));
@@ -400,6 +409,14 @@ typedef struct wrfb200_compare_result {
     long max_ulp;
 } wrfb200_compare_result;
 int wrfb200_compare(const float *a, const float *b, long n, wrfb200_compare_result *out);
+/* The same metrics over n doubles (real*8 fields), computed in binary64; the ulp distance is taken over the 64-bit
+ * ordered bit patterns (saturating at LONG_MAX, which only opposite-signed values near the infinities reach). */
+typedef struct wrfb200_compare_result_r8 {
+    long n, n_equal, n_different;
+    double max_rel, max_abs, rmse;
+    long max_ulp;
+} wrfb200_compare_result_r8;
+int wrfb200_compare_r8(const double *a, const double *b, long n, wrfb200_compare_result_r8 *out);
 
 /* Host-only description of the launch the TMA kernel makes for the tile its:ite x jts:jte of `dom` on a device with
  * `resident_blocks` resident blocks (0: a B200, 2 x 148): plan10 = {configuration TJ*10+STAGES, TJ, STAGES, tile

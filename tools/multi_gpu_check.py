@@ -8,9 +8,10 @@ Every rank runs the CUDA path on its patch (tile = patch, domain = global) and a
 between steps.  --mode fused (default): the one-cell ring moves by peer-mapped stores fused into the kernels
 (csrc/comm.cu; torch.distributed only all-gathers the bootstrap blobs).  --mode nccl: pack / NCCL send-recv /
 unpack through HaloExchanger, overlapped with the interior tile (the round-1 path).  Each rank then checks its
-patch BIT FOR BIT against the single-domain oracle loop.  --dtype float64 (fused mode only): real*8 patches
-(wrfb200_comm_init_r8 / wrfb200_comm_loop_r8) on float64 inputs with full 53-bit mantissas, checked against the
-binary64 checker loop (tests/r8_checkers.py).  Exit code 0 = every rank identical.
+patch BIT FOR BIT against the single-domain oracle loop.  --dtype float64: real*8 patches on float64 inputs with
+full 53-bit mantissas (fused: wrfb200_comm_init_r8 / wrfb200_comm_loop_r8; nccl: wrfb200_pack_halo_r8 /
+_unpack_halo_r8 around float64 NCCL send-recv), checked against the binary64 checker loop (tests/r8_checkers.py).
+Exit code 0 = every rank identical.
 """
 import argparse
 import os
@@ -90,8 +91,6 @@ def main():
     ap.add_argument("--dtype", choices=("float32", "float64"), default="float32")
     args = ap.parse_args()
     r8 = args.dtype == "float64"
-    if r8 and args.mode != "fused":
-        ap.error("--dtype float64 runs the fused mode only (the pack / unpack path is binary32)")
     rank, world = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"])
     local = int(os.environ.get("LOCAL_RANK", rank))
     torch.cuda.set_device(local)

@@ -43,6 +43,13 @@ class CompareResult(C.Structure):
                 ("max_ulp", C.c_long)]
 
 
+class CompareResultR8(C.Structure):
+    """struct wrfb200_compare_result_r8."""
+    _fields_ = [("n", C.c_long), ("n_equal", C.c_long), ("n_different", C.c_long),
+                ("max_rel", C.c_double), ("max_abs", C.c_double), ("rmse", C.c_double),
+                ("max_ulp", C.c_long)]
+
+
 class WrfB200Error(RuntimeError):
     def __init__(self, status: int, message: str):
         super().__init__(f"wrfb200 status {status}: {message}")
@@ -104,6 +111,8 @@ PROTOTYPES = {
     "wrfb200_launch_count": (C.c_int, [_P, C.POINTER(C.c_long)]),
     "wrfb200_pack_halo": (C.c_int, [_P, C.c_int, C.c_int, C.c_int] + [C.c_int] * 4 + [_P]),
     "wrfb200_unpack_halo": (C.c_int, [_P, C.c_int, C.c_int, C.c_int] + [C.c_int] * 4 + [_P]),
+    "wrfb200_pack_halo_r8": (C.c_int, [_P, C.c_int, C.c_int, C.c_int] + [C.c_int] * 4 + [_P]),
+    "wrfb200_unpack_halo_r8": (C.c_int, [_P, C.c_int, C.c_int, C.c_int] + [C.c_int] * 4 + [_P]),
     "wrfb200_standin_advance_uv": (C.c_int, [_P, C.c_int, C.c_float] + [C.c_int] * 4),
     "wrfb200_standin_advance_uv_r8": (C.c_int, [_P, C.c_int, C.c_double] + [C.c_int] * 4),
     "wrfb200_comm_info_bytes": (C.c_int, []),
@@ -123,6 +132,7 @@ PROTOTYPES = {
     "wrfb200_bounds": (C.c_int, [C.c_int] * 13 + [C.POINTER(C.c_int)] * 6),
     "wrfb200_synth_field": (C.c_int, [C.c_int, C.c_uint64, C.POINTER(Domain), C.c_float, _P]),
     "wrfb200_compare": (C.c_int, [_P, _P, C.c_long, C.POINTER(CompareResult)]),
+    "wrfb200_compare_r8": (C.c_int, [_P, _P, C.c_long, C.POINTER(CompareResultR8)]),
     "wrfb200_pipe_plan": (C.c_int, [C.POINTER(Domain)] + [C.c_int] * 7 + [C.POINTER(C.c_longlong)]),
     "wrfb200_last_error": (C.c_char_p, []),
     "wrfb200_version": (C.c_int, []),

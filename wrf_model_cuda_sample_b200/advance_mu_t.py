@@ -187,7 +187,7 @@ class Patch:
 
     ``dtype`` np.float64 (or torch.float64) makes a real*8 patch (wrfb200_create_r8): fields are float64 and the
     step runs in binary64.  Every verb with a precision calls the C verb of the patch's precision (the ``_r8``
-    entry points for float64), the fused multi-GPU verbs included; halo pack / unpack are binary32 only."""
+    entry points for float64), the fused multi-GPU and halo pack / unpack verbs included."""
 
     def __init__(self, grid: Grid, device: int = -1, allocate: bool = True, stream: Optional[int] = None,
                  dtype=np.float32):
@@ -315,13 +315,20 @@ class Patch:
         return n.value
 
     # ---- halo / stand-in ----
+    def _halo_buf(self, device_buf) -> C.c_void_p:
+        """Address of a halo buffer: a contiguous CUDA tensor of the patch's dtype."""
+        if not (hasattr(device_buf, "is_cuda") and device_buf.is_cuda and _dtype(device_buf) is self.dtype):
+            raise TypeError(f"halo buffers of a {np.dtype(self.dtype).name} patch must be CUDA tensors of that dtype, "
+                            f"got {getattr(device_buf, 'dtype', type(device_buf).__name__)}")
+        return C.c_void_p(_ptr(device_buf, self.dtype))
+
     def pack_halo(self, field: str, side: int, width: int, ips, ipe, jps, jpe, device_buf):
-        check(lib().wrfb200_pack_halo(self._h, FIELD_ID[field], side, width, ips, ipe, jps, jpe,
-                                      C.c_void_p(_ptr(device_buf))))
+        check(self._fn("wrfb200_pack_halo")(self._h, FIELD_ID[field], side, width, ips, ipe, jps, jpe,
+                                            self._halo_buf(device_buf)))
 
     def unpack_halo(self, field: str, side: int, width: int, ips, ipe, jps, jpe, device_buf):
-        check(lib().wrfb200_unpack_halo(self._h, FIELD_ID[field], side, width, ips, ipe, jps, jpe,
-                                        C.c_void_p(_ptr(device_buf))))
+        check(self._fn("wrfb200_unpack_halo")(self._h, FIELD_ID[field], side, width, ips, ipe, jps, jpe,
+                                              self._halo_buf(device_buf)))
 
     def standin_advance_uv(self, field: str, c: float, i0, i1, j0, j1):
         check(self._fn("wrfb200_standin_advance_uv")(self._h, FIELD_ID[field], float(c), i0, i1, j0, j1))
@@ -460,12 +467,19 @@ def synth_fields(grid: Grid, seed: int = 20240617, names: Iterable[str] = FIELDS
 
 
 def compare(a: np.ndarray, b: np.ndarray) -> dict:
-    """The reference's comparison metrics (common.cu:68-164) between two float32 arrays."""
-    a = np.ascontiguousarray(a, dtype=np.float32)
-    b = np.ascontiguousarray(b, dtype=np.float32)
+    """The reference's comparison metrics (common.cu:68-164) between two arrays: float32 (or anything else but
+    float64, read as float32) through wrfb200_compare, two float64 arrays through wrfb200_compare_r8 in binary64.
+    A float64 array against any other dtype raises TypeError rather than narrowing it."""
+    r8 = [getattr(x, "dtype", None) == np.float64 for x in (a, b)]
+    if any(r8) and not all(r8):
+        raise TypeError("compare needs both arrays float64 (binary64 metrics) or neither, got "
+                        f"{getattr(a, 'dtype', type(a).__name__)} and {getattr(b, 'dtype', type(b).__name__)}")
+    dt, fn, res = ((np.float64, lib().wrfb200_compare_r8, _lib.CompareResultR8()) if all(r8) else
+                   (np.float32, lib().wrfb200_compare, _lib.CompareResult()))
+    a = np.ascontiguousarray(a, dtype=dt)
+    b = np.ascontiguousarray(b, dtype=dt)
     if a.shape != b.shape:
         raise ValueError("shape mismatch")
-    r = _lib.CompareResult()
-    check(lib().wrfb200_compare(C.c_void_p(a.ctypes.data), C.c_void_p(b.ctypes.data), a.size, C.byref(r)))
-    return {"n": r.n, "n_equal": r.n_equal, "n_different": r.n_different, "max_rel": r.max_rel,
-            "max_abs": r.max_abs, "rmse": r.rmse, "max_ulp": r.max_ulp}
+    check(fn(C.c_void_p(a.ctypes.data), C.c_void_p(b.ctypes.data), a.size, C.byref(res)))
+    return {"n": res.n, "n_equal": res.n_equal, "n_different": res.n_different, "max_rel": res.max_rel,
+            "max_abs": res.max_abs, "rmse": res.rmse, "max_ulp": res.max_ulp}

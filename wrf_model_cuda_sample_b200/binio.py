@@ -3,7 +3,9 @@
 The reference drivers read one raw file per variable from an input directory (argv[1]) and compare against
 ``*_output.bin`` files in an output directory (argv[2]):  big-endian 4-byte values, stream access, Fortran
 (i,k,j) order, no headers (/root/reference/advance_mu_t_driver.f90:38-167 and :357-452,
-common.cu:166-327).  File names are the actual-argument names of WRF's solve_em
+common.cu:166-327).  A dump from WRF built with -r8 holds 8-byte reals (integers stay 4 bytes): the reader takes the
+element size of each real file from its byte length, returns float64 arrays and scalars for such a case, and
+refuses a case whose reals mix the two sizes.  File names are the actual-argument names of WRF's solve_em
 (advance_mu_t_driver.f90:193-205).  None of those files ship with the reference; with this module anyone
 holding the /data2/WRFV3_Input_Output/V3.4.1/dyn_em/advance_mu_t dump can run it through the GPU path and
 get the reference's own error report (common.cu:154-161).
@@ -44,32 +46,50 @@ def _read(path: str, dtype: str, count: int) -> np.ndarray:
     return a
 
 
+def real_kind(path: str, count: int) -> str:
+    """'>f4' or '>f8': the element size of a file of ``count`` reals, from its byte length."""
+    nbytes = os.path.getsize(path)
+    for kind in (">f4", ">f8"):
+        if nbytes == count * np.dtype(kind).itemsize:
+            return kind
+    raise ValueError(f"{path}: {nbytes} bytes are neither {count} 4-byte nor {count} 8-byte reals")
+
+
 def read_int(path: str) -> int:
     return int(_read(path, ">i4", 1)[0])
 
 
-def read_real(path: str) -> np.float32:
-    return np.float32(_read(path, ">f4", 1)[0])
+def read_real(path: str):
+    """np.float32 from a 4-byte file, np.float64 from an 8-byte one."""
+    kind = real_kind(path, 1)
+    return np.dtype(kind).newbyteorder("=").type(_read(path, kind, 1)[0])
 
 
 def read_field(path: str, shape) -> np.ndarray:
-    """Raw big-endian stream in Fortran (i,k,j) order -> native float32 array in C order [j,k,i]."""
-    a = _read(path, ">f4", int(np.prod(shape))).astype(np.float32).reshape(shape)
+    """Raw big-endian stream in Fortran (i,k,j) order -> native float32 (4-byte file) or float64 (8-byte file)
+    array in C order [j,k,i]."""
+    count = int(np.prod(shape))
+    kind = real_kind(path, count)
+    a = _read(path, kind, count).astype(np.dtype(kind).newbyteorder("=")).reshape(shape)
     if np.isnan(a).any():                                      # the reference readers flag NaNs, common.cu:39-44
         raise ValueError(f"{path}: contains NaN")
     return np.ascontiguousarray(a)
 
 
 def write_field(path: str, a: np.ndarray) -> None:
-    np.ascontiguousarray(a, dtype=np.float32).astype(">f4").tofile(path)
+    """float64 arrays as 8-byte reals, anything else as 4-byte reals."""
+    if getattr(a, "dtype", None) == np.float64:
+        np.ascontiguousarray(a).astype(">f8").tofile(path)
+    else:
+        np.ascontiguousarray(a, dtype=np.float32).astype(">f4").tofile(path)
 
 
 def write_int(path: str, v: int) -> None:
     np.array([v], dtype=">i4").tofile(path)
 
 
-def write_real(path: str, v) -> None:
-    np.array([v], dtype=">f4").tofile(path)
+def write_real(path: str, v, kind: str = ">f4") -> None:
+    np.array([v], dtype=kind).tofile(path)
 
 
 def read_case(input_dir: str) -> Tuple[Grid, tuple, Dict[str, np.ndarray]]:
@@ -80,14 +100,24 @@ def read_case(input_dir: str) -> Tuple[Grid, tuple, Dict[str, np.ndarray]]:
     for name, stem in FLAG_FILES.items():
         flags[name] = bool(read_int(j(stem))) if os.path.exists(j(stem)) else (name == "specified")
     g = Grid(**dims, **flags)
-    scalars = tuple(read_real(j(s)) for s in SCALAR_FILES)
+    kinds = {}                                   # element size of every real file, to check that they agree
+
+    def real(path, count):
+        kinds[path] = real_kind(path, count)
+        first = next(iter(kinds.values()))
+        if kinds[path] != first:
+            raise ValueError(f"{path}: {kinds[path][-1]}-byte reals in a case of {first[-1]}-byte reals "
+                             f"({next(iter(kinds))})")
+        return path
+
+    scalars = tuple(read_real(real(j(s), 1)) for s in SCALAR_FILES)
     fields = {}
     for name in FIELDS_3D + FIELDS_2D + FIELDS_1D:
         path = j(FILE_OF[name])
         if os.path.exists(path):
-            fields[name] = read_field(path, g.shape_of(name))
+            fields[name] = read_field(real(path, int(np.prod(g.shape_of(name)))), g.shape_of(name))
         elif name in OUTPUT_ONLY:
-            fields[name] = np.zeros(g.shape_of(name), dtype=np.float32)
+            fields[name] = np.zeros(g.shape_of(name), dtype=scalars[0].dtype)    # the case's precision
         else:
             raise FileNotFoundError(path)
     return g, scalars, fields
@@ -95,20 +125,25 @@ def read_case(input_dir: str) -> Tuple[Grid, tuple, Dict[str, np.ndarray]]:
 
 def write_case(directory: str, g: Grid, scalars, fields: Dict[str, np.ndarray], suffix: str = "",
                names=None) -> None:
-    """Write dims / scalars / flags (when ``suffix`` is empty) and the fields as ``<stem><suffix>.bin``."""
+    """Write dims / scalars / flags (when ``suffix`` is empty) and the fields as ``<stem><suffix>.bin``.
+    float64 fields make an 8-byte case (scalars included), others a 4-byte one; a mix raises ValueError."""
     os.makedirs(directory, exist_ok=True)
     j = lambda stem: os.path.join(directory, stem + ".bin")
+    names = [n for n in (names if names is not None else fields) if n in FILE_OF]
+    wide = {n: getattr(fields[n], "dtype", None) == np.float64 for n in names}
+    if len(set(wide.values())) > 1:
+        raise ValueError("a case holds reals of one size: got float64 fields "
+                         f"{[n for n in names if wide[n]]} beside {[n for n in names if not wide[n]]}")
     if not suffix:
         for n in DIM_NAMES:
             write_int(j(n), getattr(g, n))
         write_int(j("kds"), 1)                                # read by the C / CUDA drivers only
         for s, v in zip(SCALAR_FILES, scalars):
-            write_real(j(s), v)
+            write_real(j(s), v, ">f8" if any(wide.values()) else ">f4")
         for name, stem in FLAG_FILES.items():
             write_int(j(stem), int(getattr(g, name)))
-    for name in (names if names is not None else fields):
-        if name in FILE_OF:
-            write_field(j(FILE_OF[name] + suffix), fields[name])
+    for name in names:
+        write_field(j(FILE_OF[name] + suffix), fields[name])
 
 
 def compare_with_golden(g: Grid, fields: Dict[str, np.ndarray], golden_dir: str) -> Dict[str, dict]:

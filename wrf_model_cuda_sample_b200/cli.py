@@ -1,6 +1,7 @@
 """Command-line twin of the reference drivers (advance_mu_t_driver.{f90,c,cu}): read the reference-format
 .bin inputs from argv[1], run advance_mu_t on the GPU through the C ABI, time it, and -- if argv[2] holds
-``*_output.bin`` goldens -- print the reference's error report.
+``*_output.bin`` goldens -- print the reference's error report.  A case of 8-byte reals (a dump of WRF built with
+-r8) runs the real*8 operator, writes 8-byte outputs and is reported with the binary64 metrics.
 
     python -m wrf_model_cuda_sample_b200.cli INPUT_DIR [GOLDEN_DIR] [--write OUT_DIR] [--steps N]
 """

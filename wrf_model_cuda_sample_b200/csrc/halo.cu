@@ -11,10 +11,10 @@
 namespace {
 
 // Copy the box [i0,i0+ni) x [0,nk) x [j0,j0+nj) (memory indices) between a field and a dense
-// [j][k][i] buffer.
-template <bool PACK>
-__global__ void box_copy_kernel(float *field, float *buf, long long pitch, long long jstride,
-                                int i0, int j0, int ni, int nk, int nj)
+// [j][k][i] buffer.  T = float or double: a plain copy, no arithmetic on the values.
+template <class T, bool PACK>
+__device__ __forceinline__ void box_copy(T *field, T *buf, long long pitch, long long jstride,
+                                         int i0, int j0, int ni, int nk, int nj)
 {
     const long long n = (long long)ni * nk * nj;
     for (long long x = blockIdx.x * (long long)blockDim.x + threadIdx.x; x < n;
@@ -27,6 +27,21 @@ __global__ void box_copy_kernel(float *field, float *buf, long long pitch, long 
         if (PACK) buf[x] = field[o];
         else field[o] = buf[x];
     }
+}
+
+template <bool PACK>
+__global__ void box_copy_kernel(float *field, float *buf, long long pitch, long long jstride,
+                                int i0, int j0, int ni, int nk, int nj)
+{
+    box_copy<float, PACK>(field, buf, pitch, jstride, i0, j0, ni, nk, nj);
+}
+
+// the same box on a real*8 handle (a kernel of its own, so the float kernels keep their names)
+template <bool PACK>
+__global__ void box_copy_kernel_r8(double *field, double *buf, long long pitch, long long jstride,
+                                   int i0, int j0, int ni, int nk, int nj)
+{
+    box_copy<double, PACK>(field, buf, pitch, jstride, i0, j0, ni, nk, nj);
 }
 
 // u(i,k,j) += c*(mudf(i,j)-mudf(i-1,j))   or   v(i,k,j) += c*(mudf(i,j)-mudf(i,j-1)); one block per (k,j) row
@@ -88,11 +103,20 @@ int halo_box(const wrfb200_handle *h, int side, int width, bool inside,
     return WRFB200_OK;
 }
 
+// pack (device field -> dense buffer) or unpack (buffer -> halo) on the handle's stream; `r8` names the verb the
+// caller used: the binary32 verbs refuse a real*8 handle, the _r8 verbs a real*4 one
 int halo_copy(wrfb200_handle *h, int field, int side, int width, int ips, int ipe, int jps, int jpe,
-              float *buf, bool pack)
+              void *buf, bool pack, bool r8)
 {
     if (!h || !buf) return wrfb200_fail(WRFB200_ERR_INVALID_ARG, "null argument");
-    if (int rc = wrfb200_require_r4(h, pack ? "wrfb200_pack_halo" : "wrfb200_unpack_halo")) return rc;
+    if (r8) {
+        if (h->esize != 8)
+            return wrfb200_fail(WRFB200_ERR_STATE, "%s: this is a real*4 handle (created by wrfb200_create); use %s",
+                                pack ? "wrfb200_pack_halo_r8" : "wrfb200_unpack_halo_r8",
+                                pack ? "wrfb200_pack_halo" : "wrfb200_unpack_halo");
+    } else if (int rc = wrfb200_require_r4(h, pack ? "wrfb200_pack_halo" : "wrfb200_unpack_halo")) {
+        return rc;
+    }
     const bool f3 = field >= WRFB200_WW && field <= WRFB200_FT;
     const bool f2 = field >= WRFB200_MU && field <= WRFB200_MSFTY;
     if (!f3 && !f2) return wrfb200_fail(WRFB200_ERR_INVALID_ARG, "field %d has no horizontal halo", field);
@@ -103,18 +127,26 @@ int halo_copy(wrfb200_handle *h, int field, int side, int width, int ips, int ip
     const long long pitch = f3 ? h->pitch3 : h->pitch2;
     const long long jstride = f3 ? pitch * h->kdim : pitch;
     const long long n = (long long)ni * nk * nj;
+    const int mi = i0 - h->dom.ims, mj = j0 - h->dom.jms;
     int prev = -1;
     cudaGetDevice(&prev);
     if (prev != h->device) cudaSetDevice(h->device);
     const int threads = 256;
     const unsigned blocks = (unsigned)((n + threads - 1) / threads < 1184 ? (n + threads - 1) / threads : 1184);
     (void)cudaGetLastError();   // a launch status must not inherit a stale error of some earlier, unrelated call
-    if (pack)
-        box_copy_kernel<true><<<blocks, threads, 0, h->stream>>>(h->d[field], buf, pitch, jstride,
-                                                                 i0 - h->dom.ims, j0 - h->dom.jms, ni, nk, nj);
-    else
-        box_copy_kernel<false><<<blocks, threads, 0, h->stream>>>(h->d[field], buf, pitch, jstride,
-                                                                  i0 - h->dom.ims, j0 - h->dom.jms, ni, nk, nj);
+    if (r8) {
+        double *f = reinterpret_cast<double *>(h->d[field]), *b = static_cast<double *>(buf);
+        if (pack)
+            box_copy_kernel_r8<true><<<blocks, threads, 0, h->stream>>>(f, b, pitch, jstride, mi, mj, ni, nk, nj);
+        else
+            box_copy_kernel_r8<false><<<blocks, threads, 0, h->stream>>>(f, b, pitch, jstride, mi, mj, ni, nk, nj);
+    } else {
+        float *b = static_cast<float *>(buf);
+        if (pack)
+            box_copy_kernel<true><<<blocks, threads, 0, h->stream>>>(h->d[field], b, pitch, jstride, mi, mj, ni, nk, nj);
+        else
+            box_copy_kernel<false><<<blocks, threads, 0, h->stream>>>(h->d[field], b, pitch, jstride, mi, mj, ni, nk, nj);
+    }
     cudaError_t e = cudaGetLastError();
     if (prev != h->device && prev >= 0) cudaSetDevice(prev);
     if (e != cudaSuccess) return wrfb200_fail(WRFB200_ERR_CUDA, "halo kernel launch failed: %s", cudaGetErrorString(e));
@@ -146,19 +178,33 @@ cudaError_t wrfb200_halo_preload()
     if (e == cudaSuccess) e = cudaFuncGetAttributes(&a, (const void *)standin_uv_kernel_r8);
     if (e == cudaSuccess) e = cudaFuncGetAttributes(&a, (const void *)box_copy_kernel<true>);
     if (e == cudaSuccess) e = cudaFuncGetAttributes(&a, (const void *)box_copy_kernel<false>);
+    if (e == cudaSuccess) e = cudaFuncGetAttributes(&a, (const void *)box_copy_kernel_r8<true>);
+    if (e == cudaSuccess) e = cudaFuncGetAttributes(&a, (const void *)box_copy_kernel_r8<false>);
     return e;
 }
 
 extern "C" int wrfb200_pack_halo(wrfb200_handle *h, int field, int side, int width,
                                  int ips, int ipe, int jps, int jpe, float *device_buf)
 {
-    return halo_copy(h, field, side, width, ips, ipe, jps, jpe, device_buf, true);
+    return halo_copy(h, field, side, width, ips, ipe, jps, jpe, device_buf, true, false);
 }
 
 extern "C" int wrfb200_unpack_halo(wrfb200_handle *h, int field, int side, int width,
                                    int ips, int ipe, int jps, int jpe, const float *device_buf)
 {
-    return halo_copy(h, field, side, width, ips, ipe, jps, jpe, const_cast<float *>(device_buf), false);
+    return halo_copy(h, field, side, width, ips, ipe, jps, jpe, const_cast<float *>(device_buf), false, false);
+}
+
+extern "C" int wrfb200_pack_halo_r8(wrfb200_handle *h, int field, int side, int width,
+                                    int ips, int ipe, int jps, int jpe, double *device_buf)
+{
+    return halo_copy(h, field, side, width, ips, ipe, jps, jpe, device_buf, true, true);
+}
+
+extern "C" int wrfb200_unpack_halo_r8(wrfb200_handle *h, int field, int side, int width,
+                                      int ips, int ipe, int jps, int jpe, const double *device_buf)
+{
+    return halo_copy(h, field, side, width, ips, ipe, jps, jpe, const_cast<double *>(device_buf), false, true);
 }
 
 namespace {

@@ -3,9 +3,10 @@
 //     reads its inputs from /data2/WRFV3_Input_Output/V3.4.1/dyn_em/advance_mu_t/*.bin
 //     (advance_mu_t_driver.f90:36-167), which are not shipped; these fields have the same roles and magnitudes.
 //   * wrfb200_compare     : the reference's error report, /root/reference/common.cu:68-164 (metric set only;
-//     the reference prints and has no pass/fail threshold).
+//     the reference prints and has no pass/fail threshold); wrfb200_compare_r8 is the same over doubles.
 #include <cmath>
 #include <cstdint>
+#include <climits>
 #include <cstring>
 #include <thread>
 #include <vector>
@@ -152,6 +153,48 @@ inline long ulp_distance(float a, float b)
     return (long)(dlt < 0 ? -dlt : dlt);
 }
 
+inline long ulp_distance(double a, double b)
+{
+    // the same over the 64-bit patterns: distance of the magnitudes on one side of zero, their sum across it;
+    // only opposite-signed values near the infinities exceed LONG_MAX, and saturate there
+    uint64_t ai, bi;
+    std::memcpy(&ai, &a, 8);
+    std::memcpy(&bi, &b, 8);
+    const uint64_t sign = 0x8000000000000000ull, am = ai & ~sign, bm = bi & ~sign;
+    const uint64_t d = ((ai ^ bi) & sign) ? am + bm : (am > bm ? am - bm : bm - am);
+    return d > (uint64_t)LONG_MAX ? LONG_MAX : (long)d;
+}
+
+// wrfb200_compare / _compare_r8: T is the element type, R the result struct of that precision
+template <class T, class R>
+int compare_values(const T *a, const T *b, long n, R *out)
+{
+    if (!a || !b || !out || n < 0) return wrfb200_fail(WRFB200_ERR_INVALID_ARG, "bad argument");
+    R r{};
+    r.n = n;
+    double sq = 0.0;
+    for (long x = 0; x < n; ++x) {
+        const T va = a[x], vb = b[x];
+        if (std::isnan(va) || std::isnan(vb))
+            return wrfb200_fail(WRFB200_ERR_INVALID_ARG, "NaN at element %ld (a=%g b=%g)", x, (double)va, (double)vb);
+        const T abs_err = std::fabs(va - vb);
+        T rel;
+        if (std::fabs(va) != (T)0 && std::fabs(vb) != (T)0)
+            rel = abs_err / std::fmax(std::fabs(va), std::fabs(vb));
+        else
+            rel = std::fmax(std::fabs(va), std::fabs(vb));
+        if (rel > r.max_rel) r.max_rel = rel;
+        if (abs_err > r.max_abs) r.max_abs = abs_err;
+        const long ulp = ulp_distance(va, vb);
+        if (ulp > r.max_ulp) r.max_ulp = ulp;
+        sq += (double)abs_err * (double)abs_err;
+        if (va == vb) r.n_equal++; else r.n_different++;
+    }
+    r.rmse = n > 0 ? (T)std::sqrt(sq / (double)n) : (T)0;
+    *out = r;
+    return WRFB200_OK;
+}
+
 }  // namespace
 
 extern "C" int wrfb200_synth_field(int field, uint64_t seed, const wrfb200_domain *dom, float dx_m, float *out)
@@ -184,28 +227,10 @@ extern "C" int wrfb200_synth_field(int field, uint64_t seed, const wrfb200_domai
 
 extern "C" int wrfb200_compare(const float *a, const float *b, long n, wrfb200_compare_result *out)
 {
-    if (!a || !b || !out || n < 0) return wrfb200_fail(WRFB200_ERR_INVALID_ARG, "bad argument");
-    wrfb200_compare_result r{};
-    r.n = n;
-    double sq = 0.0;
-    for (long x = 0; x < n; ++x) {
-        const float va = a[x], vb = b[x];
-        if (std::isnan(va) || std::isnan(vb))
-            return wrfb200_fail(WRFB200_ERR_INVALID_ARG, "NaN at element %ld (a=%g b=%g)", x, (double)va, (double)vb);
-        const float abs_err = std::fabs(va - vb);
-        float rel;
-        if (std::fabs(va) != 0.0f && std::fabs(vb) != 0.0f)
-            rel = abs_err / std::fmax(std::fabs(va), std::fabs(vb));
-        else
-            rel = std::fmax(std::fabs(va), std::fabs(vb));
-        if (rel > r.max_rel) r.max_rel = rel;
-        if (abs_err > r.max_abs) r.max_abs = abs_err;
-        const long ulp = ulp_distance(va, vb);
-        if (ulp > r.max_ulp) r.max_ulp = ulp;
-        sq += (double)abs_err * (double)abs_err;
-        if (va == vb) r.n_equal++; else r.n_different++;
-    }
-    r.rmse = n > 0 ? (float)std::sqrt(sq / (double)n) : 0.0f;
-    *out = r;
-    return WRFB200_OK;
+    return compare_values(a, b, n, out);
+}
+
+extern "C" int wrfb200_compare_r8(const double *a, const double *b, long n, wrfb200_compare_result_r8 *out)
+{
+    return compare_values(a, b, n, out);
 }

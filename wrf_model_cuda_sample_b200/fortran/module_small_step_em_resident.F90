@@ -1,6 +1,6 @@
 !-----------------------------------------------------------------------------------------------------------
 ! module_small_step_em_resident.F90 -- ISO_C_BINDING interfaces of the DEVICE-RESIDENT and MULTI-GPU entry
-! points of libwrfb200.so (include/wrfb200.h sections 1, 2 and 3b), for a Fortran host that wants more than
+! points of libwrfb200.so (include/wrfb200.h sections 1, 2, 3 and 3b), for a Fortran host that wants more than
 ! the one-call drop-in of module_small_step_em.F90:
 !
 !   (A) acoustic-loop residency with the UNCHANGED 48-argument call (smallest source change in solve_em):
@@ -49,6 +49,18 @@
 !           st = wrfb200_comm_connect( h, C_LOC(everyone), nproc )
 !           st = wrfb200_comm_push_constants( h )
 !           st = wrfb200_comm_loop_r8( h, number_of_small_timesteps, 0_c_int, 0.0_c_double, 1_c_int )
+!
+!   (D) ranks on several hosts, or any transport of the caller's own (WRF's MPI): pack the edge a neighbour
+!       needs into a dense DEVICE buffer, move it, unpack it into the halo (include/wrfb200.h section 3;
+!       INTEGRATION.md section 4).  -r8 builds use the _r8 pair with REAL(c_double) buffers:
+!
+!           ! u's east halo: this rank's west column goes west, the east neighbour's west column arrives
+!           ! (field 2 = u, side 0 = west, 1 = east; send_buf, recv_buf: n = 1*nk*(jpe-jps+1) doubles on the device)
+!           st = wrfb200_pack_halo_r8( h, 2_c_int, 0_c_int, 1_c_int, ips, ipe, jps, jpe, C_LOC(send_buf) )
+!           st = wrfb200_sync( h )                                  ! the pack runs on the handle's stream
+!           CALL MPI_Sendrecv( send_buf, n, MPI_DOUBLE_PRECISION, west, 0, recv_buf, n, MPI_DOUBLE_PRECISION,  &
+!                              east, 0, comm, stat, ierr )          ! CUDA-aware MPI
+!           st = wrfb200_unpack_halo_r8( h, 2_c_int, 1_c_int, 1_c_int, ips, ipe, jps, jpe, C_LOC(recv_buf) )
 !
 ! Source only: no Fortran compiler exists in the build image (INTEGRATION.md); tests/c_abi_harness.c,
 ! tests/c_comm_harness.c and tests/c_comm_harness_r8.c drive exactly these entry points from C, and tests/test_cabi_host.py checks that every
@@ -281,6 +293,40 @@ INTERFACE
       INTEGER(c_int), VALUE :: field
       REAL(c_double), VALUE :: c
       INTEGER(c_int), VALUE :: i0, i1, j0, j1
+      INTEGER(c_int) :: status
+   END FUNCTION
+
+   ! ---- (D) halo pack / unpack around the caller's own transport; buffers are device addresses ----
+   FUNCTION wrfb200_pack_halo(handle, field, side, width, ips, ipe, jps, jpe, device_buf)             &
+            BIND(C, NAME="wrfb200_pack_halo") RESULT(status)
+      IMPORT :: c_int, c_ptr
+      TYPE(c_ptr), VALUE :: handle
+      INTEGER(c_int), VALUE :: field, side, width, ips, ipe, jps, jpe
+      TYPE(c_ptr), VALUE :: device_buf                    ! REAL(c_float) on the device
+      INTEGER(c_int) :: status
+   END FUNCTION
+   FUNCTION wrfb200_unpack_halo(handle, field, side, width, ips, ipe, jps, jpe, device_buf)           &
+            BIND(C, NAME="wrfb200_unpack_halo") RESULT(status)
+      IMPORT :: c_int, c_ptr
+      TYPE(c_ptr), VALUE :: handle
+      INTEGER(c_int), VALUE :: field, side, width, ips, ipe, jps, jpe
+      TYPE(c_ptr), VALUE :: device_buf                    ! REAL(c_float) on the device
+      INTEGER(c_int) :: status
+   END FUNCTION
+   FUNCTION wrfb200_pack_halo_r8(handle, field, side, width, ips, ipe, jps, jpe, device_buf)          &
+            BIND(C, NAME="wrfb200_pack_halo_r8") RESULT(status)
+      IMPORT :: c_int, c_ptr
+      TYPE(c_ptr), VALUE :: handle
+      INTEGER(c_int), VALUE :: field, side, width, ips, ipe, jps, jpe
+      TYPE(c_ptr), VALUE :: device_buf                    ! REAL(c_double) on the device
+      INTEGER(c_int) :: status
+   END FUNCTION
+   FUNCTION wrfb200_unpack_halo_r8(handle, field, side, width, ips, ipe, jps, jpe, device_buf)        &
+            BIND(C, NAME="wrfb200_unpack_halo_r8") RESULT(status)
+      IMPORT :: c_int, c_ptr
+      TYPE(c_ptr), VALUE :: handle
+      INTEGER(c_int), VALUE :: field, side, width, ips, ipe, jps, jpe
+      TYPE(c_ptr), VALUE :: device_buf                    ! REAL(c_double) on the device
       INTEGER(c_int) :: status
    END FUNCTION
 

@@ -20,6 +20,8 @@ from __future__ import annotations
 from dataclasses import dataclass
 from typing import Callable, Dict, List, Optional, Sequence, Tuple
 
+import numpy as np
+
 from ._lib import EAST, NORTH, SOUTH, WEST
 from .advance_mu_t import Grid
 
@@ -183,7 +185,8 @@ class HaloExchanger:
 
 
 class GpuPatchHalo:
-    """pack / recv_buffer / unpack for a device-resident ``Patch`` with preallocated torch buffers."""
+    """pack / recv_buffer / unpack for a device-resident ``Patch`` with preallocated torch buffers of the patch's
+    dtype (float64 for a real*8 patch)."""
 
     def __init__(self, patch, decomp: Decomposition, rank: int, device):
         self.patch = patch
@@ -200,7 +203,8 @@ class GpuPatchHalo:
             ips, ipe, jps, jpe = self.ext
             nk = self.grid.shape3[1] if field in FIELDS_3D else 1
             n = (width * nk * (jpe - jps + 1)) if side in (WEST, EAST) else ((ipe - ips + 1) * nk * width)
-            self._bufs[key] = torch.empty(n, dtype=torch.float32, device=self.device)
+            dtype = torch.float64 if self.patch.dtype is np.float64 else torch.float32
+            self._bufs[key] = torch.empty(n, dtype=dtype, device=self.device)
         return self._bufs[key]
 
     def pack(self, field, side, width):
