@@ -1,5 +1,5 @@
 """The fused multi-GPU path (csrc/comm.cu) on real*8 patches: wrfb200_comm_init_r8 / wrfb200_comm_loop_r8 and the
-fused double2 tile kernel (amt_tile_kernel_r8_fused).  As in tests/test_fused_comm.py the ranks are handles of ONE
+fused double2 tile kernel (amt_tile_kernel_r8<TJ, true>).  As in tests/test_fused_comm.py the ranks are handles of ONE
 process on device 0, so the flag protocol, the peer stores and the kernels are those of the multi-process runs
 (tests/c_comm_harness_r8.c, tools/multi_gpu_check.py --dtype float64).
 Bar: every rank's patch BIT-IDENTICAL to the binary64 checker loop over the whole domain, halos poisoned beforehand;

@@ -198,7 +198,6 @@ bool amt_build_tma_maps(const AmtParams &p, AmtTmaMaps *maps);                  
 cudaError_t amt_launch_pipe(const AmtParams &p, const AmtTmaMaps &maps, cudaStream_t stream);
 // real*8 kernels (amt_column.cu, amt_tile_r8.cu)
 cudaError_t amt_launch_column(const AmtParamsR8 &p, cudaStream_t stream);
-cudaError_t amt_launch_tile(const AmtParamsR8 &p, cudaStream_t stream);
+cudaError_t amt_launch_tile(const AmtParamsR8 &p, cudaStream_t stream);       // p.halo.enabled: the multi-GPU kernel
 bool amt_tile_supported(const AmtParamsR8 &p);
-cudaError_t amt_launch_tile_fused(const AmtParamsR8 &p, cudaStream_t stream);    // p.halo.enabled: multi-GPU
 cudaError_t amt_tile_r8_preload();                                               // see amt_pipe_preload

@@ -64,6 +64,31 @@ int check_domain(const wrfb200_domain &d)
 
 }  // namespace
 
+template <class P>
+void wrfb200_fill_fields(const wrfb200_handle *h, P *p)
+{
+    using T = std::remove_pointer_t<decltype(P::ww)>;
+    auto F = [h](int f) { return reinterpret_cast<T *>(h->d[f]); };
+    p->ww = F(WRFB200_WW);       p->ww_1 = F(WRFB200_WW_1);
+    p->u = F(WRFB200_U);         p->u_1 = F(WRFB200_U_1);
+    p->v = F(WRFB200_V);         p->v_1 = F(WRFB200_V_1);
+    p->t = F(WRFB200_T);         p->t_1 = F(WRFB200_T_1);
+    p->t_ave = F(WRFB200_T_AVE); p->ft = F(WRFB200_FT);
+    p->mu = F(WRFB200_MU);       p->mut = F(WRFB200_MUT);
+    p->muave = F(WRFB200_MUAVE); p->muts = F(WRFB200_MUTS);
+    p->muu = F(WRFB200_MUU);     p->muv = F(WRFB200_MUV);
+    p->mudf = F(WRFB200_MUDF);   p->mu_tend = F(WRFB200_MU_TEND);
+    p->msfuy = F(WRFB200_MSFUY); p->msfvx_inv = F(WRFB200_MSFVX_INV);
+    p->msftx = F(WRFB200_MSFTX); p->msfty = F(WRFB200_MSFTY);
+    p->dnw = F(WRFB200_DNW);     p->fnm = F(WRFB200_FNM);
+    p->fnp = F(WRFB200_FNP);     p->rdnw = F(WRFB200_RDNW);
+    p->pitch = h->pitch3;
+    p->jstride = h->pitch3 * (long long)h->kdim;
+    p->pitch2 = h->pitch2;
+}
+template void wrfb200_fill_fields(const wrfb200_handle *h, AmtParams *p);
+template void wrfb200_fill_fields(const wrfb200_handle *h, AmtParamsR8 *p);
+
 namespace {
 
 // Build the kernel argument block for the tile its:ite x jts:jte.  Returns >0 status on error,
@@ -91,25 +116,9 @@ int make_params(const wrfb200_handle *h, int its, int ite, int jts, int jte, int
     if (!h->scalars_set)
         return fail(WRFB200_ERR_STATE, "rdx/rdy/dts/epssm not set (wrfb200_set_scalars%s)", sizeof(T) == 8 ? "_r8" : "");
 
-    auto F = [h](int f) { return reinterpret_cast<T *>(h->d[f]); };
     P p{};
-    p.ww = F(WRFB200_WW);       p.ww_1 = F(WRFB200_WW_1);
-    p.u = F(WRFB200_U);         p.u_1 = F(WRFB200_U_1);
-    p.v = F(WRFB200_V);         p.v_1 = F(WRFB200_V_1);
-    p.t = F(WRFB200_T);         p.t_1 = F(WRFB200_T_1);
-    p.t_ave = F(WRFB200_T_AVE); p.ft = F(WRFB200_FT);
-    p.mu = F(WRFB200_MU);       p.mut = F(WRFB200_MUT);
-    p.muave = F(WRFB200_MUAVE); p.muts = F(WRFB200_MUTS);
-    p.muu = F(WRFB200_MUU);     p.muv = F(WRFB200_MUV);
-    p.mudf = F(WRFB200_MUDF);   p.mu_tend = F(WRFB200_MU_TEND);
-    p.msfuy = F(WRFB200_MSFUY); p.msfvx_inv = F(WRFB200_MSFVX_INV);
-    p.msftx = F(WRFB200_MSFTX); p.msfty = F(WRFB200_MSFTY);
-    p.dnw = F(WRFB200_DNW);     p.fnm = F(WRFB200_FNM);
-    p.fnp = F(WRFB200_FNP);     p.rdnw = F(WRFB200_RDNW);
+    wrfb200_fill_fields(h, &p);
     p.rdx = (T)h->rdx; p.rdy = (T)h->rdy; p.dts = (T)h->dts; p.epssm = (T)h->epssm;   // exact: stored from a T
-    p.pitch = h->pitch3;
-    p.jstride = h->pitch3 * (long long)h->kdim;
-    p.pitch2 = h->pitch2;
     p.i0 = is - d.ims; p.i1 = ie - d.ims;
     p.j0 = js - d.jms; p.j1 = je - d.jms;
     p.k0 = ks - d.kms;
@@ -181,7 +190,7 @@ int launch(wrfb200_handle *h, const AmtParamsR8 &p, cudaStream_t s, int kernel)
         // checked that the patch's layout and level count suit it
         if (!amt_tile_supported(p))
             return fail(WRFB200_ERR_UNSUPPORTED, "the fused real*8 exchange needs the tile kernel's layout and nk <= 220 (nk=%d)", p.nk);
-        e = amt_launch_tile_fused(p, s);
+        e = amt_launch_tile(p, s);
         ran = WRFB200_KERNEL_TILE;
     } else if (kernel == WRFB200_KERNEL_PIPE) {
         return fail(WRFB200_ERR_UNSUPPORTED, "the pipe kernel is binary32 only; a real*8 handle runs the tile or column kernel");
@@ -633,115 +642,107 @@ extern "C" int wrfb200_download_r8(wrfb200_handle *h, int field, double *host)
 
 // Resident-state verbs (SURVEY.md section 8b): the groups of arrays a host-resident caller moves at the three
 // cadences of the acoustic loop.  A null pointer skips that array.  Replaces the per-call copies of every field,
-// advance_mu_t_no_async.cu:245-306 (H2D) and :366-390 (D2H).
+// advance_mu_t_no_async.cu:245-306 (H2D) and :366-390 (D2H).  Each verb has a binary32 and an _r8 form (WRF built
+// with -r8) that run one body with the verb's element size and name.
+namespace {
+
+const int kConstantFields[] = {WRFB200_WW_1, WRFB200_U_1, WRFB200_V_1, WRFB200_T_1, WRFB200_FT, WRFB200_MUT,
+                               WRFB200_MUU, WRFB200_MUV, WRFB200_MU_TEND, WRFB200_MSFUY, WRFB200_MSFVX_INV,
+                               WRFB200_MSFTX, WRFB200_MSFTY, WRFB200_DNW, WRFB200_FNM, WRFB200_FNP, WRFB200_RDNW};
+const int kStateFields[] = {WRFB200_WW, WRFB200_T, WRFB200_MU};
+const int kUVFields[] = {WRFB200_U, WRFB200_V};
+const int kOutputFields[] = {WRFB200_WW, WRFB200_T, WRFB200_T_AVE, WRFB200_MU, WRFB200_MUAVE, WRFB200_MUTS,
+                             WRFB200_MUDF};
+
+// a binary32 verb refuses a real*8 handle as binary32 only; an _r8 verb names the real*4 handle it was given
+int resident_precision(const wrfb200_handle *h, int esize, const char *verb)
+{
+    if (!h) return fail(WRFB200_ERR_INVALID_ARG, "null handle");
+    if (esize == 4) return wrfb200_require_r4(h, verb);
+    return h->esize == 8 ? WRFB200_OK : wrong_precision(h, verb);
+}
+
+template <size_t N>
+int upload_fields(wrfb200_handle *h, int esize, const char *verb, const int (&ids)[N], const void *const (&host)[N])
+{
+    if (int rc = resident_precision(h, esize, verb)) return rc;
+    for (size_t x = 0; x < N; ++x)
+        if (host[x]) if (int rc = copy_verb_all(h, esize, verb, ids[x], host[x], nullptr)) return rc;
+    return WRFB200_OK;
+}
+
+// Downloads exactly the cells the routine writes for the tile its:ite x jts:jte (everything else in the
+// caller's arrays keeps its bytes, as with the Fortran).
+int download_outputs(wrfb200_handle *h, int esize, const char *verb, int its, int ite, int jts, int jte, int kts,
+                     int kte, void *const (&host)[7])
+{
+    if (int rc = resident_precision(h, esize, verb)) return rc;
+    const wrfb200_domain &d = h->dom;
+    int is, ie, js, je, ks, ke;
+    wrfb200_bounds(d.periodic_x, d.specified, d.nested, d.ids, d.ide, d.jds, d.jde,
+                   its, ite, jts, jte, kts, kte, &is, &ie, &js, &je, &ks, &ke);
+    if (is > ie || js > je || ks > ke) return WRFB200_OK;
+    for (int x = 0; x < 7; ++x)
+        if (host[x])
+            if (int rc = copy_verb(h, esize, verb, kOutputFields[x], nullptr, host[x], is, ie, ks, ke, js, je)) return rc;
+    return WRFB200_OK;
+}
+
+}  // namespace
+
 extern "C" int wrfb200_upload_constants(
     wrfb200_handle *h, const float *ww_1, const float *u_1, const float *v_1, const float *t_1, const float *ft,
     const float *mut, const float *muu, const float *muv, const float *mu_tend,
     const float *msfuy, const float *msfvx_inv, const float *msftx, const float *msfty,
     const float *dnw, const float *fnm, const float *fnp, const float *rdnw)
 {
-    if (!h) return fail(WRFB200_ERR_INVALID_ARG, "null handle");
-    if (int rc = wrfb200_require_r4(h, "wrfb200_upload_constants")) return rc;
-    const int ids[] = {WRFB200_WW_1, WRFB200_U_1, WRFB200_V_1, WRFB200_T_1, WRFB200_FT, WRFB200_MUT, WRFB200_MUU,
-                       WRFB200_MUV, WRFB200_MU_TEND, WRFB200_MSFUY, WRFB200_MSFVX_INV, WRFB200_MSFTX, WRFB200_MSFTY,
-                       WRFB200_DNW, WRFB200_FNM, WRFB200_FNP, WRFB200_RDNW};
-    const float *ptr[] = {ww_1, u_1, v_1, t_1, ft, mut, muu, muv, mu_tend, msfuy, msfvx_inv, msftx, msfty, dnw, fnm, fnp, rdnw};
-    for (int x = 0; x < 17; ++x)
-        if (ptr[x]) if (int rc = wrfb200_upload(h, ids[x], ptr[x])) return rc;
-    return WRFB200_OK;
+    return upload_fields(h, 4, "wrfb200_upload_constants", kConstantFields,
+                         {ww_1, u_1, v_1, t_1, ft, mut, muu, muv, mu_tend, msfuy, msfvx_inv, msftx, msfty, dnw, fnm, fnp, rdnw});
 }
 
 extern "C" int wrfb200_upload_state(wrfb200_handle *h, const float *ww, const float *t, const float *mu)
 {
-    if (!h) return fail(WRFB200_ERR_INVALID_ARG, "null handle");
-    if (int rc = wrfb200_require_r4(h, "wrfb200_upload_state")) return rc;
-    if (ww) if (int rc = wrfb200_upload(h, WRFB200_WW, ww)) return rc;
-    if (t) if (int rc = wrfb200_upload(h, WRFB200_T, t)) return rc;
-    if (mu) if (int rc = wrfb200_upload(h, WRFB200_MU, mu)) return rc;
-    return WRFB200_OK;
+    return upload_fields(h, 4, "wrfb200_upload_state", kStateFields, {ww, t, mu});
 }
 
 extern "C" int wrfb200_set_uv(wrfb200_handle *h, const float *u, const float *v)
 {
-    if (!h) return fail(WRFB200_ERR_INVALID_ARG, "null handle");
-    if (int rc = wrfb200_require_r4(h, "wrfb200_set_uv")) return rc;
-    if (u) if (int rc = wrfb200_upload(h, WRFB200_U, u)) return rc;
-    if (v) if (int rc = wrfb200_upload(h, WRFB200_V, v)) return rc;
-    return WRFB200_OK;
+    return upload_fields(h, 4, "wrfb200_set_uv", kUVFields, {u, v});
 }
 
-// Downloads exactly the cells the routine writes for the tile its:ite x jts:jte (everything else in the
-// caller's arrays keeps its bytes, as with the Fortran).
 extern "C" int wrfb200_download_outputs(wrfb200_handle *h, int its, int ite, int jts, int jte, int kts, int kte,
                                         float *ww, float *t, float *t_ave, float *mu, float *muave, float *muts, float *mudf)
 {
-    if (!h) return fail(WRFB200_ERR_INVALID_ARG, "null handle");
-    if (int rc = wrfb200_require_r4(h, "wrfb200_download_outputs")) return rc;
-    const wrfb200_domain &d = h->dom;
-    int is, ie, js, je, ks, ke;
-    wrfb200_bounds(d.periodic_x, d.specified, d.nested, d.ids, d.ide, d.jds, d.jde,
-                   its, ite, jts, jte, kts, kte, &is, &ie, &js, &je, &ks, &ke);
-    if (is > ie || js > je || ks > ke) return WRFB200_OK;
-    const int ids[] = {WRFB200_WW, WRFB200_T, WRFB200_T_AVE, WRFB200_MU, WRFB200_MUAVE, WRFB200_MUTS, WRFB200_MUDF};
-    float *ptr[] = {ww, t, t_ave, mu, muave, muts, mudf};
-    for (int x = 0; x < 7; ++x)
-        if (ptr[x]) if (int rc = wrfb200_download_range(h, ids[x], ptr[x], is, ie, ks, ke, js, je)) return rc;
-    return WRFB200_OK;
+    return download_outputs(h, 4, "wrfb200_download_outputs", its, ite, jts, jte, kts, kte,
+                            {ww, t, t_ave, mu, muave, muts, mudf});
 }
 
-// The same four verbs for real*8 handles (WRF built with -r8): double arrays, the _r8 copies.
 extern "C" int wrfb200_upload_constants_r8(
     wrfb200_handle *h, const double *ww_1, const double *u_1, const double *v_1, const double *t_1, const double *ft,
     const double *mut, const double *muu, const double *muv, const double *mu_tend,
     const double *msfuy, const double *msfvx_inv, const double *msftx, const double *msfty,
     const double *dnw, const double *fnm, const double *fnp, const double *rdnw)
 {
-    if (!h) return fail(WRFB200_ERR_INVALID_ARG, "null handle");
-    if (h->esize != 8) return wrong_precision(h, "wrfb200_upload_constants_r8");
-    const int ids[] = {WRFB200_WW_1, WRFB200_U_1, WRFB200_V_1, WRFB200_T_1, WRFB200_FT, WRFB200_MUT, WRFB200_MUU,
-                       WRFB200_MUV, WRFB200_MU_TEND, WRFB200_MSFUY, WRFB200_MSFVX_INV, WRFB200_MSFTX, WRFB200_MSFTY,
-                       WRFB200_DNW, WRFB200_FNM, WRFB200_FNP, WRFB200_RDNW};
-    const double *ptr[] = {ww_1, u_1, v_1, t_1, ft, mut, muu, muv, mu_tend, msfuy, msfvx_inv, msftx, msfty, dnw, fnm, fnp, rdnw};
-    for (int x = 0; x < 17; ++x)
-        if (ptr[x]) if (int rc = wrfb200_upload_r8(h, ids[x], ptr[x])) return rc;
-    return WRFB200_OK;
+    return upload_fields(h, 8, "wrfb200_upload_constants_r8", kConstantFields,
+                         {ww_1, u_1, v_1, t_1, ft, mut, muu, muv, mu_tend, msfuy, msfvx_inv, msftx, msfty, dnw, fnm, fnp, rdnw});
 }
 
 extern "C" int wrfb200_upload_state_r8(wrfb200_handle *h, const double *ww, const double *t, const double *mu)
 {
-    if (!h) return fail(WRFB200_ERR_INVALID_ARG, "null handle");
-    if (h->esize != 8) return wrong_precision(h, "wrfb200_upload_state_r8");
-    if (ww) if (int rc = wrfb200_upload_r8(h, WRFB200_WW, ww)) return rc;
-    if (t) if (int rc = wrfb200_upload_r8(h, WRFB200_T, t)) return rc;
-    if (mu) if (int rc = wrfb200_upload_r8(h, WRFB200_MU, mu)) return rc;
-    return WRFB200_OK;
+    return upload_fields(h, 8, "wrfb200_upload_state_r8", kStateFields, {ww, t, mu});
 }
 
 extern "C" int wrfb200_set_uv_r8(wrfb200_handle *h, const double *u, const double *v)
 {
-    if (!h) return fail(WRFB200_ERR_INVALID_ARG, "null handle");
-    if (h->esize != 8) return wrong_precision(h, "wrfb200_set_uv_r8");
-    if (u) if (int rc = wrfb200_upload_r8(h, WRFB200_U, u)) return rc;
-    if (v) if (int rc = wrfb200_upload_r8(h, WRFB200_V, v)) return rc;
-    return WRFB200_OK;
+    return upload_fields(h, 8, "wrfb200_set_uv_r8", kUVFields, {u, v});
 }
 
 extern "C" int wrfb200_download_outputs_r8(wrfb200_handle *h, int its, int ite, int jts, int jte, int kts, int kte,
                                            double *ww, double *t, double *t_ave, double *mu, double *muave,
                                            double *muts, double *mudf)
 {
-    if (!h) return fail(WRFB200_ERR_INVALID_ARG, "null handle");
-    if (h->esize != 8) return wrong_precision(h, "wrfb200_download_outputs_r8");
-    const wrfb200_domain &d = h->dom;
-    int is, ie, js, je, ks, ke;
-    wrfb200_bounds(d.periodic_x, d.specified, d.nested, d.ids, d.ide, d.jds, d.jde,
-                   its, ite, jts, jte, kts, kte, &is, &ie, &js, &je, &ks, &ke);
-    if (is > ie || js > je || ks > ke) return WRFB200_OK;
-    const int ids[] = {WRFB200_WW, WRFB200_T, WRFB200_T_AVE, WRFB200_MU, WRFB200_MUAVE, WRFB200_MUTS, WRFB200_MUDF};
-    double *ptr[] = {ww, t, t_ave, mu, muave, muts, mudf};
-    for (int x = 0; x < 7; ++x)
-        if (ptr[x]) if (int rc = wrfb200_download_range_r8(h, ids[x], ptr[x], is, ie, ks, ke, js, je)) return rc;
-    return WRFB200_OK;
+    return download_outputs(h, 8, "wrfb200_download_outputs_r8", its, ite, jts, jte, kts, kte,
+                            {ww, t, t_ave, mu, muave, muts, mudf});
 }
 
 // -------------------------------------------------------------------------------------------------

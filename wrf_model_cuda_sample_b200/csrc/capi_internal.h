@@ -38,6 +38,9 @@ int wrfb200_launch_params(wrfb200_handle *h, const AmtParams &p, cudaStream_t s,
 int wrfb200_make_params(const wrfb200_handle *h, int its, int ite, int jts, int jte, int kts, int kte,
                         AmtParamsR8 *out, bool *empty);
 int wrfb200_launch_params(wrfb200_handle *h, const AmtParamsR8 &p, cudaStream_t s, int kernel);
+// the handle's field pointers and strides into *p, whose element type must be the handle's (AmtParams or AmtParamsR8)
+template <class P>
+void wrfb200_fill_fields(const wrfb200_handle *h, P *p);
 // comm.cu: called by wrfb200_destroy
 void wrfb200_comm_release(wrfb200_handle *h);
 

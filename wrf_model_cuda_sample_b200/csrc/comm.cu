@@ -38,9 +38,9 @@
 //                                       it no longer reads the u / v halo I filled for step n
 //
 // Real*8 ranks (wrfb200_create_r8 + wrfb200_comm_init_r8) run the same protocol with the same flags: the step is
-// the fused double2 tile kernel (amt_tile_kernel_r8_fused, amt_tile_r8.cu), the peer addresses are computed with
-// the element size, and push_kernel moves double edges as pairs of 4-byte words.  Both ranks of a pair must hold
-// the same precision (checked at connect).
+// the double2 tile kernel with the exchange fused in (amt_tile_kernel_r8<TJ, true>, amt_tile_r8.cu), the peer
+// addresses are computed with the element size, and push_kernel moves double edges as pairs of 4-byte words.  Both
+// ranks of a pair must hold the same precision (checked at connect).
 #include <unistd.h>
 
 #include <cstdint>
@@ -619,14 +619,7 @@ extern "C" int wrfb200_comm_init_r8(wrfb200_handle *h, int px, int py, int rank,
     // every step runs the fused tile kernel: refuse a patch it cannot take now rather than at the first step.
     // Handle-owned mirrors are 128-byte aligned with even pitches, so the level count is what can fail.
     AmtParamsR8 p{};
-    auto F = [h](int f) { return reinterpret_cast<double *>(h->d[f]); };
-    p.ww = F(WRFB200_WW); p.ww_1 = F(WRFB200_WW_1); p.u = F(WRFB200_U); p.u_1 = F(WRFB200_U_1);
-    p.v = F(WRFB200_V); p.v_1 = F(WRFB200_V_1); p.t = F(WRFB200_T); p.t_1 = F(WRFB200_T_1);
-    p.t_ave = F(WRFB200_T_AVE); p.ft = F(WRFB200_FT); p.mu = F(WRFB200_MU); p.mut = F(WRFB200_MUT);
-    p.muave = F(WRFB200_MUAVE); p.muts = F(WRFB200_MUTS); p.muu = F(WRFB200_MUU); p.muv = F(WRFB200_MUV);
-    p.mudf = F(WRFB200_MUDF); p.mu_tend = F(WRFB200_MU_TEND); p.msfuy = F(WRFB200_MSFUY);
-    p.msfvx_inv = F(WRFB200_MSFVX_INV); p.msftx = F(WRFB200_MSFTX); p.msfty = F(WRFB200_MSFTY);
-    p.pitch = h->pitch3; p.jstride = h->pitch3 * (long long)h->kdim; p.pitch2 = h->pitch2;
+    wrfb200_fill_fields(h, &p);
     p.nk = h->dom.kde - 1;                                      // levels 1 .. kde-1
     if (!amt_tile_supported(p))
         return wrfb200_fail(WRFB200_ERR_UNSUPPORTED, "the real*8 multi-GPU path runs the double2 tile kernel, which "

@@ -6,6 +6,8 @@
 // advance_mu_t only reads a ONE-cell ring (u,u_1,muu,msfuy at i+1; v,v_1,muv,msfvx_inv at j+1; t_1 at
 // i+-1, j+-1 -- module_small_step_em.f90:143-146, :241-245), so a one-wide halo is packed into a dense
 // buffer here, moved between ranks by the host layer (NCCL send/recv), and unpacked on the other side.
+#include <type_traits>
+
 #include "capi_internal.h"
 
 namespace {
@@ -13,8 +15,8 @@ namespace {
 // Copy the box [i0,i0+ni) x [0,nk) x [j0,j0+nj) (memory indices) between a field and a dense
 // [j][k][i] buffer.  T = float or double: a plain copy, no arithmetic on the values.
 template <class T, bool PACK>
-__device__ __forceinline__ void box_copy(T *field, T *buf, long long pitch, long long jstride,
-                                         int i0, int j0, int ni, int nk, int nj)
+__global__ void box_copy_kernel(T *field, T *buf, long long pitch, long long jstride,
+                                int i0, int j0, int ni, int nk, int nj)
 {
     const long long n = (long long)ni * nk * nj;
     for (long long x = blockIdx.x * (long long)blockDim.x + threadIdx.x; x < n;
@@ -29,48 +31,20 @@ __device__ __forceinline__ void box_copy(T *field, T *buf, long long pitch, long
     }
 }
 
-template <bool PACK>
-__global__ void box_copy_kernel(float *field, float *buf, long long pitch, long long jstride,
-                                int i0, int j0, int ni, int nk, int nj)
-{
-    box_copy<float, PACK>(field, buf, pitch, jstride, i0, j0, ni, nk, nj);
-}
-
-// the same box on a real*8 handle (a kernel of its own, so the float kernels keep their names)
-template <bool PACK>
-__global__ void box_copy_kernel_r8(double *field, double *buf, long long pitch, long long jstride,
-                                   int i0, int j0, int ni, int nk, int nj)
-{
-    box_copy<double, PACK>(field, buf, pitch, jstride, i0, j0, ni, nk, nj);
-}
-
-// u(i,k,j) += c*(mudf(i,j)-mudf(i-1,j))   or   v(i,k,j) += c*(mudf(i,j)-mudf(i,j-1)); one block per (k,j) row
-__global__ void standin_uv_kernel(float *f, const float *mudf, long long pitch, long long jstride,
-                                  long long pitch2, long long dshift, float c,
+// u(i,k,j) += c*(mudf(i,j)-mudf(i-1,j))   or   v(i,k,j) += c*(mudf(i,j)-mudf(i,j-1)); one block per (k,j) row,
+// one rounding per operation in the handle's precision T
+template <class T>
+__global__ void standin_uv_kernel(T *f, const T *mudf, long long pitch, long long jstride,
+                                  long long pitch2, long long dshift, T c,
                                   int i0, int j0, int ni, int nk, int nj)
 {
     for (long long r = blockIdx.x; r < (long long)nk * nj; r += gridDim.x) {
         const int k = (int)(r % nk);
         const int j = (int)(r / nk);
-        float *row = f + (long long)(j0 + j) * jstride + (long long)k * pitch + i0;
-        const float *m = mudf + (long long)(j0 + j) * pitch2 + i0;
+        T *row = f + (long long)(j0 + j) * jstride + (long long)k * pitch + i0;
+        const T *m = mudf + (long long)(j0 + j) * pitch2 + i0;
         for (int i = threadIdx.x; i < ni; i += blockDim.x)
-            row[i] = __fadd_rn(row[i], __fmul_rn(c, __fsub_rn(m[i], m[i - dshift])));
-    }
-}
-
-// the same in binary64 (real*8 handles): one rounding per operation, as the float kernel
-__global__ void standin_uv_kernel_r8(double *f, const double *mudf, long long pitch, long long jstride,
-                                     long long pitch2, long long dshift, double c,
-                                     int i0, int j0, int ni, int nk, int nj)
-{
-    for (long long r = blockIdx.x; r < (long long)nk * nj; r += gridDim.x) {
-        const int k = (int)(r % nk);
-        const int j = (int)(r / nk);
-        double *row = f + (long long)(j0 + j) * jstride + (long long)k * pitch + i0;
-        const double *m = mudf + (long long)(j0 + j) * pitch2 + i0;
-        for (int i = threadIdx.x; i < ni; i += blockDim.x)
-            row[i] = __dadd_rn(row[i], __dmul_rn(c, __dsub_rn(m[i], m[i - dshift])));
+            row[i] = f_add(row[i], f_mul(c, f_sub(m[i], m[i - dshift])));
     }
 }
 
@@ -134,19 +108,16 @@ int halo_copy(wrfb200_handle *h, int field, int side, int width, int ips, int ip
     const int threads = 256;
     const unsigned blocks = (unsigned)((n + threads - 1) / threads < 1184 ? (n + threads - 1) / threads : 1184);
     (void)cudaGetLastError();   // a launch status must not inherit a stale error of some earlier, unrelated call
-    if (r8) {
-        double *f = reinterpret_cast<double *>(h->d[field]), *b = static_cast<double *>(buf);
+    auto run = [&](auto *f) {
+        using T = std::remove_pointer_t<decltype(f)>;
+        T *b = static_cast<T *>(buf);
         if (pack)
-            box_copy_kernel_r8<true><<<blocks, threads, 0, h->stream>>>(f, b, pitch, jstride, mi, mj, ni, nk, nj);
+            box_copy_kernel<T, true><<<blocks, threads, 0, h->stream>>>(f, b, pitch, jstride, mi, mj, ni, nk, nj);
         else
-            box_copy_kernel_r8<false><<<blocks, threads, 0, h->stream>>>(f, b, pitch, jstride, mi, mj, ni, nk, nj);
-    } else {
-        float *b = static_cast<float *>(buf);
-        if (pack)
-            box_copy_kernel<true><<<blocks, threads, 0, h->stream>>>(h->d[field], b, pitch, jstride, mi, mj, ni, nk, nj);
-        else
-            box_copy_kernel<false><<<blocks, threads, 0, h->stream>>>(h->d[field], b, pitch, jstride, mi, mj, ni, nk, nj);
-    }
+            box_copy_kernel<T, false><<<blocks, threads, 0, h->stream>>>(f, b, pitch, jstride, mi, mj, ni, nk, nj);
+    };
+    if (h->esize == 8) run(reinterpret_cast<double *>(h->d[field]));
+    else run(h->d[field]);
     cudaError_t e = cudaGetLastError();
     if (prev != h->device && prev >= 0) cudaSetDevice(prev);
     if (e != cudaSuccess) return wrfb200_fail(WRFB200_ERR_CUDA, "halo kernel launch failed: %s", cudaGetErrorString(e));
@@ -174,12 +145,12 @@ cudaError_t wrfb200_repitch_rows(float *dst, const float *src, long long pitch, 
 cudaError_t wrfb200_halo_preload()
 {
     cudaFuncAttributes a;
-    cudaError_t e = cudaFuncGetAttributes(&a, (const void *)standin_uv_kernel);
-    if (e == cudaSuccess) e = cudaFuncGetAttributes(&a, (const void *)standin_uv_kernel_r8);
-    if (e == cudaSuccess) e = cudaFuncGetAttributes(&a, (const void *)box_copy_kernel<true>);
-    if (e == cudaSuccess) e = cudaFuncGetAttributes(&a, (const void *)box_copy_kernel<false>);
-    if (e == cudaSuccess) e = cudaFuncGetAttributes(&a, (const void *)box_copy_kernel_r8<true>);
-    if (e == cudaSuccess) e = cudaFuncGetAttributes(&a, (const void *)box_copy_kernel_r8<false>);
+    cudaError_t e = cudaFuncGetAttributes(&a, (const void *)standin_uv_kernel<float>);
+    if (e == cudaSuccess) e = cudaFuncGetAttributes(&a, (const void *)standin_uv_kernel<double>);
+    if (e == cudaSuccess) e = cudaFuncGetAttributes(&a, (const void *)box_copy_kernel<float, true>);
+    if (e == cudaSuccess) e = cudaFuncGetAttributes(&a, (const void *)box_copy_kernel<float, false>);
+    if (e == cudaSuccess) e = cudaFuncGetAttributes(&a, (const void *)box_copy_kernel<double, true>);
+    if (e == cudaSuccess) e = cudaFuncGetAttributes(&a, (const void *)box_copy_kernel<double, false>);
     return e;
 }
 
@@ -229,14 +200,14 @@ int standin(wrfb200_handle *h, int field, double c, int i0, int i1, int j0, int 
     const unsigned blocks = (unsigned)(rows < 148 * 64 ? rows : 148 * 64);
     const long long jstride = h->pitch3 * (long long)h->kdim, dshift = field == WRFB200_U ? 1 : h->pitch2;
     (void)cudaGetLastError();   // a launch status must not inherit a stale error of some earlier, unrelated call
-    if (h->esize == 8)
-        standin_uv_kernel_r8<<<blocks, threads, 0, h->stream>>>(
-            reinterpret_cast<double *>(h->d[field]), reinterpret_cast<const double *>(h->d[WRFB200_MUDF]), h->pitch3,
-            jstride, h->pitch2, dshift, c, i0 - d.ims, j0 - d.jms, ni, nk, nj);
-    else
-        standin_uv_kernel<<<blocks, threads, 0, h->stream>>>(
-            h->d[field], h->d[WRFB200_MUDF], h->pitch3, jstride, h->pitch2, dshift, (float)c, i0 - d.ims, j0 - d.jms,
-            ni, nk, nj);
+    auto run = [&](auto *f) {
+        using T = std::remove_pointer_t<decltype(f)>;
+        standin_uv_kernel<T><<<blocks, threads, 0, h->stream>>>(f, reinterpret_cast<const T *>(h->d[WRFB200_MUDF]),
+                                                                h->pitch3, jstride, h->pitch2, dshift, (T)c,
+                                                                i0 - d.ims, j0 - d.jms, ni, nk, nj);
+    };
+    if (h->esize == 8) run(reinterpret_cast<double *>(h->d[field]));
+    else run(h->d[field]);
     cudaError_t e = cudaGetLastError();
     if (prev != h->device && prev >= 0) cudaSetDevice(prev);
     if (e != cudaSuccess) return wrfb200_fail(WRFB200_ERR_CUDA, "stand-in kernel launch failed: %s", cudaGetErrorString(e));
