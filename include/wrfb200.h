@@ -172,7 +172,8 @@ int wrfb200_advance_mu_t_loop_r8(
 int wrfb200_set_default_stream(void *cuda_stream);
 int wrfb200_set_default_kernel(int kernel /* wrfb200_kernel */);
 
-/* Release the per-thread device mirrors cached by the host-pointer form (and every host registration). */
+/* Release the per-thread device mirrors cached by the host-pointer form (and every host registration), and the
+ * shared patches of shared-tiles mode (wrfb200_set_shared_tiles) with every thread's state for them. */
 int wrfb200_release_cache(void);
 
 /* Acoustic-loop residency for HOST-pointer callers of wrfb200_advance_mu_t (thread-local).  Between begin and
@@ -211,6 +212,34 @@ int wrfb200_default_last_kernel(int *kernel);
  * n < 0, n > 64, devices == NULL with n > 0, or an id outside [0, device count): WRFB200_ERR_INVALID_ARG; no
  * device at all: WRFB200_ERR_CUDA.  Changing the list releases this thread's cached mirrors. */
 int wrfb200_set_default_devices(const int *devices, int n);
+
+/* Shared-tiles mode, for WRF's OpenMP builds (smpar, dm+sm), which cut a patch into tiles and make the HOST-pointer
+ * call once per tile from the threads of a `!$OMP PARALLEL DO`.  Process-wide and opt-in (default off, or
+ * WRFB200_SHARED_TILES=1); while it is off nothing behaves differently from the per-thread caches described above.
+ * While it is on, host-pointer calls of wrfb200_advance_mu_t / _loop (and the _r8 pair) from ANY thread that pass
+ * the same 26 arrays and the same memory extents are tiles of one patch:
+ *   - One set of device mirrors per (precision, patch device, memory extents, 26 arrays), created by whichever tile
+ *     arrives first.  Each thread keeps its own streams, staging buffers and handle bound to those mirrors, so its
+ *     default stream (synchronised before the call) and kernel choice still apply.
+ *   - The patch device is the calling thread's current device when the mode is enabled (with the environment
+ *     variable: that of the first thread to call wrfb200_acoustic_loop_begin or a host-pointer entry point).
+ *     Every shared call runs there whatever the calling thread's current device is, which is unchanged on return.
+ *   - A tile's call uploads only what no concurrent tile reads or writes: t, mu and ww at level kts (read and
+ *     written by the routine) over the tile's own columns, the read-only inputs over the tile's rows plus the
+ *     one-cell ring.  It downloads the cells it writes, as always.
+ *   - wrfb200_acoustic_loop_begin / _end (from any one thread, e.g. the master in the serial part of solve_em) act
+ *     on every thread: the first call of a tile (its..ite x jts..jte) in the loop uploads that tile's set, later
+ *     calls of the same tile with the same arrays and scalars upload only its rows of u and v plus the ring,
+ *     whichever thread makes them.  The residency contract above applies per tile.
+ *   - Contract: tiles of one patch must not overlap in computed cells (as in the Fortran); the caller changes no
+ *     array while a tile's call runs.  Disabling the mode and wrfb200_release_cache free the shared mirrors and
+ *     every thread's shared-call state: no call may be in flight then.
+ *   - A shared call from a thread whose device list (wrfb200_set_default_devices) names several devices or another
+ *     device than the patch device fails with WRFB200_ERR_UNSUPPORTED.  Device-pointer calls, handles (section 2)
+ *     and the multi-GPU comm path (3b) are not affected.
+ * Enabling without a CUDA device returns WRFB200_ERR_CUDA; enabling again on another device frees the patches of
+ * the previous one. */
+int wrfb200_set_shared_tiles(int enable);
 
 /* Host-only: how a host-pointer call of this tile is split over n parts (1 <= n <= 64).  rows4[4p..4p+3] =
  * {first computed row, last computed row, first memory row, last memory row} of part p (Fortran j; a part

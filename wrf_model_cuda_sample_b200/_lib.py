@@ -76,6 +76,7 @@ PROTOTYPES = {
     "wrfb200_host_unregister_all": (C.c_int, []),
     "wrfb200_default_last_kernel": (C.c_int, [C.POINTER(C.c_int)]),
     "wrfb200_set_default_devices": (C.c_int, [C.POINTER(C.c_int), C.c_int]),
+    "wrfb200_set_shared_tiles": (C.c_int, [C.c_int]),
     "wrfb200_host_split_plan": (C.c_int, [C.POINTER(Domain)] + [C.c_int] * 7 + [C.POINTER(C.c_int)]),
     "wrfb200_upload_constants": (C.c_int, [_P] + [_P] * 17),
     "wrfb200_upload_state": (C.c_int, [_P, _P, _P, _P]),

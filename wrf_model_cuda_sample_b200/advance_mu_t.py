@@ -16,6 +16,7 @@ from __future__ import annotations
 
 import contextlib
 import ctypes as C
+import os
 import threading
 from dataclasses import dataclass, replace
 from types import SimpleNamespace
@@ -423,6 +424,36 @@ def default_devices(devices: Optional[Sequence[int]]):
         yield
     finally:
         set_default_devices(prev)
+
+
+def _env_on(name: str) -> bool:
+    try:
+        return int(os.environ.get(name, "0")) > 0
+    except ValueError:
+        return False
+
+
+_shared_state = {"on": _env_on("WRFB200_SHARED_TILES")}    # the library reads the same variable
+
+
+def set_shared_tiles(enable: bool) -> None:
+    """Process-wide shared-tiles mode (wrfb200_set_shared_tiles): host-array ``advance_mu_t`` calls from any thread
+    with the same arrays and memory extents are tiles of one device-resident patch on the device that is current in
+    the calling thread now, with acoustic-loop residency kept per tile.  Off frees the shared patches; no call may
+    be in flight when it is turned off."""
+    check(lib().wrfb200_set_shared_tiles(int(bool(enable))))
+    _shared_state["on"] = bool(enable)
+
+
+@contextlib.contextmanager
+def shared_tiles(enable: bool = True):
+    """``with shared_tiles():`` -- ``set_shared_tiles`` for the block, then the previous state."""
+    prev = _shared_state["on"]
+    set_shared_tiles(enable)
+    try:
+        yield
+    finally:
+        set_shared_tiles(prev)
 
 
 def host_split_plan(grid: Grid, n: int):

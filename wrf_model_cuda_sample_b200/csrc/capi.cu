@@ -9,6 +9,7 @@
 // returned instead of exit() (:22-32).
 #include <cuda_runtime.h>
 
+#include <atomic>
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
@@ -815,6 +816,7 @@ namespace {
 
 thread_local cudaStream_t g_default_stream = nullptr;
 thread_local int g_default_kernel = WRFB200_KERNEL_AUTO;
+thread_local std::vector<int> g_default_devices;      // wrfb200_set_default_devices; empty: the current device only
 
 constexpr int kMaxSlabs = 16;
 
@@ -856,6 +858,123 @@ struct CompatCache {
     ~CompatCache() { release(); }
 };
 thread_local CompatCache g_cache[2];        // [0]: binary32 calls, [1]: real*8 calls
+
+// the same arrays, index sets and scalars as the call that primed a resident tile
+bool same_call(const Args &p, const Args &a)
+{
+    return std::memcmp(p.f, a.f, sizeof(a.f)) == 0 && std::memcmp(&p.dom, &a.dom, sizeof(a.dom)) == 0 &&
+           p.its == a.its && p.ite == a.ite && p.jts == a.jts && p.jte == a.jte && p.kts == a.kts &&
+           p.kte == a.kte && p.rdx == a.rdx && p.rdy == a.rdy && p.dts == a.dts && p.epssm == a.epssm;
+}
+
+// ---- shared-tiles mode (wrfb200_set_shared_tiles) ----------------------------------------------------
+// The host-array calls of every thread that pass the same 26 arrays and memory extents are tiles of ONE patch:
+// one set of mirrors on the patch device, and acoustic-loop residency kept per tile (its..ite x jts..jte) in the
+// patch rather than per thread, since an OpenMP schedule may hand a tile to another thread each step.  Each thread
+// keeps its own lanes, events, staging buffers and a handle (allocate=0) bound to the shared mirrors, so that no
+// handle field is written by two threads.
+std::atomic<int> g_shared_mode{-1};          // -1: read WRFB200_SHARED_TILES on first use; 0 off; 1 on
+std::atomic<int> g_shared_device{-1};        // the patch device (-1: not yet recorded)
+std::atomic<bool> g_shared_loop{false};      // between wrfb200_acoustic_loop_begin and _end
+std::mutex g_shared_mutex;                   // guards g_shared, g_shared_next_id and g_tile_threads
+
+struct SharedPatch {
+    wrfb200_handle *h = nullptr;             // owns the 26 mirrors
+    int prec = 0;
+    long id = 0;                             // unique in the process: a thread's handle re-binds when it changes
+    void *ptrs[WRFB200_NUM_FIELDS] = {};     // the caller's 26 host arrays
+    std::mutex mutex;                       // guards `primed`
+    std::map<std::tuple<int, int, int, int>, Args> primed;   // tiles whose state is device-resident
+
+    static std::tuple<int, int, int, int> key(const Args &a) { return std::make_tuple(a.its, a.ite, a.jts, a.jte); }
+    // true when this tile was primed by the same call in the current loop; the tile counts as not primed until
+    // this call has completed
+    bool take(const Args &a)
+    {
+        std::lock_guard<std::mutex> lock(mutex);
+        auto it = primed.find(key(a));
+        if (it == primed.end()) return false;
+        const bool same = same_call(it->second, a);
+        primed.erase(it);
+        return same && g_shared_loop.load();
+    }
+    void put(const Args &a)
+    {
+        std::lock_guard<std::mutex> lock(mutex);
+        primed[key(a)] = a;
+    }
+    void forget()
+    {
+        std::lock_guard<std::mutex> lock(mutex);
+        primed.clear();
+    }
+};
+std::vector<std::unique_ptr<SharedPatch>> g_shared;
+long g_shared_next_id = 1;
+
+// A thread's state for shared calls, listed process-wide so that wrfb200_set_shared_tiles(0) and
+// wrfb200_release_cache can free it whichever thread calls them.
+struct TileThread;
+std::vector<TileThread *> g_tile_threads;
+struct TileThread {
+    CompatCache c[2];                        // indexed like g_cache
+    long bound[2] = {0, 0};                  // SharedPatch::id the handle's fields are bound to (0: none)
+    bool listed = false;
+    void enlist()
+    {
+        if (listed) return;
+        std::lock_guard<std::mutex> lock(g_shared_mutex);
+        g_tile_threads.push_back(this);
+        listed = true;
+    }
+    void release()
+    {
+        for (int p = 0; p < 2; ++p) { c[p].release(); bound[p] = 0; }
+    }
+    ~TileThread()
+    {
+        std::lock_guard<std::mutex> lock(g_shared_mutex);
+        for (size_t x = 0; x < g_tile_threads.size(); ++x)
+            if (g_tile_threads[x] == this) { g_tile_threads.erase(g_tile_threads.begin() + x); break; }
+        release();
+    }
+};
+thread_local TileThread g_tiles;
+
+bool shared_enabled()
+{
+    int m = g_shared_mode.load();
+    if (m < 0) {
+        const char *e = getenv("WRFB200_SHARED_TILES");
+        g_shared_mode.compare_exchange_strong(m, (e && atoi(e) > 0) ? 1 : 0);
+        m = g_shared_mode.load();
+    }
+    return m == 1;
+}
+
+// The patch device.  wrfb200_set_shared_tiles(1) records it; when the environment turned the mode on, the first
+// thread that asks (wrfb200_acoustic_loop_begin or a host-array call) records its current device.
+int shared_device(int *dev)
+{
+    int d = g_shared_device.load();
+    if (d < 0) {
+        int cur = 0;
+        CU(cudaGetDevice(&cur));
+        g_shared_device.compare_exchange_strong(d, cur);
+        d = g_shared_device.load();
+    }
+    *dev = d;
+    return WRFB200_OK;
+}
+
+// frees every shared patch and every thread's state for shared calls; no call may be in flight
+void release_shared()
+{
+    std::lock_guard<std::mutex> lock(g_shared_mutex);
+    for (TileThread *t : g_tile_threads) t->release();
+    for (auto &sp : g_shared) wrfb200_destroy(sp->h);
+    g_shared.clear();
+}
 
 // Device-pointer callers: the handle that wraps the caller's arrays (and its six TMA tensor maps) is kept
 // between calls and re-used while the pointers and extents stay the same -- a 25-830 us step must not pay
@@ -973,9 +1092,20 @@ int run_device_in_place(const Args &a, int prec)
 // previous output or a loop constant) -- the per-small-step drop-in pattern of a host-resident model:
 // 0.76 GB up and 1.15 GB down per step on 1800x1060x50 instead of 3.2 GB up.
 //
-// `part`: this is one device's share of a split call (run_host_split), whose calling thread has already
-// synchronised the caller's stream and page-locked the caller's whole arrays.
-int run_host_compat_body(const Args &a, int nsteps, wrfb200_handle *h, CompatCache &cc, bool part)
+// `part`: this is one device's share of a split call (run_host_split), or a shared-tiles call (run_host_shared),
+// whose calling thread has already synchronised the caller's stream and page-locked the caller's whole arrays.
+//
+// `sp`: a tile of a shared patch (shared-tiles mode), whose mirrors other threads' tiles read and write
+// concurrently.  A tile then writes to the device only what no other tile reads or writes in between:
+//   - t, mu and ww at level kts (the fields the routine reads AND writes, each read at its own column only):
+//     the tile's own columns i_start..i_end x j_start..j_end.  The full-field mu / ww copies and the ring rows
+//     of t would overwrite a neighbouring tile's fresh outputs;
+//   - the read-only inputs: the tile's rows plus the one-cell ring (all of i), 2-D ones over the same rows.  Two
+//     tiles that both copy a ring row write the same bytes from the same host array, which the caller does not
+//     change during the loop's steps (u, v only between them); that is why those copies may overlap;
+//   - residency is kept per tile in `sp` (SharedPatch::take / put), whichever thread makes the call.
+int run_host_compat_body(const Args &a, int nsteps, wrfb200_handle *h, CompatCache &cc, bool part,
+                         SharedPatch *sp = nullptr)
 {
     const wrfb200_domain &d = a.dom;
     int is, ie, js, je, ks, ke;
@@ -991,6 +1121,8 @@ int run_host_compat_body(const Args &a, int nsteps, wrfb200_handle *h, CompatCac
     static const int in3_all[] = {WRFB200_WW_1, WRFB200_U, WRFB200_U_1, WRFB200_V, WRFB200_V_1,
                                   WRFB200_T, WRFB200_T_1, WRFB200_FT};
     static const int in3_uv[] = {WRFB200_U, WRFB200_V};
+    static const int in3_ring[] = {WRFB200_WW_1, WRFB200_U, WRFB200_U_1, WRFB200_V, WRFB200_V_1,
+                                   WRFB200_T_1, WRFB200_FT};      // shared tiles: the read-only ones (t per slab)
     static const int in2[] = {WRFB200_MU, WRFB200_MUT, WRFB200_MUU, WRFB200_MUV, WRFB200_MU_TEND,
                               WRFB200_MSFUY, WRFB200_MSFVX_INV, WRFB200_MSFTX, WRFB200_MSFTY};
     static const int in1[] = {WRFB200_DNW, WRFB200_FNM, WRFB200_FNP, WRFB200_RDNW};
@@ -998,15 +1130,10 @@ int run_host_compat_body(const Args &a, int nsteps, wrfb200_handle *h, CompatCac
     static const int out2[] = {WRFB200_MU, WRFB200_MUAVE, WRFB200_MUTS, WRFB200_MUDF};
 
     // resident step: same arrays, same index sets, same scalars as the call that primed the mirrors
-    const bool resident = cc.loop_active && cc.primed && std::memcmp(cc.primed_args.f, a.f, sizeof(a.f)) == 0 &&
-                          same_domain(cc.primed_args.dom, a.dom) && cc.primed_args.its == a.its &&
-                          cc.primed_args.ite == a.ite && cc.primed_args.jts == a.jts && cc.primed_args.jte == a.jte &&
-                          cc.primed_args.kts == a.kts && cc.primed_args.kte == a.kte &&
-                          cc.primed_args.rdx == a.rdx && cc.primed_args.rdy == a.rdy &&
-                          cc.primed_args.dts == a.dts && cc.primed_args.epssm == a.epssm;
+    const bool resident = sp ? sp->take(a) : cc.loop_active && cc.primed && same_call(cc.primed_args, a);
     cc.primed = false;                                    // until this call has completed
-    const int *in3 = resident ? in3_uv : in3_all;
-    const int n_in3 = resident ? 2 : 8;
+    const int *in3 = resident ? in3_uv : sp ? in3_ring : in3_all;
+    const int n_in3 = resident ? 2 : sp ? 7 : 8;
 
     if (pin_enabled() && !part)
         for (int f = 0; f < WRFB200_NUM_FIELDS; ++f) pin_host(a.f[f], field_bytes(d, f, h->esize));
@@ -1014,10 +1141,17 @@ int run_host_compat_body(const Args &a, int nsteps, wrfb200_handle *h, CompatCac
     // small operands first: 2-D and 1-D inputs, and ww at level 1 (the only level of ww the routine
     // reads, module_small_step_em.f90:159-161)
     h->stream = cc.up;
-    if (!resident) {
+    if (!resident && !sp) {
         for (int f : in2) if (int rc = copy_field(h, f, a.f[f], nullptr)) return rc;
         for (int f : in1) if (int rc = copy_field(h, f, a.f[f], nullptr)) return rc;
         if (int rc = copy_range(h, WRFB200_WW, a.f[WRFB200_WW], nullptr, d.ims, d.ime, a.kts, a.kts, d.jms, d.jme)) return rc;
+    } else if (!resident) {
+        for (int f : in2)
+            if (f != WRFB200_MU)
+                if (int rc = copy_range(h, f, a.f[f], nullptr, d.ims, d.ime, 0, 0, js - 1, je + 1)) return rc;
+        for (int f : in1) if (int rc = copy_field(h, f, a.f[f], nullptr)) return rc;
+        if (int rc = copy_range(h, WRFB200_MU, a.f[WRFB200_MU], nullptr, is, ie, 0, 0, js, je)) return rc;
+        if (int rc = copy_range(h, WRFB200_WW, a.f[WRFB200_WW], nullptr, is, ie, a.kts, a.kts, js, je)) return rc;
     }
 
     const int nj = je - js + 1;
@@ -1065,6 +1199,9 @@ int run_host_compat_body(const Args &a, int nsteps, wrfb200_handle *h, CompatCac
             }
             next_row = hi + 1;
         }
+        // shared tiles: t over the slab's own columns (all levels: no tile reads or writes t outside its columns)
+        if (sp && !resident)
+            if (int rc = copy_range(h, WRFB200_T, a.f[WRFB200_T], nullptr, is, ie, d.kms, d.kme, ja, jb)) return rc;
         CU(cudaEventRecord(cc.ev_up[s], cc.up));
         // all steps of this slab
         CU(cudaStreamWaitEvent(cc.comp, cc.ev_up[s], 0));
@@ -1081,7 +1218,12 @@ int run_host_compat_body(const Args &a, int nsteps, wrfb200_handle *h, CompatCac
     CU(cudaStreamSynchronize(cc.up));
     CU(cudaStreamSynchronize(cc.comp));
     CU(cudaStreamSynchronize(cc.down));
-    if (cc.loop_active) { cc.primed = true; cc.primed_args = a; }
+    if (sp) {
+        if (g_shared_loop.load()) sp->put(a);
+    } else if (cc.loop_active) {
+        cc.primed = true;
+        cc.primed_args = a;
+    }
     return WRFB200_OK;
 }
 
@@ -1089,26 +1231,29 @@ int run_host_compat_body(const Args &a, int nsteps, wrfb200_handle *h, CompatCac
 // current device, and a cache of the same memory shape is re-used wherever it lives (the single-device call);
 // device >= 0: the cache is re-created when it lives on another device.  `kernel` is the calling thread's
 // choice, passed in because a part may run in a worker thread.
-int run_host_part(const Args &a, int nsteps, int prec, CompatCache &cc, int device, int kernel, bool part)
+// The cache's handle (mirrors allocated or, with allocate=0, to be bound) and its lanes and events.
+int open_cache(CompatCache &cc, const wrfb200_domain &dom, int device, int allocate, int prec)
 {
-    if (int rc = check_domain(a.dom)) return rc;
-    if (cc.h && (!same_shape(cc.h->dom, a.dom) || (device >= 0 && cc.h->device != device))) cc.release();
-    if (!cc.h) {
-        if (int rc = create(&cc.h, &a.dom, device, 1, prec ? 8 : 4)) return rc;
-        DeviceGuard g(cc.h->device);
-        for (cudaStream_t *st : {&cc.up, &cc.comp, &cc.down})
-            CU(cudaStreamCreateWithFlags(st, cudaStreamNonBlocking));
-        for (int i = 0; i < kMaxSlabs; ++i) {
-            CU(cudaEventCreateWithFlags(&cc.ev_up[i], cudaEventDisableTiming));
-            CU(cudaEventCreateWithFlags(&cc.ev_comp[i], cudaEventDisableTiming));
-        }
+    if (int rc = create(&cc.h, &dom, device, allocate, prec ? 8 : 4)) return rc;
+    DeviceGuard g(cc.h->device);
+    for (cudaStream_t *st : {&cc.up, &cc.comp, &cc.down})
+        CU(cudaStreamCreateWithFlags(st, cudaStreamNonBlocking));
+    for (int i = 0; i < kMaxSlabs; ++i) {
+        CU(cudaEventCreateWithFlags(&cc.ev_up[i], cudaEventDisableTiming));
+        CU(cudaEventCreateWithFlags(&cc.ev_comp[i], cudaEventDisableTiming));
     }
+    return WRFB200_OK;
+}
+
+// run_host_compat_body on the cache's handle, with the calling thread's kernel choice and the call's scalars
+int run_on_cache(const Args &a, int nsteps, CompatCache &cc, int kernel, bool part, SharedPatch *sp)
+{
     wrfb200_handle *h = cc.h;
     GUARD(h);
     h->dom = a.dom;                       // same extents; domain dims / flags may differ between calls
     h->kernel = kernel;
     set_scalars(h, a.rdx, a.rdy, a.dts, a.epssm);
-    const int rc = run_host_compat_body(a, nsteps, h, cc, part);
+    const int rc = run_host_compat_body(a, nsteps, h, cc, part, sp);
     if (rc != WRFB200_OK) {
         // an early return must not leave copies on the caller's arrays in flight, nor the cached handle
         // pointing at one of the internal lanes
@@ -1122,10 +1267,68 @@ int run_host_part(const Args &a, int nsteps, int prec, CompatCache &cc, int devi
     return rc;
 }
 
+int run_host_part(const Args &a, int nsteps, int prec, CompatCache &cc, int device, int kernel, bool part)
+{
+    if (int rc = check_domain(a.dom)) return rc;
+    if (cc.h && (!same_shape(cc.h->dom, a.dom) || (device >= 0 && cc.h->device != device))) cc.release();
+    if (!cc.h)
+        if (int rc = open_cache(cc, a.dom, device, 1, prec)) return rc;
+    return run_on_cache(a, nsteps, cc, kernel, part, nullptr);
+}
+
+// One host-pointer call in shared-tiles mode: a tile of the shared patch of these arrays on the patch device,
+// created by whichever tile comes first, run from this thread's own lanes and handle.
+int run_host_shared(const Args &a, int nsteps, int prec)
+{
+    if (int rc = check_domain(a.dom)) return rc;
+    int dev = 0;
+    if (int rc = shared_device(&dev)) return rc;
+    if (!g_default_devices.empty() && (g_default_devices.size() > 1 || g_default_devices[0] != dev))
+        return fail(WRFB200_ERR_UNSUPPORTED,
+                    "shared-tiles mode runs every host-array call on the patch device %d; this thread's device list "
+                    "(wrfb200_set_default_devices: %zu device(s), first %d) names another or several",
+                    dev, g_default_devices.size(), g_default_devices[0]);
+    CU(cudaStreamSynchronize(g_default_stream));          // the caller's earlier work on its stream is done
+    const size_t es = prec ? 8 : 4;
+    if (pin_enabled())
+        for (int f = 0; f < WRFB200_NUM_FIELDS; ++f) pin_host(a.f[f], field_bytes(a.dom, f, es));
+
+    SharedPatch *sp = nullptr;
+    {
+        std::lock_guard<std::mutex> lock(g_shared_mutex);
+        for (auto &q : g_shared)
+            if (q->prec == prec && q->h->device == dev && same_shape(q->h->dom, a.dom) &&
+                std::memcmp(q->ptrs, a.f, sizeof(a.f)) == 0) { sp = q.get(); break; }
+        if (!sp) {
+            std::unique_ptr<SharedPatch> q(new (std::nothrow) SharedPatch());
+            if (!q) return fail(WRFB200_ERR_NOMEM, "out of host memory");
+            if (int rc = create(&q->h, &a.dom, dev, 1, (int)es)) return rc;
+            q->prec = prec;
+            q->id = g_shared_next_id++;
+            std::memcpy(q->ptrs, a.f, sizeof(a.f));
+            sp = q.get();
+            g_shared.push_back(std::move(q));
+        }
+    }
+
+    TileThread &tt = g_tiles;
+    tt.enlist();
+    CompatCache &cc = tt.c[prec];
+    if (cc.h && (!same_shape(cc.h->dom, a.dom) || cc.h->device != dev)) { cc.release(); tt.bound[prec] = 0; }
+    if (!cc.h)
+        if (int rc = open_cache(cc, a.dom, dev, 0, prec)) return rc;
+    if (tt.bound[prec] != sp->id) {
+        tt.bound[prec] = 0;
+        for (int f = 0; f < WRFB200_NUM_FIELDS; ++f)
+            if (int rc = bind_device(cc.h, f, sp->h->d[f], is3d(f) ? sp->h->pitch3 : sp->h->pitch2)) return rc;
+        tt.bound[prec] = sp->id;
+    }
+    return run_on_cache(a, nsteps, cc, g_default_kernel, true, sp);
+}
+
 // ---- one host-pointer call split over several devices (wrfb200_set_default_devices) --------------------
 constexpr int kMaxParts = 64;
 
-thread_local std::vector<int> g_default_devices;                         // empty: the current device only
 // parts 1.. of a split call (part 0 is g_cache), indexed like g_cache
 thread_local std::vector<std::unique_ptr<CompatCache>> g_parts[2];
 
@@ -1230,6 +1433,7 @@ int run_host_split(const Args &a, int nsteps, int prec)
 
 int run_host_compat(const Args &a, int nsteps, int prec)
 {
+    if (shared_enabled()) return run_host_shared(a, nsteps, prec);
     if (!g_default_devices.empty()) {
         int cur = 0;
         CU(cudaGetDevice(&cur));
@@ -1416,16 +1620,33 @@ extern "C" int wrfb200_host_split_plan(const wrfb200_domain *dom, int its, int i
 extern "C" int wrfb200_release_cache(void)
 {
     release_parts();
+    release_shared();
     for (DeviceCallCache &c : g_devcall) c.valid = false;
     unpin_all();
     return WRFB200_OK;
 }
+
+namespace {
+
+// the shared patches' residency follows the loop whichever thread begins or ends it
+void shared_loop(bool active)
+{
+    if (!shared_enabled()) return;
+    int dev = 0;
+    if (active && shared_device(&dev) != WRFB200_OK) (void)cudaGetLastError();   // records the patch device
+    g_shared_loop.store(active);
+    std::lock_guard<std::mutex> lock(g_shared_mutex);
+    for (auto &sp : g_shared) sp->forget();
+}
+
+}  // namespace
 
 extern "C" int wrfb200_acoustic_loop_begin(void)
 {
     for (CompatCache &c : g_cache) { c.loop_active = true; c.primed = false; }
     for (auto &pool : g_parts)
         for (auto &c : pool) { c->loop_active = true; c->primed = false; }
+    shared_loop(true);
     return WRFB200_OK;
 }
 
@@ -1434,6 +1655,27 @@ extern "C" int wrfb200_acoustic_loop_end(void)
     for (CompatCache &c : g_cache) { c.loop_active = false; c.primed = false; }
     for (auto &pool : g_parts)
         for (auto &c : pool) { c->loop_active = false; c->primed = false; }
+    shared_loop(false);
+    return WRFB200_OK;
+}
+
+extern "C" int wrfb200_set_shared_tiles(int enable)
+{
+    if (!enable) {
+        g_shared_mode.store(0);
+        g_shared_device.store(-1);
+        release_shared();
+        return WRFB200_OK;
+    }
+    int ndev = 0, dev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0 || cudaGetDevice(&dev) != cudaSuccess) {
+        cudaGetLastError();
+        return fail(WRFB200_ERR_CUDA, "no CUDA device available (this library has no CPU fallback)");
+    }
+    if (g_shared_mode.load() == 1 && g_shared_device.load() == dev) return WRFB200_OK;
+    release_shared();                                      // patches of another device, if any
+    g_shared_device.store(dev);
+    g_shared_mode.store(1);
     return WRFB200_OK;
 }
 
@@ -1485,7 +1727,7 @@ extern "C" int wrfb200_default_last_kernel(int *kernel)
 {
     if (!kernel) return fail(WRFB200_ERR_INVALID_ARG, "null argument");
     const DeviceCallCache &dc = g_devcall[g_last_prec];
-    const CompatCache &cc = g_cache[g_last_prec];
+    const CompatCache &cc = shared_enabled() ? g_tiles.c[g_last_prec] : g_cache[g_last_prec];
     *kernel = dc.valid ? dc.h.last_kernel : (cc.h ? cc.h->last_kernel : 0);
     return WRFB200_OK;
 }

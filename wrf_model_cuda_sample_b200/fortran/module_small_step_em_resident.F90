@@ -107,6 +107,14 @@ INTERFACE
       IMPORT :: c_int
       INTEGER(c_int) :: status
    END FUNCTION
+   ! OpenMP builds (smpar, dm+sm): the tiles of the !$OMP PARALLEL DO share one device-resident patch.  Call once,
+   ! after the rank has picked its GPU; the loop begin / end and the per-tile advance_mu_t calls are unchanged
+   ! (INTEGRATION.md section 1)
+   FUNCTION wrfb200_set_shared_tiles(enable) BIND(C, NAME="wrfb200_set_shared_tiles") RESULT(status)
+      IMPORT :: c_int
+      INTEGER(c_int), VALUE :: enable
+      INTEGER(c_int) :: status
+   END FUNCTION
    ! the host-array call split over several GPUs of the box: call once at start-up (e.g. ids 0..7 on an
    ! 8-GPU box), the advance_mu_t call itself is unchanged
    FUNCTION wrfb200_set_default_devices(devices, n) BIND(C, NAME="wrfb200_set_default_devices") RESULT(status)
