@@ -384,16 +384,31 @@ int wrfb200_standin_advance_uv_r8(wrfb200_handle *h, int field, double c, int i0
  *     the double2 tile kernel with the exchange fused in, so wrfb200_comm_init_r8 fails with
  *     WRFB200_ERR_UNSUPPORTED when the patch has more than 220 computed levels.  All ranks must hold the same
  *     precision: connect rejects a neighbour's blob of the other one with WRFB200_ERR_INVALID_ARG.
+ *
+ *     Periodic domains (WRF's periodic_x, and periodic_x + periodic_y on an open domain): call
+ *     wrfb200_comm_set_wrap before wrfb200_comm_init[_r8] to make the exchange cyclic across the domain edge, so
+ *     the ring of a periodic domain is refreshed inside the loop as WRF refreshes it every small step
+ *     (u(ide) = u(ids), t_1(ids-1) = t_1(ide-1), t_1(ide) = t_1(ids), the same in j, and mu, muts, mudf after the
+ *     step).  Without the call an edge rank's ring past the domain edge is never written.  wrap_x needs the
+ *     domain's periodic_x; wrap_y needs specified == 0 and nested == 0.  The patches follow WRF's convention: the
+ *     west-edge rank starts at ids, the east-edge rank ends at ide and computes at least one column (likewise in
+ *     j); that rank's column ide (row jde) receives the wrap.  px = 1 (py = 1) makes a rank its own neighbour,
+ *     which costs one extra copy launch per step.  comm_init fails with WRFB200_ERR_INVALID_ARG on a request that
+ *     breaks these rules, connect on a neighbour with other wrap flags or other global extents.  The stand-in
+ *     advance_uv then updates u from i_start (v from j_start) on a wrapped axis.
  * ---------------------------------------------------------------------------------------------- */
 #define WRFB200_COMM_INFO_BYTES 2048
 int wrfb200_comm_info_bytes(void);
+/* periodic wrap of the exchange (0/1 each); before wrfb200_comm_init / _init_r8, kept for both precisions */
+int wrfb200_comm_set_wrap(wrfb200_handle *h, int wrap_x, int wrap_y);
 int wrfb200_comm_init(wrfb200_handle *h, int px, int py, int rank,
                       int ips, int ipe, int jps, int jpe, void *info_out /* WRFB200_COMM_INFO_BYTES */);
 int wrfb200_comm_connect(wrfb200_handle *h, const void *all_infos /* nranks blobs, rank order */, int nranks);
 int wrfb200_comm_barrier(wrfb200_handle *h);          /* stream-ordered barrier with the neighbours */
 int wrfb200_comm_push_constants(wrfb200_handle *h);
-int wrfb200_comm_push_uv(wrfb200_handle *h);          /* u west column -> west neighbour (px > 1); the v south row is
-                                                         pushed by wrfb200_comm_step itself */
+int wrfb200_comm_push_uv(wrfb200_handle *h);          /* u west column -> west neighbour (px > 1, or wrap_x); the v
+                                                         south row is pushed by wrfb200_comm_step itself, except to a
+                                                         rank that is its own south neighbour (wrap_y, py = 1) */
 int wrfb200_comm_wait_outputs(wrfb200_handle *h);     /* west / south halos of mu, muts, mudf have arrived */
 int wrfb200_comm_step(wrfb200_handle *h);             /* advance_mu_t over the patch, fused with its exchange */
 /* stand-in advance_uv (see wrfb200_standin_advance_uv) over this patch's share of the global update boxes,

@@ -117,6 +117,7 @@ PROTOTYPES = {
     "wrfb200_standin_advance_uv": (C.c_int, [_P, C.c_int, C.c_float] + [C.c_int] * 4),
     "wrfb200_standin_advance_uv_r8": (C.c_int, [_P, C.c_int, C.c_double] + [C.c_int] * 4),
     "wrfb200_comm_info_bytes": (C.c_int, []),
+    "wrfb200_comm_set_wrap": (C.c_int, [_P, C.c_int, C.c_int]),
     "wrfb200_comm_init": (C.c_int, [_P, C.c_int, C.c_int, C.c_int] + [C.c_int] * 4 + [_P]),
     "wrfb200_comm_connect": (C.c_int, [_P, _P, C.c_int]),
     "wrfb200_comm_barrier": (C.c_int, [_P]),

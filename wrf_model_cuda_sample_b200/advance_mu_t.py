@@ -335,6 +335,10 @@ class Patch:
         check(self._fn("wrfb200_standin_advance_uv")(self._h, FIELD_ID[field], float(c), i0, i1, j0, j1))
 
     # ---- multi-GPU: halo exchange fused into the kernels over peer-mapped memory (csrc/comm.cu) ----
+    def comm_set_wrap(self, wrap_x: bool, wrap_y: bool) -> None:
+        """Periodic exchange across the domain edge (WRF's periodic_x / periodic_y); call before comm_init."""
+        check(lib().wrfb200_comm_set_wrap(self._h, int(bool(wrap_x)), int(bool(wrap_y))))
+
     def comm_init(self, px: int, py: int, rank: int, ips, ipe, jps, jpe) -> bytes:
         """-> this rank's opaque info blob; all-gather the blobs in rank order and pass them to comm_connect."""
         n = lib().wrfb200_comm_info_bytes()

@@ -28,6 +28,7 @@ struct wrfb200_handle {
     // graphs keyed by (its, ite, jts, jte, kte, nsteps, kernel)
     std::map<std::tuple<int, int, int, int, int, int, int>, cudaGraphExec_t> graphs;
     wrfb200_comm *comm = nullptr;      // non-null after wrfb200_comm_init
+    int wrap_x = 0, wrap_y = 0;        // periodic exchange across the domain edge (wrfb200_comm_set_wrap)
 };
 
 // capi.cu: kernel argument block for a tile / kernel launch (shared with comm.cu)

@@ -41,6 +41,14 @@
 // the double2 tile kernel with the exchange fused in (amt_tile_kernel_r8<TJ, true>, amt_tile_r8.cu), the peer
 // addresses are computed with the element size, and push_kernel moves double edges as pairs of 4-byte words.  Both
 // ranks of a pair must hold the same precision (checked at connect).
+//
+// Periodic wrap (wrfb200_comm_set_wrap): on a wrapped axis the neighbours are cyclic and the edge rank's column ide
+// (row jde) is the cell that receives the wrap -- WRF's u(ide) = u(ids) -- so that rank exchanges over ips..ide-1
+// (jps..jde-1) as if its patch ended there.  A peer then addresses a cell at my Fortran index + (di, dj), the period
+// on a wrapped side and 0 otherwise.  A rank can be its own neighbour (px = 1 or py = 1): no flag wait may depend on
+// a block of the same launch, so a self side is served by stream order alone -- its u / v edge goes through
+// push_kernel before the step, its outputs are plain stores into this rank's own arrays, and it has no wait and no
+// signal.  With px = 2 (py = 2) the same rank sits on both sides and uses the two per-side flag slots.
 #include <unistd.h>
 
 #include <cstdint>
@@ -76,7 +84,9 @@ struct CommInfo {
     int esize;                       // bytes per element: 4 (binary32) or 8 (real*8); neighbours must agree
     uint64_t host_id;
     int ims, ime, jms, jme, kms, kme;
-    int ips, ipe, jps, jpe;
+    int ips, ipe, jps, jpe;          // exchange extents (ipe = ide-1 / jpe = jde-1 on a wrapped edge)
+    int wrap_x, wrap_y;
+    int ids, ide, jds, jde;
     long long pitch3, pitch2;
     uint64_t ptr[kNX + 1];           // device addresses in the exporting process (last: flag block)
     uint64_t offset[kNX + 1];        // address - base of its allocation (IPC handles name allocations)
@@ -86,6 +96,8 @@ static_assert(sizeof(CommInfo) <= WRFB200_COMM_INFO_BYTES, "info blob too small"
 
 struct Peer {
     bool present = false;
+    bool self = false;               // this rank is its own neighbour on that side: stream order, no flags
+    int di = 0, dj = 0;              // the peer's Fortran index of my cell (i, j) is (i + di, j + dj)
     CommInfo info{};
     float *f[WRFB200_NUM_FIELDS] = {};
     unsigned *flags = nullptr;
@@ -148,7 +160,8 @@ std::mutex &ipc_mutex()
 
 struct wrfb200_comm {
     int px = 1, py = 1, rank = 0, nranks = 1;
-    int ips = 0, ipe = 0, jps = 0, jpe = 0;
+    int ips = 0, ipe = 0, jps = 0, jpe = 0;    // exchange extents
+    int wrap_x = 0, wrap_y = 0;
     int nbr[4] = {-1, -1, -1, -1};
     Peer peer[4];
     unsigned *flags = nullptr;                 // this rank's flag block (device memory)
@@ -326,7 +339,7 @@ Box edge_box(const wrfb200_handle *h, const Peer &pr, int field, int side)
     }
     Box b{};
     b.src = h->d[field] + ((long long)(j0 - d.jms) * sj + (i0 - d.ims)) * w;
-    b.dst = pr.f[field] + ((long long)(j0 - q.jms) * dj + (i0 - q.ims)) * w;
+    b.dst = pr.f[field] + ((long long)(j0 + pr.dj - q.jms) * dj + (i0 + pr.di - q.ims)) * w;
     b.sp = sp * w; b.sj = sj * w; b.dp = dp * w; b.dj = dj * w;
     b.ni = (i1 - i0 + 1) * w; b.nk = nk; b.nj = j1 - j0 + 1;
     return b;
@@ -395,7 +408,8 @@ int map_peer(wrfb200_handle *h, Peer *pr)
 }
 
 // the advance_uv stand-in boxes of this patch: u over i_start+1..i_end, v over j_start+1..j_end of the
-// GLOBAL computed range (tests/cases.py standin_boxes)
+// GLOBAL computed range (tests/cases.py standin_boxes); on a wrapped axis from i_start / j_start, whose mudf at
+// i-1 / j-1 is the wrapped ring
 void standin_boxes(const wrfb200_handle *h, int ub[4], int vb[4])
 {
     const wrfb200_domain &d = h->dom;
@@ -405,8 +419,9 @@ void standin_boxes(const wrfb200_handle *h, int ub[4], int vb[4])
                    d.ids, d.ide, d.jds, d.jde, 1, d.kde, &gi0, &gi1, &gj0, &gj1, &k0, &k1);
     auto mx = [](int a, int b) { return a > b ? a : b; };
     auto mn = [](int a, int b) { return a < b ? a : b; };
-    ub[0] = mx(c->ips, gi0 + 1); ub[1] = mn(c->ipe, gi1); ub[2] = mx(c->jps, gj0); ub[3] = mn(c->jpe, gj1);
-    vb[0] = mx(c->ips, gi0); vb[1] = mn(c->ipe, gi1); vb[2] = mx(c->jps, gj0 + 1); vb[3] = mn(c->jpe, gj1);
+    const int su = c->wrap_x ? 0 : 1, sv = c->wrap_y ? 0 : 1;
+    ub[0] = mx(c->ips, gi0 + su); ub[1] = mn(c->ipe, gi1); ub[2] = mx(c->jps, gj0); ub[3] = mn(c->jpe, gj1);
+    vb[0] = mx(c->ips, gi0); vb[1] = mn(c->ipe, gi1); vb[2] = mx(c->jps, gj0 + sv); vb[3] = mn(c->jpe, gj1);
 }
 
 int enqueue_push_uv(wrfb200_handle *h, cudaStream_t s, unsigned index)
@@ -416,12 +431,16 @@ int enqueue_push_uv(wrfb200_handle *h, cudaStream_t s, unsigned index)
     const Peer &w = c->peer[WRFB200_WEST];
     if (w.present) {
         a.box[a.nbox++] = edge_box(h, w, WRFB200_U, WRFB200_WEST);
-        a.wait0 = c->flags + F_OUT_W;
-        a.sig0 = w.flags + F_UV_E;
+        if (!w.self) {
+            a.wait0 = c->flags + F_OUT_W;
+            a.sig0 = w.flags + F_UV_E;
+        }
     }
     // (the v south row goes to the south neighbour from inside advance_mu_t itself: its south-row blocks push it
     // before they start, amt_pipe.cu for binary32 and amt_tile_r8.cu for real*8 -- no separate launch for j-slab
-    // decompositions)
+    // decompositions.  A self south side cannot: its north-row blocks, which read that row, run in the same launch.)
+    const Peer &so = c->peer[WRFB200_SOUTH];
+    if (so.present && so.self) a.box[a.nbox++] = edge_box(h, so, WRFB200_V, WRFB200_SOUTH);
     if (a.nbox == 0) return WRFB200_OK;
     a.epoch = c->flags + F_EPOCH;
     a.index = index;
@@ -437,8 +456,9 @@ int enqueue_push_uv(wrfb200_handle *h, cudaStream_t s, unsigned index)
 int enqueue_wait_outputs(wrfb200_handle *h, cudaStream_t s, unsigned done_index)
 {
     wrfb200_comm *c = h->comm;
-    const unsigned *w0 = c->peer[WRFB200_WEST].present ? c->flags + F_OUT_W : nullptr;
-    const unsigned *w1 = c->peer[WRFB200_SOUTH].present ? c->flags + F_OUT_S : nullptr;
+    auto waits = [&](int side) { return c->peer[side].present && !c->peer[side].self; };   // a self side: stream order
+    const unsigned *w0 = waits(WRFB200_WEST) ? c->flags + F_OUT_W : nullptr;
+    const unsigned *w1 = waits(WRFB200_SOUTH) ? c->flags + F_OUT_S : nullptr;
     if (!w0 && !w1) return WRFB200_OK;
     (void)cudaGetLastError();
     wait_outputs_kernel<<<1, 32, 0, s>>>(w0, w1, c->flags + F_EPOCH, done_index, c->flags + F_STATUS, c->timeout_ns);
@@ -543,6 +563,27 @@ int comm_init(wrfb200_handle *h, int px, int py, int rank, int ips, int ipe, int
         return wrfb200_fail(WRFB200_ERR_INVALID_ARG,
                             "patch i=%d..%d j=%d..%d needs a one-cell halo inside memory i=%d..%d j=%d..%d",
                             ips, ipe, jps, jpe, d.ims, d.ime, d.jms, d.jme);
+    const int pi = rank % px, pj = rank / px;
+    if (h->wrap_x) {
+        if (!d.periodic_x)
+            return wrfb200_fail(WRFB200_ERR_INVALID_ARG, "wrap_x needs a periodic_x domain");
+        if ((pi == 0 && ips != d.ids) || (pi == px - 1 && (ipe != d.ide || ipe - 1 < ips)))
+            return wrfb200_fail(WRFB200_ERR_INVALID_ARG, "wrap_x: rank %d (i=%d..%d) must start at ids=%d when on the "
+                                "west edge, and end at ide=%d with at least one computed column when on the east edge",
+                                rank, ips, ipe, d.ids, d.ide);
+    }
+    if (h->wrap_y) {
+        if (d.specified || d.nested)
+            return wrfb200_fail(WRFB200_ERR_INVALID_ARG, "wrap_y needs specified == 0 and nested == 0: otherwise the "
+                                "j range is clamped at the domain edge");
+        if ((pj == 0 && jps != d.jds) || (pj == py - 1 && (jpe != d.jde || jpe - 1 < jps)))
+            return wrfb200_fail(WRFB200_ERR_INVALID_ARG, "wrap_y: rank %d (j=%d..%d) must start at jds=%d when on the "
+                                "south edge, and end at jde=%d with at least one computed row when on the north edge",
+                                rank, jps, jpe, d.jds, d.jde);
+    }
+    // on a wrapped axis the edge rank's column ide / row jde receives the wrap: it is halo to the exchange
+    if (h->wrap_x && pi == px - 1) ipe = d.ide - 1;
+    if (h->wrap_y && pj == py - 1) jpe = d.jde - 1;
     for (int x = 0; x < kNX; ++x)
         if (!h->d[kXf[x]] || !h->owned[kXf[x]])
             return wrfb200_fail(WRFB200_ERR_STATE, "field %d must be a handle-owned mirror (wrfb200_create with allocate=1): "
@@ -556,11 +597,11 @@ int comm_init(wrfb200_handle *h, int px, int py, int rank, int ips, int ipe, int
     h->comm = c;
     c->px = px; c->py = py; c->rank = rank; c->nranks = px * py;
     c->ips = ips; c->ipe = ipe; c->jps = jps; c->jpe = jpe;
-    const int pi = rank % px, pj = rank / px;
-    c->nbr[WRFB200_WEST] = pi > 0 ? rank - 1 : -1;
-    c->nbr[WRFB200_EAST] = pi + 1 < px ? rank + 1 : -1;
-    c->nbr[WRFB200_SOUTH] = pj > 0 ? rank - px : -1;
-    c->nbr[WRFB200_NORTH] = pj + 1 < py ? rank + px : -1;
+    c->wrap_x = h->wrap_x; c->wrap_y = h->wrap_y;
+    c->nbr[WRFB200_WEST] = pi > 0 ? rank - 1 : (c->wrap_x ? rank + px - 1 : -1);
+    c->nbr[WRFB200_EAST] = pi + 1 < px ? rank + 1 : (c->wrap_x ? rank - px + 1 : -1);
+    c->nbr[WRFB200_SOUTH] = pj > 0 ? rank - px : (c->wrap_y ? rank + px * (py - 1) : -1);
+    c->nbr[WRFB200_NORTH] = pj + 1 < py ? rank + px : (c->wrap_y ? rank - px * (py - 1) : -1);
     if (const char *e = getenv("WRFB200_FLAG_TIMEOUT_MS")) {
         const long ms = atol(e);
         if (ms > 0) c->timeout_ns = (unsigned long long)ms * 1000000ull;
@@ -580,6 +621,8 @@ int comm_init(wrfb200_handle *h, int px, int py, int rank, int ips, int ipe, int
     q.pid = (int)getpid(); q.device = h->device; q.esize = h->esize; q.host_id = host_id();
     q.ims = d.ims; q.ime = d.ime; q.jms = d.jms; q.jme = d.jme; q.kms = d.kms; q.kme = d.kme;
     q.ips = ips; q.ipe = ipe; q.jps = jps; q.jpe = jpe;
+    q.wrap_x = c->wrap_x; q.wrap_y = c->wrap_y;
+    q.ids = d.ids; q.ide = d.ide; q.jds = d.jds; q.jde = d.jde;
     q.pitch3 = h->pitch3; q.pitch2 = h->pitch2;
     for (int x = 0; x <= kNX; ++x) {
         void *p = x < kNX ? (void *)h->d[kXf[x]] : (void *)c->flags;
@@ -600,6 +643,14 @@ int comm_init(wrfb200_handle *h, int px, int py, int rank, int ips, int ipe, int
 }
 
 }  // namespace
+
+extern "C" int wrfb200_comm_set_wrap(wrfb200_handle *h, int wrap_x, int wrap_y)
+{
+    if (!h) return wrfb200_fail(WRFB200_ERR_INVALID_ARG, "null handle");
+    h->wrap_x = wrap_x ? 1 : 0;
+    h->wrap_y = wrap_y ? 1 : 0;
+    return WRFB200_OK;
+}
 
 extern "C" int wrfb200_comm_init(wrfb200_handle *h, int px, int py, int rank,
                                  int ips, int ipe, int jps, int jpe, void *info_out)
@@ -663,18 +714,32 @@ extern "C" int wrfb200_comm_connect(wrfb200_handle *h, const void *all_infos, in
                                 h->esize == 8 ? "real*8" : "binary32");
         if (q.kms != d.kms || q.kme - q.kms + 1 != kdim)
             return wrfb200_fail(WRFB200_ERR_INVALID_ARG, "rank %d has different vertical memory extents", q.rank);
+        if (q.wrap_x != c->wrap_x || q.wrap_y != c->wrap_y || q.ids != d.ids || q.ide != d.ide || q.jds != d.jds ||
+            q.jde != d.jde)
+            return wrfb200_fail(WRFB200_ERR_INVALID_ARG, "rank %d has wrap (%d,%d) on i=%d..%d j=%d..%d, this rank (%d,%d) "
+                                "on i=%d..%d j=%d..%d: all ranks must set the same wrap on the same domain", q.rank,
+                                q.wrap_x, q.wrap_y, q.ids, q.ide, q.jds, q.jde, c->wrap_x, c->wrap_y, d.ids, d.ide,
+                                d.jds, d.jde);
+        // across the domain edge the peer's index of my cell is shifted by the period
+        const int pi = c->rank % c->px, pj = c->rank / c->px;
+        if (side == WRFB200_WEST && pi == 0) pr.di = d.ide - d.ids;
+        if (side == WRFB200_EAST && pi == c->px - 1) pr.di = -(d.ide - d.ids);
+        if (side == WRFB200_SOUTH && pj == 0) pr.dj = d.jde - d.jds;
+        if (side == WRFB200_NORTH && pj == c->py - 1) pr.dj = -(d.jde - d.jds);
+        const int ips = c->ips + pr.di, ipe = c->ipe + pr.di, jps = c->jps + pr.dj, jpe = c->jpe + pr.dj;
         bool adjacent = false;
         switch (side) {
-        case WRFB200_WEST:  adjacent = q.ipe + 1 == c->ips && q.jps == c->jps && q.jpe == c->jpe && q.ime >= c->ips; break;
-        case WRFB200_EAST:  adjacent = q.ips - 1 == c->ipe && q.jps == c->jps && q.jpe == c->jpe && q.ims <= c->ipe; break;
-        case WRFB200_SOUTH: adjacent = q.jpe + 1 == c->jps && q.ips == c->ips && q.ipe == c->ipe && q.jme >= c->jps; break;
-        default:            adjacent = q.jps - 1 == c->jpe && q.ips == c->ips && q.ipe == c->ipe && q.jms <= c->jpe; break;
+        case WRFB200_WEST:  adjacent = q.ipe + 1 == ips && q.jps == jps && q.jpe == jpe && q.ime >= ips; break;
+        case WRFB200_EAST:  adjacent = q.ips - 1 == ipe && q.jps == jps && q.jpe == jpe && q.ims <= ipe; break;
+        case WRFB200_SOUTH: adjacent = q.jpe + 1 == jps && q.ips == ips && q.ipe == ipe && q.jme >= jps; break;
+        default:            adjacent = q.jps - 1 == jpe && q.ips == ips && q.ipe == ipe && q.jms <= jpe; break;
         }
         if (!adjacent)
             return wrfb200_fail(WRFB200_ERR_INVALID_ARG, "rank %d (i=%d..%d j=%d..%d) is not the side-%d neighbour of i=%d..%d j=%d..%d",
                                 q.rank, q.ips, q.ipe, q.jps, q.jpe, side, c->ips, c->ipe, c->jps, c->jpe);
         if (int rc = map_peer(h, &pr)) return rc;
         pr.present = true;
+        pr.self = c->nbr[side] == c->rank;
     }
 
     // peer addresses: element offsets into the neighbour's arrays, scaled to 4-byte words (the kernels read the
@@ -686,11 +751,14 @@ extern "C" int wrfb200_comm_connect(wrfb200_handle *h, const void *all_infos, in
     hx.jpe_mem = c->jpe - d.jms;
     hx.ips_mem = c->ips - d.ims;
     hx.jps_mem = c->jps - d.jms;
+    // A self side keeps the output stores (into this rank's own ring, read by later launches only) and drops every
+    // flag: its u / v edge is copied by push_kernel ahead of the step (enqueue_push_uv).
     const Peer &so = c->peer[WRFB200_SOUTH];
-    if (so.present) {
+    if (so.present && !so.self) {
         const CommInfo &q = so.info;
         // south neighbour's v at (my memory column 0, level 0, Fortran row jps = its north halo row)
-        hx.s_v = so.f[WRFB200_V] + ((long long)(c->jps - q.jms) * (q.kme - q.kms + 1) * q.pitch3 + (d.ims - q.ims)) * w;
+        hx.s_v = so.f[WRFB200_V] + ((long long)(c->jps + so.dj - q.jms) * (q.kme - q.kms + 1) * q.pitch3 +
+                                    (d.ims + so.di - q.ims)) * w;
         hx.s_pitch3 = q.pitch3;
         hx.war_flag_south = c->flags + F_OUT_S;
         hx.uv_flag_to_south = so.flags + F_UV_N;
@@ -699,19 +767,25 @@ extern "C" int wrfb200_comm_connect(wrfb200_handle *h, const void *all_infos, in
     const Peer &e = c->peer[WRFB200_EAST], &n = c->peer[WRFB200_NORTH];
     if (e.present) {
         const CommInfo &q = e.info;
-        hx.uv_flag_east = c->flags + F_UV_E;
-        const long long o = ((long long)(d.jms - q.jms) * q.pitch2 + (c->ipe - q.ims)) * w;  // my memory row 0, column ipe
+        // my memory row 0, column ipe
+        const long long o = ((long long)(d.jms + e.dj - q.jms) * q.pitch2 + (c->ipe + e.di - q.ims)) * w;
         hx.e_mu = e.f[WRFB200_MU] + o; hx.e_muts = e.f[WRFB200_MUTS] + o; hx.e_mudf = e.f[WRFB200_MUDF] + o;
         hx.e_pitch2 = q.pitch2;
     }
     if (n.present) {
         const CommInfo &q = n.info;
-        hx.uv_flag_north = c->flags + F_UV_N;
-        const long long o = ((long long)(c->jpe - q.jms) * q.pitch2 + (d.ims - q.ims)) * w;  // row jpe, my memory column 0
+        // row jpe, my memory column 0
+        const long long o = ((long long)(c->jpe + n.dj - q.jms) * q.pitch2 + (d.ims + n.di - q.ims)) * w;
         hx.n_mu = n.f[WRFB200_MU] + o; hx.n_muts = n.f[WRFB200_MUTS] + o; hx.n_mudf = n.f[WRFB200_MUDF] + o;
     }
-    if (e.present) { hx.out_flag_to_east = e.flags + F_OUT_W; hx.east_counter = c->flags + F_EAST_DONE; }
-    if (n.present) { hx.out_flag_to_north = n.flags + F_OUT_S; hx.north_counter = c->flags + F_NORTH_DONE; }
+    if (e.present && !e.self) {
+        hx.uv_flag_east = c->flags + F_UV_E;
+        hx.out_flag_to_east = e.flags + F_OUT_W; hx.east_counter = c->flags + F_EAST_DONE;
+    }
+    if (n.present && !n.self) {
+        hx.uv_flag_north = c->flags + F_UV_N;
+        hx.out_flag_to_north = n.flags + F_OUT_S; hx.north_counter = c->flags + F_NORTH_DONE;
+    }
     hx.epoch = c->flags + F_EPOCH;
     {
         const char *e = getenv("WRFB200_NORTH_SECOND");               // A/B switch; default on
@@ -734,7 +808,7 @@ extern "C" int wrfb200_comm_barrier(wrfb200_handle *h)
     BarrierArgs a{};
     bool any = false;
     for (int side = 0; side < 4; ++side) {
-        if (!c->peer[side].present) continue;
+        if (!c->peer[side].present || c->peer[side].self) continue;    // stream order covers a self side
         a.to[side] = c->peer[side].flags + F_BAR + opposite(side);
         a.from[side] = c->flags + F_BAR + side;
         any = true;

@@ -34,6 +34,13 @@
 !           st = wrfb200_comm_push_constants( h )
 !           st = wrfb200_comm_loop( h, number_of_small_timesteps, 0_c_int, 0.0_c_float, 1_c_int )
 !
+!       A periodic domain refreshes its ring inside the loop only when the exchange wraps across the domain
+!       edge: set it from the namelist before comm_init (wrap_y needs specified = nested = .FALSE.), with the
+!       patches of WRF's own decomposition (the east-edge rank ends at ide, the north-edge rank at jde):
+!
+!           st = wrfb200_comm_set_wrap( h, MERGE(1_c_int, 0_c_int, config_flags%periodic_x),               &
+!                                          MERGE(1_c_int, 0_c_int, config_flags%periodic_y) )
+!
 !       In a build configured with -r8 the same sequence uses the real*8 patch (section (B') below): create_r8,
 !       the _r8 uploads, comm_init_r8 and comm_loop_r8; connect, push_constants, push_uv, step and status are
 !       shared by both precisions.  All ranks must be built alike (connect rejects a rank of the other precision):
@@ -339,6 +346,12 @@ INTERFACE
    END FUNCTION
 
    ! ---- (C) one rank per GPU: halo exchange fused into the kernels over peer-mapped memory ----
+   FUNCTION wrfb200_comm_set_wrap(handle, wrap_x, wrap_y) BIND(C, NAME="wrfb200_comm_set_wrap") RESULT(status)
+      IMPORT :: c_int, c_ptr
+      TYPE(c_ptr), VALUE :: handle
+      INTEGER(c_int), VALUE :: wrap_x, wrap_y             ! 0 / 1; before wrfb200_comm_init[_r8]
+      INTEGER(c_int) :: status
+   END FUNCTION
    FUNCTION wrfb200_comm_init(handle, px, py, rank, ips, ipe, jps, jpe, info_out)                     &
             BIND(C, NAME="wrfb200_comm_init") RESULT(status)
       IMPORT :: c_int, c_ptr

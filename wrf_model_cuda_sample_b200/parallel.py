@@ -65,11 +65,18 @@ def choose_process_grid(world: int, nx: int, ny: int) -> Tuple[int, int]:
 
 @dataclass(frozen=True)
 class Decomposition:
-    """A px x py process grid over the global domain of ``global_grid``."""
+    """A px x py process grid over the global domain of ``global_grid``.
+
+    ``wrap_x`` / ``wrap_y`` make the exchange periodic across the domain edge (WRF's periodic_x / periodic_y): the
+    neighbours are cyclic, and the edge rank's column ide (row jde), a copy of column ids (row jds), is halo to the
+    exchange -- see ``exchange_extents``.  A rank can then be its own neighbour (px = 1 / py = 1) or the same rank
+    can sit on both sides of an axis (px = 2 / py = 2)."""
     global_grid: Grid
     px: int
     py: int
     halo: int = 1
+    wrap_x: bool = False
+    wrap_y: bool = False
 
     @property
     def world(self) -> int:
@@ -79,6 +86,10 @@ class Decomposition:
         return rank % self.px, rank // self.px
 
     def rank_of(self, pi: int, pj: int) -> Optional[int]:
+        if self.wrap_x:
+            pi %= self.px
+        if self.wrap_y:
+            pj %= self.py
         if 0 <= pi < self.px and 0 <= pj < self.py:
             return pj * self.px + pi
         return None
@@ -100,6 +111,18 @@ class Decomposition:
         jps, jpe = split_range(g.jds, g.jde, self.py, pj)
         return ips, ipe, jps, jpe
 
+    def exchange_extents(self, rank: int) -> Tuple[int, int, int, int]:
+        """The patch as the halo exchange sees it: on a wrapped axis the edge rank ends at ide-1 (jde-1), and its
+        column ide (row jde) is the halo cell that receives the wrap (csrc/comm.cu does the same)."""
+        g = self.global_grid
+        pi, pj = self.coords(rank)
+        ips, ipe, jps, jpe = self.patch_extents(rank)
+        if self.wrap_x and pi == self.px - 1:
+            ipe = g.ide - 1
+        if self.wrap_y and pj == self.py - 1:
+            jpe = g.jde - 1
+        return ips, ipe, jps, jpe
+
     def patch_grid(self, rank: int) -> Grid:
         """The rank's call: global domain extents, memory = patch + halo, tile = patch."""
         g = self.global_grid
@@ -109,10 +132,10 @@ class Decomposition:
                     ips, ipe, jps, jpe, g.kts, g.kte, g.periodic_x, g.specified, g.nested)
 
     def interior_and_boundary_tiles(self, rank: int):
-        """Split the rank's tile into the part that reads no per-step halo (interior) and the strips that
-        do: the last column if there is an east neighbour (u at i+1), the last row if there is a north
-        neighbour (v at j+1).  Returns (interior | None, [strips])."""
-        ips, ipe, jps, jpe = self.patch_extents(rank)
+        """Split the rank's tile (its exchange extents) into the part that reads no per-step halo (interior) and
+        the strips that do: the last column if there is an east neighbour (u at i+1), the last row if there is a
+        north neighbour (v at j+1).  Returns (interior | None, [strips])."""
+        ips, ipe, jps, jpe = self.exchange_extents(rank)
         east = self.neighbour(rank, EAST) is not None
         north = self.neighbour(rank, NORTH) is not None
         ie = ipe - 1 if east else ipe
@@ -160,11 +183,15 @@ class HaloExchanger:
         return ops
 
     def start(self, halos, width: int = 1):
-        """Pack and post all sends/receives; returns an opaque token for ``finish``."""
+        """Pack and post all sends/receives; returns an opaque token for ``finish``.  A rank that is its own
+        neighbour (a wrapped axis with one rank on it) packs and unpacks locally, with no point-to-point op."""
         import torch.distributed as dist
         p2p, recvs = [], []
         for kind, field, side, peer in self.plan(halos):
-            if kind == "send":
+            if peer == self.rank:
+                if kind == "send":                   # my inside edge on `side` is my own halo on the opposite side
+                    recvs.append((field, OPPOSITE[side], self.pack(field, side, width)))
+            elif kind == "send":
                 p2p.append(dist.P2POp(dist.isend, self.pack(field, side, width), peer, self.group))
             else:
                 buf = self.recv_buffer(field, side, width)
@@ -190,7 +217,7 @@ class GpuPatchHalo:
 
     def __init__(self, patch, decomp: Decomposition, rank: int, device):
         self.patch = patch
-        self.ext = decomp.patch_extents(rank)
+        self.ext = decomp.exchange_extents(rank)
         self.grid = decomp.patch_grid(rank)
         self.device = device
         self._bufs: Dict[Tuple[str, int, str], object] = {}
@@ -225,8 +252,10 @@ def connect_fused(patch, decomp: Decomposition, rank: int, allgather: Callable[[
     ``allgather(blob) -> [blob of rank 0, blob of rank 1, ...]`` is the caller's transport (torch.distributed
     in bench.py; MPI_Allgather in a WRF host; a list when several ranks live in one process).  After this the
     acoustic loop needs no collective library: ``patch.comm_push_constants()`` once per RK sub-step, then
-    ``patch.comm_loop(n)`` or ``comm_push_uv(); comm_step()`` per step."""
+    ``patch.comm_loop(n)`` or ``comm_push_uv(); comm_step()`` per step.  The decomposition's wrap flags are set on
+    the patch first."""
     ips, ipe, jps, jpe = decomp.patch_extents(rank)
+    patch.comm_set_wrap(decomp.wrap_x, decomp.wrap_y)
     info = patch.comm_init(decomp.px, decomp.py, rank, ips, ipe, jps, jpe)
     patch.comm_connect(allgather(info))
 
