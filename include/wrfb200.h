@@ -87,7 +87,19 @@ typedef struct wrfb200_domain {
                                             module_configure.f90:434,436,447 */
 } wrfb200_domain;
 
-/* Kernel selection (testing / benchmarking; AUTO is the product default). */
+/* Kernel selection (testing / benchmarking; AUTO is the product default).
+ *
+ * Level limits.  Each kernel holds all nk = kte-kts computed levels of its columns in shared memory, so nk bounds
+ * which kernels can run:
+ *                 binary32        real*8
+ *   PIPE          nk <= 337       --
+ *   TILE          nk <= 223       nk <= 220
+ *   COLUMN        nk <= 454       nk <= 227
+ * AUTO runs the pipe kernel (binary32) / tile kernel (real*8) where the layout and nk allow it, otherwise the column
+ * kernel: binary32 nk 338 .. 454 and real*8 nk 221 .. 227 always run the column kernel.  A request past a kernel's
+ * limit -- explicit, or AUTO past the column kernel's -- fails with WRFB200_ERR_UNSUPPORTED before anything is
+ * launched, and the message quotes nk and the limit.  The multi-GPU path (section 3b) runs the pipe kernel for
+ * binary32 and the tile kernel for real*8: wrfb200_comm_init / _init_r8 refuse a larger nk. */
 typedef enum wrfb200_kernel {
     WRFB200_KERNEL_AUTO = 0,
     WRFB200_KERNEL_COLUMN = 1,   /* one thread per (i,j) column, any layout */
@@ -376,7 +388,9 @@ int wrfb200_standin_advance_uv_r8(wrfb200_handle *h, int field, double c, int i0
  *     reads those halos must be preceded by wrfb200_comm_wait_outputs on the same stream.  Everything is
  *     asynchronous on the handle's stream; there is no host synchronisation and no NCCL call inside the loop.
  *     All ranks must issue the same sequence of steps (the flags are step counters).  A halo wait gives up
- *     after 5 s (WRFB200_FLAG_TIMEOUT_MS) and is reported by wrfb200_comm_status.
+ *     after 5 s (WRFB200_FLAG_TIMEOUT_MS) and is reported by wrfb200_comm_status.  Each binary32 step runs the
+ *     TMA pipe kernel, so wrfb200_comm_init fails with WRFB200_ERR_UNSUPPORTED when the patch has more than 337
+ *     computed levels.
  *
  *     Real*8 ranks (wrfb200_create_r8, allocate=1): wrfb200_comm_init_r8 instead of wrfb200_comm_init, and the
  *     _r8 forms of the loop and the stand-in (double c).  connect, barrier, push_constants, push_uv,
@@ -465,7 +479,9 @@ int wrfb200_compare_r8(const double *a, const double *b, long n, wrfb200_compare
 /* Host-only description of the launch the TMA kernel makes for the tile its:ite x jts:jte of `dom` on a device with
  * `resident_blocks` resident blocks (0: a B200, 2 x 148): plan10 = {configuration TJ*10+STAGES, TJ, STAGES, tile
  * columns, block rows of 2-row tiles, block rows of 1-row tiles, remainder-strip blocks, first strip column (memory
- * index), grid size, dynamic shared memory in bytes}.  Needs no GPU; the launch geometry is unit-tested with it. */
+ * index), grid size, dynamic shared memory in bytes}; configuration 62 is <1, 2> with the level tables read from
+ * L2.  WRFB200_ERR_UNSUPPORTED past the pipe kernel's level limit (nk > 337).  Needs no GPU; the launch geometry is
+ * unit-tested with it. */
 int wrfb200_pipe_plan(const wrfb200_domain *dom, int its, int ite, int jts, int jte, int kts, int kte,
                       int resident_blocks, long long *plan10);
 

@@ -8,9 +8,17 @@ import pytest
 
 import wrf_model_cuda_sample_b200 as wrf
 from tests import cases
+from wrf_model_cuda_sample_b200._lib import ERR_UNSUPPORTED
 
 TI, STRIP_W, STRIP_ROWS, SLOTS = 128, 16, 2, 2 * 148
 KEYS = ("cfg", "tj", "stages", "nbx", "nby2", "nby1", "strip_blocks", "strip_i0", "grid", "smem")
+SMEM_SM, SMEM_RESERVE = 227 * 1024, 1024                 # usable shared memory per SM; reserved per resident block
+PIPE_MAX_NK = 337
+
+
+def pipe_smem(tj, stages, nk, tabs=True):
+    """Dynamic shared memory of a pipe block (csrc/amt_pipe.cu pipe_smem): ring + stash + level tables + barriers."""
+    return (8 * stages * 832 + tj * nk * TI + (4 * nk if tabs else 0)) * 4 + 8 * stages * 8
 
 
 def plan(g, slots=SLOTS):
@@ -39,10 +47,13 @@ def check_cover(g, p):
     assert 2 * p["nby2"] + p["nby1"] >= nj and 2 * (p["nby2"] - 1) + p["nby1"] < nj if p["nby1"] == 0 else \
         2 * p["nby2"] + p["nby1"] == nj
     assert p["grid"] == p["strip_blocks"] + p["nbx"] * (p["nby2"] + p["nby1"])
-    # shared memory: two resident blocks per SM for the two-block configurations, one otherwise
-    per_sm = 227 * 1024
-    blocks = 2 if p["cfg"] in (22, 13, 12, 62) else 1
-    assert blocks * (p["smem"] + 1024) <= per_sm
+    # shared memory: at least one block fits an SM, and two whenever the leanest two-block configuration (the level
+    # tables in L2) would fit twice
+    blocks = SMEM_SM // (p["smem"] + SMEM_RESERVE)
+    assert blocks >= 1
+    nk = k1 - k0 + 1
+    if 2 * (pipe_smem(1, 2, nk, tabs=False) + SMEM_RESERVE) <= SMEM_SM:
+        assert blocks >= 2, (nk, p)
 
 
 def test_baseline_shapes_match_the_profiled_launches():
@@ -63,7 +74,7 @@ def test_baseline_shapes_match_the_profiled_launches():
 def test_every_column_and_row_is_covered_exactly_once(variant):
     rs = np.random.RandomState(hash(variant) % 1000)
     for _ in range(150):
-        nx, ny, nz = int(rs.randint(5, 2100)), int(rs.randint(5, 400)), int(rs.randint(2, 130))
+        nx, ny, nz = int(rs.randint(5, 2100)), int(rs.randint(5, 400)), int(rs.randint(2, 471))
         halo = int(rs.randint(1, 8))
         g = cases.grid(nx, ny, nz, halo=halo, variant=variant)
         i0, i1, j0, j1, _, _ = g.bounds()
@@ -77,15 +88,55 @@ def test_every_column_and_row_is_covered_exactly_once(variant):
             i0, i1, j0, j1, _, _ = g.bounds()
             if i0 > i1 or j0 > j1:
                 continue
-        if nz - 1 > 400:
-            continue
         out = (C.c_longlong * 10)()
         d = g.domain()
         rc = wrf.lib().wrfb200_pipe_plan(C.byref(d), g.its, g.ite, g.jts, g.jte, g.kts, g.kte,
                                          int(rs.choice([SLOTS, 2 * 132, 64])), out)
-        if rc != 0:
+        if nz - 1 > PIPE_MAX_NK:
+            assert rc == ERR_UNSUPPORTED, (nx, ny, nz, rc)
             continue
+        assert rc == 0, wrf.lib().wrfb200_last_error()
         check_cover(g, dict(zip(KEYS, list(out))))
+
+
+# The ladder of the pipe kernel's configurations over the level count nk: (cfg at nj >= 2, cfg at nj = 1).
+LADDER = {59: (22, 13), 60: (13, 13), 66: (13, 13), 67: (12, 12), 117: (12, 12), 118: (62, 62), 120: (62, 62),
+          121: (14, 14), 236: (14, 14), 237: (12, 12), 337: (12, 12)}
+
+
+def plan_rc(g, slots=SLOTS):
+    out = (C.c_longlong * 10)()
+    d = g.domain()
+    rc = wrf.lib().wrfb200_pipe_plan(C.byref(d), g.its, g.ite, g.jts, g.jte, g.kts, g.kte, slots, out)
+    return rc, dict(zip(KEYS, list(out)))
+
+
+def test_level_ladder_boundaries():
+    """Both ends of every configuration, for 2-row-capable tiles and for a single row; refused past nk = 337."""
+    for nk, (cfg, cfg_one_row) in LADDER.items():
+        for ny, want in ((40, cfg), (4, cfg_one_row)):            # specified: 37 computed rows, or one
+            g = cases.grid(300, ny, nk + 1)
+            p = plan(g)
+            assert p["cfg"] == want, (nk, ny, p)
+            # one block per SM from nk = 121 on (the last-resort 12 included), two before
+            assert SMEM_SM // (p["smem"] + SMEM_RESERVE) == (1 if nk >= 121 else 2), (nk, p)
+            check_cover(g, p)
+    for ny in (40, 4):
+        rc, _ = plan_rc(cases.grid(300, ny, PIPE_MAX_NK + 2))
+        assert rc == ERR_UNSUPPORTED
+        msg = wrf.lib().wrfb200_last_error().decode()
+        assert "338" in msg and "337" in msg, msg
+
+
+def test_no_plan_selects_the_two_row_four_stage_configuration():
+    """cfg 24 (<2, 4>) would need nk <= 119 and is only considered from nk = 121 on: it must never appear."""
+    for ny in (4, 5, 200):                                         # specified: nj = 1, 2, 197
+        for nk in range(1, 461):
+            rc, p = plan_rc(cases.grid(140, ny, nk + 1))
+            if nk > PIPE_MAX_NK:
+                assert rc == ERR_UNSUPPORTED, nk
+            else:
+                assert rc == 0 and p["cfg"] in (22, 13, 12, 62, 14), (nk, ny, p)
 
 
 def test_plan_rejects_empty_and_unsupported_calls():

@@ -68,7 +68,19 @@ cudaError_t launch_column(const P &p, K kernel, bool (&raised)[64], cudaStream_t
     return cudaGetLastError();
 }
 
+template <class P, class T>
+bool column_levels_fit(const P &p, int *max_levels)
+{
+    const int most = kMaxDynSmemOptIn / (int)(kColThreads * sizeof(T));
+    if (max_levels) *max_levels = most;
+    return p.nk <= most;
+}
+
 }  // namespace
+
+// the [nk][128] dvdxi slab in dynamic shared memory: 512 B per level in binary32, 1 KB in binary64
+bool amt_column_levels_fit(const AmtParams &p, int *max_levels) { return column_levels_fit<AmtParams, float>(p, max_levels); }
+bool amt_column_levels_fit(const AmtParamsR8 &p, int *max_levels) { return column_levels_fit<AmtParamsR8, double>(p, max_levels); }
 
 cudaError_t amt_launch_column(const AmtParams &p, cudaStream_t stream)
 {
@@ -76,7 +88,6 @@ cudaError_t amt_launch_column(const AmtParams &p, cudaStream_t stream)
     return launch_column<AmtParams, float>(p, amt_column_kernel, raised, stream);
 }
 
-// At 128 threads a block holds 1 KB of dvdxi per level: up to 227 levels (nk) in double.
 cudaError_t amt_launch_column(const AmtParamsR8 &p, cudaStream_t stream)
 {
     static bool raised[64] = {};

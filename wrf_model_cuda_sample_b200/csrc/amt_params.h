@@ -194,6 +194,13 @@ cudaError_t amt_launch_column(const AmtParams &p, cudaStream_t stream);
 cudaError_t amt_launch_tile(const AmtParams &p, cudaStream_t stream);
 bool amt_tile_supported(const AmtParams &p);
 bool amt_pipe_supported(const AmtParams &p);
+// Level limits: every kernel keeps a per-column slab of all p.nk levels in shared memory, so the level count decides
+// whether a kernel can run at all.  true when p.nk fits; *max_levels (if given) receives the kernel's largest nk.
+bool amt_pipe_levels_fit(const AmtParams &p, int *max_levels = nullptr);             // 337
+bool amt_tile_levels_fit(const AmtParams &p, int *max_levels = nullptr);             // 223
+bool amt_column_levels_fit(const AmtParams &p, int *max_levels = nullptr);           // 454
+bool amt_tile_levels_fit(const AmtParamsR8 &p, int *max_levels = nullptr);           // 220
+bool amt_column_levels_fit(const AmtParamsR8 &p, int *max_levels = nullptr);         // 227
 bool amt_build_tma_maps(const AmtParams &p, AmtTmaMaps *maps);                    // cached: rebuilds only on change
 cudaError_t amt_launch_pipe(const AmtParams &p, const AmtTmaMaps &maps, cudaStream_t stream);
 // real*8 kernels (amt_column.cu, amt_tile_r8.cu)

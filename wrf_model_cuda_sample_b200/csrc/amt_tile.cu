@@ -325,6 +325,14 @@ size_t tile_smem(int tj, int nk) { return ((size_t)2 * tj * nk * TI + 4 * (size_
 
 }  // namespace
 
+// a one-row tile: 1040 B per level
+bool amt_tile_levels_fit(const AmtParams &p, int *max_levels)
+{
+    const int most = (int)(kSmemMax / tile_smem(1, 1));
+    if (max_levels) *max_levels = most;
+    return p.nk <= most;
+}
+
 bool amt_tile_supported(const AmtParams &p)
 {
     const void *ptrs3[] = {p.ww, p.ww_1, p.u, p.u_1, p.v, p.v_1, p.t, p.t_1, p.t_ave, p.ft};
@@ -333,8 +341,7 @@ bool amt_tile_supported(const AmtParams &p)
     for (const void *q : ptrs3) if ((reinterpret_cast<uintptr_t>(q) & 15u) != 0) return false;
     for (const void *q : ptrs2) if ((reinterpret_cast<uintptr_t>(q) & 15u) != 0) return false;
     if (p.pitch % 4 != 0 || p.pitch2 % 4 != 0 || p.jstride % 4 != 0) return false;
-    if (tile_smem(1, p.nk) > kSmemMax) return false;
-    return true;
+    return amt_tile_levels_fit(p);
 }
 
 cudaError_t amt_launch_tile(const AmtParams &p, cudaStream_t stream)

@@ -404,6 +404,14 @@ cudaError_t launch(const AmtParamsR8 &p, cudaStream_t stream)
 
 }  // namespace
 
+// a one-row tile: 1056 B per level
+bool amt_tile_levels_fit(const AmtParamsR8 &p, int *max_levels)
+{
+    const int most = (int)((size_t)kMaxDynSmemOptIn / tile_smem_r8(1, 1));
+    if (max_levels) *max_levels = most;
+    return p.nk <= most;
+}
+
 bool amt_tile_supported(const AmtParamsR8 &p)
 {
     const void *ptrs3[] = {p.ww, p.ww_1, p.u, p.u_1, p.v, p.v_1, p.t, p.t_1, p.t_ave, p.ft};
@@ -412,8 +420,7 @@ bool amt_tile_supported(const AmtParamsR8 &p)
     for (const void *q : ptrs3) if ((reinterpret_cast<uintptr_t>(q) & 15u) != 0) return false;
     for (const void *q : ptrs2) if ((reinterpret_cast<uintptr_t>(q) & 15u) != 0) return false;
     if (p.pitch % 2 != 0 || p.pitch2 % 2 != 0 || p.jstride % 2 != 0) return false;
-    if (tile_smem_r8(1, p.nk) > (size_t)kMaxDynSmemOptIn) return false;        // nk <= 220
-    return true;
+    return amt_tile_levels_fit(p);                                               // nk <= 220
 }
 
 cudaError_t amt_launch_tile(const AmtParamsR8 &p, cudaStream_t stream)

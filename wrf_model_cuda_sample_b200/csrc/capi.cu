@@ -146,17 +146,27 @@ int wrfb200_make_params(const wrfb200_handle *h, int its, int ite, int jts, int 
 
 namespace {
 
+// a kernel whose shared memory cannot hold the call's level count (amt_*_levels_fit)
+int too_many_levels(const char *what, int nk, int max_levels)
+{
+    return fail(WRFB200_ERR_UNSUPPORTED, "the %s holds at most %d levels (nk=%d)", what, max_levels, nk);
+}
+
 int launch(wrfb200_handle *h, const AmtParams &p, cudaStream_t s, int kernel)
 {
     cudaError_t e;
     int ran = kernel;
+    int most = 0;
     if (kernel == WRFB200_KERNEL_COLUMN) {
+        if (!amt_column_levels_fit(p, &most)) return too_many_levels("column kernel", p.nk, most);
         e = amt_launch_column(p, s);
     } else if (kernel == WRFB200_KERNEL_TILE) {
+        if (!amt_tile_levels_fit(p, &most)) return too_many_levels("tile kernel", p.nk, most);
         if (!amt_tile_supported(p))
             return fail(WRFB200_ERR_UNSUPPORTED, "tile kernel needs 16-byte aligned fields and pitches that are multiples of 4");
         e = amt_launch_tile(p, s);
     } else if (kernel == WRFB200_KERNEL_PIPE) {
+        if (!amt_pipe_levels_fit(p, &most)) return too_many_levels("pipe kernel", p.nk, most);
         if (!amt_pipe_supported(p))
             return fail(WRFB200_ERR_UNSUPPORTED, "pipe kernel needs 16-byte aligned fields and pitches that are multiples of 4");
         if (!amt_build_tma_maps(p, &h->maps)) return fail(WRFB200_ERR_CUDA, "cuTensorMapEncodeTiled failed");
@@ -166,10 +176,12 @@ int launch(wrfb200_handle *h, const AmtParams &p, cudaStream_t s, int kernel)
         // of columns (e.g. the one-column strips behind an east halo) would stage 128-wide rows for
         // nothing, and unaligned caller layouts cannot be bulk-copied: those take the column kernel.
         const bool wide = (p.i1 - p.i0 + 1) >= 32;
+        // Past the pipe kernel's level limit the column kernel runs, up to its own.
         if (wide && amt_pipe_supported(p) && amt_build_tma_maps(p, &h->maps)) {
             e = amt_launch_pipe(p, h->maps, s);
             ran = WRFB200_KERNEL_PIPE;
         } else {
+            if (!amt_column_levels_fit(p, &most)) return too_many_levels("column kernel (AUTO's fallback)", p.nk, most);
             e = amt_launch_column(p, s);
             ran = WRFB200_KERNEL_COLUMN;
         }
@@ -186,6 +198,7 @@ int launch(wrfb200_handle *h, const AmtParamsR8 &p, cudaStream_t s, int kernel)
 {
     cudaError_t e;
     int ran = kernel;
+    int most = 0;
     if (p.halo.enabled) {
         // a multi-GPU rank (comm.cu): the tile kernel with the halo exchange fused in; wrfb200_comm_init_r8 has
         // checked that the patch's layout and level count suit it
@@ -196,19 +209,23 @@ int launch(wrfb200_handle *h, const AmtParamsR8 &p, cudaStream_t s, int kernel)
     } else if (kernel == WRFB200_KERNEL_PIPE) {
         return fail(WRFB200_ERR_UNSUPPORTED, "the pipe kernel is binary32 only; a real*8 handle runs the tile or column kernel");
     } else if (kernel == WRFB200_KERNEL_COLUMN) {
+        if (!amt_column_levels_fit(p, &most)) return too_many_levels("real*8 column kernel", p.nk, most);
         e = amt_launch_column(p, s);
     } else if (kernel == WRFB200_KERNEL_TILE) {
+        if (!amt_tile_levels_fit(p, &most)) return too_many_levels("real*8 tile kernel", p.nk, most);
         if (!amt_tile_supported(p))
-            return fail(WRFB200_ERR_UNSUPPORTED, "real*8 tile kernel needs 16-byte aligned fields, pitches of an even "
-                                                 "number of doubles and at most 220 levels (nk=%d)", p.nk);
+            return fail(WRFB200_ERR_UNSUPPORTED, "real*8 tile kernel needs 16-byte aligned fields and pitches of an even "
+                                                 "number of doubles");
         e = amt_launch_tile(p, s);
     } else {
-        // AUTO: tiles narrower than a warp of columns take the column kernel, as for binary32
+        // AUTO: tiles narrower than a warp of columns take the column kernel, as for binary32; so do level counts
+        // past the tile kernel's limit, up to the column kernel's own
         const bool wide = (p.i1 - p.i0 + 1) >= 32;
         if (wide && amt_tile_supported(p)) {
             e = amt_launch_tile(p, s);
             ran = WRFB200_KERNEL_TILE;
         } else {
+            if (!amt_column_levels_fit(p, &most)) return too_many_levels("real*8 column kernel (AUTO's fallback)", p.nk, most);
             e = amt_launch_column(p, s);
             ran = WRFB200_KERNEL_COLUMN;
         }
@@ -1711,6 +1728,8 @@ extern "C" int wrfb200_pipe_plan(const wrfb200_domain *dom, int its, int ite, in
     p.i0 = is - dom->ims; p.i1 = ie - dom->ims;
     p.j0 = js - dom->jms; p.j1 = je - dom->jms;
     p.k0 = ks - dom->kms; p.nk = ke - ks + 1;
+    int most = 0;
+    if (!amt_pipe_levels_fit(p, &most)) return too_many_levels("pipe kernel", p.nk, most);
     if (!amt_pipe_plan(p, resident_blocks > 0 ? resident_blocks : 2 * 148, plan10))
         return fail(WRFB200_ERR_INVALID_ARG, "empty index sets");
     return WRFB200_OK;

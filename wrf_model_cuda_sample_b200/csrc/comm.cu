@@ -657,6 +657,14 @@ extern "C" int wrfb200_comm_init(wrfb200_handle *h, int px, int py, int rank,
 {
     if (!h || !info_out) return wrfb200_fail(WRFB200_ERR_INVALID_ARG, "null argument");
     if (int rc = wrfb200_require_r4(h, "multi-GPU halo exchange (wrfb200_comm_*)")) return rc;
+    // every step runs the TMA pipe kernel: refuse a level count it cannot hold now, before any neighbour connects,
+    // rather than at the first step
+    AmtParams p{};
+    p.nk = h->dom.kde - 1;                                      // levels 1 .. kde-1
+    int most = 0;
+    if (!amt_pipe_levels_fit(p, &most))
+        return wrfb200_fail(WRFB200_ERR_UNSUPPORTED, "the binary32 multi-GPU path runs the TMA pipe kernel, which holds "
+                            "at most %d levels (nk=%d)", most, p.nk);
     return comm_init(h, px, py, rank, ips, ipe, jps, jpe, info_out);
 }
 
