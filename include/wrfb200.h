@@ -185,7 +185,8 @@ int wrfb200_set_default_stream(void *cuda_stream);
 int wrfb200_set_default_kernel(int kernel /* wrfb200_kernel */);
 
 /* Release the per-thread device mirrors cached by the host-pointer form (and every host registration), and the
- * shared patches of shared-tiles mode (wrfb200_set_shared_tiles) with every thread's state for them. */
+ * shared patches of shared-tiles mode (wrfb200_set_shared_tiles) with every thread's state for them.  It also stops
+ * and joins the host threads of the staged route (wrfb200_set_host_pinning); no call may be in flight then. */
 int wrfb200_release_cache(void);
 
 /* Acoustic-loop residency for HOST-pointer callers of wrfb200_advance_mu_t (thread-local).  Between begin and
@@ -200,9 +201,16 @@ int wrfb200_acoustic_loop_end(void);
 
 /* Page-locking of the caller's host arrays (process-wide; default off, or WRFB200_PIN_HOST=1).  When on,
  * every host array of a compat call is cudaHostRegister'ed the first time it is seen and stays registered
- * until wrfb200_release_cache / wrfb200_host_unregister_all: copies then run at the pinned link rate.  The
- * caller must keep registered arrays allocated until then.  wrfb200_host_register pins one array explicitly
- * (the role of cudaHostAlloc in advance_mu_t_driver.cu:97-167). */
+ * until wrfb200_release_cache / wrfb200_host_unregister_all, and is then copied directly at the pinned link
+ * rate.  The caller must keep registered arrays allocated until then.  wrfb200_host_register pins one array
+ * explicitly (the role of cudaHostAlloc in advance_mu_t_driver.cu:97-167).
+ * Without it, pageable arrays take the staged route: host threads of the library copy them through pinned bounce
+ * buffers it owns, overlapped with the transfers, so nothing of the caller's is registered.  What pinning still
+ * buys over that route is the host-side copy that cannot overlap (DESIGN.md section 5 has the measured numbers).
+ * The route is chosen per array from whether it is page-locked; wrfb200_default_last_transfer reports it.  The
+ * staged route's pool of host threads (one per process, one thread per CPU of the process's affinity mask, at
+ * most 16) starts with the first staged call and is stopped by wrfb200_release_cache and at unload; a process
+ * forked after a staged call has no pool until its own first staged call. */
 int wrfb200_set_host_pinning(int enable);
 int wrfb200_host_register(const float *host, size_t bytes);
 int wrfb200_host_unregister_all(void);
@@ -210,6 +218,13 @@ int wrfb200_host_unregister_all(void);
 /* Kernel the most recent wrfb200_advance_mu_t call of this thread ran (a wrfb200_kernel id; AUTO resolved; for a
  * call split over several devices, the first part's). */
 int wrfb200_default_last_kernel(int *kernel);
+
+/* How the most recent host-pointer call of wrfb200_advance_mu_t / _loop (or the _r8 pair) of this thread moved its
+ * arrays (thread-local): *route = 0 every array direct (page-locked: by the caller, e.g. cudaHostAlloc or torch
+ * pin_memory, or by wrfb200_set_host_pinning), 1 some arrays staged through the library's pinned bounce buffers
+ * (pageable ones), 2 every array staged.  The four 1-D arrays, a few hundred bytes, are copied directly even when
+ * pageable but count by what they are.  No host-pointer call on this thread yet: WRFB200_ERR_STATE. */
+int wrfb200_default_last_transfer(int *route);
 
 /* Devices the HOST-pointer form of wrfb200_advance_mu_t / _loop (and the _r8 pair) spreads its j-rows over.
  * Thread-local, like wrfb200_set_default_stream / _kernel.  n = 0 (devices may be NULL): back to the current

@@ -26,6 +26,8 @@ FORTRAN_ARRAY_ORDER_B = ("dnw", "fnm", "fnp", "rdnw", "msfuy", "msfvx_inv", "msf
 
 OK, ERR_INVALID_ARG, ERR_UNSUPPORTED, ERR_CUDA, ERR_NOMEM, ERR_STATE = range(6)
 KERNEL_AUTO, KERNEL_COLUMN, KERNEL_TILE, KERNEL_PIPE = 0, 1, 2, 3
+# wrfb200_default_last_transfer: every array copied directly / some staged through bounce buffers / all staged
+TRANSFER_DIRECT, TRANSFER_MIXED, TRANSFER_STAGED = 0, 1, 2
 WEST, EAST, SOUTH, NORTH = 0, 1, 2, 3
 
 
@@ -75,6 +77,7 @@ PROTOTYPES = {
     "wrfb200_host_register": (C.c_int, [_P, C.c_size_t]),
     "wrfb200_host_unregister_all": (C.c_int, []),
     "wrfb200_default_last_kernel": (C.c_int, [C.POINTER(C.c_int)]),
+    "wrfb200_default_last_transfer": (C.c_int, [C.POINTER(C.c_int)]),
     "wrfb200_set_default_devices": (C.c_int, [C.POINTER(C.c_int), C.c_int]),
     "wrfb200_set_shared_tiles": (C.c_int, [C.c_int]),
     "wrfb200_host_split_plan": (C.c_int, [C.POINTER(Domain)] + [C.c_int] * 7 + [C.POINTER(C.c_int)]),

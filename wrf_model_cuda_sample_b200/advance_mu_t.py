@@ -477,6 +477,16 @@ def default_last_kernel() -> int:
     return k.value
 
 
+def default_last_transfer() -> int:
+    """How the most recent host-array ``advance_mu_t`` call of this thread moved its arrays: ``TRANSFER_DIRECT``
+    (every array page-locked, copied directly), ``TRANSFER_MIXED`` (some pageable ones staged through the library's
+    pinned bounce buffers) or ``TRANSFER_STAGED`` (all of them).  Raises ``WrfB200Error`` (``ERR_STATE``) before the
+    thread's first host-array call."""
+    r = C.c_int()
+    check(lib().wrfb200_default_last_transfer(C.byref(r)))
+    return r.value
+
+
 def synth_fields(grid: Grid, seed: int = 20240617, names: Iterable[str] = FIELDS, pinned: bool = False,
                  dx_m: float = 12000.0) -> Dict[str, np.ndarray]:
     """Deterministic atmosphere-like fields for ``grid``'s memory extents (wrfb200_synth_field).

@@ -8,12 +8,17 @@
 // not per acoustic step), launches are asynchronous on a caller-visible stream, and errors are
 // returned instead of exit() (:22-32).
 #include <cuda_runtime.h>
+#include <sched.h>
+#include <unistd.h>
 
 #include <atomic>
+#include <condition_variable>
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <deque>
+#include <functional>
 #include <map>
 #include <memory>
 #include <mutex>
@@ -836,6 +841,9 @@ thread_local int g_default_kernel = WRFB200_KERNEL_AUTO;
 thread_local std::vector<int> g_default_devices;      // wrfb200_set_default_devices; empty: the current device only
 
 constexpr int kMaxSlabs = 16;
+// Bounce buffers of the staged route: 0, 1 take uploads in turn; 2..4 the downloads of ww, t, t_ave; 5..8 those of
+// the four 2-D outputs.  0..4 hold one slab of one 3-D field, 5..8 the same rows of a 2-D one.
+constexpr int kBounceUp = 2, kBounce3 = 5, kBounce = 9;
 
 struct Args {
     void *f[WRFB200_NUM_FIELDS];       // float or double arrays (the entry point's precision)
@@ -852,6 +860,12 @@ struct CompatCache {
     cudaEvent_t ev_up[kMaxSlabs] = {}, ev_comp[kMaxSlabs] = {};
     void *stage[2] = {nullptr, nullptr};                            // dense landing buffers for H2D slabs
     size_t stage_bytes = 0;
+    // staged route (pageable caller arrays): pinned bounce buffers, allocated on first use, and per buffer the
+    // event of the device copy that last read or filled it
+    void *bounce[kBounce] = {};
+    cudaEvent_t ev_bounce[kBounce] = {};
+    size_t bounce3_bytes = 0, bounce2_bytes = 0;
+    int next_up = 0;                                                // the upload buffer filled next
     // acoustic-loop residency (wrfb200_acoustic_loop_begin/end): after the first call of a loop the device
     // mirrors hold everything; later calls with the SAME arrays and index sets move only u, v up
     bool loop_active = false, primed = false;
@@ -866,6 +880,9 @@ struct CompatCache {
             h = nullptr;
             for (void *&b : stage) if (b) { cudaFree(b); b = nullptr; }
             stage_bytes = 0;
+            for (void *&b : bounce) if (b) { cudaFreeHost(b); b = nullptr; }
+            for (cudaEvent_t &e : ev_bounce) if (e) { cudaEventDestroy(e); e = nullptr; }
+            bounce3_bytes = bounce2_bytes = 0;
             for (cudaEvent_t &e : ev_up) if (e) { cudaEventDestroy(e); e = nullptr; }
             for (cudaEvent_t &e : ev_comp) if (e) { cudaEventDestroy(e); e = nullptr; }
             for (cudaStream_t *st : {&up, &comp, &down}) if (*st) { cudaStreamDestroy(*st); *st = nullptr; }
@@ -1068,6 +1085,278 @@ size_t field_bytes(const wrfb200_domain &d, int f, size_t esize)
     return (is3d(f) ? idim * kdim * jdim : is2d(f) ? idim * jdim : kdim) * esize;
 }
 
+// ---- staged route for pageable caller arrays --------------------------------------------------------
+// The driver stages a pageable cudaMemcpyAsync itself, from the calling thread, at a fraction of the link rate.
+// The staged route copies pageable arrays itself: host workers move a box of rows between the caller's array and
+// a pinned bounce buffer of the cache, and the device copy starts or ends in that buffer, so it runs at the pinned
+// rate while the workers fill the other buffer.  The caller's memory is never registered, so it may be freed and
+// re-allocated at any time between calls.
+
+// Host threads for those copies: one pool per process, shared by concurrent calls, sized to the CPUs the process may
+// run on (a WRF MPI rank bound to a few cores gets a few threads), at most 16.  The workers make no CUDA call.
+class HostPool {
+public:
+    const pid_t owner = getpid();
+
+    explicit HostPool(int n)
+    {
+        for (int t = 0; t < n; ++t) {
+            try {
+                threads_.emplace_back([this] { work(); });
+            } catch (const std::exception &) {
+                break;                                    // fewer workers: slower, still correct
+            }
+        }
+    }
+    ~HostPool()
+    {
+        {
+            std::lock_guard<std::mutex> lock(m_);
+            stop_ = true;
+        }
+        work_cv_.notify_all();
+        for (std::thread &t : threads_) t.join();
+    }
+    // fn(lo, hi) over [0, n) cut into contiguous ranges, one per worker, each of at least `grain`; returns when all
+    // have run.  A job of one range runs in the calling thread.
+    void run(long n, long grain, const std::function<void(long, long)> &fn)
+    {
+        long parts = grain > 0 ? n / grain : n;
+        if (parts > (long)threads_.size()) parts = (long)threads_.size();
+        if (parts <= 1) {
+            if (n > 0) fn(0, n);
+            return;
+        }
+        int left = (int)parts;
+        {
+            std::lock_guard<std::mutex> lock(m_);
+            for (long p = 0; p < parts; ++p) q_.push_back(Task{&fn, n * p / parts, n * (p + 1) / parts, &left});
+        }
+        work_cv_.notify_all();
+        std::unique_lock<std::mutex> lock(m_);
+        done_cv_.wait(lock, [&] { return left == 0; });
+    }
+
+private:
+    struct Task {
+        const std::function<void(long, long)> *fn;
+        long lo, hi;
+        int *left;                                        // ranges of the job still running, under m_
+    };
+    void work()
+    {
+        std::unique_lock<std::mutex> lock(m_);
+        for (;;) {
+            work_cv_.wait(lock, [this] { return stop_ || !q_.empty(); });
+            if (q_.empty()) return;
+            const Task t = q_.front();
+            q_.pop_front();
+            lock.unlock();
+            (*t.fn)(t.lo, t.hi);
+            lock.lock();
+            if (--*t.left == 0) done_cv_.notify_all();
+        }
+    }
+    std::mutex m_;
+    std::condition_variable work_cv_, done_cv_;
+    std::deque<Task> q_;
+    bool stop_ = false;
+    std::vector<std::thread> threads_;
+};
+
+std::mutex g_pool_mutex;
+HostPool *g_pool = nullptr;
+
+int pool_size()
+{
+    cpu_set_t set;
+    int n = sched_getaffinity(0, sizeof(set), &set) == 0 ? CPU_COUNT(&set) : (int)std::thread::hardware_concurrency();
+    return n < 1 ? 1 : n > 16 ? 16 : n;
+}
+
+// the pool, started on first use
+HostPool *host_pool()
+{
+    std::lock_guard<std::mutex> lock(g_pool_mutex);
+    if (g_pool && g_pool->owner != getpid()) g_pool = nullptr;      // inherited across fork(): no threads here
+    if (!g_pool) g_pool = new (std::nothrow) HostPool(pool_size());
+    return g_pool;
+}
+
+// Stops and joins the pool.  A pool inherited across fork() has no threads in this process: it is forgotten.
+void stop_pool()
+{
+    std::lock_guard<std::mutex> lock(g_pool_mutex);
+    if (g_pool && g_pool->owner == getpid()) delete g_pool;
+    g_pool = nullptr;
+}
+
+struct PoolReaper {
+    ~PoolReaper() { stop_pool(); }                        // library unload / process exit
+} g_pool_reaper;
+
+// A box of one field, Fortran-numbered: i0..i1 x k0..k1 x j0..j1 (k0 = k1 = 0 for a 2-D field).  In a bounce
+// buffer it is dense in the caller's order: rows of i, k next, j slowest.
+struct Box {
+    int f, i0, i1, k0, k1, j0, j1;
+};
+
+// Moves box b between the caller's array `arr` and the dense buffer `buf` on the pool's workers.
+void host_box(HostPool *pool, const wrfb200_handle *h, const Box &b, char *arr, char *buf, bool gather)
+{
+    const wrfb200_domain &d = h->dom;
+    const size_t es = (size_t)h->esize;
+    const long kh = is3d(b.f) ? h->kdim : 1, kb = is3d(b.f) ? d.kms : 0;
+    const long nk = b.k1 - b.k0 + 1, nrows = nk * (b.j1 - b.j0 + 1);
+    const size_t w = (size_t)(b.i1 - b.i0 + 1) * es;
+    char *first = arr + (((size_t)(b.j0 - d.jms) * kh + (b.k0 - kb)) * h->idim + (b.i0 - d.ims)) * es;
+    const bool dense = w == (size_t)h->idim * es && nk == kh;       // one contiguous range of the array
+    const std::function<void(long, long)> fn = [&](long lo, long hi) {
+        if (dense) {
+            if (gather) std::memcpy(buf + lo * w, first + lo * w, (hi - lo) * w);
+            else        std::memcpy(first + lo * w, buf + lo * w, (hi - lo) * w);
+            return;
+        }
+        for (long r = lo; r < hi; ++r) {
+            char *row = first + ((size_t)(r / nk) * kh + (size_t)(r % nk)) * h->idim * es;
+            if (gather) std::memcpy(buf + r * w, row, w);
+            else        std::memcpy(row, buf + r * w, w);
+        }
+    };
+    // ranges of at least 1 MB: a smaller copy is not worth waking a worker
+    const long grain = (long)(((size_t)1 << 20) / w) + 1;
+    if (pool) pool->run(nrows, grain, fn);
+    else      fn(0, nrows);
+}
+
+// The device half: box b between the dense buffer `buf` (pinned) and the mirror, on stream s.
+int device_box(wrfb200_handle *h, const Box &b, char *buf, bool to_dev, cudaStream_t s)
+{
+    const wrfb200_domain &d = h->dom;
+    const size_t es = (size_t)h->esize;
+    const bool three = is3d(b.f);
+    const size_t dpitch = (size_t)(three ? h->pitch3 : h->pitch2) * es;
+    const size_t kd = three ? h->kdim : 1;
+    const long kb = three ? d.kms : 0;
+    const size_t nk = b.k1 - b.k0 + 1, nj = b.j1 - b.j0 + 1, w = (size_t)(b.i1 - b.i0 + 1) * es;
+    char *dev = reinterpret_cast<char *>(h->d[b.f]) +
+                ((size_t)(b.j0 - d.jms) * kd + (size_t)(b.k0 - kb)) * dpitch + (size_t)(b.i0 - d.ims) * es;
+    const cudaMemcpyKind kind = to_dev ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToHost;
+    if (nk == kd) {
+        // whole columns: rows equally spaced across k and j
+        if (to_dev) CU(cudaMemcpy2DAsync(dev, dpitch, buf, w, w, nk * nj, kind, s));
+        else        CU(cudaMemcpy2DAsync(buf, w, dev, dpitch, w, nk * nj, kind, s));
+        return WRFB200_OK;
+    }
+    cudaMemcpy3DParms cp{};
+    const cudaPitchedPtr bufp = make_cudaPitchedPtr(buf, w, w, nk);
+    const cudaPitchedPtr devp = make_cudaPitchedPtr(dev, dpitch, dpitch, kd);
+    cp.srcPtr = to_dev ? bufp : devp;
+    cp.dstPtr = to_dev ? devp : bufp;
+    cp.extent = make_cudaExtent(w, nk, nj);
+    cp.kind = kind;
+    CU(cudaMemcpy3DAsync(&cp, s));
+    return WRFB200_OK;
+}
+
+// The cache's bounce buffers, at least b3 bytes (0..4) and b2 bytes (5..8), and their events.
+int ensure_bounce(CompatCache &cc, size_t b3, size_t b2)
+{
+    if (cc.bounce3_bytes >= b3 && cc.bounce2_bytes >= b2) return WRFB200_OK;
+    for (void *&b : cc.bounce) if (b) { cudaFreeHost(b); b = nullptr; }
+    cc.bounce3_bytes = cc.bounce2_bytes = 0;
+    for (int x = 0; x < kBounce; ++x) {
+        // portable: a part of a split call copies on its own device
+        CU(cudaHostAlloc(&cc.bounce[x], x < kBounce3 ? b3 : b2, cudaHostAllocPortable));
+        if (!cc.ev_bounce[x]) CU(cudaEventCreateWithFlags(&cc.ev_bounce[x], cudaEventDisableTiming));
+    }
+    cc.bounce3_bytes = b3;
+    cc.bounce2_bytes = b2;
+    return WRFB200_OK;
+}
+
+// Staged upload of box b of the caller's array `arr`, in runs of j-planes that fit one upload buffer.  A buffer is
+// refilled only after the copy that last read it has finished.  `land` (a device staging buffer; 3-D boxes of
+// whole rows and columns only): each run lands there densely and is re-pitched into the mirror.
+int upload_box(CompatCache &cc, wrfb200_handle *h, HostPool *pool, const Box &b, const void *arr, void *land)
+{
+    const size_t es = (size_t)h->esize;
+    const size_t plane = (size_t)(b.i1 - b.i0 + 1) * (b.k1 - b.k0 + 1) * es;
+    const int per = cc.bounce3_bytes / plane > 0 ? (int)(cc.bounce3_bytes / plane) : 1;
+    for (int j = b.j0; j <= b.j1; j += per) {
+        Box c = b;
+        c.j0 = j;
+        c.j1 = j + per - 1 < b.j1 ? j + per - 1 : b.j1;
+        const int x = cc.next_up;
+        cc.next_up = (x + 1) % kBounceUp;
+        char *buf = static_cast<char *>(cc.bounce[x]);
+        CU(cudaEventSynchronize(cc.ev_bounce[x]));
+        host_box(pool, h, c, const_cast<char *>(static_cast<const char *>(arr)), buf, true);
+        if (land) {
+            const long long nrows = (long long)(c.j1 - c.j0 + 1) * h->kdim;
+            const int fpe = h->esize / (int)sizeof(float);
+            CU(cudaMemcpyAsync(land, buf, (size_t)nrows * h->idim * es, cudaMemcpyHostToDevice, cc.up));
+            CU(cudaEventRecord(cc.ev_bounce[x], cc.up));
+            const size_t doff = (size_t)(c.j0 - h->dom.jms) * h->kdim * h->pitch3;
+            CU(wrfb200_repitch_rows(h->d[b.f] + doff * fpe, static_cast<float *>(land), h->pitch3 * fpe,
+                                    h->idim * fpe, nrows, cc.up));
+            h->launches += 1;
+            continue;
+        }
+        if (int rc = device_box(h, c, buf, true, cc.up)) return rc;
+        CU(cudaEventRecord(cc.ev_bounce[x], cc.up));
+    }
+    return WRFB200_OK;
+}
+
+// A staged download whose host half has not run yet: box `b` waits in bounce buffer x for the scatter into `arr`.
+struct PendingDown {
+    bool live = false;
+    Box b{};
+    void *arr = nullptr;
+};
+
+// The host half of the download waiting in buffer x, if any: waits for its device copy, then the workers write the
+// box's cells, and no others, into the caller's array.
+int finish_down(CompatCache &cc, const wrfb200_handle *h, HostPool *pool, PendingDown *pend, int x)
+{
+    if (!pend[x].live) return WRFB200_OK;
+    pend[x].live = false;
+    CU(cudaEventSynchronize(cc.ev_bounce[x]));
+    host_box(pool, h, pend[x].b, static_cast<char *>(pend[x].arr), static_cast<char *>(cc.bounce[x]), false);
+    return WRFB200_OK;
+}
+
+// Staged download of box b into buffer x on the download lane; its host half runs when x is needed again or at the
+// end of the call (finish_down).
+int download_box(CompatCache &cc, wrfb200_handle *h, HostPool *pool, PendingDown *pend, int x, const Box &b, void *arr)
+{
+    if (int rc = finish_down(cc, h, pool, pend, x)) return rc;
+    if (int rc = device_box(h, b, static_cast<char *>(cc.bounce[x]), false, cc.down)) return rc;
+    CU(cudaEventRecord(cc.ev_bounce[x], cc.down));
+    pend[x].live = true;
+    pend[x].b = b;
+    pend[x].arr = arr;
+    return WRFB200_OK;
+}
+
+// an array that is neither page-locked nor device memory takes the staged route
+bool pageable(const void *p)
+{
+    bool pinned = false;
+    return classify(p, &pinned) == PTR_HOST && !pinned;
+}
+
+// wrfb200_default_last_transfer of a host-array call: how many of its 26 arrays are pageable
+thread_local int g_last_route = -1;                       // -1: no host-array call on this thread yet
+
+int transfer_route(const Args &a)
+{
+    int n = 0;
+    for (int f = 0; f < WRFB200_NUM_FIELDS; ++f) n += pageable(a.f[f]) ? 1 : 0;
+    return n == 0 ? 0 : n < WRFB200_NUM_FIELDS ? 1 : 2;
+}
+
 int run_device_in_place(const Args &a, int prec)
 {
     // Caller-owned device arrays in the dense Fortran layout, wrapped in a (cached) handle.
@@ -1108,6 +1397,9 @@ int run_device_in_place(const Args &a, int prec)
 // arrays upload only u and v (what advance_uv changed; everything else on the device is this routine's own
 // previous output or a loop constant) -- the per-small-step drop-in pattern of a host-resident model:
 // 0.76 GB up and 1.15 GB down per step on 1800x1060x50 instead of 3.2 GB up.
+//
+// Page-locked arrays are copied directly; pageable 2-D and 3-D arrays take the staged route (upload_box,
+// download_box): every such copy goes through the cache's pinned bounce buffers.
 //
 // `part`: this is one device's share of a split call (run_host_split), or a shared-tiles call (run_host_shared),
 // whose calling thread has already synchronised the caller's stream and page-locked the caller's whole arrays.
@@ -1155,34 +1447,65 @@ int run_host_compat_body(const Args &a, int nsteps, wrfb200_handle *h, CompatCac
     if (pin_enabled() && !part)
         for (int f = 0; f < WRFB200_NUM_FIELDS; ++f) pin_host(a.f[f], field_bytes(d, f, h->esize));
 
-    // small operands first: 2-D and 1-D inputs, and ww at level 1 (the only level of ww the routine
-    // reads, module_small_step_em.f90:159-161)
-    h->stream = cc.up;
-    if (!resident && !sp) {
-        for (int f : in2) if (int rc = copy_field(h, f, a.f[f], nullptr)) return rc;
-        for (int f : in1) if (int rc = copy_field(h, f, a.f[f], nullptr)) return rc;
-        if (int rc = copy_range(h, WRFB200_WW, a.f[WRFB200_WW], nullptr, d.ims, d.ime, a.kts, a.kts, d.jms, d.jme)) return rc;
-    } else if (!resident) {
-        for (int f : in2)
-            if (f != WRFB200_MU)
-                if (int rc = copy_range(h, f, a.f[f], nullptr, d.ims, d.ime, 0, 0, js - 1, je + 1)) return rc;
-        for (int f : in1) if (int rc = copy_field(h, f, a.f[f], nullptr)) return rc;
-        if (int rc = copy_range(h, WRFB200_MU, a.f[WRFB200_MU], nullptr, is, ie, 0, 0, js, je)) return rc;
-        if (int rc = copy_range(h, WRFB200_WW, a.f[WRFB200_WW], nullptr, is, ie, a.kts, a.kts, js, je)) return rc;
-    }
-
     const int nj = je - js + 1;
     const size_t es = (size_t)h->esize;
     const size_t bytes3 = (size_t)h->idim * h->kdim * h->jdim * es;
     int nslab = 1;
     if (bytes3 >= ((size_t)16 << 20) && nj >= 32) nslab = nj / 16 < kMaxSlabs ? nj / 16 : kMaxSlabs;
     if (nslab > kMaxSlabs) nslab = kMaxSlabs;             // one event pair per slab
+    const size_t slab_bytes = (size_t)(nj / nslab + 3) * h->kdim * h->idim * es;
+
+    // The route of each array: page-locked ones (by the caller or by opt-in pinning) are copied directly, pageable
+    // 2-D and 3-D ones through the cache's bounce buffers (the 1-D ones, a few hundred bytes, directly as well).
+    bool bounce[WRFB200_NUM_FIELDS];
+    bool any_bounce = false;
+    for (int f = 0; f < WRFB200_NUM_FIELDS; ++f) {
+        bounce[f] = !is1d(f) && pageable(a.f[f]);
+        any_bounce = any_bounce || bounce[f];
+    }
+    HostPool *pool = nullptr;
+    PendingDown pend[kBounce];
+    if (any_bounce) {
+        if (int rc = ensure_bounce(cc, slab_bytes, (size_t)(nj / nslab + 3) * h->idim * es)) return rc;
+        pool = host_pool();
+    }
+
+    // small operands first: 2-D and 1-D inputs, and ww at level 1 (the only level of ww the routine
+    // reads, module_small_step_em.f90:159-161)
+    h->stream = cc.up;
+    if (!resident && !sp) {
+        for (int f : in2) {
+            if (bounce[f]) {
+                if (int rc = upload_box(cc, h, pool, Box{f, d.ims, d.ime, 0, 0, d.jms, d.jme}, a.f[f], nullptr)) return rc;
+            } else if (int rc = copy_field(h, f, a.f[f], nullptr)) return rc;
+        }
+        for (int f : in1) if (int rc = copy_field(h, f, a.f[f], nullptr)) return rc;
+        if (bounce[WRFB200_WW]) {
+            const Box b{WRFB200_WW, d.ims, d.ime, a.kts, a.kts, d.jms, d.jme};
+            if (int rc = upload_box(cc, h, pool, b, a.f[WRFB200_WW], nullptr)) return rc;
+        } else if (int rc = copy_range(h, WRFB200_WW, a.f[WRFB200_WW], nullptr, d.ims, d.ime, a.kts, a.kts, d.jms, d.jme)) return rc;
+    } else if (!resident) {
+        for (int f : in2) {
+            if (f == WRFB200_MU) continue;
+            if (bounce[f]) {
+                if (int rc = upload_box(cc, h, pool, Box{f, d.ims, d.ime, 0, 0, js - 1, je + 1}, a.f[f], nullptr)) return rc;
+            } else if (int rc = copy_range(h, f, a.f[f], nullptr, d.ims, d.ime, 0, 0, js - 1, je + 1)) return rc;
+        }
+        for (int f : in1) if (int rc = copy_field(h, f, a.f[f], nullptr)) return rc;
+        if (bounce[WRFB200_MU]) {
+            if (int rc = upload_box(cc, h, pool, Box{WRFB200_MU, is, ie, 0, 0, js, je}, a.f[WRFB200_MU], nullptr)) return rc;
+        } else if (int rc = copy_range(h, WRFB200_MU, a.f[WRFB200_MU], nullptr, is, ie, 0, 0, js, je)) return rc;
+        if (bounce[WRFB200_WW]) {
+            const Box b{WRFB200_WW, is, ie, a.kts, a.kts, js, je};
+            if (int rc = upload_box(cc, h, pool, b, a.f[WRFB200_WW], nullptr)) return rc;
+        } else if (int rc = copy_range(h, WRFB200_WW, a.f[WRFB200_WW], nullptr, is, ie, a.kts, a.kts, js, je)) return rc;
+    }
+
     int next_row = js - 1;                                // first row of the 3-D inputs not yet uploaded
     // A row-pitched (2-D) host->device copy runs ~18 % below a contiguous one on this link (40 vs 49 GB/s
     // measured, tools/pcie_probe.py).  When the mirror is padded, land each slab densely in a staging buffer
     // with ONE contiguous copy and re-pitch it on the device (HBM speed, negligible).
     const bool staged = (h->pitch3 != h->idim) && nslab > 1;
-    const size_t slab_bytes = (size_t)(nj / nslab + 3) * h->kdim * h->idim * es;
     if (staged && cc.stage_bytes < slab_bytes) {
         for (void *&b : cc.stage) { if (b) cudaFree(b); b = nullptr; }
         cc.stage_bytes = 0;
@@ -1203,6 +1526,13 @@ int run_host_compat_body(const Args &a, int nsteps, wrfb200_handle *h, CompatCac
             const size_t doff = (size_t)(next_row - d.jms) * h->kdim * h->pitch3;
             for (int x = 0; x < n_in3; ++x) {
                 const int f = in3[x];
+                if (bounce[f]) {
+                    void *land = staged ? cc.stage[flip] : nullptr;
+                    if (staged) flip ^= 1;
+                    const Box b{f, d.ims, d.ime, d.kms, d.kme, next_row, hi};
+                    if (int rc = upload_box(cc, h, pool, b, a.f[f], land)) return rc;
+                    continue;
+                }
                 if (!staged) {
                     if (int rc = copy_range(h, f, a.f[f], nullptr, d.ims, d.ime, d.kms, d.kme, next_row, hi)) return rc;
                     continue;
@@ -1217,7 +1547,10 @@ int run_host_compat_body(const Args &a, int nsteps, wrfb200_handle *h, CompatCac
             next_row = hi + 1;
         }
         // shared tiles: t over the slab's own columns (all levels: no tile reads or writes t outside its columns)
-        if (sp && !resident)
+        if (sp && !resident && bounce[WRFB200_T]) {
+            const Box b{WRFB200_T, is, ie, d.kms, d.kme, ja, jb};
+            if (int rc = upload_box(cc, h, pool, b, a.f[WRFB200_T], nullptr)) return rc;
+        } else if (sp && !resident)
             if (int rc = copy_range(h, WRFB200_T, a.f[WRFB200_T], nullptr, is, ie, d.kms, d.kme, ja, jb)) return rc;
         CU(cudaEventRecord(cc.ev_up[s], cc.up));
         // all steps of this slab
@@ -1229,9 +1562,21 @@ int run_host_compat_body(const Args &a, int nsteps, wrfb200_handle *h, CompatCac
         // outputs: exactly the cells the Fortran writes
         CU(cudaStreamWaitEvent(cc.down, cc.ev_comp[s], 0));
         h->stream = cc.down;
-        for (int f : out3) if (int rc = copy_range(h, f, nullptr, a.f[f], is, ie, ks, ke, ja, jb)) return rc;
-        for (int f : out2) if (int rc = copy_range(h, f, nullptr, a.f[f], is, ie, 0, 0, ja, jb)) return rc;
+        for (int x = 0; x < 3; ++x) {
+            const int f = out3[x];
+            if (bounce[f]) {
+                if (int rc = download_box(cc, h, pool, pend, kBounceUp + x, Box{f, is, ie, ks, ke, ja, jb}, a.f[f])) return rc;
+            } else if (int rc = copy_range(h, f, nullptr, a.f[f], is, ie, ks, ke, ja, jb)) return rc;
+        }
+        for (int x = 0; x < 4; ++x) {
+            const int f = out2[x];
+            if (bounce[f]) {
+                if (int rc = download_box(cc, h, pool, pend, kBounce3 + x, Box{f, is, ie, 0, 0, ja, jb}, a.f[f])) return rc;
+            } else if (int rc = copy_range(h, f, nullptr, a.f[f], is, ie, 0, 0, ja, jb)) return rc;
+        }
     }
+    for (int x = 0; x < kBounce; ++x)
+        if (int rc = finish_down(cc, h, pool, pend, x)) return rc;
     CU(cudaStreamSynchronize(cc.up));
     CU(cudaStreamSynchronize(cc.comp));
     CU(cudaStreamSynchronize(cc.down));
@@ -1491,7 +1836,9 @@ int dispatch(Args &a, int nsteps, bool allow_device, int prec)
         return run_device_in_place(a, prec);
     }
     dc.valid = false;
-    return run_host_compat(a, nsteps, prec);
+    const int rc = run_host_compat(a, nsteps, prec);
+    g_last_route = transfer_route(a);                     // after the call: opt-in pinning may have locked the arrays
+    return rc;
 }
 
 }  // namespace
@@ -1640,6 +1987,7 @@ extern "C" int wrfb200_release_cache(void)
     release_shared();
     for (DeviceCallCache &c : g_devcall) c.valid = false;
     unpin_all();
+    stop_pool();
     return WRFB200_OK;
 }
 
@@ -1748,5 +2096,13 @@ extern "C" int wrfb200_default_last_kernel(int *kernel)
     const DeviceCallCache &dc = g_devcall[g_last_prec];
     const CompatCache &cc = shared_enabled() ? g_tiles.c[g_last_prec] : g_cache[g_last_prec];
     *kernel = dc.valid ? dc.h.last_kernel : (cc.h ? cc.h->last_kernel : 0);
+    return WRFB200_OK;
+}
+
+extern "C" int wrfb200_default_last_transfer(int *route)
+{
+    if (!route) return fail(WRFB200_ERR_INVALID_ARG, "null argument");
+    if (g_last_route < 0) return fail(WRFB200_ERR_STATE, "no host-array call on this thread yet");
+    *route = g_last_route;
     return WRFB200_OK;
 }

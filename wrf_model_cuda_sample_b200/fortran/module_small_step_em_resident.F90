@@ -114,6 +114,13 @@ INTERFACE
       IMPORT :: c_int
       INTEGER(c_int) :: status
    END FUNCTION
+   ! how this thread's last advance_mu_t call moved its arrays: 0 all direct (page-locked), 1 some staged through
+   ! the library's pinned bounce buffers (pageable), 2 all staged
+   FUNCTION wrfb200_default_last_transfer(route) BIND(C, NAME="wrfb200_default_last_transfer") RESULT(status)
+      IMPORT :: c_int
+      INTEGER(c_int), INTENT(OUT) :: route
+      INTEGER(c_int) :: status
+   END FUNCTION
    ! OpenMP builds (smpar, dm+sm): the tiles of the !$OMP PARALLEL DO share one device-resident patch.  Call once,
    ! after the rank has picked its GPU; the loop begin / end and the per-tile advance_mu_t calls are unchanged
    ! (INTEGRATION.md section 1)
