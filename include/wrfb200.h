@@ -113,6 +113,13 @@ typedef enum wrfb200_kernel {
 /* Halo sides of a patch. */
 typedef enum wrfb200_side { WRFB200_WEST = 0, WRFB200_EAST = 1, WRFB200_SOUTH = 2, WRFB200_NORTH = 3 } wrfb200_side;
 
+/* What a wrfb200_advance_mu_t call did with the calling thread's cache (wrfb200_default_last_cache). */
+typedef enum wrfb200_cache {
+    WRFB200_CACHE_REUSED = 0,   /* the device state of its domain (or its device-pointer wrapper) was already there */
+    WRFB200_CACHE_CREATED = 1,  /* it was created */
+    WRFB200_CACHE_EVICTED = 2   /* it was created after the least recently used domain(s) had been freed */
+} wrfb200_cache;
+
 typedef struct wrfb200_handle wrfb200_handle;
 
 /* ------------------------------------------------------------------------------------------------
@@ -120,8 +127,9 @@ typedef struct wrfb200_handle wrfb200_handle;
  *    (module_small_step_em.f90:7-18; config_flags expanded to its three used members).
  *
  *    Pointers may be HOST pointers (compat mode: upload -> step -> download of the written ranges ->
- *    sync; device mirrors are cached per thread and re-used by later calls with the same extents) or
- *    DEVICE pointers (launched in place on the current wrfb200 stream, returns without host sync).
+ *    sync; device mirrors are cached per thread and precision, one set per domain -- device and memory
+ *    extents -- for up to 8 domains, and re-used by later calls of that domain) or DEVICE pointers
+ *    (launched in place on the current wrfb200 stream, returns without host sync).
  *    All array pointers of one call must be of the same kind.  Writes exactly the cells the Fortran
  *    writes: ww,t,t_ave for k<=kte-1 and mu,muave,muts,mudf, inside i_start..i_end x j_start..j_end only.
  * ---------------------------------------------------------------------------------------------- */
@@ -184,9 +192,23 @@ int wrfb200_advance_mu_t_loop_r8(
 int wrfb200_set_default_stream(void *cuda_stream);
 int wrfb200_set_default_kernel(int kernel /* wrfb200_kernel */);
 
-/* Release the per-thread device mirrors cached by the host-pointer form (and every host registration), and the
- * shared patches of shared-tiles mode (wrfb200_set_shared_tiles) with every thread's state for them.  It also stops
- * and joins the host threads of the staged route (wrfb200_set_host_pinning); no call may be in flight then. */
+/* Domain caches.  A nested run calls the host-pointer form for the parent and each nest in turn, with other memory
+ * extents (and often another kde).  The calling thread keeps, per precision, the device state of up to 8 domains,
+ * keyed by device and memory extents ims..ime, jms..jme, kms..kme (not by array addresses), most recently used
+ * first: its mirrors, device staging buffers and acoustic-loop residency.  A call for a domain seen before
+ * allocates nothing.  The thread's lanes and pinned bounce buffers serve all its domains; the buffers only grow,
+ * to the largest slab any of them needs.  Before a new domain is created, the least recently used ones are freed:
+ * beyond 8, and on the domain's device while the free memory there cannot hold the new mirrors and staging buffers;
+ * if the allocation still runs out of memory, every other domain of the thread is freed and it is tried once more,
+ * then the call fails with WRFB200_ERR_NOMEM.  Each entry of a split call's device list (wrfb200_set_default_devices)
+ * keeps its domains the same way, in a cache of its own.  Device-pointer calls keep the wrapping handle and
+ * tensor maps of the thread's 4 most recent sets of (26 pointers, domain) per precision.
+ *
+ * wrfb200_release_cache frees all of it: every domain of the calling thread's caches, its device-pointer wrappers,
+ * every host registration, and the shared patches of shared-tiles mode (wrfb200_set_shared_tiles) with every
+ * thread's state for them.  Call it to hand the device memory back to the model, e.g. before a phase that needs it
+ * or at the end of a run.  It also stops and joins the host threads of the staged route (wrfb200_set_host_pinning);
+ * no call may be in flight then. */
 int wrfb200_release_cache(void);
 
 /* Acoustic-loop residency for HOST-pointer callers of wrfb200_advance_mu_t (thread-local).  Between begin and
@@ -195,7 +217,8 @@ int wrfb200_release_cache(void);
  * downloads the seven outputs.  Contract: between those calls the caller changes nothing but u and v (ww, t,
  * mu on the device are this routine's own previous outputs; the rest are constants of the RK sub-step).
  * This is the reference's per-call H2D of all 26 arrays (advance_mu_t_no_async.cu:245-306) reduced to the
- * two that change. */
+ * two that change.  Residency is kept per domain, and begin / end act on every domain of the thread: the first
+ * call of each domain in a loop uploads everything, whatever another domain did in between. */
 int wrfb200_acoustic_loop_begin(void);
 int wrfb200_acoustic_loop_end(void);
 
@@ -225,6 +248,19 @@ int wrfb200_default_last_kernel(int *kernel);
  * (pageable ones), 2 every array staged.  The four 1-D arrays, a few hundred bytes, are copied directly even when
  * pageable but count by what they are.  No host-pointer call on this thread yet: WRFB200_ERR_STATE. */
 int wrfb200_default_last_transfer(int *route);
+
+/* What the most recent wrfb200_advance_mu_t / _loop call of this thread (either precision, host or device pointers)
+ * did with its cache (thread-local): *state is a wrfb200_cache -- 0 re-used its domain's device state (or
+ * device-pointer wrapper), 1 created it, 2 created it after freeing the least recently used domain(s).  A call split
+ * over several devices reports the most any part did; a shared-tiles call, 1 when it created the shared patch or
+ * the thread's handle for it.  No call on this thread has reached its cache yet (or the last one was refused
+ * before): WRFB200_ERR_STATE. */
+int wrfb200_default_last_cache(int *state);
+
+/* How many times the host-pointer caches of this process have allocated their pinned bounce buffers (the staged
+ * route's nine cudaHostAlloc buffers), first allocations and growth alike.  A diagnostic: the buffers only grow, to
+ * the largest slab each cache has seen, so calls that alternate between domains a cache already holds allocate none. */
+int wrfb200_bounce_allocations(long *count);
 
 /* Devices the HOST-pointer form of wrfb200_advance_mu_t / _loop (and the _r8 pair) spreads its j-rows over.
  * Thread-local, like wrfb200_set_default_stream / _kernel.  n = 0 (devices may be NULL): back to the current

@@ -28,6 +28,8 @@ OK, ERR_INVALID_ARG, ERR_UNSUPPORTED, ERR_CUDA, ERR_NOMEM, ERR_STATE = range(6)
 KERNEL_AUTO, KERNEL_COLUMN, KERNEL_TILE, KERNEL_PIPE = 0, 1, 2, 3
 # wrfb200_default_last_transfer: every array copied directly / some staged through bounce buffers / all staged
 TRANSFER_DIRECT, TRANSFER_MIXED, TRANSFER_STAGED = 0, 1, 2
+# enum wrfb200_cache (wrfb200_default_last_cache): the domain's device state re-used / created / created after evicting
+CACHE_REUSED, CACHE_CREATED, CACHE_EVICTED = 0, 1, 2
 WEST, EAST, SOUTH, NORTH = 0, 1, 2, 3
 
 
@@ -78,6 +80,8 @@ PROTOTYPES = {
     "wrfb200_host_unregister_all": (C.c_int, []),
     "wrfb200_default_last_kernel": (C.c_int, [C.POINTER(C.c_int)]),
     "wrfb200_default_last_transfer": (C.c_int, [C.POINTER(C.c_int)]),
+    "wrfb200_default_last_cache": (C.c_int, [C.POINTER(C.c_int)]),
+    "wrfb200_bounce_allocations": (C.c_int, [C.POINTER(C.c_long)]),
     "wrfb200_set_default_devices": (C.c_int, [C.POINTER(C.c_int), C.c_int]),
     "wrfb200_set_shared_tiles": (C.c_int, [C.c_int]),
     "wrfb200_host_split_plan": (C.c_int, [C.POINTER(Domain)] + [C.c_int] * 7 + [C.POINTER(C.c_int)]),

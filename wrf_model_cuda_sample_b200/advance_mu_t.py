@@ -487,6 +487,16 @@ def default_last_transfer() -> int:
     return r.value
 
 
+def default_last_cache() -> int:
+    """What the most recent ``advance_mu_t`` call of this thread (either precision, host arrays or device tensors)
+    did with its cache: ``CACHE_REUSED`` (its domain's device state, or device-pointer wrapper, was already there),
+    ``CACHE_CREATED`` or ``CACHE_EVICTED`` (created after the least recently used domains were freed).  Raises
+    ``WrfB200Error`` (``ERR_STATE``) when no call of this thread has reached its cache yet."""
+    r = C.c_int()
+    check(lib().wrfb200_default_last_cache(C.byref(r)))
+    return r.value
+
+
 def synth_fields(grid: Grid, seed: int = 20240617, names: Iterable[str] = FIELDS, pinned: bool = False,
                  dx_m: float = 12000.0) -> Dict[str, np.ndarray]:
     """Deterministic atmosphere-like fields for ``grid``'s memory extents (wrfb200_synth_field).

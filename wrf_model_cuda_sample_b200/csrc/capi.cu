@@ -11,6 +11,7 @@
 #include <sched.h>
 #include <unistd.h>
 
+#include <algorithm>
 #include <atomic>
 #include <condition_variable>
 #include <cstdarg>
@@ -411,6 +412,21 @@ extern "C" int wrfb200_bounds(int periodic_x, int specified, int nested,
 // -------------------------------------------------------------------------------------------------
 namespace {
 
+// elements of the device mirror of field f: rows of `pitch` elements
+size_t mirror_elems(int f, long pitch, long kdim, long jdim)
+{
+    return is3d(f) ? (size_t)pitch * kdim * jdim : is2d(f) ? (size_t)pitch * jdim : (size_t)kdim;
+}
+
+// bytes of the 26 mirrors create() allocates for the memory extents of d
+size_t mirror_bytes(const wrfb200_domain &d, int esize)
+{
+    const long pitch = round_up(d.ime - d.ims + 1, 128 / esize), jdim = d.jme - d.jms + 1, kdim = d.kme - d.kms + 1;
+    size_t n = 0;
+    for (int f = 0; f < WRFB200_NUM_FIELDS; ++f) n += mirror_elems(f, pitch, kdim, jdim);
+    return n * esize;
+}
+
 int create(wrfb200_handle **out, const wrfb200_domain *dom, int device, int allocate, int esize)
 {
     if (!out || !dom) return fail(WRFB200_ERR_INVALID_ARG, "null argument");
@@ -434,9 +450,7 @@ int create(wrfb200_handle **out, const wrfb200_domain *dom, int device, int allo
         if (!g.ok) { delete h; return fail(WRFB200_ERR_CUDA, "cannot select CUDA device %d", device); }
         h->pitch3 = h->pitch2 = round_up(h->idim, 128 / esize);  // 128-byte rows
         for (int f = 0; f < WRFB200_NUM_FIELDS; ++f) {
-            size_t n = is3d(f) ? (size_t)h->pitch3 * h->kdim * h->jdim
-                     : is2d(f) ? (size_t)h->pitch2 * h->jdim
-                               : (size_t)h->kdim;
+            const size_t n = mirror_elems(f, is3d(f) ? h->pitch3 : h->pitch2, h->kdim, h->jdim);
             cudaError_t e = cudaMalloc(&h->d[f], n * esize);
             if (e == cudaSuccess) e = cudaMemsetAsync(h->d[f], 0, n * esize, nullptr);
             if (e != cudaSuccess) {
@@ -852,46 +866,77 @@ struct Args {
     int its, ite, jts, jte, kts, kte;
 };
 
-// Per-thread cache of device mirrors for host-pointer callers (the reference allocates and frees
-// 29 buffers on every call; we allocate once per distinct memory shape).
-struct CompatCache {
-    wrfb200_handle *h = nullptr;
-    cudaStream_t up = nullptr, comp = nullptr, down = nullptr;      // upload / compute / download lanes
-    cudaEvent_t ev_up[kMaxSlabs] = {}, ev_comp[kMaxSlabs] = {};
+// Per-thread cache of device mirrors for host-pointer callers (the reference allocates and frees 29 buffers on every
+// call; we allocate once per domain).  A nested WRF run calls the routine for the parent and for each nest in turn,
+// with other memory extents, so a cache keeps the mirrors of up to kMaxDomains domains, most recently used first,
+// and a switch back to one of them allocates nothing.  Each domain owns its mirrors, device staging buffers and
+// residency; the lanes, their events and the pinned bounce buffers belong to the cache and serve all its domains
+// one call at a time, so N domains do not mean N sets of page-locked memory.
+constexpr size_t kMaxDomains = 8;
+
+// One domain of a cache, keyed by its device and memory extents (not by the caller's array addresses: solve_em
+// passes locals that may move between calls).
+struct DomainEntry {
+    wrfb200_handle *h = nullptr;                                    // owns the 26 mirrors
     void *stage[2] = {nullptr, nullptr};                            // dense landing buffers for H2D slabs
     size_t stage_bytes = 0;
-    // staged route (pageable caller arrays): pinned bounce buffers, allocated on first use, and per buffer the
-    // event of the device copy that last read or filled it
+    // acoustic-loop residency (wrfb200_acoustic_loop_begin/end): after the first call of a loop the device
+    // mirrors hold everything; later calls with the SAME arrays and index sets move only u, v up
+    bool primed = false;
+    Args primed_args{};
+    ~DomainEntry()
+    {
+        if (!h) return;
+        DeviceGuard g(h->device);
+        h->stream = nullptr;               // never synchronise on a lane (they outlive the entry or are gone)
+        wrfb200_destroy(h);                // device-wide sync, frees the mirrors
+        for (void *b : stage) if (b) cudaFree(b);
+        (void)cudaGetLastError();
+    }
+};
+
+struct CompatCache {
+    std::vector<std::unique_ptr<DomainEntry>> doms;                 // most recently used first
+    int lane_device = -1;                                           // the device of the lanes and events
+    cudaStream_t up = nullptr, comp = nullptr, down = nullptr;      // upload / compute / download lanes
+    cudaEvent_t ev_up[kMaxSlabs] = {}, ev_comp[kMaxSlabs] = {};
+    // staged route (pageable caller arrays): pinned bounce buffers, allocated on first use and grown to the largest
+    // slab seen, and per buffer the event of the device copy that last read or filled it
     void *bounce[kBounce] = {};
     cudaEvent_t ev_bounce[kBounce] = {};
     size_t bounce3_bytes = 0, bounce2_bytes = 0;
     int next_up = 0;                                                // the upload buffer filled next
-    // acoustic-loop residency (wrfb200_acoustic_loop_begin/end): after the first call of a loop the device
-    // mirrors hold everything; later calls with the SAME arrays and index sets move only u, v up
-    bool loop_active = false, primed = false;
-    Args primed_args{};
+    bool loop_active = false;                                       // between wrfb200_acoustic_loop_begin and _end
+    void forget()
+    {
+        for (auto &e : doms) e->primed = false;
+    }
+    void release_lanes()
+    {
+        if (lane_device < 0) return;
+        DeviceGuard g(lane_device);
+        for (cudaStream_t st : {up, comp, down}) if (st) cudaStreamSynchronize(st);
+        for (void *&b : bounce) if (b) { cudaFreeHost(b); b = nullptr; }
+        for (cudaEvent_t &e : ev_bounce) if (e) { cudaEventDestroy(e); e = nullptr; }
+        bounce3_bytes = bounce2_bytes = 0;
+        for (cudaEvent_t &e : ev_up) if (e) { cudaEventDestroy(e); e = nullptr; }
+        for (cudaEvent_t &e : ev_comp) if (e) { cudaEventDestroy(e); e = nullptr; }
+        for (cudaStream_t *st : {&up, &comp, &down}) if (*st) { cudaStreamDestroy(*st); *st = nullptr; }
+        lane_device = -1;
+        (void)cudaGetLastError();
+    }
     void release()
     {
-        primed = false;
-        if (h) {
-            DeviceGuard g(h->device);
-            h->stream = nullptr;               // never synchronise on one of the lanes destroyed below
-            wrfb200_destroy(h);                // device-wide sync, frees the mirrors
-            h = nullptr;
-            for (void *&b : stage) if (b) { cudaFree(b); b = nullptr; }
-            stage_bytes = 0;
-            for (void *&b : bounce) if (b) { cudaFreeHost(b); b = nullptr; }
-            for (cudaEvent_t &e : ev_bounce) if (e) { cudaEventDestroy(e); e = nullptr; }
-            bounce3_bytes = bounce2_bytes = 0;
-            for (cudaEvent_t &e : ev_up) if (e) { cudaEventDestroy(e); e = nullptr; }
-            for (cudaEvent_t &e : ev_comp) if (e) { cudaEventDestroy(e); e = nullptr; }
-            for (cudaStream_t *st : {&up, &comp, &down}) if (*st) { cudaStreamDestroy(*st); *st = nullptr; }
-            (void)cudaGetLastError();
-        }
+        doms.clear();
+        release_lanes();
     }
     ~CompatCache() { release(); }
 };
 thread_local CompatCache g_cache[2];        // [0]: binary32 calls, [1]: real*8 calls
+
+// wrfb200_default_last_cache: what the thread's last call did with its cache (wrfb200_cache; -1: no call has
+// reached its cache yet)
+thread_local int g_last_cache = -1;
 
 // the same arrays, index sets and scalars as the call that primed a resident tile
 bool same_call(const Args &p, const Args &a)
@@ -1012,15 +1057,34 @@ void release_shared()
 
 // Device-pointer callers: the handle that wraps the caller's arrays (and its six TMA tensor maps) is kept
 // between calls and re-used while the pointers and extents stay the same -- a 25-830 us step must not pay
-// six cuTensorMapEncodeTiled and 26 cudaPointerGetAttributes every time.
+// six cuTensorMapEncodeTiled and 26 cudaPointerGetAttributes every time.  A thread keeps kDeviceCalls of them
+// per precision, the least recently used one replaced first, so that a nested run alternating its domains keeps
+// the wrapper of each.  A host-pointer call drops them all.
+constexpr int kDeviceCalls = 4;
 struct DeviceCallCache {
     wrfb200_handle h;
     void *ptrs[WRFB200_NUM_FIELDS] = {};
     wrfb200_domain dom{};
     bool valid = false;
+    long used = 0;                           // g_devcall_clock at its last call
 };
-thread_local DeviceCallCache g_devcall[2];   // indexed like g_cache
+thread_local DeviceCallCache g_devcall[2][kDeviceCalls];   // indexed like g_cache
+thread_local long g_devcall_clock = 0;
 thread_local int g_last_prec = 0;              // which of the two the most recent call used
+
+// the entry of the thread's most recent device-pointer call of precision prec, if none has been dropped since
+const DeviceCallCache *last_devcall(int prec)
+{
+    const DeviceCallCache *last = nullptr;
+    for (const DeviceCallCache &c : g_devcall[prec])
+        if (c.valid && (!last || c.used > last->used)) last = &c;
+    return last;
+}
+
+void drop_devcalls(int prec)
+{
+    for (DeviceCallCache &c : g_devcall[prec]) c.valid = false;
+}
 
 bool same_shape(const wrfb200_domain &a, const wrfb200_domain &b)
 {
@@ -1259,10 +1323,18 @@ int device_box(wrfb200_handle *h, const Box &b, char *buf, bool to_dev, cudaStre
     return WRFB200_OK;
 }
 
-// The cache's bounce buffers, at least b3 bytes (0..4) and b2 bytes (5..8), and their events.
+// wrfb200_bounce_allocations: sets of bounce buffers allocated by every cache of the process
+std::atomic<long> g_bounce_allocs{0};
+
+// The cache's bounce buffers, at least b3 bytes (0..4) and b2 bytes (5..8), and their events.  They only grow, each
+// size to the largest seen, so that calls of the cache's domains in turn find them large enough whichever of the two
+// sizes each domain needs more of.
 int ensure_bounce(CompatCache &cc, size_t b3, size_t b2)
 {
     if (cc.bounce3_bytes >= b3 && cc.bounce2_bytes >= b2) return WRFB200_OK;
+    b3 = std::max(b3, cc.bounce3_bytes);
+    b2 = std::max(b2, cc.bounce2_bytes);
+    g_bounce_allocs.fetch_add(1);
     for (void *&b : cc.bounce) if (b) { cudaFreeHost(b); b = nullptr; }
     cc.bounce3_bytes = cc.bounce2_bytes = 0;
     for (int x = 0; x < kBounce; ++x) {
@@ -1361,11 +1433,19 @@ int run_device_in_place(const Args &a, int prec)
 {
     // Caller-owned device arrays in the dense Fortran layout, wrapped in a (cached) handle.
     if (int rc = check_domain(a.dom)) return rc;
-    DeviceCallCache &c = g_devcall[prec];
     int dev = 0;
     CU(cudaGetDevice(&dev));
-    const bool hit = c.valid && c.h.device == dev && same_domain(c.dom, a.dom) &&
-                     std::memcmp(c.ptrs, a.f, sizeof(c.ptrs)) == 0;
+    DeviceCallCache *hit = nullptr, *oldest = &g_devcall[prec][0];
+    for (DeviceCallCache &x : g_devcall[prec]) {
+        if (x.valid && x.h.device == dev && same_domain(x.dom, a.dom) && std::memcmp(x.ptrs, a.f, sizeof(x.ptrs)) == 0) {
+            hit = &x;
+            break;
+        }
+        if (oldest->valid && (!x.valid || x.used < oldest->used)) oldest = &x;    // a free entry first
+    }
+    DeviceCallCache &c = hit ? *hit : *oldest;
+    g_last_cache = hit ? WRFB200_CACHE_REUSED : c.valid ? WRFB200_CACHE_EVICTED : WRFB200_CACHE_CREATED;
+    c.used = ++g_devcall_clock;
     if (!hit) {
         c.valid = false;
         c.h.dom = a.dom;
@@ -1413,9 +1493,24 @@ int run_device_in_place(const Args &a, int prec)
 //     tiles that both copy a ring row write the same bytes from the same host array, which the caller does not
 //     change during the loop's steps (u, v only between them); that is why those copies may overlap;
 //   - residency is kept per tile in `sp` (SharedPatch::take / put), whichever thread makes the call.
-int run_host_compat_body(const Args &a, int nsteps, wrfb200_handle *h, CompatCache &cc, bool part,
+// The slab pipeline's cut of nj computed rows of a call on memory extents d: nslab slabs of at most `rows` rows each,
+// ring rows included (the rows of a staging buffer and of a bounce buffer).
+struct SlabPlan {
+    int nslab;
+    size_t rows;
+};
+SlabPlan slab_plan(const wrfb200_domain &d, int nj, size_t es)
+{
+    const size_t idim = d.ime - d.ims + 1, jdim = d.jme - d.jms + 1, kdim = d.kme - d.kms + 1;
+    int nslab = 1;
+    if (idim * kdim * jdim * es >= ((size_t)16 << 20) && nj >= 32) nslab = nj / 16 < kMaxSlabs ? nj / 16 : kMaxSlabs;
+    return SlabPlan{nslab, (size_t)(nj / nslab + 3)};         // at most kMaxSlabs: one event pair per slab
+}
+
+int run_host_compat_body(const Args &a, int nsteps, DomainEntry &e, CompatCache &cc, bool part,
                          SharedPatch *sp = nullptr)
 {
+    wrfb200_handle *h = e.h;
     const wrfb200_domain &d = a.dom;
     int is, ie, js, je, ks, ke;
     wrfb200_bounds(d.periodic_x, d.specified, d.nested, d.ids, d.ide, d.jds, d.jde,
@@ -1439,8 +1534,8 @@ int run_host_compat_body(const Args &a, int nsteps, wrfb200_handle *h, CompatCac
     static const int out2[] = {WRFB200_MU, WRFB200_MUAVE, WRFB200_MUTS, WRFB200_MUDF};
 
     // resident step: same arrays, same index sets, same scalars as the call that primed the mirrors
-    const bool resident = sp ? sp->take(a) : cc.loop_active && cc.primed && same_call(cc.primed_args, a);
-    cc.primed = false;                                    // until this call has completed
+    const bool resident = sp ? sp->take(a) : cc.loop_active && e.primed && same_call(e.primed_args, a);
+    e.primed = false;                                     // until this call has completed
     const int *in3 = resident ? in3_uv : sp ? in3_ring : in3_all;
     const int n_in3 = resident ? 2 : sp ? 7 : 8;
 
@@ -1449,11 +1544,9 @@ int run_host_compat_body(const Args &a, int nsteps, wrfb200_handle *h, CompatCac
 
     const int nj = je - js + 1;
     const size_t es = (size_t)h->esize;
-    const size_t bytes3 = (size_t)h->idim * h->kdim * h->jdim * es;
-    int nslab = 1;
-    if (bytes3 >= ((size_t)16 << 20) && nj >= 32) nslab = nj / 16 < kMaxSlabs ? nj / 16 : kMaxSlabs;
-    if (nslab > kMaxSlabs) nslab = kMaxSlabs;             // one event pair per slab
-    const size_t slab_bytes = (size_t)(nj / nslab + 3) * h->kdim * h->idim * es;
+    const SlabPlan plan = slab_plan(d, nj, es);
+    const int nslab = plan.nslab;
+    const size_t slab_bytes = plan.rows * h->kdim * h->idim * es;
 
     // The route of each array: page-locked ones (by the caller or by opt-in pinning) are copied directly, pageable
     // 2-D and 3-D ones through the cache's bounce buffers (the 1-D ones, a few hundred bytes, directly as well).
@@ -1466,7 +1559,7 @@ int run_host_compat_body(const Args &a, int nsteps, wrfb200_handle *h, CompatCac
     HostPool *pool = nullptr;
     PendingDown pend[kBounce];
     if (any_bounce) {
-        if (int rc = ensure_bounce(cc, slab_bytes, (size_t)(nj / nslab + 3) * h->idim * es)) return rc;
+        if (int rc = ensure_bounce(cc, slab_bytes, plan.rows * h->idim * es)) return rc;
         pool = host_pool();
     }
 
@@ -1506,11 +1599,11 @@ int run_host_compat_body(const Args &a, int nsteps, wrfb200_handle *h, CompatCac
     // measured, tools/pcie_probe.py).  When the mirror is padded, land each slab densely in a staging buffer
     // with ONE contiguous copy and re-pitch it on the device (HBM speed, negligible).
     const bool staged = (h->pitch3 != h->idim) && nslab > 1;
-    if (staged && cc.stage_bytes < slab_bytes) {
-        for (void *&b : cc.stage) { if (b) cudaFree(b); b = nullptr; }
-        cc.stage_bytes = 0;
-        for (void *&b : cc.stage) CU(cudaMalloc(&b, slab_bytes));
-        cc.stage_bytes = slab_bytes;
+    if (staged && e.stage_bytes < slab_bytes) {
+        for (void *&b : e.stage) { if (b) cudaFree(b); b = nullptr; }
+        e.stage_bytes = 0;
+        for (void *&b : e.stage) CU(cudaMalloc(&b, slab_bytes));
+        e.stage_bytes = slab_bytes;
     }
     const int fpe = h->esize / (int)sizeof(float);         // the re-pitch kernel moves 4-byte words
     int flip = 0;
@@ -1527,7 +1620,7 @@ int run_host_compat_body(const Args &a, int nsteps, wrfb200_handle *h, CompatCac
             for (int x = 0; x < n_in3; ++x) {
                 const int f = in3[x];
                 if (bounce[f]) {
-                    void *land = staged ? cc.stage[flip] : nullptr;
+                    void *land = staged ? e.stage[flip] : nullptr;
                     if (staged) flip ^= 1;
                     const Box b{f, d.ims, d.ime, d.kms, d.kme, next_row, hi};
                     if (int rc = upload_box(cc, h, pool, b, a.f[f], land)) return rc;
@@ -1537,7 +1630,7 @@ int run_host_compat_body(const Args &a, int nsteps, wrfb200_handle *h, CompatCac
                     if (int rc = copy_range(h, f, a.f[f], nullptr, d.ims, d.ime, d.kms, d.kme, next_row, hi)) return rc;
                     continue;
                 }
-                float *st = static_cast<float *>(cc.stage[flip]);
+                float *st = static_cast<float *>(e.stage[flip]);
                 flip ^= 1;
                 CU(cudaMemcpyAsync(st, static_cast<const char *>(a.f[f]) + hoff * es, (size_t)nrows * h->idim * es,
                                    cudaMemcpyHostToDevice, cc.up));
@@ -1583,59 +1676,139 @@ int run_host_compat_body(const Args &a, int nsteps, wrfb200_handle *h, CompatCac
     if (sp) {
         if (g_shared_loop.load()) sp->put(a);
     } else if (cc.loop_active) {
-        cc.primed = true;
-        cc.primed_args = a;
+        e.primed = true;
+        e.primed_args = a;
     }
     return WRFB200_OK;
 }
 
-// One host-pointer call, or one device's share of a split call, on the cached mirrors `cc`.  device < 0: the
-// current device, and a cache of the same memory shape is re-used wherever it lives (the single-device call);
-// device >= 0: the cache is re-created when it lives on another device.  `kernel` is the calling thread's
-// choice, passed in because a part may run in a worker thread.
-// The cache's handle (mirrors allocated or, with allocate=0, to be bound) and its lanes and events.
-int open_cache(CompatCache &cc, const wrfb200_domain &dom, int device, int allocate, int prec)
+// The cache's lanes and their events on `device`.  They move when a domain of the cache lives on another device
+// than the last one (a single-device caller that changed its current device).
+int open_lanes(CompatCache &cc, int device)
 {
-    if (int rc = create(&cc.h, &dom, device, allocate, prec ? 8 : 4)) return rc;
-    DeviceGuard g(cc.h->device);
-    for (cudaStream_t *st : {&cc.up, &cc.comp, &cc.down})
-        CU(cudaStreamCreateWithFlags(st, cudaStreamNonBlocking));
-    for (int i = 0; i < kMaxSlabs; ++i) {
-        CU(cudaEventCreateWithFlags(&cc.ev_up[i], cudaEventDisableTiming));
-        CU(cudaEventCreateWithFlags(&cc.ev_comp[i], cudaEventDisableTiming));
+    if (cc.lane_device == device) return WRFB200_OK;
+    cc.release_lanes();
+    DeviceGuard g(device);
+    if (!g.ok) return fail(WRFB200_ERR_CUDA, "cannot select CUDA device %d", device);
+    cc.lane_device = device;
+    const int rc = [&]() -> int {
+        for (cudaStream_t *st : {&cc.up, &cc.comp, &cc.down})
+            CU(cudaStreamCreateWithFlags(st, cudaStreamNonBlocking));
+        for (int i = 0; i < kMaxSlabs; ++i) {
+            CU(cudaEventCreateWithFlags(&cc.ev_up[i], cudaEventDisableTiming));
+            CU(cudaEventCreateWithFlags(&cc.ev_comp[i], cudaEventDisableTiming));
+        }
+        return WRFB200_OK;
+    }();
+    if (rc != WRFB200_OK) {
+        const std::string msg = wrfb200_last_error();
+        cc.release_lanes();
+        wrfb200_fail(rc, "%s", msg.c_str());
     }
+    return rc;
+}
+
+// A new domain at the front of the cache: its handle (mirrors allocated or, with allocate=0, to be bound).
+int open_domain(CompatCache &cc, const wrfb200_domain &dom, int device, int allocate, int prec)
+{
+    std::unique_ptr<DomainEntry> e(new (std::nothrow) DomainEntry());
+    if (!e) return fail(WRFB200_ERR_NOMEM, "out of host memory");
+    if (int rc = create(&e->h, &dom, device, allocate, prec ? 8 : 4)) return rc;
+    cc.doms.insert(cc.doms.begin(), std::move(e));
     return WRFB200_OK;
 }
 
-// run_host_compat_body on the cache's handle, with the calling thread's kernel choice and the call's scalars
-int run_on_cache(const Args &a, int nsteps, CompatCache &cc, int kernel, bool part, SharedPatch *sp)
+// The domain of the call's memory extents at the front of cache cc, found or created; *state tells which
+// (wrfb200_cache).  device < 0 (the single-device call): an entry of the same extents is re-used wherever it
+// lives, a new one goes on the current device; device >= 0 (a part of a split call): the entry must live there.
+// Before creating, the cache gives up its least recently used domains: beyond kMaxDomains, and on the target
+// device while its free memory cannot hold the new mirrors and the staging buffers the call will allocate.  If the allocation still runs out of memory, every
+// other domain of the cache (and of the thread's other precision, unless this is a part of a split call running
+// beside the thread's other parts) is freed and it is tried once more.
+int find_domain(CompatCache &cc, const Args &a, int device, int prec, bool part, int *state)
 {
-    wrfb200_handle *h = cc.h;
+    const wrfb200_domain &dom = a.dom;
+    for (size_t x = 0; x < cc.doms.size(); ++x) {
+        const wrfb200_handle *h = cc.doms[x]->h;
+        if (same_shape(h->dom, dom) && (device < 0 || h->device == device)) {
+            std::rotate(cc.doms.begin(), cc.doms.begin() + x, cc.doms.begin() + x + 1);
+            *state = WRFB200_CACHE_REUSED;
+            return WRFB200_OK;
+        }
+    }
+    if (device < 0) CU(cudaGetDevice(&device));
+    *state = WRFB200_CACHE_CREATED;
+    if (cc.doms.size() >= kMaxDomains) {
+        cc.doms.pop_back();
+        *state = WRFB200_CACHE_EVICTED;
+    }
+    {
+        DeviceGuard g(device);
+        if (!g.ok) return fail(WRFB200_ERR_CUDA, "cannot select CUDA device %d", device);
+        const int es = prec ? 8 : 4;
+        size_t need = mirror_bytes(dom, es);
+        int is, ie, js, je, ks, ke;
+        wrfb200_bounds(dom.periodic_x, dom.specified, dom.nested, dom.ids, dom.ide, dom.jds, dom.jde,
+                       a.its, a.ite, a.jts, a.jte, a.kts, a.kte, &is, &ie, &js, &je, &ks, &ke);
+        const long idim = dom.ime - dom.ims + 1, kdim = dom.kme - dom.kms + 1;
+        const SlabPlan plan = slab_plan(dom, js <= je ? je - js + 1 : 0, es);
+        if (round_up(idim, 128 / es) != idim && plan.nslab > 1)      // run_host_compat_body's staging buffers
+            need += 2 * plan.rows * kdim * idim * es;
+        for (;;) {
+            size_t free_bytes = 0, total = 0;
+            if (cudaMemGetInfo(&free_bytes, &total) != cudaSuccess) { (void)cudaGetLastError(); break; }
+            if (free_bytes >= need) break;
+            size_t x = cc.doms.size();
+            while (x > 0 && cc.doms[x - 1]->h->device != device) --x;
+            if (x == 0) break;
+            cc.doms.erase(cc.doms.begin() + (x - 1));
+            *state = WRFB200_CACHE_EVICTED;
+        }
+    }
+    int rc = open_domain(cc, dom, device, 1, prec);
+    CompatCache *other = part ? nullptr : &g_cache[1 - prec];
+    if (rc == WRFB200_ERR_NOMEM && (!cc.doms.empty() || (other && !other->doms.empty()))) {
+        (void)cudaGetLastError();
+        cc.doms.clear();
+        if (other) other->doms.clear();
+        *state = WRFB200_CACHE_EVICTED;
+        rc = open_domain(cc, dom, device, 1, prec);
+    }
+    return rc;
+}
+
+// run_host_compat_body on domain e of cache cc, with the calling thread's kernel choice and the call's scalars
+int run_on_cache(const Args &a, int nsteps, CompatCache &cc, DomainEntry &e, int kernel, bool part, SharedPatch *sp)
+{
+    wrfb200_handle *h = e.h;
     GUARD(h);
     h->dom = a.dom;                       // same extents; domain dims / flags may differ between calls
     h->kernel = kernel;
     set_scalars(h, a.rdx, a.rdy, a.dts, a.epssm);
-    const int rc = run_host_compat_body(a, nsteps, h, cc, part, sp);
+    const int rc = run_host_compat_body(a, nsteps, e, cc, part, sp);
     if (rc != WRFB200_OK) {
         // an early return must not leave copies on the caller's arrays in flight, nor the cached handle
         // pointing at one of the internal lanes
         const std::string msg = wrfb200_last_error();
         for (cudaStream_t st : {cc.up, cc.comp, cc.down}) if (st) cudaStreamSynchronize(st);
         (void)cudaGetLastError();
-        cc.primed = false;
+        e.primed = false;
         wrfb200_fail(rc, "%s", msg.c_str());
     }
     h->stream = part ? nullptr : g_default_stream;
     return rc;
 }
 
-int run_host_part(const Args &a, int nsteps, int prec, CompatCache &cc, int device, int kernel, bool part)
+// One host-pointer call, or one device's share of a split call, on its domain of cache `cc` (find_domain).
+// `kernel` is the calling thread's choice, passed in because a part may run in a worker thread; *state receives
+// what the call did with the cache.
+int run_host_part(const Args &a, int nsteps, int prec, CompatCache &cc, int device, int kernel, bool part, int *state)
 {
     if (int rc = check_domain(a.dom)) return rc;
-    if (cc.h && (!same_shape(cc.h->dom, a.dom) || (device >= 0 && cc.h->device != device))) cc.release();
-    if (!cc.h)
-        if (int rc = open_cache(cc, a.dom, device, 1, prec)) return rc;
-    return run_on_cache(a, nsteps, cc, kernel, part, nullptr);
+    if (int rc = find_domain(cc, a, device, prec, part, state)) return rc;
+    DomainEntry &e = *cc.doms.front();
+    if (int rc = open_lanes(cc, e.h->device)) return rc;
+    return run_on_cache(a, nsteps, cc, e, kernel, part, nullptr);
 }
 
 // One host-pointer call in shared-tiles mode: a tile of the shared patch of these arrays on the patch device,
@@ -1656,6 +1829,7 @@ int run_host_shared(const Args &a, int nsteps, int prec)
         for (int f = 0; f < WRFB200_NUM_FIELDS; ++f) pin_host(a.f[f], field_bytes(a.dom, f, es));
 
     SharedPatch *sp = nullptr;
+    g_last_cache = WRFB200_CACHE_REUSED;
     {
         std::lock_guard<std::mutex> lock(g_shared_mutex);
         for (auto &q : g_shared)
@@ -1670,22 +1844,31 @@ int run_host_shared(const Args &a, int nsteps, int prec)
             std::memcpy(q->ptrs, a.f, sizeof(a.f));
             sp = q.get();
             g_shared.push_back(std::move(q));
+            g_last_cache = WRFB200_CACHE_CREATED;
         }
     }
 
+    // the thread's one handle for shared calls, bound to the patch's mirrors
     TileThread &tt = g_tiles;
     tt.enlist();
     CompatCache &cc = tt.c[prec];
-    if (cc.h && (!same_shape(cc.h->dom, a.dom) || cc.h->device != dev)) { cc.release(); tt.bound[prec] = 0; }
-    if (!cc.h)
-        if (int rc = open_cache(cc, a.dom, dev, 0, prec)) return rc;
+    if (!cc.doms.empty() && (!same_shape(cc.doms[0]->h->dom, a.dom) || cc.doms[0]->h->device != dev)) {
+        cc.release();
+        tt.bound[prec] = 0;
+    }
+    if (cc.doms.empty()) {
+        if (int rc = open_domain(cc, a.dom, dev, 0, prec)) return rc;
+        g_last_cache = WRFB200_CACHE_CREATED;
+    }
+    if (int rc = open_lanes(cc, dev)) return rc;
+    DomainEntry &e = *cc.doms.front();
     if (tt.bound[prec] != sp->id) {
         tt.bound[prec] = 0;
         for (int f = 0; f < WRFB200_NUM_FIELDS; ++f)
-            if (int rc = bind_device(cc.h, f, sp->h->d[f], is3d(f) ? sp->h->pitch3 : sp->h->pitch2)) return rc;
+            if (int rc = bind_device(e.h, f, sp->h->d[f], is3d(f) ? sp->h->pitch3 : sp->h->pitch2)) return rc;
         tt.bound[prec] = sp->id;
     }
-    return run_on_cache(a, nsteps, cc, g_default_kernel, true, sp);
+    return run_on_cache(a, nsteps, cc, e, g_default_kernel, true, sp);
 }
 
 // ---- one host-pointer call split over several devices (wrfb200_set_default_devices) --------------------
@@ -1736,9 +1919,18 @@ int run_host_split(const Args &a, int nsteps, int prec)
     if (pin_enabled())
         for (int f = 0; f < WRFB200_NUM_FIELDS; ++f) pin_host(a.f[f], field_bytes(a.dom, f, es));
 
+    // the cache of part p, whether or not a call uses it: p's device list entry, so that each cache keeps serving one
+    // device for every domain, also when a domain with fewer rows than devices leaves parts unused
+    std::vector<std::unique_ptr<CompatCache>> &pool = g_parts[prec];
+    while ((int)pool.size() + 1 < n) {
+        pool.emplace_back(new (std::nothrow) CompatCache());
+        if (!pool.back()) { pool.pop_back(); return fail(WRFB200_ERR_NOMEM, "out of host memory"); }
+        pool.back()->loop_active = g_cache[prec].loop_active;
+    }
     struct Part {
         Args a;
-        int device, rc = WRFB200_OK;
+        CompatCache *cache;
+        int device, rc = WRFB200_OK, state = -1;
         std::string err;
     };
     std::vector<Part> parts;
@@ -1747,6 +1939,7 @@ int run_host_split(const Args &a, int nsteps, int prec)
         if (r[0] > r[1]) continue;                        // no rows: not used
         Part q;
         q.a = a;
+        q.cache = p == 0 ? &g_cache[prec] : pool[p - 1].get();      // taken here: g_cache is the calling thread's
         q.device = g_default_devices[p];
         const size_t row3 = field_bytes(a.dom, WRFB200_U, es) / (a.dom.jme - a.dom.jms + 1);
         const size_t row2 = field_bytes(a.dom, WRFB200_MU, es) / (a.dom.jme - a.dom.jms + 1);
@@ -1758,17 +1951,10 @@ int run_host_split(const Args &a, int nsteps, int prec)
     }
     if (parts.empty()) return WRFB200_OK;
 
-    std::vector<std::unique_ptr<CompatCache>> &pool = g_parts[prec];
-    while (pool.size() + 1 < parts.size()) {
-        pool.emplace_back(new (std::nothrow) CompatCache());
-        if (!pool.back()) { pool.pop_back(); return fail(WRFB200_ERR_NOMEM, "out of host memory"); }
-        pool.back()->loop_active = g_cache[prec].loop_active;
-    }
-    auto cache = [&](size_t q) -> CompatCache & { return q == 0 ? g_cache[prec] : *pool[q - 1]; };
     const int kernel = g_default_kernel;
     auto run = [&](size_t q) {
         Part &p = parts[q];
-        p.rc = run_host_part(p.a, nsteps, prec, cache(q), p.device, kernel, true);
+        p.rc = run_host_part(p.a, nsteps, prec, *p.cache, p.device, kernel, true, &p.state);
         if (p.rc != WRFB200_OK) p.err = wrfb200_last_error();
     };
     std::vector<std::thread> workers;
@@ -1784,9 +1970,10 @@ int run_host_split(const Args &a, int nsteps, int prec)
     run(0);
     for (std::thread &t : workers) t.join();
 
+    for (const Part &p : parts) g_last_cache = std::max(g_last_cache, p.state);     // the most any part did
     for (size_t q = 0; q < parts.size(); ++q) {
         if (parts[q].rc == WRFB200_OK) continue;
-        for (size_t r = 0; r < parts.size(); ++r) cache(r).primed = false;
+        for (const Part &r : parts) r.cache->forget();
         const Part &p = parts[q];
         return fail(p.rc, "device %d, rows j=%d..%d: %s", p.device, p.a.jts, p.a.jte, p.err.c_str());
     }
@@ -1801,7 +1988,7 @@ int run_host_compat(const Args &a, int nsteps, int prec)
         CU(cudaGetDevice(&cur));
         if (g_default_devices.size() > 1 || g_default_devices[0] != cur) return run_host_split(a, nsteps, prec);
     }
-    return run_host_part(a, nsteps, prec, g_cache[prec], -1, g_default_kernel, false);
+    return run_host_part(a, nsteps, prec, g_cache[prec], -1, g_default_kernel, false, &g_last_cache);
 }
 
 void release_parts()
@@ -1815,10 +2002,11 @@ void release_parts()
 int dispatch(Args &a, int nsteps, bool allow_device, int prec)
 {
     g_last_prec = prec;
-    DeviceCallCache &dc = g_devcall[prec];
-    // device-pointer fast path: the very same arrays as the previous call need no re-classification
-    if (allow_device && nsteps == 1 && dc.valid && std::memcmp(dc.ptrs, a.f, sizeof(a.f)) == 0)
-        return run_device_in_place(a, prec);
+    g_last_cache = -1;
+    // device-pointer fast path: the very same arrays as a recent call need no re-classification
+    if (allow_device && nsteps == 1)
+        for (const DeviceCallCache &dc : g_devcall[prec])
+            if (dc.valid && std::memcmp(dc.ptrs, a.f, sizeof(a.f)) == 0) return run_device_in_place(a, prec);
     PtrKind kind = classify(a.f[0]);
     for (int f = 0; f < WRFB200_NUM_FIELDS; ++f) {
         PtrKind k = classify(a.f[f]);
@@ -1835,7 +2023,7 @@ int dispatch(Args &a, int nsteps, bool allow_device, int prec)
             return fail(WRFB200_ERR_INVALID_ARG, "this entry point takes host pointers; device-resident callers use wrfb200_step");
         return run_device_in_place(a, prec);
     }
-    dc.valid = false;
+    drop_devcalls(prec);
     const int rc = run_host_compat(a, nsteps, prec);
     g_last_route = transfer_route(a);                     // after the call: opt-in pinning may have locked the arrays
     return rc;
@@ -1985,7 +2173,7 @@ extern "C" int wrfb200_release_cache(void)
 {
     release_parts();
     release_shared();
-    for (DeviceCallCache &c : g_devcall) c.valid = false;
+    for (int prec = 0; prec < 2; ++prec) drop_devcalls(prec);
     unpin_all();
     stop_pool();
     return WRFB200_OK;
@@ -2008,18 +2196,18 @@ void shared_loop(bool active)
 
 extern "C" int wrfb200_acoustic_loop_begin(void)
 {
-    for (CompatCache &c : g_cache) { c.loop_active = true; c.primed = false; }
+    for (CompatCache &c : g_cache) { c.loop_active = true; c.forget(); }
     for (auto &pool : g_parts)
-        for (auto &c : pool) { c->loop_active = true; c->primed = false; }
+        for (auto &c : pool) { c->loop_active = true; c->forget(); }
     shared_loop(true);
     return WRFB200_OK;
 }
 
 extern "C" int wrfb200_acoustic_loop_end(void)
 {
-    for (CompatCache &c : g_cache) { c.loop_active = false; c.primed = false; }
+    for (CompatCache &c : g_cache) { c.loop_active = false; c.forget(); }
     for (auto &pool : g_parts)
-        for (auto &c : pool) { c->loop_active = false; c->primed = false; }
+        for (auto &c : pool) { c->loop_active = false; c->forget(); }
     shared_loop(false);
     return WRFB200_OK;
 }
@@ -2093,9 +2281,9 @@ extern "C" int wrfb200_last_kernel(wrfb200_handle *h, int *kernel)
 extern "C" int wrfb200_default_last_kernel(int *kernel)
 {
     if (!kernel) return fail(WRFB200_ERR_INVALID_ARG, "null argument");
-    const DeviceCallCache &dc = g_devcall[g_last_prec];
+    const DeviceCallCache *dc = last_devcall(g_last_prec);
     const CompatCache &cc = shared_enabled() ? g_tiles.c[g_last_prec] : g_cache[g_last_prec];
-    *kernel = dc.valid ? dc.h.last_kernel : (cc.h ? cc.h->last_kernel : 0);
+    *kernel = dc ? dc->h.last_kernel : (cc.doms.empty() ? 0 : cc.doms.front()->h->last_kernel);
     return WRFB200_OK;
 }
 
@@ -2104,5 +2292,20 @@ extern "C" int wrfb200_default_last_transfer(int *route)
     if (!route) return fail(WRFB200_ERR_INVALID_ARG, "null argument");
     if (g_last_route < 0) return fail(WRFB200_ERR_STATE, "no host-array call on this thread yet");
     *route = g_last_route;
+    return WRFB200_OK;
+}
+
+extern "C" int wrfb200_default_last_cache(int *state)
+{
+    if (!state) return fail(WRFB200_ERR_INVALID_ARG, "null argument");
+    if (g_last_cache < 0) return fail(WRFB200_ERR_STATE, "no advance_mu_t call on this thread has reached its cache yet");
+    *state = g_last_cache;
+    return WRFB200_OK;
+}
+
+extern "C" int wrfb200_bounce_allocations(long *count)
+{
+    if (!count) return fail(WRFB200_ERR_INVALID_ARG, "null argument");
+    *count = g_bounce_allocs.load();
     return WRFB200_OK;
 }

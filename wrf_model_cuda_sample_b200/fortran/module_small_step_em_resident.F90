@@ -110,6 +110,8 @@ INTERFACE
       INTEGER(c_size_t), VALUE :: bytes
       INTEGER(c_int) :: status
    END FUNCTION
+   ! frees every domain's device state this thread keeps (nested runs keep up to 8 per precision), e.g. at the end
+   ! of the run, to hand the device memory back to the model
    FUNCTION wrfb200_release_cache() BIND(C, NAME="wrfb200_release_cache") RESULT(status)
       IMPORT :: c_int
       INTEGER(c_int) :: status
@@ -119,6 +121,13 @@ INTERFACE
    FUNCTION wrfb200_default_last_transfer(route) BIND(C, NAME="wrfb200_default_last_transfer") RESULT(status)
       IMPORT :: c_int
       INTEGER(c_int), INTENT(OUT) :: route
+      INTEGER(c_int) :: status
+   END FUNCTION
+   ! what this thread's last advance_mu_t call did with its cache: 0 re-used its domain's device state, 1 created
+   ! it, 2 created it after freeing the least recently used domain(s) (nested runs: one entry per domain)
+   FUNCTION wrfb200_default_last_cache(state) BIND(C, NAME="wrfb200_default_last_cache") RESULT(status)
+      IMPORT :: c_int
+      INTEGER(c_int), INTENT(OUT) :: state
       INTEGER(c_int) :: status
    END FUNCTION
    ! OpenMP builds (smpar, dm+sm): the tiles of the !$OMP PARALLEL DO share one device-resident patch.  Call once,
